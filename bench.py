@@ -42,6 +42,8 @@ sys.path.insert(0, ROOT)
 
 SHARD_ROWS = 1
 FLOP_PER_TEST, FLOP_PER_SEGMENT = 17, 5  # SURVEY.md 8d
+DUMP_BYTES = 64 * 10 ** 6        # --dump-outputs writes at most this much
+DUMP_SAMPLE_PIXELS = 1 << 20     # pixels kept when the whole image does not fit in DUMP_BYTES
 
 
 def workloads():
@@ -149,6 +151,30 @@ def config_of(wl, world, cam, world_size):
             "parallelism": f"rows interleaved over {world_size} GPU(s), tiles of {SHARD_ROWS} rows"}
 
 
+def dump_outputs(dirname, lin, rgb8, world_size, rank):
+    """Writes what the timed call left in its device buffers, so that two builds can be compared output for
+    output: linear.npy (float64 radiance) and rgb8.npy (the 8-bit image as float32), both [H, W, 3].  An image
+    larger than DUMP_BYTES is cut to a fixed, seeded sample of DUMP_SAMPLE_PIXELS pixels: then both are
+    [pixels, 3] and pixel_index.npy holds the row-major index (y * W + x) of each pixel."""
+    import numpy as np
+    import torch.distributed as dist
+    if world_size > 1:  # each rank wrote only its own rows of zero-initialised full-size buffers
+        lin, rgb8 = lin.clone(), rgb8.clone()
+        dist.all_reduce(lin)
+        dist.all_reduce(rgb8)
+    if rank != 0:
+        return
+    lin = lin.cpu().numpy()
+    rgb8 = rgb8.cpu().numpy().astype(np.float32)
+    out = {"linear": lin, "rgb8": rgb8}
+    if lin.nbytes + rgb8.nbytes > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(lin.shape[0] * lin.shape[1], DUMP_SAMPLE_PIXELS, replace=False))
+        out = {"linear": lin.reshape(-1, 3)[idx], "rgb8": rgb8.reshape(-1, 3)[idx], "pixel_index": idx.astype(np.float64)}
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def run_reference(args, wl):
     rank = int(os.environ.get("RANK", "0"))
     world_size = int(os.environ.get("WORLD_SIZE", "1"))
@@ -187,6 +213,8 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip strict_order / e2e_single_process")
     ap.add_argument("--spp", type=int, default=None, help="override the workload's spp (invalid as a bench value)")
     ap.add_argument("--spu", type=int, default=0, help="samples per work unit for the timed steps (tuning; 0 = the library's choice)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the images the last timed step computed to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
     wl = workloads()[args.workload]
     if args.spp:
@@ -271,6 +299,8 @@ def main():
     total_ms, segs_per_step, kernel_ms, seg_local, spu_used = timed_device_steps(args.steps, samples_per_unit=args.spu)
     clocks = sampler.stop() if rank == 0 else None
     value = segs_per_step * args.steps / (total_ms * 1e-3)
+    if args.dump_outputs:  # now: the strict-order and e2e legs below render into the same buffers
+        dump_outputs(args.dump_outputs, out_lin, out_rgb, world_size, rank)
 
     # ---- the reference's strict summation order (one sequential sum per pixel), same timing rules
     strict = None
@@ -282,7 +312,8 @@ def main():
 
     # ---- e2e: host buffers through rtclj_render, H2D + D2H (into pinned host memory) inside the timed region
     soa = R.scenes.to_soa(world)
-    shm_path = f"/dev/shm/rtclj_bench_{os.environ.get('MASTER_PORT', 'single')}"
+    # one name per user and job: the ranks of a job share MASTER_PORT, other jobs (and users) on the host do not
+    shm_path = f"/dev/shm/rtclj_bench_{os.getuid()}_{os.environ.get('MASTER_PORT') or os.getpid()}"
     lin_bytes, rgb_bytes = H * W * 3 * 8, H * W * 3
     if rank == 0:
         with open(shm_path, "wb") as f:

@@ -1,7 +1,7 @@
-"""Regenerates tests/golden/*.npz.  Run in the BUILD container (it reads
-/root/reference, which does not exist on the GPU box):
+"""Regenerates tests/golden/*.npz from a checkout of keychera/raytracing-clj (for its two
+committed renders) and the CPU oracle:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py path/to/raytracing-clj
 
 1. reference_images.npz -- the reference's two committed renders, the only result
    pins it offers (SURVEY.md 4): scene.ppm (`-M:main`, 400x225) and scene-realm.ppm
@@ -46,8 +46,7 @@ def fixture_cases():
     }
 
 
-def main():
-    ref = "/root/reference"
+def main(ref):
     np.savez_compressed(os.path.join(HERE, "reference_images.npz"),
                         scene_main=load_p3(os.path.join(ref, "scene.ppm")),
                         scene_realm=load_p3(os.path.join(ref, "scene-realm.ppm")))
@@ -66,4 +65,6 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        raise SystemExit(__doc__)
+    main(sys.argv[1])

@@ -41,15 +41,23 @@ def _has_gpu():
     return _abi.lib().rtclj_device_count(C.byref(n)) == 0 and n.value > 0
 
 
-def test_no_cpu_fallback():
-    if _has_gpu():
-        pytest.skip("a GPU is present")
+def check_no_cpu_fallback():
+    assert not _has_gpu()
     with pytest.raises(_abi.RtcljError) as e:
         render.render(R.scenes.main_hittables(), R.camera.main_camera(16), 1, 5)
     assert e.value.code == _abi.E_NO_DEVICE
     with pytest.raises(_abi.RtcljError):
         render.Context(0)
     assert b"CUDA" in _abi.lib().rtclj_last_error() or b"device" in _abi.lib().rtclj_last_error()
+
+
+def test_no_cpu_fallback():
+    """In a child process that sees no CUDA device, so that it runs on machines with a GPU as well."""
+    import subprocess
+    import sys
+    code = "import sys; sys.path[:0] = sys.argv[1:]; import test_abi; test_abi.check_no_cpu_fallback()"
+    subprocess.run([sys.executable, "-c", code, ROOT, os.path.join(ROOT, "tests")], check=True,
+                   env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
 
 
 def test_missing_library_is_an_error(monkeypatch):
