@@ -16,6 +16,9 @@
  *                           several GPUs in, the text of scene.ppm out
  *   rtclj_ctx_*             the same loop with device-resident buffers (scene upload
  *                           once, many renders; what bench.py times as `value`)
+ *   rtclj_ctx_accum_*, rtclj_progressive_*
+ *                           the same loop run in passes of samples (progressive rendering),
+ *                           bit-identical to a one-shot render after every pass
  *   rtclj_quantise_rgb8     write-color! / linear->gamma / clamp,
  *                           src/raytracing.clj:19-26 ; realm/raytracing.clj:246-249,356-357
  *   rtclj_encode_ppm_p3     the P3 writer, src/raytracing.clj:172-175 ;
@@ -228,8 +231,52 @@ int rtclj_ctx_set_scene(rtclj_ctx *ctx, const rtclj_scene *scene);
  * carries its cull table with it (kernel parameters), the library holds no per-device state. */
 int rtclj_ctx_render(rtclj_ctx *ctx, const rtclj_camera *camera, const rtclj_params *params,
                      void *d_out_linear, void *d_out_rgb8, void *stream);
-/* Synchronises `stream` and reads the counters of the last rtclj_ctx_render. */
+/* Synchronises `stream` and reads the counters of the last rtclj_ctx_render (or accumulation pass). */
 int rtclj_ctx_stats(rtclj_ctx *ctx, void *stream, rtclj_stats *stats);
+
+/* ---- Progressive rendering: the compute-pixel loop (src/raytracing.clj:141-171) run in passes, so that
+ * an image can be shown while it refines, stopped early or extended without tracing its samples again.
+ *
+ * An accumulation is fixed at its start by a scene, a camera and params; params->spp is the TARGET
+ * sample count.  A pass of n samples adds samples [d, d + n) of every pixel to the pixel's running
+ * sum, d being the samples done before it, and writes the images of the mean over d + n samples.
+ *   - pass_unit, reported by the call that begins the accumulation: 1 in strict order
+ *     (samples_per_unit >= spp, or <= 0 for a primary-ray render: the library's default there), else
+ *     the unit size (samples_per_unit, or the library's choice when <= 0).  Every pass but the one that
+ *     reaches spp must be a multiple of pass_unit; a pass that is not, or that would go beyond spp,
+ *     returns RTCLJ_E_INVALID.
+ *   - After passes totalling d samples the images (linear and 8-bit) are bit-identical to
+ *     rtclj_ctx_render with the same camera and params but spp = d and samples_per_unit = pass_unit
+ *     (strict order: samples_per_unit = d).  At d = spp that is the one-shot render of the
+ *     accumulation's own params.  The images do not depend on the pass sizes, on the number of GPUs
+ *     or on the device list.
+ *   - RTCLJ_F_WAVE_KERNEL and RTCLJ_F_SPLIT_KERNEL are refused (RTCLJ_E_INVALID); spp is at most 2^30.
+ *     max_depth <= 0 accumulates black.
+ * Strict order holds at most 2 GiB of per-sample colours per context, whatever the image size. */
+
+/* Device-resident, on the caller's stream (a cudaStream_t, NULL = the default stream); one accumulation
+ * per context.  begin zeroes the running sums (24 B per pixel of the shard) and returns the pass unit;
+ * step enqueues one pass and returns the samples per pixel done after it.  d_out_linear / d_out_rgb8 are
+ * DEVICE pointers to full-size images, either may be NULL (the pass is still added).  rtclj_ctx_set_scene
+ * ends the accumulation (step returns RTCLJ_E_INVALID until the next begin), and so does a failed
+ * pass; rtclj_ctx_render between two steps leaves it intact.  rtclj_ctx_stats reports the last pass. */
+int rtclj_ctx_accum_begin(rtclj_ctx *ctx, const rtclj_camera *camera, const rtclj_params *params,
+                          int32_t *pass_unit, void *stream);
+int rtclj_ctx_accum_step(rtclj_ctx *ctx, int32_t samples, void *d_out_linear, void *d_out_rgb8,
+                         int32_t *samples_done, void *stream);
+
+/* Host buffers, image rows interleaved over `n_devices` GPUs as in rtclj_render_multi (tiles of
+ * params->shard_rows rows, <= 0: 1) -- what a JVM host calls to show an image while it refines.  The
+ * handle owns a context per device and uploads the scene at create.  Each step runs one pass on every
+ * device and writes the whole image into out_linear / out_rgb8 (either may be NULL); stats may be NULL.
+ * One thread at a time per handle.  A step that fails on any device ends the accumulation. */
+typedef struct rtclj_progressive rtclj_progressive; /* opaque */
+int rtclj_progressive_create(const rtclj_scene *scene, const rtclj_camera *camera,
+                             const rtclj_params *params, const int32_t *devices, int32_t n_devices,
+                             int32_t *pass_unit, rtclj_progressive **out);
+int rtclj_progressive_step(rtclj_progressive *p, int32_t samples, double *out_linear,
+                           uint8_t *out_rgb8, int32_t *samples_done, rtclj_stats *stats);
+int rtclj_progressive_destroy(rtclj_progressive *p); /* NULL is fine */
 
 /* Measures this GPU's arithmetic peaks with pure-FMA kernels (no memory traffic): scalar
  * FFMA, packed FFMA2 and fp64 DFMA, in TFLOP/s (2 flops per FMA), plus the SM count.

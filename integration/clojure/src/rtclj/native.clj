@@ -186,6 +186,77 @@
         (aset realm (+ 2 (* 3 p)) (aget c 2))))
     realm))
 
+;; ---- progressive rendering: the same loop in passes, an image that refines (rtclj_progressive_*)
+;; int rtclj_progressive_create(const rtclj_scene*, const rtclj_camera*, const rtclj_params*,
+;;                              const int32_t* devices, int32_t n_devices, int32_t* pass_unit,
+;;                              rtclj_progressive** out)
+(def ^:private rtclj-progressive-create
+  (downcall "rtclj_progressive_create"
+            (fd-int ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS
+                    ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/ADDRESS)))
+;; int rtclj_progressive_step(rtclj_progressive*, int32_t samples, double* out_linear, uint8_t* out_rgb8,
+;;                            int32_t* samples_done, rtclj_stats*)
+(def ^:private rtclj-progressive-step
+  (downcall "rtclj_progressive_step"
+            (fd-int ValueLayout/ADDRESS ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/ADDRESS
+                    ValueLayout/ADDRESS ValueLayout/ADDRESS)))
+;; int rtclj_progressive_destroy(rtclj_progressive*)
+(def ^:private rtclj-progressive-destroy
+  (downcall "rtclj_progressive_destroy" (fd-int ValueLayout/ADDRESS)))
+
+(defn- pinned-bytes
+  "n bytes of PINNED host memory (rtclj_host_alloc).  Returns [segment free-fn]."
+  [^Arena a ^long n]
+  (let [slot (.allocate a 8 8)
+        _    (check! (.invokeWithArguments rtclj-host-alloc [n slot]))
+        ^MemorySegment p (.reinterpret (.get slot ValueLayout/ADDRESS 0) n)]
+    [p #(.invokeWithArguments rtclj-host-free [p])]))
+
+(defn progressive
+  "Begins a progressive render: the compute-pixel loop (raytracing.clj:141-171) run in passes towards
+   samples-per-px samples, on :devices (default [0]), with the options of `render`.  After passes totalling
+   d samples the image is bit-identical to `render` with d samples in the same summation order.  Returns a
+   handle map; :pass-unit is the granularity of passes (every pass but the last a multiple of it).  Close it
+   with progressive-close!."
+  [bodies cam samples-per-px max-depth & {:keys [devices] :or {devices [0]} :as opts}]
+  (with-open [a (Arena/ofConfined)]
+    (let [w    (long (:image-width cam))
+          h    (long (:image-height cam))
+          [scene camera params] (marshal a bodies cam samples-per-px max-depth opts)
+          unit (.allocate a 4 4)
+          slot (.allocate a 8 8)]
+      (check! (.invokeWithArguments rtclj-progressive-create
+                                    [scene camera params
+                                     (.allocateFrom a ValueLayout/JAVA_INT (int-array devices)) (int (count devices))
+                                     unit slot]))
+      (let [handle (.get slot ValueLayout/ADDRESS 0)]
+        (try
+          (let [[linear free-linear!] (pinned-doubles a (* 3 w h))
+                [rgb8 free-rgb8!]     (pinned-bytes a (* 3 w h))]
+            {:handle handle :pass-unit (.get unit ValueLayout/JAVA_INT 0) :samples-per-px samples-per-px
+             :linear linear :rgb8 rgb8 :free! (fn [] (free-linear!) (free-rgb8!))})
+          (catch Throwable t
+            (.invokeWithArguments rtclj-progressive-destroy [handle])
+            (throw t)))))))
+
+(defn progressive-step!
+  "One pass of `samples` samples per pixel.  Returns {:linear :rgb8 :samples-done}: the image so far as
+   W*H*3 doubles (linear RGB, row-major from the top-left pixel) and W*H*3 bytes quantised like write-color!,
+   both in PINNED memory that belongs to `p`: the next step overwrites them, progressive-close! frees them."
+  [p samples]
+  (with-open [a (Arena/ofConfined)]
+    (let [done (.allocate a 4 4)]
+      (check! (.invokeWithArguments rtclj-progressive-step
+                                    [(:handle p) (int samples) (:linear p) (:rgb8 p) done MemorySegment/NULL]))
+      {:linear (:linear p) :rgb8 (:rgb8 p) :samples-done (.get done ValueLayout/JAVA_INT 0)})))
+
+(defn progressive-close!
+  "Ends a progressive render: its GPU contexts and its pinned images are released."
+  [p]
+  (try
+    (check! (.invokeWithArguments rtclj-progressive-destroy [(:handle p)]))
+    (finally ((:free! p)))))
+
 ;; int rtclj_encode_ppm_p3_gpu(int32_t device, const uint8_t* rgb8, int32_t width, int32_t height,
 ;;                             char* out, size_t capacity, size_t* len)
 (def ^:private rtclj-encode-ppm-p3-gpu

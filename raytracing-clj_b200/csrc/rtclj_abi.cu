@@ -90,6 +90,16 @@ struct rtclj_ctx {
   cudaEvent_t p3_ev0 = nullptr, p3_ev1 = nullptr;           // the P3 writer's own timing events
   cudaStream_t own_stream = nullptr;
   int last_spu = 0;
+  // the accumulation in progress (rtclj_ctx_accum_begin / _step); rtclj_ctx_set_scene ends it
+  struct Accum {
+    bool active = false;
+    bool strict = false;     // one sequential sum per pixel (pass_unit 1)
+    rtclj_camera cam;
+    rtclj_params prm;        // prm.spp: the target
+    int done = 0;            // samples per pixel so far
+    int pass_unit = 1;
+  } accum;
+  DevBuf<double> acc;                   // the accumulation's running sums: 3 per local pixel
   double prim_geom[4 * kPrimarySpheres] = {};  // exact geometry of the first spheres: parameters of render_primary_kernel
   bool have_scene = false;
   bool render_pending = false;  // a render has been enqueued since the last scene upload / stats
@@ -263,6 +273,7 @@ void rtclj_ctx_destroy(rtclj_ctx* c) {
   if (c->own_stream) cudaStreamSynchronize(c->own_stream);
   c->geom32.release(); c->geomA.release(); c->geom64.release(); c->mat.release(); c->partial.release();
   c->counters.release(); c->stack.release(); c->arrive.release(); c->sample_buf.release(); c->out_linear.release(); c->out_rgb8.release();
+  c->acc.release();
   c->p3_state.release(); c->p3_in.release(); c->p3_text.release();
   for (cudaEvent_t e : {c->ev0, c->ev1, c->ev2, c->p3_ev0, c->p3_ev1, c->pin_ev[0], c->pin_ev[1]})
     if (e) cudaEventDestroy(e);
@@ -273,6 +284,7 @@ void rtclj_ctx_destroy(rtclj_ctx* c) {
 
 int rtclj_ctx_set_scene(rtclj_ctx* c, const rtclj_scene* s) {
   if (!c || !s) return fail(RTCLJ_E_INVALID, "null ctx or scene");
+  c->accum.active = false;  // an accumulation belongs to the scene it began with
   const int n = s->n;
   if (n < 0) return fail(RTCLJ_E_INVALID, "negative sphere count");
   if (n > 0 && (!s->center_xyz || !s->radius || !s->material || !s->albedo_rgb || !s->fuzz || !s->ior))
@@ -376,33 +388,29 @@ int rtclj_ctx_set_scene(rtclj_ctx* c, const rtclj_scene* s) {
   return RTCLJ_OK;
 }
 
-int rtclj_ctx_render(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, void* d_out_linear,
-                     void* d_out_rgb8, void* stream_) {
-  if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
-  if (!c->have_scene) return fail(RTCLJ_E_INVALID, "rtclj_ctx_set_scene has not been called");
-  int rc = validate(cam, prm);
-  if (rc) return rc;
-  cudaStream_t stream = (cudaStream_t)stream_;
-  CU(cudaSetDevice(c->device));
+}  // extern "C"
 
-  const int W = cam->width, H = cam->height;
-  const int shard_count = prm->shard_count > 1 ? prm->shard_count : 1;
-  const int shard_index = shard_count > 1 ? prm->shard_index : 0;
-  const int shard_rows = shard_count > 1 ? prm->shard_rows : H;
-  const int local_rows = local_rows_of(H, shard_index, shard_count, shard_rows);
-  const unsigned long long local_pixels = (unsigned long long)local_rows * (unsigned long long)W;
-  const int grid = c->sm_count;
-  const bool run_kernel = prm->max_depth > 0;
-  const bool const_tab = use_const_table(c->nhalf) && !(prm->flags & RTCLJ_F_SMEM_TABLE);
-  const bool want_out = d_out_linear || d_out_rgb8;
-  // scenes of <= 512 spheres: four kernels produce the same image (tests); the default is the fastest
-  // measured on the bench workload (DESIGN.md section 7), the flags select the others for A/B timing
-  enum { SMALL_LANE1, SMALL_LANE2, SMALL_WAVE, SMALL_SPLIT };
+namespace {
+
+// Scenes of <= 512 spheres: four kernels produce the same image (tests); the default is the fastest measured on
+// the bench workload (DESIGN.md section 7), the flags select the others for A/B timing
+enum { SMALL_LANE1, SMALL_LANE2, SMALL_WAVE, SMALL_SPLIT };
+struct KernelChoice {
+  bool run_kernel, const_tab, primary_only;
+  int small;
+  bool wave, lane2, split;  // constant-table kernels other than render_kernel<true>
+  bool primary;             // render_primary_kernel
+};
+
+// the kernel of a launch that traces `total_samples` samples of this shard
+KernelChoice choose_kernel(const rtclj_ctx* c, const rtclj_params* prm, double total_samples) {
+  KernelChoice k;
+  k.run_kernel = prm->max_depth > 0;
+  k.const_tab = use_const_table(c->nhalf) && !(prm->flags & RTCLJ_F_SMEM_TABLE);
   // Two paths per lane pay when the cull dominates (many spheres) and the render is long enough to hide
   // the longer tail of twice as many work units in flight: measured on a B200 (profiles/r2_kernel_ab.md),
   // cover scene 1920x1080: 500 spp 543.7 vs 561.6 ms, one eighth of it (an 8-GPU shard, 1.3e8 samples) 70.85 vs
   // 71.40 ms, 16 spp (3.3e7 samples) 19.6 vs 18.6 ms; 5 spheres: 11.7 vs 11.0 ms.  Break-even near 9e7 samples.
-  const double total_samples = (double)local_pixels * (double)prm->spp;
   // (final build of round 2, 16 / 24 / 32 / 48 spp at 1920x1080: 18.48 / 26.71 / 34.86 / 51.25 against 18.50 / 27.23 /
   // 35.77 / 53.28 ms -- the break-even moved down to 3.3e7 samples; at 2e6 samples the single-path kernel is 30 % faster)
   int small = (c->n >= 64 && total_samples >= 4.0e7) ? SMALL_LANE2 : SMALL_LANE1;
@@ -413,51 +421,59 @@ int rtclj_ctx_render(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* 
   if (prm->flags & RTCLJ_F_LANE2_KERNEL) small = SMALL_LANE2;
   if (prm->flags & RTCLJ_F_WAVE_KERNEL) small = SMALL_WAVE;
   if (prm->flags & RTCLJ_F_SPLIT_KERNEL) small = SMALL_SPLIT;
-  const bool wave = run_kernel && const_tab && small == SMALL_WAVE;    // also finishes the pixels itself
-  const bool lane2 = run_kernel && const_tab && small == SMALL_LANE2;
-  const bool split = run_kernel && const_tab && small == SMALL_SPLIT;
+  k.small = small;
+  k.wave = k.run_kernel && k.const_tab && small == SMALL_WAVE;    // also finishes the pixels itself
+  k.lane2 = k.run_kernel && k.const_tab && small == SMALL_LANE2;
+  k.split = k.run_kernel && k.const_tab && small == SMALL_SPLIT;
+  k.primary_only = prm->max_depth == 1 || (prm->flags & RTCLJ_F_NORMAL_SHADING);
+  // primary rays only and a handful of spheres (config 4): a kernel without the path machinery, 1.6x faster
+  // (rtclj_primary_kernel.cuh); RTCLJ_F_LANE_KERNEL / RTCLJ_F_NO_CULL keep render_kernel for A/B and tests
+  k.primary = k.run_kernel && k.const_tab && small == SMALL_LANE1 && k.primary_only && c->n <= kPrimarySpheres &&
+              !(prm->flags & (RTCLJ_F_LANE_KERNEL | RTCLJ_F_NO_CULL));
+  return k;
+}
 
-  // Summation unit.  Primary-ray renders (max-depth 1, normal shading) are bit-exact contracts and short
-  // paths: they default to the reference's strict sequential sum (raytracing.clj:142-155,
-  // raytracing_i.clj:146-163); other renders split a pixel into chunks for load balance.
-  const bool primary_only = prm->max_depth == 1 || (prm->flags & RTCLJ_F_NORMAL_SHADING);
-  int spu = prm->samples_per_unit > 0 ? prm->samples_per_unit
-                                      : (primary_only ? prm->spp : auto_samples_per_unit(W, H, prm->spp));
-  if (spu > prm->spp) spu = prm->spp;
-  c->last_spu = spu;
-  // The strict order on long paths: one 500-sample unit lasts as long as its pixel's paths, the last ones
-  // run alone (measured: 622 vs 543 ms on one GPU, 162 vs 72 ms per GPU on eight).  Instead the samples are
-  // traced in small units and each sample's colour is STORED (32 B); finalize_kernel then adds them in
-  // sample order -- the same additions in the same order.  33 GB at 1920x1080 x 500 spp; HBM has 180 GB.
-  double* sample_buf = nullptr;
-  if (spu == prm->spp && !primary_only && prm->spp >= 64 && run_kernel && !wave && want_out && local_pixels > 0) {
-    const size_t need = (size_t)local_pixels * (size_t)prm->spp * 4u;  // doubles
-    size_t free_b = 0, total_b = 0;
-    // kept in the context between renders (allocating 33 GB per frame costs more than the frame); a render
-    // that does not need it gives a large one back (below)
-    if (need <= c->sample_buf.cap ||
-        (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need * 8 < (free_b + c->sample_buf.cap * 8) / 2 &&
-         c->sample_buf.reserve(need) == cudaSuccess)) {
-      sample_buf = c->sample_buf.p;
-      spu = auto_samples_per_unit(W, H, prm->spp);  // scheduling units; the arithmetic stays strict
-    } else {
-      cudaGetLastError();  // too large: fall back to one unit per pixel
-    }
-  } else if (c->sample_buf.cap * 8 > ((size_t)1 << 30)) {
-    c->sample_buf.release();  // (synchronises the device; only on a strict -> chunked change of mode)
-  }
-  const int nchunks = (prm->spp + spu - 1) / spu;
-  const unsigned long long total_units = local_pixels * (unsigned long long)nchunks;
+// the rows of the image one render covers (rtclj_params.shard_*)
+struct Shard { int index, count, rows; unsigned long long local_pixels; };
+Shard shard_of(const rtclj_camera* cam, const rtclj_params* prm) {
+  Shard s;
+  s.count = prm->shard_count > 1 ? prm->shard_count : 1;
+  s.index = s.count > 1 ? prm->shard_index : 0;
+  s.rows = s.count > 1 ? prm->shard_rows : cam->height;
+  s.local_pixels = (unsigned long long)local_rows_of(cam->height, s.index, s.count, s.rows) * (unsigned long long)cam->width;
+  return s;
+}
+
+// One render launch: samples [sample_base, sample_base + samples) of every pixel of the shard, in work units of
+// `spu` samples, then (finalize) finalize_kernel.
+struct Pass {
+  int sample_base = 0, samples = 0, spu = 0;
+  double* sample_buf = nullptr;  // strict order: every sample's colour, added in sample order by finalize_kernel
+  double* acc = nullptr;         // an accumulation's running sums (FParams::acc)
+  bool seeded = false;           // strict accumulation on render_primary_kernel: the seeded variant
+  int mean_n = 0;                // divisor of the pixel mean
+  bool first = true;             // resets the counters and starts the timing: the first launch of a call
+  bool finalize = false;
+  double* out_linear = nullptr;
+  unsigned char* out_rgb8 = nullptr;
+};
+
+int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, const KernelChoice& ch, const Shard& sh,
+                const Pass& ps, cudaStream_t stream) {
+  const int grid = c->sm_count;
+  const int nchunks = (ps.samples + ps.spu - 1) / ps.spu;
+  const unsigned long long total_units = sh.local_pixels * (unsigned long long)nchunks;
   if (total_units > 0xffffffffull) {
     return fail(RTCLJ_E_INVALID, "%llu work units: raise samples_per_unit", total_units);
   }
 
-  CU(cudaMemsetAsync(c->counters.p, 0, 8 * sizeof(unsigned long long), stream));
+  // a later launch of the same call resets the ticket queue only: the counters add up over the call
+  CU(cudaMemsetAsync(c->counters.p, 0, (ps.first ? 8 : 1) * sizeof(unsigned long long), stream));
   if (total_units == 0) return RTCLJ_OK;
 
-  if ((!wave || nchunks > 1) && !sample_buf) CU(c->partial.reserve((size_t)total_units * 3));
-  CU(cudaEventRecord(c->ev0, stream));
-  if (!run_kernel) {
+  if ((!ch.wave || nchunks > 1) && !ps.sample_buf) CU(c->partial.reserve((size_t)total_units * 3));
+  if (ps.first) CU(cudaEventRecord(c->ev0, stream));
+  if (!ch.run_kernel) {
     CU(cudaMemsetAsync(c->partial.p, 0, (size_t)total_units * 3 * sizeof(double), stream));  // depth <= 0: black
   } else {
     KParams& P = c->kparams;  // 8.4 KB with the table: kept in the context, not on the stack of a JVM thread
@@ -468,57 +484,55 @@ int rtclj_ctx_render(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* 
       P.shift[a] = c->shift[a];
     }
     P.use_defocus = !(cam->defocus_angle <= 0.0);
-    P.W = W; P.H = H; P.spp = prm->spp; P.max_depth = prm->max_depth;
+    P.W = cam->width; P.H = cam->height; P.spp = ps.sample_base + ps.samples; P.max_depth = prm->max_depth;
     P.flags = prm->flags; P.k0 = (unsigned)prm->seed; P.k1 = (unsigned)(prm->seed >> 32);
     for (unsigned r = 0; r < 10; ++r) { P.rk[2 * r] = P.k0 + r * 0x9E3779B9u; P.rk[2 * r + 1] = P.k1 + r * 0xBB67AE85u; }
     // A handful of spheres: the exhaustive fp64 scan (the same lexicographic minimum, tests) beats cull +
     // prefilter.  Measured at 1920x1080 x 16 spp on prefixes of the default scene: path tracing 1 / 2 / 3 / 4
     // spheres 2.24 / 4.86 / 7.08 / 9.43 ms against 2.78 / 5.24 / 7.12 / 9.31 with the cull; primary rays only
     // 2 / 5 / 6 / 8 spheres 0.96 / 1.16 / 1.20 / 1.30 ms against 1.19 / 1.26 / 1.25 / 1.26.
-    if (const_tab && small == SMALL_LANE1 && (c->n <= 2 || (primary_only && c->n <= kPrimarySpheres))) P.flags |= RTCLJ_F_NO_CULL;
+    if (ch.const_tab && ch.small == SMALL_LANE1 && (c->n <= 2 || (ch.primary_only && c->n <= kPrimarySpheres))) P.flags |= RTCLJ_F_NO_CULL;
     P.n = c->n; P.nblocks = c->nhalf / 2; P.tail8 = c->nhalf & 1;
     P.nconst = (c->n + 2 * kCBP - 1) / (2 * kCBP);
     P.smem_blocks = smem_table_blocks(c->smem_optin);
     P.geom_bytes = (unsigned)std::min((size_t)c->nhalf * 256, (size_t)P.smem_blocks * 512);  // staged part
-    P.shard_index = shard_index; P.shard_count = shard_count; P.shard_rows = shard_rows;
-    P.nchunks = nchunks; P.spu = spu; P.total_units = total_units;
+    P.shard_index = sh.index; P.shard_count = sh.count; P.shard_rows = sh.rows;
+    P.nchunks = nchunks; P.spu = ps.spu; P.sample_base = ps.sample_base; P.total_units = total_units;
     P.geom32 = c->geom32.p; P.geomA = c->geomA.p; P.geom64 = c->geom64.p; P.mat = c->mat.p;
-    P.partial = c->partial.p; P.queue = c->counters.p; P.stats = c->counters.p + 1;
-    P.sample_buf = sample_buf; P.sample_stride = local_pixels;
-    if (const_tab && !c->ctab_host.empty())
+    P.partial = c->partial.p; P.acc = ps.acc; P.queue = c->counters.p; P.stats = c->counters.p + 1;
+    P.sample_buf = ps.sample_buf; P.sample_stride = sh.local_pixels;
+    if (ch.const_tab && !c->ctab_host.empty())
       std::memcpy(P.ctab, c->ctab_host.data(), std::min(sizeof P.ctab, c->ctab_host.size() * sizeof(float)));
-    // primary rays only and a handful of spheres (config 4): a kernel without the path machinery, 1.6x faster
-    // (rtclj_primary_kernel.cuh); RTCLJ_F_LANE_KERNEL / RTCLJ_F_NO_CULL keep render_kernel for A/B and tests
-    const bool primary = const_tab && small == SMALL_LANE1 && primary_only && c->n <= kPrimarySpheres &&
-                         !(prm->flags & (RTCLJ_F_LANE_KERNEL | RTCLJ_F_NO_CULL));
-    if (primary) {
+    if (ch.primary) {
       std::memcpy(P.ctab, c->prim_geom, sizeof c->prim_geom);
       const unsigned long long want = (total_units + kPrimaryThreads - 1) / kPrimaryThreads;
       const unsigned blocks = (unsigned)std::min<unsigned long long>(want, (unsigned long long)grid * (unsigned long long)(2048 / kPrimaryThreads));
-      if (P.use_defocus) render_primary_kernel<true><<<blocks, kPrimaryThreads, 0, stream>>>(P);
+      if (ps.seeded && P.use_defocus) render_primary_seeded_kernel<true><<<blocks, kPrimaryThreads, 0, stream>>>(P);
+      else if (ps.seeded) render_primary_seeded_kernel<false><<<blocks, kPrimaryThreads, 0, stream>>>(P);
+      else if (P.use_defocus) render_primary_kernel<true><<<blocks, kPrimaryThreads, 0, stream>>>(P);
       else render_primary_kernel<false><<<blocks, kPrimaryThreads, 0, stream>>>(P);
-    } else if (wave) {
+    } else if (ch.wave) {
       P.stack_stride = (unsigned)grid * (unsigned)kWS;
       if (prm->max_depth > 1) {  // the attenuating hits of a path, for either product order
         CU(c->stack.reserve((size_t)prm->max_depth * P.stack_stride));
         P.stack = c->stack.p;
       }
-      P.out_linear = (double*)d_out_linear; P.out_rgb8 = (unsigned char*)d_out_rgb8;
-      if (nchunks > 1 && want_out) {
-        CU(c->arrive.reserve((size_t)local_pixels));
-        CU(cudaMemsetAsync(c->arrive.p, 0, (size_t)local_pixels * sizeof(unsigned), stream));
+      P.out_linear = ps.out_linear; P.out_rgb8 = ps.out_rgb8;
+      if (nchunks > 1 && (ps.out_linear || ps.out_rgb8)) {
+        CU(c->arrive.reserve((size_t)sh.local_pixels));
+        CU(cudaMemsetAsync(c->arrive.p, 0, (size_t)sh.local_pixels * sizeof(unsigned), stream));
         P.arrive = c->arrive.p;
       }
       render_wave_kernel<<<grid, kWT, WaveSmem::total, stream>>>(P);
-    } else if (split) {
+    } else if (ch.split) {
       P.stack_stride = (unsigned)grid * (unsigned)kSplitW * 2u;
       if (prm->max_depth > 1) {
         CU(c->stack.reserve((size_t)prm->max_depth * P.stack_stride));
         P.stack = c->stack.p;
       }
-      if (sample_buf) render_split_kernel<true><<<grid, kSplitThreads, SplitSmem::total, stream>>>(P);
+      if (ps.sample_buf) render_split_kernel<true><<<grid, kSplitThreads, SplitSmem::total, stream>>>(P);
       else render_split_kernel<false><<<grid, kSplitThreads, SplitSmem::total, stream>>>(P);
-    } else if (lane2) {
+    } else if (ch.lane2) {
       P.stack_stride = (unsigned)grid * (unsigned)kT2 * 2u;
       if (prm->max_depth > 1) {
         CU(c->stack.reserve((size_t)prm->max_depth * P.stack_stride));
@@ -530,7 +544,7 @@ int rtclj_ctx_render(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* 
       CU(cudaMemsetAsync(c->arrive.p, 0, probe_words * sizeof(unsigned), stream));
       P.arrive = c->arrive.p;
 #endif
-      if (sample_buf) render_lane2_kernel<true><<<grid, kT2, Lane2Smem::total, stream>>>(P);
+      if (ps.sample_buf) render_lane2_kernel<true><<<grid, kT2, Lane2Smem::total, stream>>>(P);
       else render_lane2_kernel<false><<<grid, kT2, Lane2Smem::total, stream>>>(P);
 #ifdef RTCLJ_TAIL_PROBE
       if (const char* path = std::getenv("RTCLJ_TAIL_PROBE_FILE")) {
@@ -543,6 +557,7 @@ int rtclj_ctx_render(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* 
     } else {
       // scenes of fewer than 64 spheres: their own instantiation (packed prefilter candidates, 768 threads), measured
       // per regime -- rtclj_kernels.cuh, render_kernel / threads_of
+      const bool const_tab = ch.const_tab, sample_buf = ps.sample_buf != nullptr;
       const bool packed = RTCLJ_PACKED_CANDS && const_tab && c->n < 64;
       P.stack_stride = (unsigned)grid * (unsigned)threads_of(const_tab, packed);
       if (prm->flags & RTCLJ_F_REVERSE_PRODUCT) {
@@ -560,20 +575,74 @@ int rtclj_ctx_render(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* 
     CU(cudaGetLastError());
   }
   CU(cudaEventRecord(c->ev1, stream));
-  if (!wave && want_out) {
+  if (ps.finalize) {
     FParams F;
-    F.sample_buf = sample_buf; F.sample_stride = local_pixels;
-    F.partial = c->partial.p; F.out_linear = (double*)d_out_linear; F.out_rgb8 = (unsigned char*)d_out_rgb8;
-    F.W = W; F.spp = prm->spp; F.nchunks = nchunks;
-    F.shard_index = shard_index; F.shard_count = shard_count; F.shard_rows = shard_rows;
-    F.flags = prm->flags; F.local_pixels = local_pixels;
-    const unsigned blocks = (unsigned)((local_pixels + 255) / 256);
+    F.sample_buf = ps.sample_buf; F.sample_stride = sh.local_pixels;
+    F.partial = c->partial.p; F.out_linear = ps.out_linear; F.out_rgb8 = ps.out_rgb8;
+    F.W = cam->width; F.spp = ps.samples; F.nchunks = nchunks;
+    F.shard_index = sh.index; F.shard_count = sh.count; F.shard_rows = sh.rows;
+    F.flags = prm->flags; F.local_pixels = sh.local_pixels;
+    F.acc = ps.acc; F.seeded = ps.seeded; F.mean_n = ps.mean_n;
+    const unsigned blocks = (unsigned)((sh.local_pixels + 255) / 256);
     finalize_kernel<<<blocks, 256, 0, stream>>>(F);
     CU(cudaGetLastError());
   }
   CU(cudaEventRecord(c->ev2, stream));
   c->render_pending = true;
   return RTCLJ_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int rtclj_ctx_render(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, void* d_out_linear,
+                     void* d_out_rgb8, void* stream_) {
+  if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
+  if (!c->have_scene) return fail(RTCLJ_E_INVALID, "rtclj_ctx_set_scene has not been called");
+  int rc = validate(cam, prm);
+  if (rc) return rc;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  CU(cudaSetDevice(c->device));
+
+  const int W = cam->width, H = cam->height;
+  const Shard sh = shard_of(cam, prm);
+  const bool want_out = d_out_linear || d_out_rgb8;
+  const KernelChoice ch = choose_kernel(c, prm, (double)sh.local_pixels * (double)prm->spp);
+
+  // Summation unit.  Primary-ray renders (max-depth 1, normal shading) are bit-exact contracts and short
+  // paths: they default to the reference's strict sequential sum (raytracing.clj:142-155,
+  // raytracing_i.clj:146-163); other renders split a pixel into chunks for load balance.
+  int spu = prm->samples_per_unit > 0 ? prm->samples_per_unit
+                                      : (ch.primary_only ? prm->spp : auto_samples_per_unit(W, H, prm->spp));
+  if (spu > prm->spp) spu = prm->spp;
+  c->last_spu = spu;
+  // The strict order on long paths: one 500-sample unit lasts as long as its pixel's paths, the last ones
+  // run alone (measured: 622 vs 543 ms on one GPU, 162 vs 72 ms per GPU on eight).  Instead the samples are
+  // traced in small units and each sample's colour is STORED (32 B); finalize_kernel then adds them in
+  // sample order -- the same additions in the same order.  33 GB at 1920x1080 x 500 spp; HBM has 180 GB.
+  double* sample_buf = nullptr;
+  if (spu == prm->spp && !ch.primary_only && prm->spp >= 64 && ch.run_kernel && !ch.wave && want_out && sh.local_pixels > 0) {
+    const size_t need = (size_t)sh.local_pixels * (size_t)prm->spp * 4u;  // doubles
+    size_t free_b = 0, total_b = 0;
+    // kept in the context between renders (allocating 33 GB per frame costs more than the frame); a render
+    // that does not need it gives a large one back (below)
+    if (need <= c->sample_buf.cap ||
+        (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need * 8 < (free_b + c->sample_buf.cap * 8) / 2 &&
+         c->sample_buf.reserve(need) == cudaSuccess)) {
+      sample_buf = c->sample_buf.p;
+      spu = auto_samples_per_unit(W, H, prm->spp);  // scheduling units; the arithmetic stays strict
+    } else {
+      cudaGetLastError();  // too large: fall back to one unit per pixel
+    }
+  } else if (c->sample_buf.cap * 8 > ((size_t)1 << 30)) {
+    c->sample_buf.release();  // (synchronises the device; only on a strict -> chunked change of mode)
+  }
+  Pass ps;
+  ps.samples = prm->spp; ps.spu = spu; ps.sample_buf = sample_buf; ps.mean_n = prm->spp;
+  ps.finalize = !ch.wave && want_out;
+  ps.out_linear = (double*)d_out_linear; ps.out_rgb8 = (unsigned char*)d_out_rgb8;
+  return launch_pass(c, cam, prm, ch, sh, ps, stream);
 }
 
 int rtclj_ctx_stats(rtclj_ctx* c, void* stream_, rtclj_stats* st) {
@@ -738,6 +807,36 @@ int render_shard_hostbuf(const rtclj_scene* scene, const rtclj_camera* cam, cons
   return RTCLJ_OK;
 }
 
+// the device list of a multi-GPU call: not empty, every ordinal valid and listed once
+int check_devices(const int32_t* devices, int32_t n_devices) {
+  if (n_devices <= 0 || !devices) return fail(RTCLJ_E_INVALID, "empty device list");
+  int ndev = 0;
+  int rc = rtclj_device_count(&ndev);
+  if (rc) return rc;
+  if (ndev == 0) return fail(RTCLJ_E_NO_DEVICE, "no CUDA device (this library has no CPU fallback)");
+  for (int d = 0; d < n_devices; ++d) {
+    if (devices[d] < 0 || devices[d] >= ndev) return fail(RTCLJ_E_INVALID, "device %d out of range [0,%d)", devices[d], ndev);
+    for (int e = 0; e < d; ++e)
+      if (devices[e] == devices[d]) return fail(RTCLJ_E_INVALID, "device %d listed twice", devices[d]);
+  }
+  return RTCLJ_OK;
+}
+
+// the counters of a multi-GPU call: the devices' counts add up, the times are the slowest device's
+rtclj_stats sum_stats(const std::vector<rtclj_stats>& st) {
+  rtclj_stats total;
+  std::memset(&total, 0, sizeof total);
+  for (const rtclj_stats& s : st) {
+    total.samples += s.samples; total.segments += s.segments; total.exact_tests += s.exact_tests;
+    total.list_overflows += s.list_overflows; total.prefilter_tests += s.prefilter_tests;
+    total.device_ms = std::max(total.device_ms, s.device_ms);
+    total.kernel_ms = std::max(total.kernel_ms, s.kernel_ms);
+    total.samples_per_unit = s.samples_per_unit;
+  }
+  total.n_devices = (int32_t)st.size();
+  return total;
+}
+
 // nothing may throw across the C boundary (a JVM host would die): bad_alloc etc. become error codes
 template <class F>
 int guarded(F&& f) {
@@ -763,16 +862,8 @@ int rtclj_render_multi(const rtclj_scene* scene, const rtclj_camera* cam, const 
     if (!scene) return fail(RTCLJ_E_INVALID, "null scene");
     int rc = validate(cam, prm);
     if (rc) return rc;
-    if (n_devices <= 0 || !devices) return fail(RTCLJ_E_INVALID, "empty device list");
-    int ndev = 0;
-    rc = rtclj_device_count(&ndev);
+    rc = check_devices(devices, n_devices);
     if (rc) return rc;
-    if (ndev == 0) return fail(RTCLJ_E_NO_DEVICE, "no CUDA device (this library has no CPU fallback)");
-    for (int d = 0; d < n_devices; ++d) {
-      if (devices[d] < 0 || devices[d] >= ndev) return fail(RTCLJ_E_INVALID, "device %d out of range [0,%d)", devices[d], ndev);
-      for (int e = 0; e < d; ++e)
-        if (devices[e] == devices[d]) return fail(RTCLJ_E_INVALID, "device %d listed twice", devices[d]);
-    }
     std::vector<rtclj_params> p((size_t)n_devices, *prm);
     std::vector<rtclj_stats> st((size_t)n_devices);
     std::vector<int> rcs((size_t)n_devices, RTCLJ_OK);
@@ -795,18 +886,9 @@ int rtclj_render_multi(const rtclj_scene* scene, const rtclj_camera* cam, const 
     for (int d = 1; d < n_devices; ++d) pool.emplace_back(work, d);
     work(0);
     for (std::thread& t : pool) t.join();
-    rtclj_stats total;
-    std::memset(&total, 0, sizeof total);
-    for (int d = 0; d < n_devices; ++d) {
+    for (int d = 0; d < n_devices; ++d)
       if (rcs[(size_t)d]) { rtclj_error_set(msgs[(size_t)d].c_str()); return rcs[(size_t)d]; }
-      const rtclj_stats& s = st[(size_t)d];
-      total.samples += s.samples; total.segments += s.segments; total.exact_tests += s.exact_tests;
-      total.list_overflows += s.list_overflows; total.prefilter_tests += s.prefilter_tests;
-      total.device_ms = std::max(total.device_ms, s.device_ms);
-      total.kernel_ms = std::max(total.kernel_ms, s.kernel_ms);
-      total.samples_per_unit = s.samples_per_unit;
-    }
-    total.n_devices = n_devices;
+    rtclj_stats total = sum_stats(st);
     total.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (stats) *stats = total;
     return RTCLJ_OK;
@@ -822,6 +904,214 @@ int rtclj_render(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_
     rc = render_shard_hostbuf(scene, cam, prm, out_linear, out_rgb8, stats);
     if (rc == RTCLJ_OK && stats) stats->n_devices = 1;
     return rc;
+  });
+}
+
+// ---------------------------------------------------------------- accumulation over passes
+// The compute-pixel loop (src/raytracing.clj:141-171) run in passes: a pass adds samples [d, d + n) of every
+// pixel to the pixel's running sum, in the order a one-shot render adds them (DESIGN.md section 4.9).
+
+// The strict order of the general kernels goes through sample_buf (32 B per pixel and sample); an
+// accumulation's pass that needs more is cut into sub-passes of at most this many bytes, each followed by its
+// fold.  A one-shot strict render of 1920x1080 x 500 spp holds 33 GB; a strict accumulation never more than this.
+constexpr size_t kAccumSampleBufBytes = (size_t)2 << 30;
+
+int rtclj_ctx_accum_begin(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, int32_t* pass_unit,
+                          void* stream_) {
+  return guarded([&]() -> int {
+    if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
+    if (!c->have_scene) return fail(RTCLJ_E_INVALID, "rtclj_ctx_set_scene has not been called");
+    int rc = validate(cam, prm);
+    if (rc) return rc;
+    if (prm->flags & (RTCLJ_F_WAVE_KERNEL | RTCLJ_F_SPLIT_KERNEL))
+      return fail(RTCLJ_E_INVALID, "the wavefront and split kernels do not accumulate over passes");
+    // the kernels hold sample indices in 32-bit ints (render_lane2_kernel keeps k and k_end in shared memory
+    // as 32-bit words) and compute k + samples_per_unit: keep that sum below 2^31
+    if (prm->spp > (1 << 30)) return fail(RTCLJ_E_INVALID, "target of %d samples per pixel: at most 2^30", prm->spp);
+    c->accum.active = false;
+    CU(cudaSetDevice(c->device));
+    const bool primary_only = prm->max_depth == 1 || (prm->flags & RTCLJ_F_NORMAL_SHADING);
+    const bool strict = prm->samples_per_unit >= prm->spp || (prm->samples_per_unit <= 0 && primary_only);
+    const int unit = strict ? 1
+                            : (prm->samples_per_unit > 0 ? prm->samples_per_unit
+                                                         : auto_samples_per_unit(cam->width, cam->height, prm->spp));
+    const Shard sh = shard_of(cam, prm);
+    CU(c->acc.reserve(std::max<size_t>((size_t)sh.local_pixels * 3, 1)));
+    CU(cudaMemsetAsync(c->acc.p, 0, (size_t)sh.local_pixels * 3 * sizeof(double), (cudaStream_t)stream_));
+    c->accum.strict = strict;
+    c->accum.cam = *cam;
+    c->accum.prm = *prm;
+    c->accum.done = 0;
+    c->accum.pass_unit = unit;
+    c->accum.active = true;
+    if (pass_unit) *pass_unit = unit;
+    return RTCLJ_OK;
+  });
+}
+
+int rtclj_ctx_accum_step(rtclj_ctx* c, int32_t samples, void* d_out_linear, void* d_out_rgb8, int32_t* samples_done,
+                         void* stream_) {
+  return guarded([&]() -> int {
+    if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
+    auto& A = c->accum;
+    if (!A.active) return fail(RTCLJ_E_INVALID, "no accumulation: call rtclj_ctx_accum_begin (rtclj_ctx_set_scene ends one)");
+    const rtclj_params* prm = &A.prm;
+    const rtclj_camera* cam = &A.cam;
+    if (samples <= 0) return fail(RTCLJ_E_INVALID, "a pass needs a positive sample count, got %d", samples);
+    if ((long long)A.done + samples > (long long)prm->spp)
+      return fail(RTCLJ_E_INVALID, "pass of %d samples after %d: beyond the target of %d", samples, A.done, prm->spp);
+    if (A.done + samples != prm->spp && samples % A.pass_unit != 0)
+      return fail(RTCLJ_E_INVALID, "pass of %d samples: every pass but the last must be a multiple of pass_unit = %d",
+                  samples, A.pass_unit);
+    cudaStream_t stream = (cudaStream_t)stream_;
+    CU(cudaSetDevice(c->device));
+    const Shard sh = shard_of(cam, prm);
+    const KernelChoice ch = choose_kernel(c, prm, (double)sh.local_pixels * (double)samples);
+    const int d = A.done + samples;  // samples per pixel after this pass: the mean's divisor
+    Pass ps;
+    ps.sample_base = A.done; ps.samples = samples; ps.acc = c->acc.p; ps.mean_n = d; ps.finalize = true;
+    ps.out_linear = (double*)d_out_linear; ps.out_rgb8 = (unsigned char*)d_out_rgb8;
+    int rc = RTCLJ_OK;
+    if (!A.strict || !ch.run_kernel) {
+      // chunks of pass_unit samples, folded onto the running sums in chunk order (depth <= 0: one unit of black)
+      ps.spu = ch.run_kernel ? std::min(A.pass_unit, samples) : samples;
+      rc = launch_pass(c, cam, prm, ch, sh, ps, stream);
+    } else if (ch.primary) {
+      // one unit per pixel whose sums continue from the running sums: the reference's sequential sum in registers
+      ps.spu = samples; ps.seeded = true;
+      rc = launch_pass(c, cam, prm, ch, sh, ps, stream);
+    } else {
+      // every sample's colour through sample_buf, added in sample order by the fold: sub-passes of at most
+      // kAccumSampleBufBytes, the fold is sequential per sample, so the cut changes no bit
+      const size_t per_sample = (size_t)sh.local_pixels * 32u;
+      const int per = per_sample ? (int)std::min<size_t>(kAccumSampleBufBytes / per_sample, (size_t)samples) : samples;
+      if (per <= 0)
+        return fail(RTCLJ_E_TOO_LARGE, "%llu pixels: one sample of each exceeds the %zu-byte strict buffer; use chunks "
+                    "(samples_per_unit < spp)", sh.local_pixels, kAccumSampleBufBytes);
+      CU(c->sample_buf.reserve(std::max<size_t>((size_t)per * per_sample / 8u, 1)));
+      for (int b = 0; b < samples && rc == RTCLJ_OK; b += per) {
+        Pass sub = ps;
+        sub.sample_base = A.done + b;
+        sub.samples = std::min(per, samples - b);
+        sub.spu = auto_samples_per_unit(cam->width, cam->height, sub.samples);  // scheduling units only
+        sub.sample_buf = c->sample_buf.p;
+        sub.first = b == 0;
+        if (b + per < samples) { sub.out_linear = nullptr; sub.out_rgb8 = nullptr; }  // fold only
+        rc = launch_pass(c, cam, prm, ch, sh, sub, stream);
+      }
+    }
+    if (rc) { A.active = false; return rc; }  // the running sums may hold part of the pass
+    c->last_spu = A.strict ? d : A.pass_unit;
+    A.done = d;
+    if (samples_done) *samples_done = d;
+    return RTCLJ_OK;
+  });
+}
+
+// A progressive render into host buffers, rows interleaved over several GPUs as in rtclj_render_multi.  Each
+// device has a context of its own (not the cached one of rtclj_render, which other calls would give another
+// scene and with it end the accumulation), accumulating its shard of the rows.
+struct rtclj_progressive {
+  std::vector<rtclj_ctx*> ctxs;
+  std::vector<rtclj_params> prm;  // per device: its shard
+  rtclj_camera cam;
+  int spp = 0, pass_unit = 1, done = 0;
+  bool failed = false;  // a step failed on some device: the devices' running sums no longer agree
+  ~rtclj_progressive() { for (rtclj_ctx* c : ctxs) rtclj_ctx_destroy(c); }
+};
+
+int rtclj_progressive_create(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm,
+                             const int32_t* devices, int32_t n_devices, int32_t* pass_unit, rtclj_progressive** out) {
+  return guarded([&]() -> int {
+    if (!out) return fail(RTCLJ_E_INVALID, "null out");
+    *out = nullptr;
+    if (!scene) return fail(RTCLJ_E_INVALID, "null scene");
+    int rc = validate(cam, prm);
+    if (rc) return rc;
+    rc = check_devices(devices, n_devices);
+    if (rc) return rc;
+    std::unique_ptr<rtclj_progressive> p(new rtclj_progressive());
+    p->cam = *cam;
+    p->spp = prm->spp;
+    for (int d = 0; d < n_devices; ++d) {
+      rtclj_params q = *prm;
+      q.device = devices[d];
+      if (n_devices > 1) {
+        q.shard_index = d; q.shard_count = n_devices;
+        q.shard_rows = prm->shard_rows > 0 ? prm->shard_rows : 1;  // 1-row tiles balance best (DESIGN.md 6)
+      } else {
+        q.shard_index = 0; q.shard_count = 1; q.shard_rows = 0;
+      }
+      rtclj_ctx* c = nullptr;
+      rc = rtclj_ctx_create(devices[d], &c);
+      if (rc) return rc;
+      p->ctxs.push_back(c);
+      p->prm.push_back(q);
+      rc = rtclj_ctx_set_scene(c, scene);
+      if (rc) return rc;
+      rc = rtclj_ctx_accum_begin(c, cam, &q, &p->pass_unit, c->own_stream);
+      if (rc) return rc;
+    }
+    if (pass_unit) *pass_unit = p->pass_unit;
+    *out = p.release();
+    return RTCLJ_OK;
+  });
+}
+
+int rtclj_progressive_step(rtclj_progressive* p, int32_t samples, double* out_linear, uint8_t* out_rgb8,
+                           int32_t* samples_done, rtclj_stats* stats) {
+  return guarded([&]() -> int {
+    const auto t0 = std::chrono::steady_clock::now();
+    if (!p) return fail(RTCLJ_E_INVALID, "null progressive handle");
+    if (p->failed) return fail(RTCLJ_E_INVALID, "an earlier step failed: destroy this handle and create a new one");
+    // rtclj_ctx_accum_step's checks, made before any device starts, so that the devices stay in step
+    if (samples <= 0) return fail(RTCLJ_E_INVALID, "a pass needs a positive sample count, got %d", samples);
+    if ((long long)p->done + samples > (long long)p->spp)
+      return fail(RTCLJ_E_INVALID, "pass of %d samples after %d: beyond the target of %d", samples, p->done, p->spp);
+    if (p->done + samples != p->spp && samples % p->pass_unit != 0)
+      return fail(RTCLJ_E_INVALID, "pass of %d samples: every pass but the last must be a multiple of pass_unit = %d",
+                  samples, p->pass_unit);
+    const size_t n = p->ctxs.size();
+    const size_t npix = (size_t)p->cam.width * (size_t)p->cam.height;
+    std::vector<rtclj_stats> st(n);
+    std::vector<int> rcs(n, RTCLJ_OK);
+    std::vector<std::string> msgs(n);
+    auto shard = [&](size_t d) -> int {  // pass -> this device's rows of the caller's images -> counters
+      rtclj_ctx* c = p->ctxs[d];
+      const rtclj_params& q = p->prm[d];
+      CU(cudaSetDevice(c->device));
+      if (out_linear) CU(c->out_linear.reserve(npix * 3));
+      if (out_rgb8) CU(c->out_rgb8.reserve(npix * 3));
+      int r = rtclj_ctx_accum_step(c, samples, out_linear ? c->out_linear.p : nullptr, out_rgb8 ? c->out_rgb8.p : nullptr,
+                                   nullptr, c->own_stream);
+      if (r) return r;
+      r = download_rows(c, &p->cam, q.shard_index, q.shard_count, q.shard_rows, out_linear, out_rgb8, c->own_stream);
+      if (r) return r;
+      return rtclj_ctx_stats(c, c->own_stream, &st[d]);  // synchronises the stream: the direct copies have landed
+    };
+    auto work = [&](size_t d) {
+      rcs[d] = guarded([&]() { return shard(d); });
+      if (rcs[d]) msgs[d] = rtclj_error_get();  // the message is thread-local: carry it over
+    };
+    std::vector<std::thread> pool;
+    for (size_t d = 1; d < n; ++d) pool.emplace_back(work, d);
+    work(0);
+    for (std::thread& t : pool) t.join();
+    for (size_t d = 0; d < n; ++d)
+      if (rcs[d]) { p->failed = true; rtclj_error_set(msgs[d].c_str()); return rcs[d]; }
+    p->done += samples;
+    if (samples_done) *samples_done = p->done;
+    rtclj_stats total = sum_stats(st);
+    total.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = total;
+    return RTCLJ_OK;
+  });
+}
+
+int rtclj_progressive_destroy(rtclj_progressive* p) {
+  return guarded([&]() -> int {
+    delete p;  // (destroying the contexts waits for their streams)
+    return RTCLJ_OK;
   });
 }
 
@@ -906,18 +1196,9 @@ int rtclj_render_multi_ppm(const rtclj_scene* scene, const rtclj_camera* cam, co
     for (int d = 1; d < n_devices; ++d) pool.emplace_back(work, d);
     work(0);
     for (std::thread& t : pool) t.join();
-    rtclj_stats total;
-    std::memset(&total, 0, sizeof total);
-    for (int d = 0; d < n_devices; ++d) {
+    for (int d = 0; d < n_devices; ++d)
       if (rcs[(size_t)d]) { rtclj_error_set(msgs[(size_t)d].c_str()); return rcs[(size_t)d]; }
-      const rtclj_stats& s = st[(size_t)d];
-      total.samples += s.samples; total.segments += s.segments; total.exact_tests += s.exact_tests;
-      total.list_overflows += s.list_overflows; total.prefilter_tests += s.prefilter_tests;
-      total.device_ms = std::max(total.device_ms, s.device_ms);
-      total.kernel_ms = std::max(total.kernel_ms, s.kernel_ms);
-      total.samples_per_unit = s.samples_per_unit;
-    }
-    total.n_devices = n_devices;
+    rtclj_stats total = sum_stats(st);
     // the write-color! loop on the assembled image, then the text alone goes to the host
     CU(cudaSetDevice(root->device));
     size_t need = 0;

@@ -291,7 +291,7 @@ __device__ __forceinline__ void path_step(const KParams& P, PathRegs& pr, PathCo
           const int tile = lr / P.shard_rows;
           const int pj = (tile * P.shard_count + P.shard_index) * P.shard_rows + (lr - tile * P.shard_rows);
           pixel = (unsigned)pj * (unsigned)P.W + (unsigned)pi;
-          k = chunk * P.spu;
+          k = P.sample_base + chunk * P.spu;
           k_end = min(k + P.spu, P.spp);
           sums[0] = 0.0; sums[kSumStride] = 0.0; sums[2 * kSumStride] = 0.0;
           need_cam = true;

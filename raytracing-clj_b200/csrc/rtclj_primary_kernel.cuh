@@ -28,8 +28,12 @@ constexpr int kPrimarySpheres = 6;    // the measured crossover of scan vs cull 
 #endif
 constexpr int kPrimaryThreads = RTCLJ_PRIM_THREADS;
 
-template <bool kDefocus>  // (as a run-time branch the unused disk draw still costs its conversions: 3 % of a sample)
-__global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_primary_kernel(const __grid_constant__ KParams P) {
+// kSeeded: an accumulation's strict pass (rtclj_ctx_accum_step).  One unit per pixel, whose three sums start
+// from the pixel's running sums P.acc instead of 0.0, so that the pass continues the sequential sum of the
+// passes before it; finalize_kernel stores the unit sum back.  Its own kernel (render_primary_seeded_kernel),
+// so that render_primary_kernel's code stays as it is.
+template <bool kDefocus, bool kSeeded>
+__device__ __forceinline__ void render_primary_body(const KParams& P) {
   constexpr unsigned FULL = 0xffffffffu;
   const int lane = threadIdx.x & 31;
   const bool normal_shading = (P.flags & F_NORMAL_SHADING) != 0;
@@ -54,11 +58,13 @@ __global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_prima
     const int tile = lr / P.shard_rows;
     const int pj = (tile * P.shard_count + P.shard_index) * P.shard_rows + (lr - tile * P.shard_rows);
     const unsigned pixel = (unsigned)pj * (unsigned)P.W + (unsigned)pi;
-    const int k_end = min(chunk * P.spu + P.spu, P.spp);
+    const int k_begin = P.sample_base + chunk * P.spu;
+    const int k_end = min(k_begin + P.spu, P.spp);
     double sum_r = 0.0, sum_g = 0.0, sum_b = 0.0;
+    if (kSeeded) { const double* a = P.acc + (size_t)p_local * 3u; sum_r = a[0]; sum_g = a[1]; sum_b = a[2]; }
 
 #pragma unroll 1
-    for (int k = chunk * P.spu; k < k_end; ++k) {
+    for (int k = k_begin; k < k_end; ++k) {
       // ---- camera ray: raytracing.clj:144-151, realm/raytracing.clj:332-339, raytracing_i.clj:150-158
       uint4 w = RTCLJ_PHILOX(P, pixel, (unsigned)k, 0u, 0u);
       const double sx = (double)pi + (u24(w.x) - 0.5);
@@ -138,6 +144,16 @@ __global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_prima
       atomicAdd(P.stats + 2, s * (unsigned long long)n);
     }
   }
+}
+
+template <bool kDefocus>  // (as a run-time branch the unused disk draw still costs its conversions: 3 % of a sample)
+__global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_primary_kernel(const __grid_constant__ KParams P) {
+  render_primary_body<kDefocus, false>(P);
+}
+
+template <bool kDefocus>
+__global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_primary_seeded_kernel(const __grid_constant__ KParams P) {
+  render_primary_body<kDefocus, true>(P);
 }
 
 }  // namespace rtclj

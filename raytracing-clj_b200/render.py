@@ -150,6 +150,29 @@ class Context:
         _abi.check(_abi.lib().rtclj_ctx_stats(self._h, C.c_void_p(stream or None), C.byref(st)))
         return st.as_dict()
 
+    def accum_begin(self, cam, samples_per_px: int, max_depth: int, *, seed: int = 1, flags: int = _abi.FLAGS_MAIN,
+                    samples_per_unit: int = 0, shard: Optional[tuple] = None, stream: int = 0) -> int:
+        """Begins an accumulation over passes (rtclj_ctx_accum_begin) towards `samples_per_px` samples and
+        returns its pass unit: every pass but the last must be a multiple of it."""
+        cm = _camera_struct(cam)
+        prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit),
+                          0, 0, 0, int(self.device), 0)
+        if shard is not None:
+            prm.shard_index, prm.shard_count, prm.shard_rows = (int(x) for x in shard)
+        unit = C.c_int32()
+        _abi.check(_abi.lib().rtclj_ctx_accum_begin(self._h, C.byref(cm), C.byref(prm), C.byref(unit),
+                                                    C.c_void_p(stream or None)))
+        return unit.value
+
+    def accum_step(self, samples: int, d_out_linear: int = 0, d_out_rgb8: int = 0, stream: int = 0) -> int:
+        """Enqueues one pass of `samples` samples per pixel (rtclj_ctx_accum_step); the images at the device
+        pointers are those of a one-shot render of all samples so far.  Returns the samples done."""
+        done = C.c_int32()
+        _abi.check(_abi.lib().rtclj_ctx_accum_step(self._h, int(samples), C.c_void_p(d_out_linear or None),
+                                                   C.c_void_p(d_out_rgb8 or None), C.byref(done),
+                                                   C.c_void_p(stream or None)))
+        return done.value
+
     def encode_ppm(self, d_rgb8: int, width: int, height: int, d_out: int = 0, capacity: int = 0,
                    stream: int = 0) -> int:
         """The P3 writer (raytracing.clj:172-175) as device kernels: d_rgb8 -> text at d_out, both
@@ -170,6 +193,71 @@ class Context:
         if self._h:
             _abi.lib().rtclj_ctx_destroy(self._h)
             self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class Progressive:
+    """A render that refines pass by pass (rtclj_progressive_*): the compute-pixel loop (raytracing.clj:141-171)
+    run in passes into host buffers, rows interleaved over `devices` (default [0]).  After passes totalling d
+    samples the images are bit-identical to `render(..., samples_per_px=d)` in the same summation order, so the
+    last pass gives the one-shot image of `samples_per_px` samples.
+
+        with Progressive(world, cam, 500, 50) as p:
+            n = -(-25 // p.pass_unit) * p.pass_unit   # about 25 samples a pass, a multiple of the pass unit
+            while p.samples_done < p.samples_per_px:
+                lin, rgb8, st = p.step(min(n, p.samples_per_px - p.samples_done))   # show rgb8
+    """
+
+    def __init__(self, world, cam, samples_per_px: int = 100, max_depth: int = 50, *, seed: int = 1,
+                 flags: int = _abi.FLAGS_MAIN, samples_per_unit: int = 0, devices: Optional[Sequence[int]] = None):
+        self._h = C.c_void_p()
+        soa = _as_soa(world)
+        sc, cm = _scene_struct(soa), _camera_struct(cam)
+        self.height, self.width = cm.height, cm.width
+        self.samples_per_px = int(samples_per_px)
+        prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit),
+                          0, 0, 0, 0, 0)
+        devs = list(devices) if devices else [0]
+        arr = (C.c_int32 * len(devs))(*devs)
+        unit = C.c_int32()
+        _abi.check(_abi.lib().rtclj_progressive_create(C.byref(sc), C.byref(cm), C.byref(prm), arr, len(devs),
+                                                       C.byref(unit), C.byref(self._h)))
+        self.pass_unit = unit.value
+        self.samples_done = 0
+
+    def step(self, samples: int, *, want_linear: bool = True, want_rgb8: bool = True,
+             out_linear: Optional[np.ndarray] = None, out_rgb8: Optional[np.ndarray] = None):
+        """One pass of `samples` samples per pixel (the last pass may be any size; the others a multiple of
+        pass_unit).  Returns (linear float64 [H,W,3] | None, rgb8 uint8 [H,W,3] | None, stats dict) of the
+        image so far; out_linear / out_rgb8 are reused when given."""
+        if not self._h:
+            raise _abi.RtcljError(_abi.E_INVALID, "progressive render is closed")
+        if want_linear and out_linear is None:
+            out_linear = np.zeros((self.height, self.width, 3), dtype=np.float64)
+        if want_rgb8 and out_rgb8 is None:
+            out_rgb8 = np.zeros((self.height, self.width, 3), dtype=np.uint8)
+        done, st = C.c_int32(), _abi.Stats()
+        _abi.check(_abi.lib().rtclj_progressive_step(
+            self._h, int(samples), out_linear.ctypes.data if out_linear is not None else None,
+            out_rgb8.ctypes.data if out_rgb8 is not None else None, C.byref(done), C.byref(st)))
+        self.samples_done = done.value
+        return out_linear, out_rgb8, st.as_dict()
+
+    def close(self) -> None:
+        if self._h:
+            _abi.check(_abi.lib().rtclj_progressive_destroy(self._h))
+            self._h = C.c_void_p()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
 
     def __del__(self):
         try:
