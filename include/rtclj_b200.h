@@ -278,6 +278,40 @@ int rtclj_progressive_step(rtclj_progressive *p, int32_t samples, double *out_li
                            uint8_t *out_rgb8, int32_t *samples_done, rtclj_stats *stats);
 int rtclj_progressive_destroy(rtclj_progressive *p); /* NULL is fine */
 
+/* ---- Adaptive sampling: an accumulation whose passes trace only the pixels that are still noisy
+ * (DESIGN.md section 4.10).  Same pass rules, refusals and target as above, plus a tolerance {abs, rel}
+ * (finite, >= 0) and min_samples (>= 2 * pass_unit), else RTCLJ_E_INVALID.
+ *   - Every pixel starts active.  A pass of n samples after d traces samples [d, d + n) of the pixels active
+ *     when it starts; at its end each traced pixel p is tested and, once stopped, keeps its sample count n_p
+ *     for good.
+ *   - After every step the images of EVERY pixel are bit-identical to rtclj_ctx_render with spp = n_p and
+ *     samples_per_unit = pass_unit (strict order: = n_p); each step rewrites the whole image.
+ *   - The rule.  A unit is pass_unit samples (one chunk sum; strict order: one sample's colour).  Per pixel and
+ *     channel S1 = the running sum and S2 = the sum of the squared unit sums in unit order; m = ceil(n_p / u)
+ *     -- the short last chunk at the target counts as a unit like the others.  stderr = sqrt(fmax(((S2 -
+ *     S1*S1/m) / (m (m - 1))) / (u u), 0)).  The pixel stays active iff n_p < spp and (n_p < min_samples or
+ *     stderr > abs + rel * |mean| in some channel, mean = its linear value).
+ *   - A pixel's decision depends on its own sums only: for one sequence of pass sizes, images, sample-count
+ *     map and noise are the same on every device list, shard_rows and kernel.  A different sequence of pass
+ *     sizes may stop pixels at other counts.
+ *   - With min_samples >= spp no pixel stops early: the plain accumulation, bit for bit.
+ * Memory: 33 bytes per pixel of the shard on top of the accumulation's 24. */
+int rtclj_ctx_accum_begin_adaptive(rtclj_ctx *ctx, const rtclj_camera *camera, const rtclj_params *params,
+                                   const double tolerance[2] /* abs, rel */, int32_t min_samples,
+                                   int32_t *pass_unit, void *stream);
+/* after a step of an adaptive accumulation: d_samples (int32 W*H) / d_stderr (double W*H*3) are DEVICE
+ * pointers to full-size images, either may be NULL (the shard's rows are written); active_pixels != NULL
+ * synchronises `stream` and returns the shard's pixels still active.  RTCLJ_E_INVALID for a non-adaptive
+ * accumulation. */
+int rtclj_ctx_accum_noise(rtclj_ctx *ctx, int32_t *d_samples, double *d_stderr, uint64_t *active_pixels, void *stream);
+/* host buffers, as rtclj_progressive_create / rtclj_progressive_step; noise writes the whole sample-count map
+ * (int32 W*H) and noise estimate (double W*H*3), either may be NULL, and the pixels still active on all devices. */
+int rtclj_progressive_create_adaptive(const rtclj_scene *scene, const rtclj_camera *camera,
+                                      const rtclj_params *params, const double tolerance[2], int32_t min_samples,
+                                      const int32_t *devices, int32_t n_devices, int32_t *pass_unit,
+                                      rtclj_progressive **out);
+int rtclj_progressive_noise(rtclj_progressive *p, int32_t *samples, double *noise, uint64_t *active_pixels);
+
 /* Measures this GPU's arithmetic peaks with pure-FMA kernels (no memory traffic): scalar
  * FFMA, packed FFMA2 and fp64 DFMA, in TFLOP/s (2 flops per FMA), plus the SM count.
  * bench.py reports the roofline against these next to the nominal figure. */

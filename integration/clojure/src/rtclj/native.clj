@@ -204,6 +204,20 @@
 (def ^:private rtclj-progressive-destroy
   (downcall "rtclj_progressive_destroy" (fd-int ValueLayout/ADDRESS)))
 
+;; ---- adaptive sampling: passes trace only the pixels whose noise is still above a tolerance (DESIGN.md 4.10)
+;; int rtclj_progressive_create_adaptive(const rtclj_scene*, const rtclj_camera*, const rtclj_params*,
+;;                                       const double tolerance[2], int32_t min_samples, const int32_t* devices,
+;;                                       int32_t n_devices, int32_t* pass_unit, rtclj_progressive** out)
+(def ^:private rtclj-progressive-create-adaptive
+  (downcall "rtclj_progressive_create_adaptive"
+            (fd-int ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS
+                    ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/JAVA_INT ValueLayout/ADDRESS
+                    ValueLayout/ADDRESS)))
+;; int rtclj_progressive_noise(rtclj_progressive*, int32_t* samples, double* noise, uint64_t* active_pixels)
+(def ^:private rtclj-progressive-noise
+  (downcall "rtclj_progressive_noise"
+            (fd-int ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS)))
+
 (defn- pinned-bytes
   "n bytes of PINNED host memory (rtclj_host_alloc).  Returns [segment free-fn]."
   [^Arena a ^long n]
@@ -238,6 +252,58 @@
           (catch Throwable t
             (.invokeWithArguments rtclj-progressive-destroy [handle])
             (throw t)))))))
+
+(declare progressive-close!)
+
+(defn progressive-adaptive
+  "Begins an adaptive progressive render: `progressive`, but every pass traces only the pixels whose noise
+   estimate (the standard error of the pixel mean, per channel) is still above abs-tol + rel-tol * |mean|, after
+   at least :min-samples samples (at least two pass units; default exactly two).  A pixel that stops keeps its
+   image, bit-identical to `render` with its own sample count.  Use progressive-step!, progressive-noise and
+   progressive-close! on the handle."
+  [bodies cam samples-per-px max-depth abs-tol rel-tol & {:keys [devices min-samples] :or {devices [0]} :as opts}]
+  (with-open [a (Arena/ofConfined)]
+    (let [w    (long (:image-width cam))
+          h    (long (:image-height cam))
+          [scene camera params] (marshal a bodies cam samples-per-px max-depth opts)
+          tol  (.allocateFrom a ValueLayout/JAVA_DOUBLE (double-array [abs-tol rel-tol]))
+          unit (.allocate a 4 4)
+          slot (.allocate a 8 8)
+          create (fn [least]
+                   (.invokeWithArguments rtclj-progressive-create-adaptive
+                                         [scene camera params tol (int least)
+                                          (.allocateFrom a ValueLayout/JAVA_INT (int-array devices)) (int (count devices))
+                                          unit slot]))]
+      ;; the default minimum is two pass units: the unit comes from a plain create of the same params
+      (if min-samples
+        (check! (create min-samples))
+        (let [probe (progressive bodies cam samples-per-px max-depth opts)
+              least (* 2 (:pass-unit probe))]
+          (progressive-close! probe)
+          (check! (create least))))
+      (let [handle (.get slot ValueLayout/ADDRESS 0)]
+        (try
+          (let [[linear free-linear!] (pinned-doubles a (* 3 w h))
+                [rgb8 free-rgb8!]     (pinned-bytes a (* 3 w h))]
+            {:handle handle :pass-unit (.get unit ValueLayout/JAVA_INT 0) :samples-per-px samples-per-px
+             :width w :height h :linear linear :rgb8 rgb8 :free! (fn [] (free-linear!) (free-rgb8!))})
+          (catch Throwable t
+            (.invokeWithArguments rtclj-progressive-destroy [handle])
+            (throw t)))))))
+
+(defn progressive-noise
+  "After a step of a progressive-adaptive render: {:samples int[W*H], the samples each pixel has, :stderr
+   double[W*H*3], its noise estimate, :active, the pixels the next pass traces (0: the render is done)}."
+  [p]
+  (with-open [a (Arena/ofConfined)]
+    (let [n       (* (long (:width p)) (long (:height p)))
+          samples (.allocate a (* 4 n) 8)
+          stderr  (.allocate a (* 24 n) 8)
+          active  (.allocate a 8 8)]
+      (check! (.invokeWithArguments rtclj-progressive-noise [(:handle p) samples stderr active]))
+      {:samples (.toArray samples ValueLayout/JAVA_INT)
+       :stderr  (.toArray stderr ValueLayout/JAVA_DOUBLE)
+       :active  (.get active ValueLayout/JAVA_LONG 0)})))
 
 (defn progressive-step!
   "One pass of `samples` samples per pixel.  Returns {:linear :rgb8 :samples-done}: the image so far as

@@ -82,6 +82,13 @@ SYMBOLS = {
     "rtclj_progressive_step": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32),
                                          C.POINTER(Stats)]),
     "rtclj_progressive_destroy": (C.c_int, [C.c_void_p]),
+    "rtclj_ctx_accum_begin_adaptive": (C.c_int, [C.c_void_p, C.POINTER(Camera), C.POINTER(Params), C.POINTER(C.c_double),
+                                                 C.c_int32, C.POINTER(C.c_int32), C.c_void_p]),
+    "rtclj_ctx_accum_noise": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64), C.c_void_p]),
+    "rtclj_progressive_create_adaptive": (C.c_int, [C.POINTER(Scene), C.POINTER(Camera), C.POINTER(Params),
+                                                    C.POINTER(C.c_double), C.c_int32, C.POINTER(C.c_int32), C.c_int32,
+                                                    C.POINTER(C.c_int32), C.POINTER(C.c_void_p)]),
+    "rtclj_progressive_noise": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)]),
     "rtclj_calibrate_peaks": (C.c_int, [C.c_int32, C.POINTER(C.c_double), C.POINTER(C.c_double),
                                         C.POINTER(C.c_double), C.POINTER(C.c_int32)]),
     "rtclj_quantise_rgb8": (C.c_int, [C.c_void_p, C.c_size_t, C.c_uint32, C.c_void_p]),

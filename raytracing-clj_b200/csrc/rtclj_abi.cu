@@ -8,6 +8,7 @@
 #include "rtclj_primary_kernel.cuh"
 #include "rtclj_split_kernel.cuh"
 #include "rtclj_p3_kernels.cuh"
+#include "rtclj_adaptive.cuh"
 #include "rtclj_error.h"
 
 #include <algorithm>
@@ -98,8 +99,20 @@ struct rtclj_ctx {
     rtclj_params prm;        // prm.spp: the target
     int done = 0;            // samples per pixel so far
     int pass_unit = 1;
+    // adaptive accumulation (rtclj_ctx_accum_begin_adaptive): the stopping rule, DESIGN.md section 4.10
+    bool adaptive = false;
+    double abs_tol = 0.0, rel_tol = 0.0;
+    int min_samples = 0;
   } accum;
   DevBuf<double> acc;                   // the accumulation's running sums: 3 per local pixel
+  // adaptive accumulation, per local pixel: sums of squared unit sums (3 doubles), sample count, live flag, and
+  // the list of the live pixels (descending) that the listed kernels trace; list_aux = [count, tile counts...]
+  DevBuf<double> acc2;
+  DevBuf<int> nsamp;
+  DevBuf<unsigned char> live;
+  DevBuf<unsigned> list, list_aux;
+  DevBuf<int> noise_samples;            // rtclj_progressive_noise: full-size staging of the exported images
+  DevBuf<double> noise_stderr;
   double prim_geom[4 * kPrimarySpheres] = {};  // exact geometry of the first spheres: parameters of render_primary_kernel
   bool have_scene = false;
   bool render_pending = false;  // a render has been enqueued since the last scene upload / stats
@@ -263,6 +276,14 @@ int rtclj_ctx_create(int32_t device, rtclj_ctx** out) {
   CU(cudaFuncSetAttribute(render_lane2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Lane2Smem::total));
   CU(cudaFuncSetAttribute(render_split_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SplitSmem::total));
   CU(cudaFuncSetAttribute(render_split_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SplitSmem::total));
+  CU(cudaFuncSetAttribute(render_listed_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
+  CU(cudaFuncSetAttribute(render_listed_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
+  CU(cudaFuncSetAttribute(render_listed_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
+  CU(cudaFuncSetAttribute(render_listed_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
+  CU(cudaFuncSetAttribute(render_listed_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
+  CU(cudaFuncSetAttribute(render_listed_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
+  CU(cudaFuncSetAttribute(render_lane2_listed_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Lane2Smem::total));
+  CU(cudaFuncSetAttribute(render_lane2_listed_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Lane2Smem::total));
   *out = guard.release();
   return RTCLJ_OK;
 }
@@ -273,7 +294,8 @@ void rtclj_ctx_destroy(rtclj_ctx* c) {
   if (c->own_stream) cudaStreamSynchronize(c->own_stream);
   c->geom32.release(); c->geomA.release(); c->geom64.release(); c->mat.release(); c->partial.release();
   c->counters.release(); c->stack.release(); c->arrive.release(); c->sample_buf.release(); c->out_linear.release(); c->out_rgb8.release();
-  c->acc.release();
+  c->acc.release(); c->acc2.release(); c->nsamp.release(); c->live.release(); c->list.release(); c->list_aux.release();
+  c->noise_samples.release(); c->noise_stderr.release();
   c->p3_state.release(); c->p3_in.release(); c->p3_text.release();
   for (cudaEvent_t e : {c->ev0, c->ev1, c->ev2, c->p3_ev0, c->p3_ev1, c->pin_ev[0], c->pin_ev[1]})
     if (e) cudaEventDestroy(e);
@@ -454,9 +476,42 @@ struct Pass {
   int mean_n = 0;                // divisor of the pixel mean
   bool first = true;             // resets the counters and starts the timing: the first launch of a call
   bool finalize = false;
+  bool listed = false;           // adaptive accumulation: listed kernels, finalize_adaptive_kernel
+  bool decide = true;            // listed: the last launch of the pass applies the stopping rule and relists
   double* out_linear = nullptr;
   unsigned char* out_rgb8 = nullptr;
 };
+
+// render_kernel, or its listed twin (the pixels of KParams::list only)
+template <bool kConstTab, bool kSampleBuf, bool kPacked>
+void launch_render_kernel(bool listed, int grid, size_t sm, cudaStream_t stream, const KParams& P) {
+  if (listed) render_listed_kernel<kConstTab, kSampleBuf, kPacked><<<grid, threads_of(kConstTab, kPacked), sm, stream>>>(P);
+  else render_kernel<kConstTab, kSampleBuf, kPacked><<<grid, threads_of(kConstTab, kPacked), sm, stream>>>(P);
+}
+
+// the fold and stopping rule of an adaptive accumulation's pass, shard `sh` (finalize_adaptive_kernel)
+AParams adaptive_params(const rtclj_ctx* c, const Shard& sh) {
+  AParams A;
+  std::memset(&A, 0, sizeof A);
+  const auto& acc = c->accum;
+  A.W = acc.cam.width; A.shard_index = sh.index; A.shard_count = sh.count; A.shard_rows = sh.rows;
+  A.flags = acc.prm.flags; A.local_pixels = sh.local_pixels; A.sample_stride = sh.local_pixels;
+  A.acc = c->acc.p; A.acc2 = c->acc2.p; A.samples = c->nsamp.p; A.live = c->live.p;
+  A.strict = acc.strict; A.unit = acc.pass_unit; A.target = acc.prm.spp; A.min_samples = acc.min_samples;
+  A.abs_tol = acc.abs_tol; A.rel_tol = acc.rel_tol;
+  return A;
+}
+
+// rebuilds the list of live pixels and its count on the device (rtclj_adaptive.cuh)
+int relist(rtclj_ctx* c, unsigned long long local_pixels, cudaStream_t stream) {
+  if (local_pixels == 0) return RTCLJ_OK;
+  const unsigned tiles = (unsigned)((local_pixels + kListTile - 1) / kListTile);
+  list_count_kernel<<<tiles, kListThreads, 0, stream>>>(c->live.p, local_pixels, c->list_aux.p + 1);
+  list_scan_kernel<<<1, 1024, 0, stream>>>(c->list_aux.p + 1, tiles, c->list_aux.p);
+  list_scatter_kernel<<<tiles, kListThreads, 0, stream>>>(c->live.p, local_pixels, c->list_aux.p + 1, c->list.p);
+  CU(cudaGetLastError());
+  return RTCLJ_OK;
+}
 
 int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, const KernelChoice& ch, const Shard& sh,
                 const Pass& ps, cudaStream_t stream) {
@@ -501,13 +556,19 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
     P.geom32 = c->geom32.p; P.geomA = c->geomA.p; P.geom64 = c->geom64.p; P.mat = c->mat.p;
     P.partial = c->partial.p; P.acc = ps.acc; P.queue = c->counters.p; P.stats = c->counters.p + 1;
     P.sample_buf = ps.sample_buf; P.sample_stride = sh.local_pixels;
+    P.list = ps.listed ? c->list.p : nullptr; P.list_count = ps.listed ? c->list_aux.p : nullptr;
+    P.acc2 = ps.listed ? c->acc2.p : nullptr;
     if (ch.const_tab && !c->ctab_host.empty())
       std::memcpy(P.ctab, c->ctab_host.data(), std::min(sizeof P.ctab, c->ctab_host.size() * sizeof(float)));
     if (ch.primary) {
       std::memcpy(P.ctab, c->prim_geom, sizeof c->prim_geom);
       const unsigned long long want = (total_units + kPrimaryThreads - 1) / kPrimaryThreads;
       const unsigned blocks = (unsigned)std::min<unsigned long long>(want, (unsigned long long)grid * (unsigned long long)(2048 / kPrimaryThreads));
-      if (ps.seeded && P.use_defocus) render_primary_seeded_kernel<true><<<blocks, kPrimaryThreads, 0, stream>>>(P);
+      if (ps.listed && ps.seeded && P.use_defocus) render_primary_seeded_listed_kernel<true><<<blocks, kPrimaryThreads, 0, stream>>>(P);
+      else if (ps.listed && ps.seeded) render_primary_seeded_listed_kernel<false><<<blocks, kPrimaryThreads, 0, stream>>>(P);
+      else if (ps.listed && P.use_defocus) render_primary_listed_kernel<true><<<blocks, kPrimaryThreads, 0, stream>>>(P);
+      else if (ps.listed) render_primary_listed_kernel<false><<<blocks, kPrimaryThreads, 0, stream>>>(P);
+      else if (ps.seeded && P.use_defocus) render_primary_seeded_kernel<true><<<blocks, kPrimaryThreads, 0, stream>>>(P);
       else if (ps.seeded) render_primary_seeded_kernel<false><<<blocks, kPrimaryThreads, 0, stream>>>(P);
       else if (P.use_defocus) render_primary_kernel<true><<<blocks, kPrimaryThreads, 0, stream>>>(P);
       else render_primary_kernel<false><<<blocks, kPrimaryThreads, 0, stream>>>(P);
@@ -544,7 +605,9 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
       CU(cudaMemsetAsync(c->arrive.p, 0, probe_words * sizeof(unsigned), stream));
       P.arrive = c->arrive.p;
 #endif
-      if (ps.sample_buf) render_lane2_kernel<true><<<grid, kT2, Lane2Smem::total, stream>>>(P);
+      if (ps.listed && ps.sample_buf) render_lane2_listed_kernel<true><<<grid, kT2, Lane2Smem::total, stream>>>(P);
+      else if (ps.listed) render_lane2_listed_kernel<false><<<grid, kT2, Lane2Smem::total, stream>>>(P);
+      else if (ps.sample_buf) render_lane2_kernel<true><<<grid, kT2, Lane2Smem::total, stream>>>(P);
       else render_lane2_kernel<false><<<grid, kT2, Lane2Smem::total, stream>>>(P);
 #ifdef RTCLJ_TAIL_PROBE
       if (const char* path = std::getenv("RTCLJ_TAIL_PROBE_FILE")) {
@@ -565,17 +628,29 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
         P.stack = c->stack.p;
       }
       const size_t sm = smem_needed(c->nhalf, const_tab, c->smem_optin, packed);
-      if (const_tab && sample_buf && packed) render_kernel<true, true, true><<<grid, threads_of(true, true), sm, stream>>>(P);
-      else if (const_tab && packed) render_kernel<true, false, true><<<grid, threads_of(true, true), sm, stream>>>(P);
-      else if (const_tab && sample_buf) render_kernel<true, true><<<grid, threads_of(true), sm, stream>>>(P);
-      else if (const_tab) render_kernel<true, false><<<grid, threads_of(true), sm, stream>>>(P);
-      else if (sample_buf) render_kernel<false, true><<<grid, threads_of(false), sm, stream>>>(P);
-      else render_kernel<false, false><<<grid, threads_of(false), sm, stream>>>(P);
+      const bool listed = ps.listed;
+      if (const_tab && sample_buf && packed) launch_render_kernel<true, true, true>(listed, grid, sm, stream, P);
+      else if (const_tab && packed) launch_render_kernel<true, false, true>(listed, grid, sm, stream, P);
+      else if (const_tab && sample_buf) launch_render_kernel<true, true, false>(listed, grid, sm, stream, P);
+      else if (const_tab) launch_render_kernel<true, false, false>(listed, grid, sm, stream, P);
+      else if (sample_buf) launch_render_kernel<false, true, false>(listed, grid, sm, stream, P);
+      else launch_render_kernel<false, false, false>(listed, grid, sm, stream, P);
     }
     CU(cudaGetLastError());
   }
   CU(cudaEventRecord(c->ev1, stream));
-  if (ps.finalize) {
+  if (ps.finalize && ps.listed) {
+    AParams A = adaptive_params(c, sh);
+    A.sample_buf = ps.sample_buf; A.partial = c->partial.p; A.out_linear = ps.out_linear; A.out_rgb8 = ps.out_rgb8;
+    A.spp = ps.samples; A.nchunks = nchunks; A.seeded = ps.seeded; A.mean_n = ps.mean_n; A.decide = ps.decide;
+    const unsigned blocks = (unsigned)((sh.local_pixels + 255) / 256);
+    finalize_adaptive_kernel<<<blocks, 256, 0, stream>>>(A);
+    CU(cudaGetLastError());
+    if (ps.decide) {
+      int rc = relist(c, sh.local_pixels, stream);
+      if (rc) return rc;
+    }
+  } else if (ps.finalize) {
     FParams F;
     F.sample_buf = ps.sample_buf; F.sample_stride = sh.local_pixels;
     F.partial = c->partial.p; F.out_linear = ps.out_linear; F.out_rgb8 = ps.out_rgb8;
@@ -916,36 +991,98 @@ int rtclj_render(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_
 // fold.  A one-shot strict render of 1920x1080 x 500 spp holds 33 GB; a strict accumulation never more than this.
 constexpr size_t kAccumSampleBufBytes = (size_t)2 << 30;
 
+}  // extern "C"
+
+namespace {
+
+// the pass unit of an accumulation: 1 in strict order, else the one-shot render's unit size
+int accum_pass_unit(const rtclj_camera* cam, const rtclj_params* prm, bool* strict_out) {
+  const bool primary_only = prm->max_depth == 1 || (prm->flags & RTCLJ_F_NORMAL_SHADING);
+  const bool strict = prm->samples_per_unit >= prm->spp || (prm->samples_per_unit <= 0 && primary_only);
+  if (strict_out) *strict_out = strict;
+  return strict ? 1
+                : (prm->samples_per_unit > 0 ? prm->samples_per_unit
+                                             : auto_samples_per_unit(cam->width, cam->height, prm->spp));
+}
+
+// the arguments of an adaptive accumulation (checked before any device is touched): tolerance = {abs, rel}, both
+// finite and >= 0; min_samples >= 2 pass units, so that the estimate has at least two units
+int check_adaptive(const rtclj_camera* cam, const rtclj_params* prm, const double* tol, int32_t min_samples) {
+  if (!tol) return fail(RTCLJ_E_INVALID, "null tolerance");
+  if (!(std::isfinite(tol[0]) && std::isfinite(tol[1]) && tol[0] >= 0.0 && tol[1] >= 0.0))
+    return fail(RTCLJ_E_INVALID, "tolerances must be finite and >= 0, got %g, %g", tol[0], tol[1]);
+  int rc = validate(cam, prm);
+  if (rc) return rc;
+  const int unit = accum_pass_unit(cam, prm, nullptr);
+  if ((long long)min_samples < 2ll * unit)
+    return fail(RTCLJ_E_INVALID, "min_samples = %d: at least two pass units (%d)", min_samples, 2 * unit);
+  return RTCLJ_OK;
+}
+
+// tol == nullptr: a plain accumulation
+int accum_begin(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, const double* tol, int32_t min_samples,
+                int32_t* pass_unit, cudaStream_t stream) {
+  if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
+  if (!c->have_scene) return fail(RTCLJ_E_INVALID, "rtclj_ctx_set_scene has not been called");
+  int rc = tol ? check_adaptive(cam, prm, tol, min_samples) : validate(cam, prm);
+  if (rc) return rc;
+  if (prm->flags & (RTCLJ_F_WAVE_KERNEL | RTCLJ_F_SPLIT_KERNEL))
+    return fail(RTCLJ_E_INVALID, "the wavefront and split kernels do not accumulate over passes");
+  // the kernels hold sample indices in 32-bit ints (render_lane2_kernel keeps k and k_end in shared memory
+  // as 32-bit words) and compute k + samples_per_unit: keep that sum below 2^31
+  if (prm->spp > (1 << 30)) return fail(RTCLJ_E_INVALID, "target of %d samples per pixel: at most 2^30", prm->spp);
+  c->accum.active = false;
+  CU(cudaSetDevice(c->device));
+  bool strict = false;
+  const int unit = accum_pass_unit(cam, prm, &strict);
+  const Shard sh = shard_of(cam, prm);
+  const size_t npix = (size_t)sh.local_pixels;
+  CU(c->acc.reserve(std::max<size_t>(npix * 3, 1)));
+  CU(cudaMemsetAsync(c->acc.p, 0, npix * 3 * sizeof(double), stream));
+  if (tol) {
+    // every pixel starts live, with no samples and S2 = 0; the list of all pixels is built by the compaction
+    const size_t tiles = (npix + kListTile - 1) / kListTile;
+    CU(c->acc2.reserve(std::max<size_t>(npix * 3, 1)));
+    CU(c->nsamp.reserve(std::max<size_t>(npix, 1)));
+    CU(c->live.reserve(std::max<size_t>(npix, 1)));
+    CU(c->list.reserve(std::max<size_t>(npix, 1)));
+    CU(c->list_aux.reserve(1 + tiles));
+    CU(cudaMemsetAsync(c->acc2.p, 0, npix * 3 * sizeof(double), stream));
+    CU(cudaMemsetAsync(c->nsamp.p, 0, npix * sizeof(int), stream));
+    CU(cudaMemsetAsync(c->live.p, 1, npix, stream));
+    CU(cudaMemsetAsync(c->list_aux.p, 0, sizeof(unsigned), stream));
+    rc = relist(c, sh.local_pixels, stream);
+    if (rc) return rc;
+  }
+  c->accum.strict = strict;
+  c->accum.cam = *cam;
+  c->accum.prm = *prm;
+  c->accum.done = 0;
+  c->accum.pass_unit = unit;
+  c->accum.adaptive = tol != nullptr;
+  c->accum.abs_tol = tol ? tol[0] : 0.0;
+  c->accum.rel_tol = tol ? tol[1] : 0.0;
+  c->accum.min_samples = tol ? min_samples : 0;
+  c->accum.active = true;
+  if (pass_unit) *pass_unit = unit;
+  return RTCLJ_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
 int rtclj_ctx_accum_begin(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, int32_t* pass_unit,
                           void* stream_) {
+  return guarded([&]() -> int { return accum_begin(c, cam, prm, nullptr, 0, pass_unit, (cudaStream_t)stream_); });
+}
+
+int rtclj_ctx_accum_begin_adaptive(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm,
+                                   const double tolerance[2], int32_t min_samples, int32_t* pass_unit, void* stream_) {
   return guarded([&]() -> int {
     if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
-    if (!c->have_scene) return fail(RTCLJ_E_INVALID, "rtclj_ctx_set_scene has not been called");
-    int rc = validate(cam, prm);
-    if (rc) return rc;
-    if (prm->flags & (RTCLJ_F_WAVE_KERNEL | RTCLJ_F_SPLIT_KERNEL))
-      return fail(RTCLJ_E_INVALID, "the wavefront and split kernels do not accumulate over passes");
-    // the kernels hold sample indices in 32-bit ints (render_lane2_kernel keeps k and k_end in shared memory
-    // as 32-bit words) and compute k + samples_per_unit: keep that sum below 2^31
-    if (prm->spp > (1 << 30)) return fail(RTCLJ_E_INVALID, "target of %d samples per pixel: at most 2^30", prm->spp);
-    c->accum.active = false;
-    CU(cudaSetDevice(c->device));
-    const bool primary_only = prm->max_depth == 1 || (prm->flags & RTCLJ_F_NORMAL_SHADING);
-    const bool strict = prm->samples_per_unit >= prm->spp || (prm->samples_per_unit <= 0 && primary_only);
-    const int unit = strict ? 1
-                            : (prm->samples_per_unit > 0 ? prm->samples_per_unit
-                                                         : auto_samples_per_unit(cam->width, cam->height, prm->spp));
-    const Shard sh = shard_of(cam, prm);
-    CU(c->acc.reserve(std::max<size_t>((size_t)sh.local_pixels * 3, 1)));
-    CU(cudaMemsetAsync(c->acc.p, 0, (size_t)sh.local_pixels * 3 * sizeof(double), (cudaStream_t)stream_));
-    c->accum.strict = strict;
-    c->accum.cam = *cam;
-    c->accum.prm = *prm;
-    c->accum.done = 0;
-    c->accum.pass_unit = unit;
-    c->accum.active = true;
-    if (pass_unit) *pass_unit = unit;
-    return RTCLJ_OK;
+    if (!tolerance) return fail(RTCLJ_E_INVALID, "null tolerance");
+    return accum_begin(c, cam, prm, tolerance, min_samples, pass_unit, (cudaStream_t)stream_);
   });
 }
 
@@ -970,6 +1107,7 @@ int rtclj_ctx_accum_step(rtclj_ctx* c, int32_t samples, void* d_out_linear, void
     const int d = A.done + samples;  // samples per pixel after this pass: the mean's divisor
     Pass ps;
     ps.sample_base = A.done; ps.samples = samples; ps.acc = c->acc.p; ps.mean_n = d; ps.finalize = true;
+    ps.listed = A.adaptive;  // only the live pixels, each folded and tested (finalize_adaptive_kernel)
     ps.out_linear = (double*)d_out_linear; ps.out_rgb8 = (unsigned char*)d_out_rgb8;
     int rc = RTCLJ_OK;
     if (!A.strict || !ch.run_kernel) {
@@ -996,6 +1134,7 @@ int rtclj_ctx_accum_step(rtclj_ctx* c, int32_t samples, void* d_out_linear, void
         sub.spu = auto_samples_per_unit(cam->width, cam->height, sub.samples);  // scheduling units only
         sub.sample_buf = c->sample_buf.p;
         sub.first = b == 0;
+        sub.decide = b + per >= samples;
         if (b + per < samples) { sub.out_linear = nullptr; sub.out_rgb8 = nullptr; }  // fold only
         rc = launch_pass(c, cam, prm, ch, sh, sub, stream);
       }
@@ -1008,6 +1147,29 @@ int rtclj_ctx_accum_step(rtclj_ctx* c, int32_t samples, void* d_out_linear, void
   });
 }
 
+int rtclj_ctx_accum_noise(rtclj_ctx* c, int32_t* d_samples, double* d_stderr, uint64_t* active_pixels, void* stream_) {
+  return guarded([&]() -> int {
+    if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
+    if (!c->accum.active || !c->accum.adaptive)
+      return fail(RTCLJ_E_INVALID, "no adaptive accumulation: call rtclj_ctx_accum_begin_adaptive");
+    cudaStream_t stream = (cudaStream_t)stream_;
+    CU(cudaSetDevice(c->device));
+    const Shard sh = shard_of(&c->accum.cam, &c->accum.prm);
+    if ((d_samples || d_stderr) && sh.local_pixels > 0) {
+      const unsigned blocks = (unsigned)((sh.local_pixels + 255) / 256);
+      noise_export_kernel<<<blocks, 256, 0, stream>>>(adaptive_params(c, sh), d_samples, d_stderr);
+      CU(cudaGetLastError());
+    }
+    if (active_pixels) {
+      unsigned n = 0;
+      CU(cudaMemcpyAsync(&n, c->list_aux.p, sizeof n, cudaMemcpyDeviceToHost, stream));
+      CU(cudaStreamSynchronize(stream));
+      *active_pixels = n;
+    }
+    return RTCLJ_OK;
+  });
+}
+
 // A progressive render into host buffers, rows interleaved over several GPUs as in rtclj_render_multi.  Each
 // device has a context of its own (not the cached one of rtclj_render, which other calls would give another
 // scene and with it end the accumulation), accumulating its shard of the rows.
@@ -1016,23 +1178,35 @@ struct rtclj_progressive {
   std::vector<rtclj_params> prm;  // per device: its shard
   rtclj_camera cam;
   int spp = 0, pass_unit = 1, done = 0;
+  bool adaptive = false;
   bool failed = false;  // a step failed on some device: the devices' running sums no longer agree
   ~rtclj_progressive() { for (rtclj_ctx* c : ctxs) rtclj_ctx_destroy(c); }
 };
 
-int rtclj_progressive_create(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm,
-                             const int32_t* devices, int32_t n_devices, int32_t* pass_unit, rtclj_progressive** out) {
+}  // extern "C"
+
+namespace {
+
+// tol == nullptr: a plain accumulation
+int progressive_create(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm, const double* tol,
+                       int32_t min_samples, const int32_t* devices, int32_t n_devices, int32_t* pass_unit,
+                       rtclj_progressive** out) {
   return guarded([&]() -> int {
     if (!out) return fail(RTCLJ_E_INVALID, "null out");
     *out = nullptr;
     if (!scene) return fail(RTCLJ_E_INVALID, "null scene");
     int rc = validate(cam, prm);
     if (rc) return rc;
+    if (tol) {
+      rc = check_adaptive(cam, prm, tol, min_samples);
+      if (rc) return rc;
+    }
     rc = check_devices(devices, n_devices);
     if (rc) return rc;
     std::unique_ptr<rtclj_progressive> p(new rtclj_progressive());
     p->cam = *cam;
     p->spp = prm->spp;
+    p->adaptive = tol != nullptr;
     for (int d = 0; d < n_devices; ++d) {
       rtclj_params q = *prm;
       q.device = devices[d];
@@ -1049,13 +1223,30 @@ int rtclj_progressive_create(const rtclj_scene* scene, const rtclj_camera* cam, 
       p->prm.push_back(q);
       rc = rtclj_ctx_set_scene(c, scene);
       if (rc) return rc;
-      rc = rtclj_ctx_accum_begin(c, cam, &q, &p->pass_unit, c->own_stream);
+      rc = accum_begin(c, cam, &q, tol, min_samples, &p->pass_unit, c->own_stream);
       if (rc) return rc;
     }
     if (pass_unit) *pass_unit = p->pass_unit;
     *out = p.release();
     return RTCLJ_OK;
   });
+}
+
+}  // namespace
+
+extern "C" {
+
+int rtclj_progressive_create(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm,
+                             const int32_t* devices, int32_t n_devices, int32_t* pass_unit, rtclj_progressive** out) {
+  return progressive_create(scene, cam, prm, nullptr, 0, devices, n_devices, pass_unit, out);
+}
+
+int rtclj_progressive_create_adaptive(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm,
+                                      const double tolerance[2], int32_t min_samples, const int32_t* devices,
+                                      int32_t n_devices, int32_t* pass_unit, rtclj_progressive** out) {
+  if (out) *out = nullptr;
+  if (!tolerance) return fail(RTCLJ_E_INVALID, "null tolerance");
+  return progressive_create(scene, cam, prm, tolerance, min_samples, devices, n_devices, pass_unit, out);
 }
 
 int rtclj_progressive_step(rtclj_progressive* p, int32_t samples, double* out_linear, uint8_t* out_rgb8,
@@ -1104,6 +1295,43 @@ int rtclj_progressive_step(rtclj_progressive* p, int32_t samples, double* out_li
     rtclj_stats total = sum_stats(st);
     total.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (stats) *stats = total;
+    return RTCLJ_OK;
+  });
+}
+
+int rtclj_progressive_noise(rtclj_progressive* p, int32_t* samples, double* stderr_, uint64_t* active_pixels) {
+  return guarded([&]() -> int {
+    if (!p) return fail(RTCLJ_E_INVALID, "null progressive handle");
+    if (!p->adaptive) return fail(RTCLJ_E_INVALID, "not an adaptive progressive render");
+    if (p->failed) return fail(RTCLJ_E_INVALID, "an earlier step failed: destroy this handle and create a new one");
+    const size_t W = (size_t)p->cam.width, H = (size_t)p->cam.height;
+    uint64_t total = 0;
+    for (size_t d = 0; d < p->ctxs.size(); ++d) {  // (small images: one device after the other)
+      rtclj_ctx* c = p->ctxs[d];
+      const rtclj_params& q = p->prm[d];
+      CU(cudaSetDevice(c->device));
+      if (samples) CU(c->noise_samples.reserve(W * H));
+      if (stderr_) CU(c->noise_stderr.reserve(W * H * 3));
+      uint64_t n = 0;
+      int rc = rtclj_ctx_accum_noise(c, samples ? c->noise_samples.p : nullptr, stderr_ ? c->noise_stderr.p : nullptr, &n,
+                                     c->own_stream);
+      if (rc) return rc;
+      total += n;
+      std::vector<Piece> pieces;
+      if (samples) {
+        plan_pieces(H, W * sizeof(int32_t), q.shard_index, q.shard_count, q.shard_rows, kStageBytes, pieces);
+        rc = download_image(c, pieces, (char*)samples, (const char*)c->noise_samples.p, c->own_stream);
+        if (rc) return rc;
+      }
+      if (stderr_) {
+        pieces.clear();
+        plan_pieces(H, W * 3 * sizeof(double), q.shard_index, q.shard_count, q.shard_rows, kStageBytes, pieces);
+        rc = download_image(c, pieces, (char*)stderr_, (const char*)c->noise_stderr.p, c->own_stream);
+        if (rc) return rc;
+      }
+      CU(cudaStreamSynchronize(c->own_stream));  // the direct copies into pinned memory have landed
+    }
+    if (active_pixels) *active_pixels = total;
     return RTCLJ_OK;
   });
 }

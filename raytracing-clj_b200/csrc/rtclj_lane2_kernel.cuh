@@ -32,8 +32,10 @@ struct Lane2Smem {
   static constexpr size_t total = u32 + (size_t)7 * kT2 * 4;
 };
 
-template <bool kSampleBuf>  // strict order through the per-sample buffer: its own instantiation (rtclj_kernels.cuh)
-__global__ void __launch_bounds__(kT2, 1) render_lane2_kernel(const __grid_constant__ KParams P) {
+// kSampleBuf: strict order through the per-sample buffer, its own instantiation (rtclj_kernels.cuh); kListed: the
+// pixels of KParams::list only (render_lane2_listed_kernel)
+template <bool kSampleBuf, bool kListed>
+__device__ __forceinline__ void render_lane2_body(const KParams& P) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int tid = threadIdx.x, lane = tid & 31;
   const unsigned gtid = blockIdx.x * kT2 + tid;
@@ -43,6 +45,7 @@ __global__ void __launch_bounds__(kT2, 1) render_lane2_kernel(const __grid_const
   unsigned* const wU = reinterpret_cast<unsigned*>(smem_raw + Lane2Smem::u32) + tid;              // [c * kT2]
   const unsigned flags = P.flags;
   const unsigned FULL = 0xffffffffu;
+  const unsigned long long total_units = kListed ? total_units_of<true>(P) : 0ull;
 
   // the path in registers
   PathRegs pr;
@@ -119,9 +122,9 @@ __global__ void __launch_bounds__(kT2, 1) render_lane2_kernel(const __grid_const
 #pragma unroll 1
     for (int path = 0; path < 2; ++path) {
       const unsigned mask_shift = path ? 16u : 0u;
-      path_step<kSampleBuf, kT2>(P, pr, pc, path ? bany1 : bany0,
-                                 [&](int j) { return ~(my_mask[j * kT2] >> mask_shift) & 0xffffu; },
-                                 my_sums + path * 3 * kT2, (size_t)gtid * 2u + (size_t)path, lane);
+      path_step<kSampleBuf, kT2, kListed>(P, pr, pc, path ? bany1 : bany0,
+                                          [&](int j) { return ~(my_mask[j * kT2] >> mask_shift) & 0xffffu; },
+                                          my_sums + path * 3 * kT2, (size_t)gtid * 2u + (size_t)path, lane, total_units);
 
       // ---- swap: this path waits in shared memory while the other one is processed / both are culled
       {
@@ -156,6 +159,16 @@ __global__ void __launch_bounds__(kT2, 1) render_lane2_kernel(const __grid_const
       if (lane == 0) atomicAdd(P.stats + q, (unsigned long long)lo + ((unsigned long long)hi << 16));
     }
   }
+}
+
+template <bool kSampleBuf>
+__global__ void __launch_bounds__(kT2, 1) render_lane2_kernel(const __grid_constant__ KParams P) {
+  render_lane2_body<kSampleBuf, false>(P);
+}
+
+template <bool kSampleBuf>
+__global__ void __launch_bounds__(kT2, 1) render_lane2_listed_kernel(const __grid_constant__ KParams P) {
+  render_lane2_body<kSampleBuf, true>(P);
 }
 
 // (The same loop with ONE path per lane built on path_step() was measured against render_kernel<true>: equal on

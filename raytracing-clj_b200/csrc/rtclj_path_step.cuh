@@ -43,9 +43,11 @@ struct PathCounters { unsigned samples, seg, exact, pref; };
 // bany: which cull blocks have a survivor for this path (block j at bit 32 - nconst + j);
 // survivors_of_block(j): the 16 survivor bits of block j (sphere s of the block -> bit 15 - s);
 // sums: the path's three unit sums, kSumStride doubles apart; stack_col: its column of the attenuation stack.
-template <bool kSampleBuf, int kSumStride, class SurvivorsOfBlock>
+// kListed: tickets go to the pixels of KParams::list, `total_units` of them (total_units_of, read once per kernel).
+template <bool kSampleBuf, int kSumStride, bool kListed = false, class SurvivorsOfBlock>
 __device__ __forceinline__ void path_step(const KParams& P, PathRegs& pr, PathCounters& pc, unsigned bany,
-                                          SurvivorsOfBlock survivors_of_block, double* sums, size_t stack_col, int lane) {
+                                          SurvivorsOfBlock survivors_of_block, double* sums, size_t stack_col, int lane,
+                                          unsigned long long total_units = 0) {
   d3& O = pr.O; d3& D = pr.D;
   unsigned& pixel = pr.pixel; unsigned& unit = pr.unit;
   int& k = pr.k; int& k_end = pr.k_end; int& depth_left = pr.depth_left; int& nstack = pr.nstack; int& status = pr.status;
@@ -281,10 +283,11 @@ __device__ __forceinline__ void path_step(const KParams& P, PathRegs& pr, PathCo
       base = __shfl_sync(FULL, base, leader);
       if (need_unit) {
         const unsigned long long ticket = base + (unsigned long long)__popc(mask & ((1u << lane) - 1u));
-        if (ticket >= P.total_units) {
+        if (ticket >= (kListed ? total_units : P.total_units)) {
           status = PS_DEAD;
         } else {
-          const unsigned p_local = unit_of_ticket(P, (unsigned)ticket, unit);
+          const unsigned p_local = kListed ? unit_of_listed_ticket(P, (unsigned)ticket, unit)
+                                           : unit_of_ticket(P, (unsigned)ticket, unit);
           const int chunk = (int)(unit - p_local * (unsigned)P.nchunks);
           const int lr = (int)(p_local / (unsigned)P.W);
           const int pi = (int)(p_local - (unsigned)lr * (unsigned)P.W);

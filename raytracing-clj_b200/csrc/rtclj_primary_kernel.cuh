@@ -32,9 +32,13 @@ constexpr int kPrimaryThreads = RTCLJ_PRIM_THREADS;
 // from the pixel's running sums P.acc instead of 0.0, so that the pass continues the sequential sum of the
 // passes before it; finalize_kernel stores the unit sum back.  Its own kernel (render_primary_seeded_kernel),
 // so that render_primary_kernel's code stays as it is.
-template <bool kDefocus, bool kSeeded>
+// kListed: the pixels of KParams::list only (an adaptive accumulation's pass, DESIGN.md section 4.10).  Seeded and
+// listed, the kernel also continues the pixel's sums of squared sample colours (KParams::acc2) in three more
+// registers, in sample order, and stores them back in place: the fold's S2 in strict order without a sample buffer.
+template <bool kDefocus, bool kSeeded, bool kListed = false>
 __device__ __forceinline__ void render_primary_body(const KParams& P) {
   constexpr unsigned FULL = 0xffffffffu;
+  constexpr bool kMoments = kSeeded && kListed;
   const int lane = threadIdx.x & 31;
   const bool normal_shading = (P.flags & F_NORMAL_SHADING) != 0;
   const double* __restrict__ G = reinterpret_cast<const double*>(P.ctab);  // [n][cx, cy, cz, r]
@@ -46,12 +50,15 @@ __device__ __forceinline__ void render_primary_body(const KParams& P) {
     unsigned long long base = 0;
     if (lane == 0) base = atomicAdd(P.queue, 32ull);
     base = __shfl_sync(FULL, base, 0);
-    if (base >= P.total_units) break;
+    // (listed: the count is read again per ticket -- an L1 hit; held across the sample loop it costs a spill at
+    // the 80 registers of three CTAs per SM)
+    const unsigned long long total_units = total_units_of<kListed>(P);
+    if (base >= total_units) break;
     const unsigned long long ticket = base + (unsigned long long)lane;
-    if (ticket >= P.total_units) continue;  // (tail of the last ticket: the lane waits at the next shuffle, which ends the loop)
+    if (ticket >= total_units) continue;  // (tail of the last ticket: the lane waits at the next shuffle, which ends the loop)
 
-    const unsigned unit = (unsigned)ticket;
-    const unsigned p_local = unit / (unsigned)P.nchunks;
+    unsigned unit = (unsigned)ticket;
+    const unsigned p_local = kListed ? unit_of_listed_ticket(P, (unsigned)ticket, unit) : unit / (unsigned)P.nchunks;
     const int chunk = (int)(unit - p_local * (unsigned)P.nchunks);
     const int lr = (int)(p_local / (unsigned)P.W);
     const int pi = (int)(p_local - (unsigned)lr * (unsigned)P.W);
@@ -62,6 +69,8 @@ __device__ __forceinline__ void render_primary_body(const KParams& P) {
     const int k_end = min(k_begin + P.spu, P.spp);
     double sum_r = 0.0, sum_g = 0.0, sum_b = 0.0;
     if (kSeeded) { const double* a = P.acc + (size_t)p_local * 3u; sum_r = a[0]; sum_g = a[1]; sum_b = a[2]; }
+    double sq_r = 0.0, sq_g = 0.0, sq_b = 0.0;
+    if (kMoments) { const double* a = P.acc2 + (size_t)p_local * 3u; sq_r = a[0]; sq_g = a[1]; sq_b = a[2]; }
 
 #pragma unroll 1
     for (int k = k_begin; k < k_end; ++k) {
@@ -128,10 +137,16 @@ __device__ __forceinline__ void render_primary_body(const KParams& P) {
         color = muls(add(N, mk(1.0, 1.0, 1.0)), 0.5);
       }
       sum_r = sum_r + color.x; sum_g = sum_g + color.y; sum_b = sum_b + color.z;  // raytracing.clj:153
+      if (kMoments) { sq_r = sq_r + color.x * color.x; sq_g = sq_g + color.y * color.y; sq_b = sq_b + color.z * color.z; }
       n_samples++;
+    }
+    if (kListed) {  // the unit again from the ticket: one load per unit instead of a register (a spill) over the loop
+      const unsigned q = (unsigned)ticket / (unsigned)P.nchunks;
+      unit = *(volatile const unsigned*)(P.list + q) * (unsigned)P.nchunks + ((unsigned)ticket - q * (unsigned)P.nchunks);
     }
     double* out = P.partial + (size_t)unit * 3u;
     out[0] = sum_r; out[1] = sum_g; out[2] = sum_b;
+    if (kMoments) { double* a = P.acc2 + (size_t)p_local * 3u; a[0] = sq_r; a[1] = sq_g; a[2] = sq_b; }
   }
 
   // ---- counters: samples = segments; every sphere is tested for every segment
@@ -154,6 +169,16 @@ __global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_prima
 template <bool kDefocus>
 __global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_primary_seeded_kernel(const __grid_constant__ KParams P) {
   render_primary_body<kDefocus, true>(P);
+}
+
+template <bool kDefocus>
+__global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_primary_listed_kernel(const __grid_constant__ KParams P) {
+  render_primary_body<kDefocus, false, true>(P);
+}
+
+template <bool kDefocus>
+__global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_primary_seeded_listed_kernel(const __grid_constant__ KParams P) {
+  render_primary_body<kDefocus, true, true>(P);
 }
 
 }  // namespace rtclj

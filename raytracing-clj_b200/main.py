@@ -4,6 +4,9 @@
     python -m raytracing_clj_b200.main main [spp] [depth]     -> scene.ppm
     python -m raytracing_clj_b200.main main [spp] [depth] --every N
                                                               -> scene.ppm, rewritten every N samples
+    python -m raytracing_clj_b200.main main [spp] [depth] --every N --tolerance ABS,REL
+                                                              -> the same with adaptive sampling, and
+                                                                 scene-samples.png (samples per pixel)
     python -m raytracing_clj_b200.main realm                  -> scene-realm.ppm
     python -m raytracing_clj_b200.main i                      -> scene-i.ppm
 
@@ -12,12 +15,19 @@ the P3 file the reference writes.  `(time ...)` is mirrored by printing the elap
 
 With --every N the image is rendered in passes of N samples (rounded up to the render's pass unit) and
 scene.ppm / scene.png are replaced after each pass, so that an open viewer shows the image refine; the
-last files are byte for byte those of a run without --every."""
+last files are byte for byte those of a run without --every.
+
+With --tolerance ABS,REL the passes trace only the pixels whose noise estimate is still above
+ABS + REL * |pixel mean| (adaptive sampling, DESIGN.md section 4.10; every pixel gets at least two pass
+units), and the run ends once no pixel is left.  scene-samples.png shows the samples each pixel received
+(white: spp)."""
 from __future__ import annotations
 
 import os
 import sys
 import time
+
+import numpy as np
 
 from . import _abi, camera, render, scenes
 
@@ -30,22 +40,42 @@ def _replace(path: str, data: bytes) -> None:
     os.replace(tmp, path)
 
 
-def main_variant(spp: int = 100, depth: int = 50, out: str = "scene.ppm", seed: int = 1, every: int = 0):
+def samples_image(samples: np.ndarray, spp: int) -> np.ndarray:
+    """The sample-count map as a grey 8-bit image: black 0, white spp samples per pixel."""
+    v = np.rint(samples.astype(np.float64) * (255.0 / spp)).clip(0, 255).astype(np.uint8)
+    return np.repeat(v[:, :, None], 3, axis=2)
+
+
+def main_variant(spp: int = 100, depth: int = 50, out: str = "scene.ppm", seed: int = 1, every: int = 0,
+                 tolerance=None):
     print("config:", {"samples-per-px": spp, "max-depth": depth})
     t0 = time.perf_counter()
+    if tolerance is not None and every <= 0:
+        every = max(1, spp // 10)
     if every > 0:
         png = out[:-4] + ".png" if out.endswith(".ppm") else out + ".png"
-        with render.Progressive(scenes.main_hittables(), camera.main_camera(), spp, depth, seed=seed,
-                                flags=_abi.FLAGS_MAIN) as p:
+        cam = camera.main_camera()
+        with render.Progressive(scenes.main_hittables(), cam, spp, depth, seed=seed, flags=_abi.FLAGS_MAIN,
+                                tolerance=tolerance) as p:
             n = -(-every // p.pass_unit) * p.pass_unit
-            segments = 0
-            while p.samples_done < spp:
+            segments = traced = 0
+            active = cam.width * cam.height
+            while p.samples_done < spp and active > 0:
                 _, rgb8, st = p.step(min(n, spp - p.samples_done), want_linear=False)
                 segments += st["segments"]
-                if p.samples_done < spp:  # the last image goes out below, as without --every
+                traced += st["samples"]
+                if p.adaptive:
+                    samples, _, active = p.noise()
+                if p.samples_done < spp and active > 0:  # the last image goes out below, as without --every
                     _replace(out, render.encode_ppm(rgb8))
                     _replace(png, render.encode_png(rgb8))
-                print(f"{p.samples_done}/{spp} samples per pixel: {out} ({1e3 * (time.perf_counter() - t0):.0f} ms)")
+                left = f", {active} pixels active" if p.adaptive else ""
+                print(f"{p.samples_done}/{spp} samples per pixel{left}: {out} ({1e3 * (time.perf_counter() - t0):.0f} ms)")
+            if p.adaptive:
+                grey = out[:-4] + "-samples.png" if out.endswith(".ppm") else out + "-samples.png"
+                render.write_png(grey, samples_image(samples, spp))
+                full = spp * cam.width * cam.height
+                print(f"samples traced: {traced} of {full} ({100.0 * traced / full:.1f} %); sample counts in {grey}")
         st["segments"] = segments
     else:
         _, rgb8, st = render.render(scenes.main_hittables(), camera.main_camera(), spp, depth, seed=seed,
@@ -75,14 +105,24 @@ def i_variant(out: str = "scene-i.ppm", seed: int = 1):
 def _cli(argv):
     which = argv[0] if argv else "main"
     if which == "main":
-        every = 0
+        every, tolerance = 0, None
+        if "--tolerance" in argv:
+            i = argv.index("--tolerance")
+            try:
+                tolerance = tuple(float(x) for x in argv[i + 1].split(","))
+            except (IndexError, ValueError):
+                tolerance = ()
+            if len(tolerance) != 2 or min(tolerance) < 0:
+                raise SystemExit("--tolerance needs ABS,REL: two numbers >= 0")
+            argv = argv[:i] + argv[i + 2:]
         if "--every" in argv:
             i = argv.index("--every")
             if i + 1 >= len(argv) or int(argv[i + 1]) <= 0:
                 raise SystemExit("--every needs a positive number of samples")
             every = int(argv[i + 1])
             argv = argv[:i] + argv[i + 2:]
-        main_variant(int(argv[1]) if len(argv) > 1 else 100, int(argv[2]) if len(argv) > 2 else 50, every=every)
+        main_variant(int(argv[1]) if len(argv) > 1 else 100, int(argv[2]) if len(argv) > 2 else 50, every=every,
+                     tolerance=tolerance)
     elif which == "realm":
         realm_variant()
     elif which == "i":

@@ -7,6 +7,7 @@ Everything here calls librtclj_b200.so; nothing is computed in Python."""
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Iterable, List, Optional, Sequence
 
 import numpy as np
@@ -118,6 +119,28 @@ def render_ppm(world, cam: Camera, samples_per_px: int = 100, max_depth: int = 5
     return bytes(memoryview(store)[: n.value]), st.as_dict()
 
 
+def pass_unit(width: int, height: int, samples_per_px: int, max_depth: int, flags: int = _abi.FLAGS_MAIN,
+              samples_per_unit: int = 0) -> int:
+    """The pass unit an accumulation of these params reports (rtclj_ctx_accum_begin): 1 in strict order, else the
+    unit size of the one-shot render (the library's choice for samples_per_unit <= 0)."""
+    primary_only = max_depth == 1 or bool(flags & _abi.F_NORMAL_SHADING)
+    if samples_per_unit >= samples_per_px or (samples_per_unit <= 0 and primary_only):
+        return 1
+    if samples_per_unit > 0:
+        return samples_per_unit
+    nchunks = math.ceil((64.0 * 148.0 * 512.0 * 8.0) / (float(width) * float(height)))  # auto_samples_per_unit
+    nchunks = max(1, min(nchunks, max(1, samples_per_px // 8)))
+    return (samples_per_px + nchunks - 1) // nchunks
+
+
+def _adaptive_args(cam, samples_per_px, max_depth, flags, samples_per_unit, tolerance, min_samples):
+    """(double[2] tolerance, min_samples) of an adaptive accumulation; min_samples <= 0: two pass units."""
+    abs_tol, rel_tol = (float(x) for x in tolerance)
+    if min_samples <= 0:
+        min_samples = 2 * pass_unit(cam.width, cam.height, samples_per_px, max_depth, flags, samples_per_unit)
+    return (C.c_double * 2)(abs_tol, rel_tol), int(min_samples)
+
+
 class Context:
     """Device-resident rendering: scene uploaded once, output left in device memory
     (pointers come from the caller, e.g. torch tensors), launches enqueued on the caller's
@@ -151,18 +174,36 @@ class Context:
         return st.as_dict()
 
     def accum_begin(self, cam, samples_per_px: int, max_depth: int, *, seed: int = 1, flags: int = _abi.FLAGS_MAIN,
-                    samples_per_unit: int = 0, shard: Optional[tuple] = None, stream: int = 0) -> int:
+                    samples_per_unit: int = 0, shard: Optional[tuple] = None, stream: int = 0,
+                    tolerance: Optional[Sequence[float]] = None, min_samples: int = 0) -> int:
         """Begins an accumulation over passes (rtclj_ctx_accum_begin) towards `samples_per_px` samples and
-        returns its pass unit: every pass but the last must be a multiple of it."""
+        returns its pass unit: every pass but the last must be a multiple of it.  tolerance = (abs, rel): an
+        adaptive accumulation (rtclj_ctx_accum_begin_adaptive) whose passes trace only the pixels whose noise
+        estimate is still above abs + rel * |mean|, after at least min_samples samples (<= 0: two pass units)."""
         cm = _camera_struct(cam)
         prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit),
                           0, 0, 0, int(self.device), 0)
         if shard is not None:
             prm.shard_index, prm.shard_count, prm.shard_rows = (int(x) for x in shard)
         unit = C.c_int32()
-        _abi.check(_abi.lib().rtclj_ctx_accum_begin(self._h, C.byref(cm), C.byref(prm), C.byref(unit),
-                                                    C.c_void_p(stream or None)))
+        if tolerance is None:
+            _abi.check(_abi.lib().rtclj_ctx_accum_begin(self._h, C.byref(cm), C.byref(prm), C.byref(unit),
+                                                        C.c_void_p(stream or None)))
+        else:
+            tol, least = _adaptive_args(cm, int(samples_per_px), int(max_depth), int(flags), int(samples_per_unit),
+                                        tolerance, int(min_samples))
+            _abi.check(_abi.lib().rtclj_ctx_accum_begin_adaptive(self._h, C.byref(cm), C.byref(prm), tol, least,
+                                                                 C.byref(unit), C.c_void_p(stream or None)))
         return unit.value
+
+    def accum_noise(self, d_samples: int = 0, d_stderr: int = 0, stream: int = 0) -> int:
+        """After a step of an adaptive accumulation: writes this context's rows of the sample-count map (int32
+        [H,W]) and of the noise estimate (float64 [H,W,3]) to the device pointers (either may be 0), and returns
+        the number of pixels still active (synchronises `stream`)."""
+        active = C.c_uint64()
+        _abi.check(_abi.lib().rtclj_ctx_accum_noise(self._h, C.c_void_p(d_samples or None), C.c_void_p(d_stderr or None),
+                                                    C.byref(active), C.c_void_p(stream or None)))
+        return active.value
 
     def accum_step(self, samples: int, d_out_linear: int = 0, d_out_rgb8: int = 0, stream: int = 0) -> int:
         """Enqueues one pass of `samples` samples per pixel (rtclj_ctx_accum_step); the images at the device
@@ -214,19 +255,27 @@ class Progressive:
     """
 
     def __init__(self, world, cam, samples_per_px: int = 100, max_depth: int = 50, *, seed: int = 1,
-                 flags: int = _abi.FLAGS_MAIN, samples_per_unit: int = 0, devices: Optional[Sequence[int]] = None):
+                 flags: int = _abi.FLAGS_MAIN, samples_per_unit: int = 0, devices: Optional[Sequence[int]] = None,
+                 tolerance: Optional[Sequence[float]] = None, min_samples: int = 0):
         self._h = C.c_void_p()
         soa = _as_soa(world)
         sc, cm = _scene_struct(soa), _camera_struct(cam)
         self.height, self.width = cm.height, cm.width
         self.samples_per_px = int(samples_per_px)
+        self.adaptive = tolerance is not None
         prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit),
                           0, 0, 0, 0, 0)
         devs = list(devices) if devices else [0]
         arr = (C.c_int32 * len(devs))(*devs)
         unit = C.c_int32()
-        _abi.check(_abi.lib().rtclj_progressive_create(C.byref(sc), C.byref(cm), C.byref(prm), arr, len(devs),
-                                                       C.byref(unit), C.byref(self._h)))
+        if tolerance is None:
+            _abi.check(_abi.lib().rtclj_progressive_create(C.byref(sc), C.byref(cm), C.byref(prm), arr, len(devs),
+                                                           C.byref(unit), C.byref(self._h)))
+        else:  # adaptive sampling (rtclj_progressive_create_adaptive): see Context.accum_begin
+            tol, least = _adaptive_args(cm, int(samples_per_px), int(max_depth), int(flags), int(samples_per_unit),
+                                        tolerance, int(min_samples))
+            _abi.check(_abi.lib().rtclj_progressive_create_adaptive(C.byref(sc), C.byref(cm), C.byref(prm), tol, least,
+                                                                    arr, len(devs), C.byref(unit), C.byref(self._h)))
         self.pass_unit = unit.value
         self.samples_done = 0
 
@@ -247,6 +296,17 @@ class Progressive:
             out_rgb8.ctypes.data if out_rgb8 is not None else None, C.byref(done), C.byref(st)))
         self.samples_done = done.value
         return out_linear, out_rgb8, st.as_dict()
+
+    def noise(self):
+        """Adaptive renders: (samples int32 [H,W], the count each pixel has; stderr float64 [H,W,3], its noise
+        estimate; active, the pixels the next pass would trace) after the last step."""
+        if not self._h:
+            raise _abi.RtcljError(_abi.E_INVALID, "progressive render is closed")
+        samples = np.zeros((self.height, self.width), dtype=np.int32)
+        stderr = np.zeros((self.height, self.width, 3), dtype=np.float64)
+        active = C.c_uint64()
+        _abi.check(_abi.lib().rtclj_progressive_noise(self._h, samples.ctypes.data, stderr.ctypes.data, C.byref(active)))
+        return samples, stderr, active.value
 
     def close(self) -> None:
         if self._h:
