@@ -290,7 +290,9 @@ int rtclj_progressive_destroy(rtclj_progressive *p); /* NULL is fine */
  *     channel S1 = the running sum and S2 = the sum of the squared unit sums in unit order; m = ceil(n_p / u)
  *     -- the short last chunk at the target counts as a unit like the others.  stderr = sqrt(fmax(((S2 -
  *     S1*S1/m) / (m (m - 1))) / (u u), 0)).  The pixel stays active iff n_p < spp and (n_p < min_samples or
- *     stderr > abs + rel * |mean| in some channel, mean = its linear value).
+ *     stderr > abs + rel * |mean| in some channel, mean = its linear value, or S1*S1 or S2 is not finite in
+ *     some channel: moments that overflowed make the variance inf - inf, which the clamp would read as 0, so
+ *     such a pixel counts as noisy).  The exported noise estimate is the clamped value.
  *   - A pixel's decision depends on its own sums only: for one sequence of pass sizes, images, sample-count
  *     map and noise are the same on every device list, shard_rows and kernel.  A different sequence of pass
  *     sizes may stop pixels at other counts.

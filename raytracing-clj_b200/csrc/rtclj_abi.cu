@@ -504,12 +504,7 @@ AParams adaptive_params(const rtclj_ctx* c, const Shard& sh) {
 
 // rebuilds the list of live pixels and its count on the device (rtclj_adaptive.cuh)
 int relist(rtclj_ctx* c, unsigned long long local_pixels, cudaStream_t stream) {
-  if (local_pixels == 0) return RTCLJ_OK;
-  const unsigned tiles = (unsigned)((local_pixels + kListTile - 1) / kListTile);
-  list_count_kernel<<<tiles, kListThreads, 0, stream>>>(c->live.p, local_pixels, c->list_aux.p + 1);
-  list_scan_kernel<<<1, 1024, 0, stream>>>(c->list_aux.p + 1, tiles, c->list_aux.p);
-  list_scatter_kernel<<<tiles, kListThreads, 0, stream>>>(c->live.p, local_pixels, c->list_aux.p + 1, c->list.p);
-  CU(cudaGetLastError());
+  CU(launch_relist(c->live.p, local_pixels, c->list_aux.p, c->list.p, stream));
   return RTCLJ_OK;
 }
 

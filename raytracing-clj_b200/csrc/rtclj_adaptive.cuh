@@ -23,6 +23,13 @@ __device__ __forceinline__ double unit_stderr(double s1, double s2, int n, int u
   return sqrt(v);
 }
 
+// Moments that overflowed: S1^2 or S2 is not finite, so the variance above is inf - inf = NaN or -inf, which the
+// clamp would turn into 0.  The stopping rule counts such a channel as noisy instead (a bright pixel is not a
+// converged one).  With finite moments both terms are finite and >= 0, so the variance is finite for m >= 2.
+__device__ __forceinline__ bool moments_overflow(double s1, double s2) {
+  return !(isfinite(s1 * s1) && isfinite(s2));
+}
+
 struct AParams {
   const double* sample_buf;      // strict order: per-sample colours [k][local pixel][4], or nullptr
   unsigned long long sample_stride;
@@ -107,7 +114,7 @@ __global__ void finalize_adaptive_kernel(const AParams A) {
     bool noisy = n < A.min_samples;
     for (int c = 0; c < 3; ++c) {
       const double t = A.abs_tol + A.rel_tol * fabs(mean[c]);
-      noisy = noisy || unit_stderr(s1[c], s2[c], n, A.unit) > t;
+      noisy = noisy || moments_overflow(s1[c], s2[c]) || unit_stderr(s1[c], s2[c], n, A.unit) > t;
     }
     A.live[p] = (n < A.target && noisy) ? 1 : 0;
   }
@@ -183,6 +190,18 @@ __global__ void __launch_bounds__(kListThreads) list_scatter_kernel(const unsign
     const unsigned long long s = s0 + (unsigned long long)e;
     if (s < n && live[n - 1 - s]) list[o++] = (unsigned)(n - 1 - s);
   }
+}
+
+// The compaction of n pixels' live flags: list[0, aux[0]) gets the live pixels in descending order, aux[0] their
+// count; aux[1, 1 + tiles) is the scan's scratch.  Asynchronous on `stream`; n == 0 launches nothing.
+inline cudaError_t launch_relist(const unsigned char* live, unsigned long long n, unsigned* aux, unsigned* list,
+                                 cudaStream_t stream) {
+  if (n == 0) return cudaSuccess;
+  const unsigned tiles = (unsigned)((n + kListTile - 1) / kListTile);
+  list_count_kernel<<<tiles, kListThreads, 0, stream>>>(live, n, aux + 1);
+  list_scan_kernel<<<1, 1024, 0, stream>>>(aux + 1, tiles, aux);
+  list_scatter_kernel<<<tiles, kListThreads, 0, stream>>>(live, n, aux + 1, list);
+  return cudaGetLastError();
 }
 
 }  // namespace rtclj

@@ -173,3 +173,15 @@ def test_primary_listed_kernels_keep_off_shared_and_local_memory(sass, key):
     assert re.search(r"\bLDG\b", text) and re.search(r"\bDFMA\b", text), key
     # one unit sum (three doubles); the seeded variant also stores the sums of squares
     assert len(re.findall(r"\bSTG\b", text)) == (6 if "seeded" in key else 3), key
+
+
+def test_kernel_harness_compiles_against_the_header(tmp_path):
+    """tests/native/adaptive_kernels.cu includes rtclj_adaptive.cuh as it is: a header change that breaks the
+    kernel tests shows here, without a GPU.  Its mirror of AParams matches the compiler's layout."""
+    sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+    import adaptive_kernels as K
+    if K.nvcc() is None:
+        pytest.skip("nvcc not installed")
+    so = C.CDLL(K.build(str(tmp_path)))
+    K.check_layout(so)
+    assert so.ak_list_tile() == 2048

@@ -156,8 +156,10 @@ def replay(colors, passes, unit, target, least, tol, strict, mean_divide):
             se = np.sqrt(v)
         num = (0.0 + s1) if strict else s1
         mean = num / n[:, None] if mean_divide else num * (1.0 / n[:, None])
-        t = tol[0] + tol[1] * np.abs(mean)
-        keep = (n < target) & ((n < least) | (se > t).any(axis=1))
+        with np.errstate(over="ignore", invalid="ignore"):
+            t = tol[0] + tol[1] * np.abs(mean)
+            overflow = ~(np.isfinite(s1 * s1) & np.isfinite(s2))  # moments that overflowed count as noisy
+        keep = (n < target) & ((n < least) | (se > t).any(axis=1) | overflow.any(axis=1))
         live[idx] = keep[idx]
         out.append((n.copy(), se.copy(), mean.copy()))
     return out
