@@ -119,7 +119,11 @@ typedef struct rtclj_scene {
 } rtclj_scene;
 
 /* The vectors the reference derives before its loop (raytracing.clj:126-139;
- * realm/raytracing.clj:306-322).  Row 0 is the top of the image. */
+ * realm/raytracing.clj:306-322).  Row 0 is the top of the image.
+ * Every value must be finite; only `center` and the defocus vectors are range-limited
+ * (|center| + |defocus_u| + |defocus_v| < 1e18 per axis).  The directions pixel00 + du*x + dv*y - origin
+ * are not: d = 0 or |d|^2 beyond the fp64 range give NaN roots, which are handled as the reference
+ * handles them (DESIGN.md 4.1). */
 typedef struct rtclj_camera {
   double pixel00[3];    /* pixel-00-loc   */
   double pixel_du[3];   /* pixel-du       */

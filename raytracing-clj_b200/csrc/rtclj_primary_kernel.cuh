@@ -94,7 +94,8 @@ __device__ __forceinline__ void render_primary_body(const KParams& P) {
       const d3 D = sub(ps, O);
 
       // ---- closest hit over every sphere in list order (hit-anything, raytracing.clj:33-43;
-      // raytracing_i.clj:48-57): the operations of exact_test_lex, geometry from the parameters
+      // raytracing_i.clj:48-57): the operations of exact_test_lex, geometry from the parameters, with the
+      // reference's acceptance of a NaN root (scan_all_ni)
       const double a = lensq(D);
       const double ya = recip_refined(a);
       const bool a_ok = recip_safe(a);
@@ -120,7 +121,9 @@ __device__ __forceinline__ void render_primary_body(const KParams& P) {
           root = div_by(h + sq, a, ya, a_ok);
           if (root <= 1e-3) continue;
         }
-        if (root < closest) { closest = root; best = i; }  // list order: on an exact tie the earlier sphere stays
+        // list order: on an exact tie the earlier sphere stays.  `!(closest <= root)`, not `root < closest`: the
+        // reference accepts a NaN root (|d|^2 = 0 or inf), and once closest is NaN every later sphere wins
+        if (!(closest <= root)) { closest = root; best = i; }
       }
 
       // ---- colour of the sample

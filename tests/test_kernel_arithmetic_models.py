@@ -255,6 +255,132 @@ def test_list_scan_with_strict_bounds_equals_the_lexicographic_minimum():
         assert (closest, best) == (c2, b2), (near, far, miss)
 
 
+def reference_pick(roots, tmin=1e-3):
+    """hit-anything's sequential scan (hittable.clj:15-21, rt_oracle.c sphere_root), which scan_all_ni restates: near
+    root, then far root, accepted when !(root <= t_min || closest <= root) -- true for a NaN root."""
+    closest, best = np.inf, -1
+    for i, r in enumerate(roots):
+        if r is None:
+            continue
+        for root in r:
+            if not (root <= tmin or closest <= root):
+                closest, best = root, i
+                break
+    return closest, best
+
+
+def lex_pick(roots, tmin=1e-3):
+    """exact_test_lex in any order (here: reversed): the near root unless it is <= t_min, then the far root unless it
+    is <= t_min; lexicographic minimum of (root_i, i), which a NaN root never is."""
+    closest, best = np.inf, -1
+    for i in reversed(range(len(roots))):
+        if roots[i] is None:
+            continue
+        root = roots[i][0]
+        if root <= tmin:
+            root = roots[i][1]
+            if root <= tmin:
+                continue
+        if root < closest or (root == closest and i < best):
+            closest, best = root, i
+    return closest, best
+
+
+def primary_pick(roots, tmin=1e-3):
+    """render_primary_kernel: exact_test_lex's choice of root, in list order, accepted when !(closest <= root)."""
+    closest, best = np.inf, -1
+    for i, r in enumerate(roots):
+        if r is None:
+            continue
+        root = r[0]
+        if root <= tmin:
+            root = r[1]
+            if root <= tmin:
+                continue
+        if not (closest <= root):
+            closest, best = root, i
+    return closest, best
+
+
+def test_scan_rules_on_nan_roots():
+    """Root pairs (h -+ sq) / a from operands drawn with NaN, +-inf, zero and exact ties at t_min = 1e-3 (a degenerate
+    direction: |d|^2 = a is 0 or inf).  reference_pick is the rule of the oracle and of the exhaustive scans
+    (exact_test_div restates it operation for operation), so the checks here are of the two rules that differ from it
+    in form: the lexicographic form of the cull path never accepts a NaN root, so it differs from the reference
+    exactly on sets with one; the primary kernel's rule (lexicographic choice of root, then `!(closest <= root)`)
+    equals the reference on every set.  The kernels' scans themselves are compared with the oracle on the GPU
+    (tests/test_gpu_degenerate_rays.py)."""
+    rng = np.random.default_rng(17)
+    hs = np.array([-np.inf, -1e300, -2.0, -0.0, 0.0, 5e-4, 1e-3, 2e-3, 1.0, 3.0, 1e300, np.inf, np.nan])
+    sqs = np.array([0.0, 1e-3, 1.0, 2.0, 1e300, np.inf, np.nan])
+    As = np.array([0.0, 1.0, 1.0, 2.0, 1e-300, 1e300, np.inf])
+    differ = with_nan = 0
+    for _ in range(20_000):
+        n = int(rng.integers(1, 6))
+        roots = []
+        for _ in range(n):
+            if rng.random() < 0.2:
+                roots.append(None)                           # negative discriminant
+                continue
+            h, sq, a = rng.choice(hs), rng.choice(sqs), rng.choice(As)
+            with np.errstate(all="ignore"):
+                roots.append((np.float64(h - sq) / a, np.float64(h + sq) / a))
+        want = reference_pick(roots)
+        got = primary_pick(roots)
+        assert got[1] == want[1] and (got[0] == want[0] or (got[0] != got[0] and want[0] != want[0])), roots
+        nan = any(r is not None and (r[0] != r[0] or r[1] != r[1]) for r in roots)
+        lex = lex_pick(roots)
+        same = lex[1] == want[1] and (lex[0] == want[0] or (lex[0] != lex[0] and want[0] != want[0]))
+        if not nan:
+            assert same, roots                               # without a NaN root the cull path's rule is exact
+        with_nan += nan
+        differ += not same
+    assert with_nan > 2000 and differ > 500, (with_nan, differ)
+
+
+def test_cull_path_never_sees_a_nan_root():
+    """Why the cull path may keep exact_test_lex: none of its roots is NaN.  The argument is the chain of bounds below,
+    each taken at its worst case from the input limits; the random rays after it only spot-check the arithmetic.
+
+    * The cull path runs only when fp32 |d|^2 lies in (1e-30, 1e30) (make_view).  fp32 rounds each component and
+      the sum by at most 2^-24 relative, so the fp64 |d|^2 = a is below 1e30 (1 + 2^-20); and some fp32 component is
+      at least sqrt(1e-30 / 3.1) > 5e-16, a normal fp32 value, so a > 2.5e-31 > 0: no 0 / 0, no x / inf.
+    * Scene coordinates and radii are below 1e18 (rtclj_ctx_set_scene); a ray starts at the camera (|center| plus the
+      defocus vectors below 1e18 per axis, validate()) or at a hit point on a sphere, below 2e18 per axis up to
+      rounding.  So each component of oc = C - O is below 3e18 (with slack: 3.1e18), |oc| below sqrt(3) 3.1e18.
+    * Then |h| <= |d| |oc|, c <= |oc|^2 + r^2, |disc| <= h^2 + a |c|: all finite, far below 1e70, so sqrt(disc),
+      h -+ sq and (h -+ sq) / a are finite numbers (or disc < 0: no root)."""
+    slack = 1.01
+    a_max, a_min = 1e30 * (1.0 + 2.0 ** -20), (1e-30 / 3.1)
+    assert np.float32(np.sqrt(a_min)) > np.finfo(np.float32).tiny                    # a normal fp32 component
+    oc_max = np.sqrt(3.0) * 3.1e18 * slack
+    h_max = np.sqrt(a_max) * oc_max * slack
+    c_max = (oc_max ** 2 + 1e18 ** 2) * slack
+    disc_max = (h_max ** 2 + a_max * c_max) * slack
+    root_max = (h_max + np.sqrt(disc_max)) / (a_min / slack)
+    assert disc_max < 1e70 and np.isfinite(root_max), (disc_max, root_max)
+    # spot check at the extremes, random directions: every intermediate finite, no NaN root
+    rng = np.random.default_rng(23)
+    for _ in range(2000):
+        u = rng.normal(size=3)
+        D = u / np.linalg.norm(u) * rng.choice([1.1e-15, 9e14])
+        O = rng.choice([-1.0, 1.0], 3) * rng.choice([0.0, 1.99e18], 3)
+        C = rng.choice([-1.0, 1.0], 3) * rng.choice([0.0, 9.9e17], 3)
+        r = rng.choice([-9.9e17, 1.0, 9.9e17])
+        oc = C - O
+        a, h, c = float(D @ D), float(D @ oc), float(oc @ oc) - r * r
+        disc = h * h - a * c
+        assert np.isfinite(h * h) and np.isfinite(a * c) and np.isfinite(disc) and abs(disc) < disc_max
+        if disc >= 0.0:
+            assert np.isfinite((h - np.sqrt(disc)) / a) and np.isfinite((h + np.sqrt(disc)) / a)
+    # and the fp32 test that routes a ray to the exhaustive scan brackets exactly that range of |d|
+    for d, degenerate in ((1e-16, True), (1.2e-15, False), (8e14, False), (1e16, True), (0.0, True), (np.inf, True)):
+        f = np.float32(d)
+        with np.errstate(over="ignore", invalid="ignore"):
+            l2 = f * f
+        assert (not (l2 > np.float32(1e-30) and l2 < np.float32(1e30))) == degenerate, d
+
+
 def test_tickets_visit_every_unit_once_from_the_last_pixel_to_the_first():
     """rtclj_kernels.cuh unit_of_ticket(): ticket -> (local pixel, chunk) with a pixel's chunks on consecutive tickets
     and the pixels handed out from the shard's last to its first (the top rows -- sky -- last, DESIGN.md section 6);
