@@ -181,6 +181,40 @@ int validate(const rtclj_camera* cam, const rtclj_params* prm) {
   return RTCLJ_OK;
 }
 
+// Every instantiation of the render kernels, indexed by its template flags: launch_pass launches from these tables
+// and rtclj_ctx_create raises the dynamic shared memory limit of every entry that takes some (kSmemLimits).
+using KernelFn = void (*)(KParams);
+// render_kernel and render_listed_kernel, [listed][const_tab][sample_buf][packed]: threads_of(const_tab, packed)
+// threads, smem_needed() bytes.  The packed instantiation exists with the constant table only.
+const KernelFn kRenderFns[2][2][2][2] = {
+    {{{render_kernel<false, false, false>, nullptr}, {render_kernel<false, true, false>, nullptr}},
+     {{render_kernel<true, false, false>, render_kernel<true, false, true>},
+      {render_kernel<true, true, false>, render_kernel<true, true, true>}}},
+    {{{render_listed_kernel<false, false, false>, nullptr}, {render_listed_kernel<false, true, false>, nullptr}},
+     {{render_listed_kernel<true, false, false>, render_listed_kernel<true, false, true>},
+      {render_listed_kernel<true, true, false>, render_listed_kernel<true, true, true>}}}};
+// render_lane2_kernel and render_lane2_listed_kernel, [listed][sample_buf]: kT2 threads, Lane2Smem::total bytes
+const KernelFn kLane2Fns[2][2] = {{render_lane2_kernel<false>, render_lane2_kernel<true>},
+                                  {render_lane2_listed_kernel<false>, render_lane2_listed_kernel<true>}};
+// render_split_kernel, [sample_buf]: kSplitThreads threads, SplitSmem::total bytes
+const KernelFn kSplitFns[2] = {render_split_kernel<false>, render_split_kernel<true>};
+// render_wave_kernel: kWT threads, WaveSmem::total bytes
+const KernelFn kWaveFns[1] = {render_wave_kernel};
+// the primary-ray kernels, [listed][seeded][defocus]: kPrimaryThreads threads, no dynamic shared memory
+const KernelFn kPrimaryFns[2][2][2] = {
+    {{render_primary_kernel<false>, render_primary_kernel<true>},
+     {render_primary_seeded_kernel<false>, render_primary_seeded_kernel<true>}},
+    {{render_primary_listed_kernel<false>, render_primary_listed_kernel<true>},
+     {render_primary_seeded_listed_kernel<false>, render_primary_seeded_listed_kernel<true>}}};
+
+// the tables of kernels with dynamic shared memory, and the most a launch asks for (0: the device's opt-in limit)
+struct SmemLimit { const KernelFn* fns; size_t count; size_t bytes; };
+const SmemLimit kSmemLimits[] = {
+    {&kRenderFns[0][0][0][0], sizeof kRenderFns / sizeof(KernelFn), 0},
+    {&kLane2Fns[0][0], sizeof kLane2Fns / sizeof(KernelFn), Lane2Smem::total},
+    {kSplitFns, sizeof kSplitFns / sizeof(KernelFn), SplitSmem::total},
+    {kWaveFns, sizeof kWaveFns / sizeof(KernelFn), WaveSmem::total}};
+
 }  // namespace
 
 // ---- arithmetic-peak calibration (pure FMA loops, 8 independent chains per thread)
@@ -265,25 +299,10 @@ int rtclj_ctx_create(int32_t device, rtclj_ctx** out) {
   CU(cudaEventCreateWithFlags(&c->pin_ev[1], cudaEventDisableTiming));
   CU(cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking));
   CU(c->counters.reserve(8));
-  CU(cudaFuncSetAttribute(render_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
-  CU(cudaFuncSetAttribute(render_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
-  CU(cudaFuncSetAttribute(render_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
-  CU(cudaFuncSetAttribute(render_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
-  CU(cudaFuncSetAttribute(render_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
-  CU(cudaFuncSetAttribute(render_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
-  CU(cudaFuncSetAttribute(render_wave_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WaveSmem::total));
-  CU(cudaFuncSetAttribute(render_lane2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Lane2Smem::total));
-  CU(cudaFuncSetAttribute(render_lane2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Lane2Smem::total));
-  CU(cudaFuncSetAttribute(render_split_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SplitSmem::total));
-  CU(cudaFuncSetAttribute(render_split_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SplitSmem::total));
-  CU(cudaFuncSetAttribute(render_listed_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
-  CU(cudaFuncSetAttribute(render_listed_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
-  CU(cudaFuncSetAttribute(render_listed_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
-  CU(cudaFuncSetAttribute(render_listed_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
-  CU(cudaFuncSetAttribute(render_listed_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
-  CU(cudaFuncSetAttribute(render_listed_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_optin));
-  CU(cudaFuncSetAttribute(render_lane2_listed_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Lane2Smem::total));
-  CU(cudaFuncSetAttribute(render_lane2_listed_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Lane2Smem::total));
+  for (const SmemLimit& t : kSmemLimits)
+    for (size_t i = 0; i < t.count; ++i)
+      if (t.fns[i])
+        CU(cudaFuncSetAttribute(t.fns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(t.bytes ? t.bytes : c->smem_optin)));
   *out = guard.release();
   return RTCLJ_OK;
 }
@@ -417,18 +436,24 @@ namespace {
 // Scenes of <= 512 spheres: four kernels produce the same image (tests); the default is the fastest measured on
 // the bench workload (DESIGN.md section 7), the flags select the others for A/B timing
 enum { SMALL_LANE1, SMALL_LANE2, SMALL_WAVE, SMALL_SPLIT };
+// the kernel a launch runs: none (max_depth <= 0, black), render_kernel with the table in shared memory or as a
+// kernel parameter, and the other constant-table kernels
+enum class Kernel { none, render_smem, render_const, lane2, wave, split, primary };
 struct KernelChoice {
-  bool run_kernel, const_tab, primary_only;
-  int small;
-  bool wave, lane2, split;  // constant-table kernels other than render_kernel<true>
-  bool primary;             // render_primary_kernel
+  Kernel kernel;
+  bool primary_only;   // max_depth 1 or normal shading
+  bool no_cull;        // the library adds RTCLJ_F_NO_CULL: the exhaustive fp64 scan
+  bool packed;         // render_kernel's instantiation for scenes of fewer than 64 spheres
+  bool finishes;       // the kernel writes the pixels itself, without finalize_kernel (wave)
+  bool sample_buf_ok;  // the kernel can store every sample's colour (sample_buf)
 };
+
+bool primary_only(const rtclj_params* prm) { return prm->max_depth == 1 || (prm->flags & RTCLJ_F_NORMAL_SHADING); }
 
 // the kernel of a launch that traces `total_samples` samples of this shard
 KernelChoice choose_kernel(const rtclj_ctx* c, const rtclj_params* prm, double total_samples) {
   KernelChoice k;
-  k.run_kernel = prm->max_depth > 0;
-  k.const_tab = use_const_table(c->nhalf) && !(prm->flags & RTCLJ_F_SMEM_TABLE);
+  const bool const_tab = use_const_table(c->nhalf) && !(prm->flags & RTCLJ_F_SMEM_TABLE);
   // Two paths per lane pay when the cull dominates (many spheres) and the render is long enough to hide
   // the longer tail of twice as many work units in flight: measured on a B200 (profiles/r2_kernel_ab.md),
   // cover scene 1920x1080: 500 spp 543.7 vs 561.6 ms, one eighth of it (an 8-GPU shard, 1.3e8 samples) 70.85 vs
@@ -443,15 +468,28 @@ KernelChoice choose_kernel(const rtclj_ctx* c, const rtclj_params* prm, double t
   if (prm->flags & RTCLJ_F_LANE2_KERNEL) small = SMALL_LANE2;
   if (prm->flags & RTCLJ_F_WAVE_KERNEL) small = SMALL_WAVE;
   if (prm->flags & RTCLJ_F_SPLIT_KERNEL) small = SMALL_SPLIT;
-  k.small = small;
-  k.wave = k.run_kernel && k.const_tab && small == SMALL_WAVE;    // also finishes the pixels itself
-  k.lane2 = k.run_kernel && k.const_tab && small == SMALL_LANE2;
-  k.split = k.run_kernel && k.const_tab && small == SMALL_SPLIT;
-  k.primary_only = prm->max_depth == 1 || (prm->flags & RTCLJ_F_NORMAL_SHADING);
+  const bool lane1 = const_tab && small == SMALL_LANE1;  // one path per lane: the primary kernel or render_kernel<true>
+  k.primary_only = primary_only(prm);
+  if (prm->max_depth <= 0) k.kernel = Kernel::none;
+  else if (!const_tab) k.kernel = Kernel::render_smem;
+  else if (small == SMALL_LANE2) k.kernel = Kernel::lane2;
+  else if (small == SMALL_WAVE) k.kernel = Kernel::wave;
+  else if (small == SMALL_SPLIT) k.kernel = Kernel::split;
   // primary rays only and a handful of spheres (config 4): a kernel without the path machinery, 1.6x faster
   // (rtclj_primary_kernel.cuh); RTCLJ_F_LANE_KERNEL / RTCLJ_F_NO_CULL keep render_kernel for A/B and tests
-  k.primary = k.run_kernel && k.const_tab && small == SMALL_LANE1 && k.primary_only && c->n <= kPrimarySpheres &&
-              !(prm->flags & (RTCLJ_F_LANE_KERNEL | RTCLJ_F_NO_CULL));
+  else if (lane1 && k.primary_only && c->n <= kPrimarySpheres && !(prm->flags & (RTCLJ_F_LANE_KERNEL | RTCLJ_F_NO_CULL)))
+    k.kernel = Kernel::primary;
+  else k.kernel = Kernel::render_const;
+  // A handful of spheres: the exhaustive fp64 scan (the same lexicographic minimum, tests) beats cull +
+  // prefilter.  Measured at 1920x1080 x 16 spp on prefixes of the default scene: path tracing 1 / 2 / 3 / 4
+  // spheres 2.24 / 4.86 / 7.08 / 9.43 ms against 2.78 / 5.24 / 7.12 / 9.31 with the cull; primary rays only
+  // 2 / 5 / 6 / 8 spheres 0.96 / 1.16 / 1.20 / 1.30 ms against 1.19 / 1.26 / 1.25 / 1.26.
+  k.no_cull = lane1 && (c->n <= 2 || (k.primary_only && c->n <= kPrimarySpheres));
+  // scenes of fewer than 64 spheres: their own instantiation (packed prefilter candidates, 768 threads), measured
+  // per regime -- rtclj_kernels.cuh, render_kernel / threads_of
+  k.packed = RTCLJ_PACKED_CANDS && k.kernel == Kernel::render_const && c->n < 64;
+  k.finishes = k.kernel == Kernel::wave;
+  k.sample_buf_ok = k.kernel != Kernel::none && k.kernel != Kernel::wave;
   return k;
 }
 
@@ -481,13 +519,6 @@ struct Pass {
   double* out_linear = nullptr;
   unsigned char* out_rgb8 = nullptr;
 };
-
-// render_kernel, or its listed twin (the pixels of KParams::list only)
-template <bool kConstTab, bool kSampleBuf, bool kPacked>
-void launch_render_kernel(bool listed, int grid, size_t sm, cudaStream_t stream, const KParams& P) {
-  if (listed) render_listed_kernel<kConstTab, kSampleBuf, kPacked><<<grid, threads_of(kConstTab, kPacked), sm, stream>>>(P);
-  else render_kernel<kConstTab, kSampleBuf, kPacked><<<grid, threads_of(kConstTab, kPacked), sm, stream>>>(P);
-}
 
 // the fold and stopping rule of an adaptive accumulation's pass, shard `sh` (finalize_adaptive_kernel)
 AParams adaptive_params(const rtclj_ctx* c, const Shard& sh) {
@@ -521,9 +552,9 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
   CU(cudaMemsetAsync(c->counters.p, 0, (ps.first ? 8 : 1) * sizeof(unsigned long long), stream));
   if (total_units == 0) return RTCLJ_OK;
 
-  if ((!ch.wave || nchunks > 1) && !ps.sample_buf) CU(c->partial.reserve((size_t)total_units * 3));
+  if ((!ch.finishes || nchunks > 1) && !ps.sample_buf) CU(c->partial.reserve((size_t)total_units * 3));
   if (ps.first) CU(cudaEventRecord(c->ev0, stream));
-  if (!ch.run_kernel) {
+  if (ch.kernel == Kernel::none) {
     CU(cudaMemsetAsync(c->partial.p, 0, (size_t)total_units * 3 * sizeof(double), stream));  // depth <= 0: black
   } else {
     KParams& P = c->kparams;  // 8.4 KB with the table: kept in the context, not on the stack of a JVM thread
@@ -537,11 +568,7 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
     P.W = cam->width; P.H = cam->height; P.spp = ps.sample_base + ps.samples; P.max_depth = prm->max_depth;
     P.flags = prm->flags; P.k0 = (unsigned)prm->seed; P.k1 = (unsigned)(prm->seed >> 32);
     for (unsigned r = 0; r < 10; ++r) { P.rk[2 * r] = P.k0 + r * 0x9E3779B9u; P.rk[2 * r + 1] = P.k1 + r * 0xBB67AE85u; }
-    // A handful of spheres: the exhaustive fp64 scan (the same lexicographic minimum, tests) beats cull +
-    // prefilter.  Measured at 1920x1080 x 16 spp on prefixes of the default scene: path tracing 1 / 2 / 3 / 4
-    // spheres 2.24 / 4.86 / 7.08 / 9.43 ms against 2.78 / 5.24 / 7.12 / 9.31 with the cull; primary rays only
-    // 2 / 5 / 6 / 8 spheres 0.96 / 1.16 / 1.20 / 1.30 ms against 1.19 / 1.26 / 1.25 / 1.26.
-    if (ch.const_tab && ch.small == SMALL_LANE1 && (c->n <= 2 || (ch.primary_only && c->n <= kPrimarySpheres))) P.flags |= RTCLJ_F_NO_CULL;
+    if (ch.no_cull) P.flags |= RTCLJ_F_NO_CULL;
     P.n = c->n; P.nblocks = c->nhalf / 2; P.tail8 = c->nhalf & 1;
     P.nconst = (c->n + 2 * kCBP - 1) / (2 * kCBP);
     P.smem_blocks = smem_table_blocks(c->smem_optin);
@@ -553,84 +580,64 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
     P.sample_buf = ps.sample_buf; P.sample_stride = sh.local_pixels;
     P.list = ps.listed ? c->list.p : nullptr; P.list_count = ps.listed ? c->list_aux.p : nullptr;
     P.acc2 = ps.listed ? c->acc2.p : nullptr;
-    if (ch.const_tab && !c->ctab_host.empty())
+    const bool const_tab = ch.kernel != Kernel::render_smem, sample_buf = ps.sample_buf != nullptr;
+    if (const_tab && !c->ctab_host.empty())
       std::memcpy(P.ctab, c->ctab_host.data(), std::min(sizeof P.ctab, c->ctab_host.size() * sizeof(float)));
-    if (ch.primary) {
-      std::memcpy(P.ctab, c->prim_geom, sizeof c->prim_geom);
-      const unsigned long long want = (total_units + kPrimaryThreads - 1) / kPrimaryThreads;
-      const unsigned blocks = (unsigned)std::min<unsigned long long>(want, (unsigned long long)grid * (unsigned long long)(2048 / kPrimaryThreads));
-      if (ps.listed && ps.seeded && P.use_defocus) render_primary_seeded_listed_kernel<true><<<blocks, kPrimaryThreads, 0, stream>>>(P);
-      else if (ps.listed && ps.seeded) render_primary_seeded_listed_kernel<false><<<blocks, kPrimaryThreads, 0, stream>>>(P);
-      else if (ps.listed && P.use_defocus) render_primary_listed_kernel<true><<<blocks, kPrimaryThreads, 0, stream>>>(P);
-      else if (ps.listed) render_primary_listed_kernel<false><<<blocks, kPrimaryThreads, 0, stream>>>(P);
-      else if (ps.seeded && P.use_defocus) render_primary_seeded_kernel<true><<<blocks, kPrimaryThreads, 0, stream>>>(P);
-      else if (ps.seeded) render_primary_seeded_kernel<false><<<blocks, kPrimaryThreads, 0, stream>>>(P);
-      else if (P.use_defocus) render_primary_kernel<true><<<blocks, kPrimaryThreads, 0, stream>>>(P);
-      else render_primary_kernel<false><<<blocks, kPrimaryThreads, 0, stream>>>(P);
-    } else if (ch.wave) {
-      P.stack_stride = (unsigned)grid * (unsigned)kWS;
-      if (prm->max_depth > 1) {  // the attenuating hits of a path, for either product order
-        CU(c->stack.reserve((size_t)prm->max_depth * P.stack_stride));
-        P.stack = c->stack.p;
+    KernelFn fn = nullptr;
+    unsigned blocks = (unsigned)grid, paths = 0;  // paths in flight per CTA: the rows of the attenuation stack
+    int threads = 0;
+    size_t sm = 0;
+    bool stack = prm->max_depth > 1;  // the attenuating hits of a path, for either product order
+    switch (ch.kernel) {
+      case Kernel::primary: {
+        std::memcpy(P.ctab, c->prim_geom, sizeof c->prim_geom);
+        const unsigned long long want = (total_units + kPrimaryThreads - 1) / kPrimaryThreads;
+        blocks = (unsigned)std::min<unsigned long long>(want, (unsigned long long)grid * (unsigned long long)(2048 / kPrimaryThreads));
+        fn = kPrimaryFns[ps.listed][ps.seeded][P.use_defocus]; threads = kPrimaryThreads; stack = false;
+        break;
       }
-      P.out_linear = ps.out_linear; P.out_rgb8 = ps.out_rgb8;
-      if (nchunks > 1 && (ps.out_linear || ps.out_rgb8)) {
-        CU(c->arrive.reserve((size_t)sh.local_pixels));
-        CU(cudaMemsetAsync(c->arrive.p, 0, (size_t)sh.local_pixels * sizeof(unsigned), stream));
-        P.arrive = c->arrive.p;
-      }
-      render_wave_kernel<<<grid, kWT, WaveSmem::total, stream>>>(P);
-    } else if (ch.split) {
-      P.stack_stride = (unsigned)grid * (unsigned)kSplitW * 2u;
-      if (prm->max_depth > 1) {
-        CU(c->stack.reserve((size_t)prm->max_depth * P.stack_stride));
-        P.stack = c->stack.p;
-      }
-      if (ps.sample_buf) render_split_kernel<true><<<grid, kSplitThreads, SplitSmem::total, stream>>>(P);
-      else render_split_kernel<false><<<grid, kSplitThreads, SplitSmem::total, stream>>>(P);
-    } else if (ch.lane2) {
-      P.stack_stride = (unsigned)grid * (unsigned)kT2 * 2u;
-      if (prm->max_depth > 1) {
-        CU(c->stack.reserve((size_t)prm->max_depth * P.stack_stride));
-        P.stack = c->stack.p;
-      }
+      case Kernel::wave:
+        fn = kWaveFns[0]; threads = kWT; sm = WaveSmem::total; paths = kWS;
+        P.out_linear = ps.out_linear; P.out_rgb8 = ps.out_rgb8;
+        if (nchunks > 1 && (ps.out_linear || ps.out_rgb8)) {
+          CU(c->arrive.reserve((size_t)sh.local_pixels));
+          CU(cudaMemsetAsync(c->arrive.p, 0, (size_t)sh.local_pixels * sizeof(unsigned), stream));
+          P.arrive = c->arrive.p;
+        }
+        break;
+      case Kernel::split:
+        fn = kSplitFns[sample_buf]; threads = kSplitThreads; sm = SplitSmem::total; paths = 2u * kSplitW;
+        break;
+      case Kernel::lane2:
+        fn = kLane2Fns[ps.listed][sample_buf]; threads = kT2; sm = Lane2Smem::total; paths = 2u * kT2;
+        break;
+      default:  // render_kernel
+        fn = kRenderFns[ps.listed][const_tab][sample_buf][ch.packed]; threads = threads_of(const_tab, ch.packed);
+        sm = smem_needed(c->nhalf, const_tab, c->smem_optin, ch.packed); paths = (unsigned)threads;
+        stack = prm->flags & RTCLJ_F_REVERSE_PRODUCT;
+    }
+    P.stack_stride = (unsigned)grid * paths;
+    if (stack) {
+      CU(c->stack.reserve((size_t)prm->max_depth * P.stack_stride));
+      P.stack = c->stack.p;
+    }
 #ifdef RTCLJ_TAIL_PROBE
-      const size_t probe_words = (size_t)grid * (kT2 / 32) * 4 * 2;
+    const size_t probe_words = (size_t)grid * (kT2 / 32) * 4 * 2;
+    if (ch.kernel == Kernel::lane2) {
       CU(c->arrive.reserve(probe_words));
       CU(cudaMemsetAsync(c->arrive.p, 0, probe_words * sizeof(unsigned), stream));
       P.arrive = c->arrive.p;
-#endif
-      if (ps.listed && ps.sample_buf) render_lane2_listed_kernel<true><<<grid, kT2, Lane2Smem::total, stream>>>(P);
-      else if (ps.listed) render_lane2_listed_kernel<false><<<grid, kT2, Lane2Smem::total, stream>>>(P);
-      else if (ps.sample_buf) render_lane2_kernel<true><<<grid, kT2, Lane2Smem::total, stream>>>(P);
-      else render_lane2_kernel<false><<<grid, kT2, Lane2Smem::total, stream>>>(P);
-#ifdef RTCLJ_TAIL_PROBE
-      if (const char* path = std::getenv("RTCLJ_TAIL_PROBE_FILE")) {
-        std::vector<unsigned> host(probe_words);
-        CU(cudaStreamSynchronize(stream));
-        CU(cudaMemcpy(host.data(), c->arrive.p, probe_words * sizeof(unsigned), cudaMemcpyDeviceToHost));
-        if (FILE* f = std::fopen(path, "wb")) { std::fwrite(host.data(), sizeof(unsigned), probe_words, f); std::fclose(f); }
-      }
-#endif
-    } else {
-      // scenes of fewer than 64 spheres: their own instantiation (packed prefilter candidates, 768 threads), measured
-      // per regime -- rtclj_kernels.cuh, render_kernel / threads_of
-      const bool const_tab = ch.const_tab, sample_buf = ps.sample_buf != nullptr;
-      const bool packed = RTCLJ_PACKED_CANDS && const_tab && c->n < 64;
-      P.stack_stride = (unsigned)grid * (unsigned)threads_of(const_tab, packed);
-      if (prm->flags & RTCLJ_F_REVERSE_PRODUCT) {
-        CU(c->stack.reserve((size_t)prm->max_depth * P.stack_stride));
-        P.stack = c->stack.p;
-      }
-      const size_t sm = smem_needed(c->nhalf, const_tab, c->smem_optin, packed);
-      const bool listed = ps.listed;
-      if (const_tab && sample_buf && packed) launch_render_kernel<true, true, true>(listed, grid, sm, stream, P);
-      else if (const_tab && packed) launch_render_kernel<true, false, true>(listed, grid, sm, stream, P);
-      else if (const_tab && sample_buf) launch_render_kernel<true, true, false>(listed, grid, sm, stream, P);
-      else if (const_tab) launch_render_kernel<true, false, false>(listed, grid, sm, stream, P);
-      else if (sample_buf) launch_render_kernel<false, true, false>(listed, grid, sm, stream, P);
-      else launch_render_kernel<false, false, false>(listed, grid, sm, stream, P);
     }
+#endif
+    fn<<<blocks, threads, sm, stream>>>(P);
+#ifdef RTCLJ_TAIL_PROBE
+    if (const char* path = std::getenv("RTCLJ_TAIL_PROBE_FILE"); path && ch.kernel == Kernel::lane2) {
+      std::vector<unsigned> host(probe_words);
+      CU(cudaStreamSynchronize(stream));
+      CU(cudaMemcpy(host.data(), c->arrive.p, probe_words * sizeof(unsigned), cudaMemcpyDeviceToHost));
+      if (FILE* f = std::fopen(path, "wb")) { std::fwrite(host.data(), sizeof(unsigned), probe_words, f); std::fclose(f); }
+    }
+#endif
     CU(cudaGetLastError());
   }
   CU(cudaEventRecord(c->ev1, stream));
@@ -692,7 +699,7 @@ int rtclj_ctx_render(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* 
   // traced in small units and each sample's colour is STORED (32 B); finalize_kernel then adds them in
   // sample order -- the same additions in the same order.  33 GB at 1920x1080 x 500 spp; HBM has 180 GB.
   double* sample_buf = nullptr;
-  if (spu == prm->spp && !ch.primary_only && prm->spp >= 64 && ch.run_kernel && !ch.wave && want_out && sh.local_pixels > 0) {
+  if (spu == prm->spp && !ch.primary_only && prm->spp >= 64 && ch.sample_buf_ok && want_out && sh.local_pixels > 0) {
     const size_t need = (size_t)sh.local_pixels * (size_t)prm->spp * 4u;  // doubles
     size_t free_b = 0, total_b = 0;
     // kept in the context between renders (allocating 33 GB per frame costs more than the frame); a render
@@ -710,7 +717,7 @@ int rtclj_ctx_render(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* 
   }
   Pass ps;
   ps.samples = prm->spp; ps.spu = spu; ps.sample_buf = sample_buf; ps.mean_n = prm->spp;
-  ps.finalize = !ch.wave && want_out;
+  ps.finalize = !ch.finishes && want_out;
   ps.out_linear = (double*)d_out_linear; ps.out_rgb8 = (unsigned char*)d_out_rgb8;
   return launch_pass(c, cam, prm, ch, sh, ps, stream);
 }
@@ -837,16 +844,23 @@ std::mutex g_ctx_mu;
 struct DeviceSlot { std::mutex mu; rtclj_ctx* ctx = nullptr; };
 std::vector<std::unique_ptr<DeviceSlot>> g_slots;
 
-int device_slot(int device, DeviceSlot** out) {
+// the cached context of `device`, created on first use; `lock` holds the device's slot when this returns
+int cached_ctx(int device, std::unique_lock<std::mutex>& lock, rtclj_ctx** ctx) {
   int ndev = 0;
   int rc = rtclj_device_count(&ndev);
   if (rc) return rc;
   if (ndev == 0) return fail(RTCLJ_E_NO_DEVICE, "no CUDA device (this library has no CPU fallback)");
   if (device < 0 || device >= ndev) return fail(RTCLJ_E_INVALID, "device %d out of range [0,%d)", device, ndev);
-  std::lock_guard<std::mutex> lk(g_ctx_mu);
-  if ((int)g_slots.size() < ndev) g_slots.resize((size_t)ndev);
-  if (!g_slots[(size_t)device]) g_slots[(size_t)device].reset(new DeviceSlot());
-  *out = g_slots[(size_t)device].get();
+  DeviceSlot* slot = nullptr;
+  {
+    std::lock_guard<std::mutex> lk(g_ctx_mu);
+    if ((int)g_slots.size() < ndev) g_slots.resize((size_t)ndev);
+    if (!g_slots[(size_t)device]) g_slots[(size_t)device].reset(new DeviceSlot());
+    slot = g_slots[(size_t)device].get();
+  }
+  lock = std::unique_lock<std::mutex>(slot->mu);
+  if (!slot->ctx) { rc = rtclj_ctx_create(device, &slot->ctx); if (rc) return rc; }
+  *ctx = slot->ctx;
   return RTCLJ_OK;
 }
 
@@ -854,12 +868,10 @@ int device_slot(int device, DeviceSlot** out) {
 int render_shard_hostbuf(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm, double* out_linear,
                          uint8_t* out_rgb8, rtclj_stats* stats) {
   const auto t0 = std::chrono::steady_clock::now();
-  DeviceSlot* slot = nullptr;
-  int rc = device_slot(prm->device, &slot);
+  std::unique_lock<std::mutex> lock;
+  rtclj_ctx* c = nullptr;
+  int rc = cached_ctx(prm->device, lock, &c);
   if (rc) return rc;
-  std::lock_guard<std::mutex> lk(slot->mu);
-  if (!slot->ctx) { rc = rtclj_ctx_create(prm->device, &slot->ctx); if (rc) return rc; }
-  rtclj_ctx* c = slot->ctx;
   rc = rtclj_ctx_set_scene(c, scene);
   if (rc) return rc;
   const size_t npix = (size_t)cam->width * (size_t)cam->height;
@@ -907,6 +919,19 @@ rtclj_stats sum_stats(const std::vector<rtclj_stats>& st) {
   return total;
 }
 
+// the rtclj_params of devices[d] in a call on n devices: its shard of the rows
+rtclj_params shard_params(const rtclj_params* prm, const int32_t* devices, int d, int n) {
+  rtclj_params q = *prm;
+  q.device = devices[d];
+  if (n > 1) {
+    q.shard_index = d; q.shard_count = n;
+    q.shard_rows = prm->shard_rows > 0 ? prm->shard_rows : 1;  // 1-row tiles balance best (DESIGN.md 6)
+  } else {
+    q.shard_index = 0; q.shard_count = 1; q.shard_rows = 0;
+  }
+  return q;
+}
+
 // nothing may throw across the C boundary (a JVM host would die): bad_alloc etc. become error codes
 template <class F>
 int guarded(F&& f) {
@@ -914,6 +939,36 @@ int guarded(F&& f) {
   catch (const std::bad_alloc&) { return fail(RTCLJ_E_CUDA, "out of host memory"); }
   catch (const std::exception& e) { return fail(RTCLJ_E_CUDA, "unexpected exception: %s", e.what()); }
   catch (...) { return fail(RTCLJ_E_CUDA, "unexpected exception"); }
+}
+
+// fn(d) for d = 0 .. n-1 at once: a worker thread for each d > 0, d = 0 on the calling thread.  Returns the code
+// of the lowest d that failed, with its message (which is thread-local: carried over)
+template <class F>
+int run_on_devices(int n, F&& fn) {
+  std::vector<int> rcs((size_t)n, RTCLJ_OK);
+  std::vector<std::string> msgs((size_t)n);
+  auto work = [&](int d) {
+    rcs[(size_t)d] = guarded([&]() { return fn(d); });
+    if (rcs[(size_t)d]) msgs[(size_t)d] = rtclj_error_get();
+  };
+  std::vector<std::thread> pool;
+  for (int d = 1; d < n; ++d) pool.emplace_back(work, d);
+  work(0);
+  for (std::thread& t : pool) t.join();
+  for (int d = 0; d < n; ++d)
+    if (rcs[(size_t)d]) { rtclj_error_set(msgs[(size_t)d].c_str()); return rcs[(size_t)d]; }
+  return RTCLJ_OK;
+}
+
+// the checks of a pass of `samples` samples per pixel after `done`, towards `spp`, in pass units of `unit`
+int check_pass(int done, int samples, int spp, int unit) {
+  if (samples <= 0) return fail(RTCLJ_E_INVALID, "a pass needs a positive sample count, got %d", samples);
+  if ((long long)done + samples > (long long)spp)
+    return fail(RTCLJ_E_INVALID, "pass of %d samples after %d: beyond the target of %d", samples, done, spp);
+  if (done + samples != spp && samples % unit != 0)
+    return fail(RTCLJ_E_INVALID, "pass of %d samples: every pass but the last must be a multiple of pass_unit = %d",
+                samples, unit);
+  return RTCLJ_OK;
 }
 
 }  // namespace
@@ -934,30 +989,12 @@ int rtclj_render_multi(const rtclj_scene* scene, const rtclj_camera* cam, const 
     if (rc) return rc;
     rc = check_devices(devices, n_devices);
     if (rc) return rc;
-    std::vector<rtclj_params> p((size_t)n_devices, *prm);
     std::vector<rtclj_stats> st((size_t)n_devices);
-    std::vector<int> rcs((size_t)n_devices, RTCLJ_OK);
-    std::vector<std::string> msgs((size_t)n_devices);
-    for (int d = 0; d < n_devices; ++d) {
-      p[(size_t)d].device = devices[d];
-      if (n_devices > 1) {
-        p[(size_t)d].shard_index = d;
-        p[(size_t)d].shard_count = n_devices;
-        p[(size_t)d].shard_rows = prm->shard_rows > 0 ? prm->shard_rows : 1;  // 1-row tiles balance best (DESIGN.md 6)
-      } else {
-        p[(size_t)d].shard_index = 0; p[(size_t)d].shard_count = 1; p[(size_t)d].shard_rows = 0;
-      }
-    }
-    auto work = [&](int d) {
-      rcs[(size_t)d] = guarded([&]() { return render_shard_hostbuf(scene, cam, &p[(size_t)d], out_linear, out_rgb8, &st[(size_t)d]); });
-      if (rcs[(size_t)d]) msgs[(size_t)d] = rtclj_error_get();  // the message is thread-local: carry it over
-    };
-    std::vector<std::thread> pool;
-    for (int d = 1; d < n_devices; ++d) pool.emplace_back(work, d);
-    work(0);
-    for (std::thread& t : pool) t.join();
-    for (int d = 0; d < n_devices; ++d)
-      if (rcs[(size_t)d]) { rtclj_error_set(msgs[(size_t)d].c_str()); return rcs[(size_t)d]; }
+    rc = run_on_devices(n_devices, [&](int d) {
+      const rtclj_params q = shard_params(prm, devices, d, n_devices);
+      return render_shard_hostbuf(scene, cam, &q, out_linear, out_rgb8, &st[(size_t)d]);
+    });
+    if (rc) return rc;
     rtclj_stats total = sum_stats(st);
     total.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (stats) *stats = total;
@@ -992,8 +1029,7 @@ namespace {
 
 // the pass unit of an accumulation: 1 in strict order, else the one-shot render's unit size
 int accum_pass_unit(const rtclj_camera* cam, const rtclj_params* prm, bool* strict_out) {
-  const bool primary_only = prm->max_depth == 1 || (prm->flags & RTCLJ_F_NORMAL_SHADING);
-  const bool strict = prm->samples_per_unit >= prm->spp || (prm->samples_per_unit <= 0 && primary_only);
+  const bool strict = prm->samples_per_unit >= prm->spp || (prm->samples_per_unit <= 0 && primary_only(prm));
   if (strict_out) *strict_out = strict;
   return strict ? 1
                 : (prm->samples_per_unit > 0 ? prm->samples_per_unit
@@ -1089,12 +1125,8 @@ int rtclj_ctx_accum_step(rtclj_ctx* c, int32_t samples, void* d_out_linear, void
     if (!A.active) return fail(RTCLJ_E_INVALID, "no accumulation: call rtclj_ctx_accum_begin (rtclj_ctx_set_scene ends one)");
     const rtclj_params* prm = &A.prm;
     const rtclj_camera* cam = &A.cam;
-    if (samples <= 0) return fail(RTCLJ_E_INVALID, "a pass needs a positive sample count, got %d", samples);
-    if ((long long)A.done + samples > (long long)prm->spp)
-      return fail(RTCLJ_E_INVALID, "pass of %d samples after %d: beyond the target of %d", samples, A.done, prm->spp);
-    if (A.done + samples != prm->spp && samples % A.pass_unit != 0)
-      return fail(RTCLJ_E_INVALID, "pass of %d samples: every pass but the last must be a multiple of pass_unit = %d",
-                  samples, A.pass_unit);
+    int rc = check_pass(A.done, samples, prm->spp, A.pass_unit);
+    if (rc) return rc;
     cudaStream_t stream = (cudaStream_t)stream_;
     CU(cudaSetDevice(c->device));
     const Shard sh = shard_of(cam, prm);
@@ -1104,12 +1136,11 @@ int rtclj_ctx_accum_step(rtclj_ctx* c, int32_t samples, void* d_out_linear, void
     ps.sample_base = A.done; ps.samples = samples; ps.acc = c->acc.p; ps.mean_n = d; ps.finalize = true;
     ps.listed = A.adaptive;  // only the live pixels, each folded and tested (finalize_adaptive_kernel)
     ps.out_linear = (double*)d_out_linear; ps.out_rgb8 = (unsigned char*)d_out_rgb8;
-    int rc = RTCLJ_OK;
-    if (!A.strict || !ch.run_kernel) {
+    if (!A.strict || ch.kernel == Kernel::none) {
       // chunks of pass_unit samples, folded onto the running sums in chunk order (depth <= 0: one unit of black)
-      ps.spu = ch.run_kernel ? std::min(A.pass_unit, samples) : samples;
+      ps.spu = ch.kernel != Kernel::none ? std::min(A.pass_unit, samples) : samples;
       rc = launch_pass(c, cam, prm, ch, sh, ps, stream);
-    } else if (ch.primary) {
+    } else if (ch.kernel == Kernel::primary) {
       // one unit per pixel whose sums continue from the running sums: the reference's sequential sum in registers
       ps.spu = samples; ps.seeded = true;
       rc = launch_pass(c, cam, prm, ch, sh, ps, stream);
@@ -1203,14 +1234,7 @@ int progressive_create(const rtclj_scene* scene, const rtclj_camera* cam, const 
     p->spp = prm->spp;
     p->adaptive = tol != nullptr;
     for (int d = 0; d < n_devices; ++d) {
-      rtclj_params q = *prm;
-      q.device = devices[d];
-      if (n_devices > 1) {
-        q.shard_index = d; q.shard_count = n_devices;
-        q.shard_rows = prm->shard_rows > 0 ? prm->shard_rows : 1;  // 1-row tiles balance best (DESIGN.md 6)
-      } else {
-        q.shard_index = 0; q.shard_count = 1; q.shard_rows = 0;
-      }
+      const rtclj_params q = shard_params(prm, devices, d, n_devices);
       rtclj_ctx* c = nullptr;
       rc = rtclj_ctx_create(devices[d], &c);
       if (rc) return rc;
@@ -1251,18 +1275,11 @@ int rtclj_progressive_step(rtclj_progressive* p, int32_t samples, double* out_li
     if (!p) return fail(RTCLJ_E_INVALID, "null progressive handle");
     if (p->failed) return fail(RTCLJ_E_INVALID, "an earlier step failed: destroy this handle and create a new one");
     // rtclj_ctx_accum_step's checks, made before any device starts, so that the devices stay in step
-    if (samples <= 0) return fail(RTCLJ_E_INVALID, "a pass needs a positive sample count, got %d", samples);
-    if ((long long)p->done + samples > (long long)p->spp)
-      return fail(RTCLJ_E_INVALID, "pass of %d samples after %d: beyond the target of %d", samples, p->done, p->spp);
-    if (p->done + samples != p->spp && samples % p->pass_unit != 0)
-      return fail(RTCLJ_E_INVALID, "pass of %d samples: every pass but the last must be a multiple of pass_unit = %d",
-                  samples, p->pass_unit);
-    const size_t n = p->ctxs.size();
+    int rc = check_pass(p->done, samples, p->spp, p->pass_unit);
+    if (rc) return rc;
     const size_t npix = (size_t)p->cam.width * (size_t)p->cam.height;
-    std::vector<rtclj_stats> st(n);
-    std::vector<int> rcs(n, RTCLJ_OK);
-    std::vector<std::string> msgs(n);
-    auto shard = [&](size_t d) -> int {  // pass -> this device's rows of the caller's images -> counters
+    std::vector<rtclj_stats> st(p->ctxs.size());
+    rc = run_on_devices((int)p->ctxs.size(), [&](int d) -> int {  // pass -> this device's rows of the caller's images
       rtclj_ctx* c = p->ctxs[d];
       const rtclj_params& q = p->prm[d];
       CU(cudaSetDevice(c->device));
@@ -1273,18 +1290,9 @@ int rtclj_progressive_step(rtclj_progressive* p, int32_t samples, double* out_li
       if (r) return r;
       r = download_rows(c, &p->cam, q.shard_index, q.shard_count, q.shard_rows, out_linear, out_rgb8, c->own_stream);
       if (r) return r;
-      return rtclj_ctx_stats(c, c->own_stream, &st[d]);  // synchronises the stream: the direct copies have landed
-    };
-    auto work = [&](size_t d) {
-      rcs[d] = guarded([&]() { return shard(d); });
-      if (rcs[d]) msgs[d] = rtclj_error_get();  // the message is thread-local: carry it over
-    };
-    std::vector<std::thread> pool;
-    for (size_t d = 1; d < n; ++d) pool.emplace_back(work, d);
-    work(0);
-    for (std::thread& t : pool) t.join();
-    for (size_t d = 0; d < n; ++d)
-      if (rcs[d]) { p->failed = true; rtclj_error_set(msgs[d].c_str()); return rcs[d]; }
+      return rtclj_ctx_stats(c, c->own_stream, &st[(size_t)d]);  // synchronises the stream: the direct copies have landed
+    });
+    if (rc) { p->failed = true; return rc; }
     p->done += samples;
     if (samples_done) *samples_done = p->done;
     rtclj_stats total = sum_stats(st);
@@ -1353,15 +1361,8 @@ int rtclj_render_multi_ppm(const rtclj_scene* scene, const rtclj_camera* cam, co
     const size_t npix = (size_t)cam->width * (size_t)cam->height;
     const size_t worst = 64 + npix * 12;  // "255 255 255\n" per pixel + header
     if (!out) { *len = worst; return RTCLJ_OK; }  // sizing call: an upper bound, nothing is rendered
-    if (n_devices <= 0 || !devices) return fail(RTCLJ_E_INVALID, "empty device list");
-    int ndev = 0;
-    rc = rtclj_device_count(&ndev);
+    rc = check_devices(devices, n_devices);
     if (rc) return rc;
-    for (int d = 0; d < n_devices; ++d) {
-      if (devices[d] < 0 || devices[d] >= ndev) return fail(RTCLJ_E_INVALID, "device %d out of range [0,%d)", devices[d], ndev);
-      for (int e = 0; e < d; ++e)
-        if (devices[e] == devices[d]) return fail(RTCLJ_E_INVALID, "device %d listed twice", devices[d]);
-    }
     // every device of the call stays locked until the text is out (the root's image is written by its peers);
     // locks are taken in ordinal order, so two such calls cannot deadlock
     std::vector<int> order(devices, devices + n_devices);
@@ -1369,28 +1370,20 @@ int rtclj_render_multi_ppm(const rtclj_scene* scene, const rtclj_camera* cam, co
     std::vector<std::unique_lock<std::mutex>> locks;
     std::vector<rtclj_ctx*> ctxs((size_t)n_devices, nullptr);
     for (int dev : order) {
-      DeviceSlot* slot = nullptr;
-      rc = device_slot(dev, &slot);
+      rtclj_ctx* c = nullptr;
+      locks.emplace_back();
+      rc = cached_ctx(dev, locks.back(), &c);
       if (rc) return rc;
-      locks.emplace_back(slot->mu);
-      if (!slot->ctx) { rc = rtclj_ctx_create(dev, &slot->ctx); if (rc) return rc; }
-      for (int d = 0; d < n_devices; ++d) if (devices[d] == dev) ctxs[(size_t)d] = slot->ctx;
+      for (int d = 0; d < n_devices; ++d) if (devices[d] == dev) ctxs[(size_t)d] = c;
     }
     rtclj_ctx* root = ctxs[0];
     CU(cudaSetDevice(root->device));
     CU(root->out_rgb8.reserve(npix * 3));
     CU(root->p3_text.reserve(worst));
-    std::vector<rtclj_params> p((size_t)n_devices, *prm);
     std::vector<rtclj_stats> st((size_t)n_devices);
-    std::vector<int> rcs((size_t)n_devices, RTCLJ_OK);
-    std::vector<std::string> msgs((size_t)n_devices);
-    const int tile = prm->shard_rows > 0 ? prm->shard_rows : 1;
-    auto shard = [&](int d) -> int {
+    rc = run_on_devices(n_devices, [&](int d) -> int {
       rtclj_ctx* c = ctxs[(size_t)d];
-      rtclj_params& q = p[(size_t)d];
-      q.device = devices[d];
-      if (n_devices > 1) { q.shard_index = d; q.shard_count = n_devices; q.shard_rows = tile; }
-      else { q.shard_index = 0; q.shard_count = 1; q.shard_rows = 0; }
+      const rtclj_params q = shard_params(prm, devices, d, n_devices);
       int r = rtclj_ctx_set_scene(c, scene);
       if (r) return r;
       if (c != root) CU(c->out_rgb8.reserve(npix * 3));
@@ -1410,17 +1403,8 @@ int rtclj_render_multi_ppm(const rtclj_scene* scene, const rtclj_camera* cam, co
         }
       }
       return rtclj_ctx_stats(c, c->own_stream, &st[(size_t)d]);  // synchronises: render and copies are done
-    };
-    auto work = [&](int d) {
-      rcs[(size_t)d] = guarded([&]() { return shard(d); });
-      if (rcs[(size_t)d]) msgs[(size_t)d] = rtclj_error_get();
-    };
-    std::vector<std::thread> pool;
-    for (int d = 1; d < n_devices; ++d) pool.emplace_back(work, d);
-    work(0);
-    for (std::thread& t : pool) t.join();
-    for (int d = 0; d < n_devices; ++d)
-      if (rcs[(size_t)d]) { rtclj_error_set(msgs[(size_t)d].c_str()); return rcs[(size_t)d]; }
+    });
+    if (rc) return rc;
     rtclj_stats total = sum_stats(st);
     // the write-color! loop on the assembled image, then the text alone goes to the host
     CU(cudaSetDevice(root->device));
@@ -1546,12 +1530,10 @@ int rtclj_ctx_encode_ms(rtclj_ctx* c, double* count_scan_ms, double* write_ms) {
 int rtclj_encode_ppm_p3_gpu(int32_t device, const uint8_t* rgb8, int32_t width, int32_t height, char* out,
                             size_t capacity, size_t* len) {
   if (width <= 0 || height <= 0 || !len || !rgb8) return fail(RTCLJ_E_INVALID, "bad image or null len");
-  DeviceSlot* slot = nullptr;
-  int rc = device_slot(device, &slot);
+  std::unique_lock<std::mutex> lock;
+  rtclj_ctx* c = nullptr;
+  int rc = cached_ctx(device, lock, &c);
   if (rc) return rc;
-  std::lock_guard<std::mutex> lk(slot->mu);
-  if (!slot->ctx) { rc = rtclj_ctx_create(device, &slot->ctx); if (rc) return rc; }
-  rtclj_ctx* c = slot->ctx;
   CU(cudaSetDevice(c->device));
   const size_t npix = (size_t)width * (size_t)height;
   CU(c->p3_in.reserve(npix * 3));
