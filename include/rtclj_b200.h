@@ -27,6 +27,9 @@
  *                           the same writer as device kernels (device / host buffers)
  *   rtclj_encode_png, rtclj_decode_ppm_p3
  *                           ppm->png, src/raytracing.clj:176 (src/ppm2png.clj:35-87): writer, reader
+ *   rtclj_ctx_encode_png, rtclj_encode_png_gpu
+ *                           a compressed PNG of the same image, written by device kernels (device / host buffers)
+ *   rtclj_render_multi_png  the render loop and ppm->png as one call: several GPUs in, a compressed PNG out
  *   rtclj_camera_main/_realm/_i
  *                           the camera let-blocks, src/raytracing.clj:105-139 ;
  *                           realm/raytracing.clj:264-280,306-322 ;
@@ -354,6 +357,55 @@ int rtclj_encode_ppm_p3_gpu(int32_t device, const uint8_t *rgb8, int32_t width, 
  * blocks.  Call with out == NULL to get the required capacity in *len. */
 int rtclj_encode_png(const uint8_t *rgb8, int32_t width, int32_t height, uint8_t *out, size_t capacity,
                      size_t *len);
+
+/* A compressed PNG of the same image, encoded on the device.  The bytes are exactly those of this definition
+ * (tests/png_model.py reproduces them; DESIGN.md section 4.11):
+ *   1. Chunks: the signature; IHDR as rtclj_encode_png's (8-bit truecolour, no interlace); an IDAT holding only the
+ *      zlib header 78 01; one IDAT per segment; an IDAT holding only the big-endian Adler-32 of the whole filtered
+ *      stream; IEND.  Each chunk's CRC-32 covers its type and data.
+ *   2. Filtering: each row is filtered with each of the five PNG filters (bpp 3; outside the image a = b = c = 0).
+ *      The cost is the sum of |byte as int8| over the filtered row, filter 0 included; the lowest cost wins, a tie
+ *      goes to the lower type.  The filtered stream F is H * (1 + 3W) bytes.
+ *   3. Segments: F is cut at multiples of 65 536 bytes (the last segment may be shorter); segments are encoded
+ *      independently, no match reaches back past a segment's first byte.
+ *   4. Tokens: a maximal run of L equal bytes starting at s within a segment is a literal at s, then
+ *      (L - 1) / 258 matches (258, distance 1), then the remainder q = (L - 1) % 258 as one match of length q if
+ *      q >= 3, else as q literals (what zlib's greedy deflate_rle emits).
+ *   5. Each segment is one dynamic block (BTYPE 2) of all its tokens plus end-of-block:
+ *      - literal/length code lengths by package-merge limited to 15 bits; items ordered by (frequency, symbol)
+ *        ascending, at equal weight leaves before packages (the end-of-block symbol and the segment's first literal
+ *        are always present);
+ *      - distance code: codes 0 and 1, length 1 each (HDIST = 2); only code 0 (distance 1) is emitted;
+ *      - HLIT = highest used literal/length symbol + 1, at least 257;
+ *      - the HLIT + HDIST lengths as one sequence: a zero run of 11..138 is symbol 18, of 3..10 symbol 17, longest
+ *        first, greedily; a non-zero length is written once, then symbol 16 covers each further run of 3..6
+ *        repeats of it; everything else is a literal length;
+ *      - code-length code by package-merge limited to 7 bits, same ordering; if only one symbol is used, the lowest
+ *        other symbol gets length 1 as well;
+ *      - HCLEN trimmed on the order 16 17 18 0 8 7 9 6 10 5 11 4 12 3 13 2 14 1 15, at least 4 entries;
+ *      - canonical codes (RFC 1951 3.2.2), packed LSB-first.
+ *   6. Stored fallback: if the dynamic encoding, flush included, is not shorter in bytes than stored blocks of at
+ *      most 65 535 bytes, the segment is written stored (incompressible noise).
+ *   7. A dynamic segment but the last is followed by an empty stored block (sync flush: 000, padding to the byte,
+ *      00 00 FF FF); a stored segment ends on a byte boundary; the last segment's last block has BFINAL = 1 and is
+ *      padded to the byte.
+ * out == NULL (d_out == NULL) is the sizing call: *len receives a sufficient capacity, the size with every segment
+ * stored, and nothing runs on the GPU.  A capacity below the exact length returns RTCLJ_E_BUFFER with *len set to
+ * the exact length.  Non-positive sizes, null pointers and images whose F would exceed 2^31 - 2 segments return
+ * RTCLJ_E_INVALID.  rtclj_ctx_encode_png reads the DEVICE image d_rgb8 and writes DEVICE memory d_out; it keeps F
+ * (the image's bytes plus one per row) and one 64 KiB staging slot per segment in the context, and synchronises
+ * `stream` (the length comes back from the device). */
+int rtclj_ctx_encode_png(rtclj_ctx *ctx, const uint8_t *d_rgb8, int32_t width, int32_t height, uint8_t *d_out,
+                         size_t capacity, size_t *len, void *stream);
+/* Host buffers in and out, the encoding on `device` (copies inside the call). */
+int rtclj_encode_png_gpu(int32_t device, const uint8_t *rgb8, int32_t width, int32_t height, uint8_t *out,
+                         size_t capacity, size_t *len);
+/* rtclj_render_multi_ppm with this PNG writer in place of the P3 writer: renders on `n_devices` GPUs, assembles the
+ * 8-bit rows on devices[0] and encodes them there; only the PNG crosses PCIe.  The bytes are those of
+ * rtclj_encode_png_gpu on rtclj_render's rgb8 image. */
+int rtclj_render_multi_png(const rtclj_scene *scene, const rtclj_camera *camera, const rtclj_params *params,
+                           const int32_t *devices, int32_t n_devices, uint8_t *out, size_t capacity, size_t *len,
+                           rtclj_stats *stats);
 
 /* The reader half of ppm->png (src/ppm2png.clj:35-87 reads "P3", "W H", a maximum <= 255 and one
  * "r g b" line per pixel; this parser accepts any whitespace between the tokens).  Call with

@@ -55,6 +55,14 @@
             (fd-int ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS
                     ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/JAVA_LONG ValueLayout/ADDRESS
                     ValueLayout/ADDRESS)))
+;; int rtclj_render_multi_png(const rtclj_scene*, const rtclj_camera*, const rtclj_params*,
+;;                            const int32_t* devices, int32_t n_devices,
+;;                            uint8_t* out, size_t capacity, size_t* len, rtclj_stats*)
+(def ^:private rtclj-render-multi-png
+  (downcall "rtclj_render_multi_png"
+            (fd-int ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS
+                    ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/JAVA_LONG ValueLayout/ADDRESS
+                    ValueLayout/ADDRESS)))
 ;; int rtclj_host_alloc(size_t bytes, void** out);  int rtclj_host_free(void* p)
 (def ^:private rtclj-host-alloc (downcall "rtclj_host_alloc" (fd-int ValueLayout/JAVA_LONG ValueLayout/ADDRESS)))
 (def ^:private rtclj-host-free (downcall "rtclj_host_free" (fd-int ValueLayout/ADDRESS)))
@@ -171,6 +179,25 @@
                                     [scene camera params
                                      (.allocateFrom a ValueLayout/JAVA_INT (int-array devices)) (int (count devices))
                                      out cap len MemorySegment/NULL]))
+      (with-open [o (java.io.FileOutputStream. path)]
+        (.write (.getChannel o) (.asByteBuffer (.asSlice out 0 (.get len ValueLayout/JAVA_LONG 0))))))))
+
+(defn render-png!
+  "render-ppm! with ppm->png (raytracing.clj:176) in place of the P3 text: the render loop on :devices (default
+   [0]), then the device PNG writer on the first of them (filtered rows, run-length deflate; DESIGN.md section
+   4.11).  The compressed file comes back and is handed to a single .write; its pixels are those of scene.ppm."
+  [^String path bodies cam samples-per-px max-depth & {:keys [devices] :or {devices [0]} :as opts}]
+  (with-open [a (Arena/ofConfined)]
+    (let [[scene camera params] (marshal a bodies cam samples-per-px max-depth opts)
+          devs (.allocateFrom a ValueLayout/JAVA_INT (int-array devices))
+          len  (.allocate a 8 8)
+          _    (check! (.invokeWithArguments rtclj-render-multi-png          ; sizing call: nothing is rendered
+                                             [scene camera params devs (int (count devices))
+                                              MemorySegment/NULL 0 len MemorySegment/NULL]))
+          cap  (.get len ValueLayout/JAVA_LONG 0)
+          out  (.allocate a cap 16)]
+      (check! (.invokeWithArguments rtclj-render-multi-png
+                                    [scene camera params devs (int (count devices)) out cap len MemorySegment/NULL]))
       (with-open [o (java.io.FileOutputStream. path)]
         (.write (.getChannel o) (.asByteBuffer (.asSlice out 0 (.get len ValueLayout/JAVA_LONG 0))))))))
 
@@ -345,3 +372,24 @@
       (let [n (.get len ValueLayout/JAVA_LONG 0)]
         (with-open [o (java.io.FileOutputStream. path)]
           (.write (.getChannel o) (.asByteBuffer (.asSlice out 0 n))))))))
+
+;; int rtclj_encode_png_gpu(int32_t device, const uint8_t* rgb8, int32_t width, int32_t height,
+;;                          uint8_t* out, size_t capacity, size_t* len)
+(def ^:private rtclj-encode-png-gpu
+  (downcall "rtclj_encode_png_gpu"
+            (fd-int ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/JAVA_INT ValueLayout/JAVA_INT
+                    ValueLayout/ADDRESS ValueLayout/JAVA_LONG ValueLayout/ADDRESS)))
+
+(defn encode-png-gpu
+  "ppm->png's writer (raytracing.clj:176) on the GPU: rgb8 is a byte[] of W*H*3 components (row-major from the
+   top-left pixel), the result a byte[] holding a compressed PNG of it (DESIGN.md section 4.11)."
+  ^bytes [^bytes rgb8 width height & {:keys [device] :or {device 0}}]
+  (with-open [a (Arena/ofConfined)]
+    (let [w   (int width) h (int height)
+          src (.allocateFrom a ValueLayout/JAVA_BYTE rgb8)
+          len (.allocate a 8 8)
+          _   (check! (.invokeWithArguments rtclj-encode-png-gpu [(int device) src w h MemorySegment/NULL 0 len]))
+          cap (.get len ValueLayout/JAVA_LONG 0)
+          out (.allocate a cap 16)]
+      (check! (.invokeWithArguments rtclj-encode-png-gpu [(int device) src w h out cap len]))
+      (.toArray (.asSlice out 0 (.get len ValueLayout/JAVA_LONG 0)) ValueLayout/JAVA_BYTE))))

@@ -103,6 +103,13 @@ SYMBOLS = {
                                       C.c_size_t]),
     "rtclj_encode_png": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_size_t,
                                    C.POINTER(C.c_size_t)]),
+    "rtclj_ctx_encode_png": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_size_t,
+                                       C.POINTER(C.c_size_t), C.c_void_p]),
+    "rtclj_encode_png_gpu": (C.c_int, [C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_size_t,
+                                       C.POINTER(C.c_size_t)]),
+    "rtclj_render_multi_png": (C.c_int, [C.POINTER(Scene), C.POINTER(Camera), C.POINTER(Params),
+                                         C.POINTER(C.c_int32), C.c_int32, C.c_void_p, C.c_size_t,
+                                         C.POINTER(C.c_size_t), C.POINTER(Stats)]),
     "rtclj_ratio_to_double": (C.c_double, [C.c_int64, C.c_int64]),
     "rtclj_camera_main": (C.c_int, [C.c_int32, C.c_int32, C.c_double, C.POINTER(C.c_double),
                                     C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_double,

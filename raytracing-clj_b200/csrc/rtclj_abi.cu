@@ -8,6 +8,7 @@
 #include "rtclj_primary_kernel.cuh"
 #include "rtclj_split_kernel.cuh"
 #include "rtclj_p3_kernels.cuh"
+#include "rtclj_png_kernels.cuh"
 #include "rtclj_adaptive.cuh"
 #include "rtclj_error.h"
 
@@ -87,6 +88,12 @@ struct rtclj_ctx {
   int p3_ctas_per_sm = 0;
   DevBuf<unsigned char> p3_in, p3_text; // staging for the host-buffer entry point
   float p3_count_ms = 0.f, p3_write_ms = 0.f;
+  // PNG writer: the filtered stream F, one staging slot and one record per 64 KiB segment, the total length
+  DevBuf<unsigned char> png_f, png_stage;
+  DevBuf<PngSegRec> png_rec;
+  DevBuf<unsigned long long> png_state;
+  DevBuf<unsigned char> png_in, png_out;  // staging for the host-buffer entry points
+  bool png_attr = false;                   // the PNG kernels' shared-memory limit is raised
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev2 = nullptr;  // render: start, kernel end, finalize end
   cudaEvent_t p3_ev0 = nullptr, p3_ev1 = nullptr;           // the P3 writer's own timing events
   cudaStream_t own_stream = nullptr;
@@ -316,6 +323,7 @@ void rtclj_ctx_destroy(rtclj_ctx* c) {
   c->acc.release(); c->acc2.release(); c->nsamp.release(); c->live.release(); c->list.release(); c->list_aux.release();
   c->noise_samples.release(); c->noise_stderr.release();
   c->p3_state.release(); c->p3_in.release(); c->p3_text.release();
+  c->png_f.release(); c->png_stage.release(); c->png_rec.release(); c->png_state.release(); c->png_in.release(); c->png_out.release();
   for (cudaEvent_t e : {c->ev0, c->ev1, c->ev2, c->p3_ev0, c->p3_ev1, c->pin_ev[0], c->pin_ev[1]})
     if (e) cudaEventDestroy(e);
   for (void* h : c->pin) if (h) cudaFreeHost(h);
@@ -1346,6 +1354,81 @@ int rtclj_progressive_destroy(rtclj_progressive* p) {
   });
 }
 
+}  // extern "C"
+
+namespace {
+
+// The render loop on several GPUs with the 8-bit image assembled on devices[0]: each device renders its shard and
+// copies its rows into the root's out_rgb8 over NVLink.  Every device of the call is locked in `locks` until the
+// caller lets go of them (the root's image is written by its peers); locks are taken in ordinal order, so two such
+// calls cannot deadlock.  *root receives devices[0]'s context, *total the summed counters.
+int render_to_root(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm, const int32_t* devices,
+                   int32_t n_devices, std::vector<std::unique_lock<std::mutex>>& locks, rtclj_ctx** root_out,
+                   rtclj_stats* total) {
+  int rc = check_devices(devices, n_devices);
+  if (rc) return rc;
+  const size_t npix = (size_t)cam->width * (size_t)cam->height;
+  std::vector<int> order(devices, devices + n_devices);
+  std::sort(order.begin(), order.end());
+  std::vector<rtclj_ctx*> ctxs((size_t)n_devices, nullptr);
+  for (int dev : order) {
+    rtclj_ctx* c = nullptr;
+    locks.emplace_back();
+    rc = cached_ctx(dev, locks.back(), &c);
+    if (rc) return rc;
+    for (int d = 0; d < n_devices; ++d) if (devices[d] == dev) ctxs[(size_t)d] = c;
+  }
+  rtclj_ctx* root = ctxs[0];
+  CU(cudaSetDevice(root->device));
+  CU(root->out_rgb8.reserve(npix * 3));
+  std::vector<rtclj_stats> st((size_t)n_devices);
+  rc = run_on_devices(n_devices, [&](int d) -> int {
+    rtclj_ctx* c = ctxs[(size_t)d];
+    const rtclj_params q = shard_params(prm, devices, d, n_devices);
+    int r = rtclj_ctx_set_scene(c, scene);
+    if (r) return r;
+    if (c != root) CU(c->out_rgb8.reserve(npix * 3));
+    r = rtclj_ctx_render(c, cam, &q, nullptr, c->out_rgb8.p, c->own_stream);
+    if (r) return r;
+    if (c != root) {  // this shard's rows -> the root's image, device to device
+      int can = 0;
+      if (cudaDeviceCanAccessPeer(&can, c->device, root->device) == cudaSuccess && can) {
+        const cudaError_t e = cudaDeviceEnablePeerAccess(root->device, 0);
+        if (e != cudaSuccess) cudaGetLastError();  // already enabled: fine; otherwise the copy is staged by the driver
+      }
+      std::vector<Piece> pieces;
+      plan_pieces((size_t)cam->height, (size_t)cam->width * 3, q.shard_index, q.shard_count, q.shard_rows, (size_t)1 << 40, pieces);
+      for (const Piece& pc : pieces) {
+        if (pc.height == 1) CU(cudaMemcpyAsync(root->out_rgb8.p + pc.off, c->out_rgb8.p + pc.off, pc.width, cudaMemcpyDefault, c->own_stream));
+        else CU(cudaMemcpy2DAsync(root->out_rgb8.p + pc.off, pc.pitch, c->out_rgb8.p + pc.off, pc.pitch, pc.width, pc.height, cudaMemcpyDefault, c->own_stream));
+      }
+    }
+    return rtclj_ctx_stats(c, c->own_stream, &st[(size_t)d]);  // synchronises: render and copies are done
+  });
+  if (rc) return rc;
+  *total = sum_stats(st);
+  *root_out = root;
+  CU(cudaSetDevice(root->device));
+  return RTCLJ_OK;
+}
+
+// The filtered stream's length and the sizing call's answer (every segment stored) of a W x H PNG;
+// RTCLJ_E_INVALID for sizes the encoder cannot take.
+int png_sizes(int32_t width, int32_t height, size_t* nf, size_t* bound) {
+  if (width <= 0 || height <= 0) return fail(RTCLJ_E_INVALID, "image size must be positive (%d x %d)", width, height);
+  const size_t N = (size_t)height * ((size_t)width * 3 + 1);  // < 2^63 for any int32 size
+  const size_t nseg = (N + kPngSeg - 1) / kPngSeg;
+  if (nseg > 0x7ffffffeull) return fail(RTCLJ_E_INVALID, "a %d x %d PNG is too large for the device encoder", width, height);
+  const size_t full = N / kPngSeg, rest = N - full * kPngSeg;
+  *nf = N;
+  *bound = kPngHead + kPngTail + full * (12 + kPngSeg + 10) + (rest ? 12 + rest + 5 * ((rest + 65534) / 65535) : 0);
+  return RTCLJ_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
 // Render on several GPUs and return the P3 TEXT -- the reference's loop plus its write-color! loop
 // (src/raytracing.clj:141-175) as one call.  The 8-bit shards are assembled on devices[0] by peer copies
 // over NVLink and the device P3 writer runs there; only the text crosses PCIe.  This is the one product for
@@ -1361,59 +1444,51 @@ int rtclj_render_multi_ppm(const rtclj_scene* scene, const rtclj_camera* cam, co
     const size_t npix = (size_t)cam->width * (size_t)cam->height;
     const size_t worst = 64 + npix * 12;  // "255 255 255\n" per pixel + header
     if (!out) { *len = worst; return RTCLJ_OK; }  // sizing call: an upper bound, nothing is rendered
-    rc = check_devices(devices, n_devices);
-    if (rc) return rc;
-    // every device of the call stays locked until the text is out (the root's image is written by its peers);
-    // locks are taken in ordinal order, so two such calls cannot deadlock
-    std::vector<int> order(devices, devices + n_devices);
-    std::sort(order.begin(), order.end());
     std::vector<std::unique_lock<std::mutex>> locks;
-    std::vector<rtclj_ctx*> ctxs((size_t)n_devices, nullptr);
-    for (int dev : order) {
-      rtclj_ctx* c = nullptr;
-      locks.emplace_back();
-      rc = cached_ctx(dev, locks.back(), &c);
-      if (rc) return rc;
-      for (int d = 0; d < n_devices; ++d) if (devices[d] == dev) ctxs[(size_t)d] = c;
-    }
-    rtclj_ctx* root = ctxs[0];
-    CU(cudaSetDevice(root->device));
-    CU(root->out_rgb8.reserve(npix * 3));
-    CU(root->p3_text.reserve(worst));
-    std::vector<rtclj_stats> st((size_t)n_devices);
-    rc = run_on_devices(n_devices, [&](int d) -> int {
-      rtclj_ctx* c = ctxs[(size_t)d];
-      const rtclj_params q = shard_params(prm, devices, d, n_devices);
-      int r = rtclj_ctx_set_scene(c, scene);
-      if (r) return r;
-      if (c != root) CU(c->out_rgb8.reserve(npix * 3));
-      r = rtclj_ctx_render(c, cam, &q, nullptr, c->out_rgb8.p, c->own_stream);
-      if (r) return r;
-      if (c != root) {  // this shard's rows -> the root's image, device to device
-        int can = 0;
-        if (cudaDeviceCanAccessPeer(&can, c->device, root->device) == cudaSuccess && can) {
-          const cudaError_t e = cudaDeviceEnablePeerAccess(root->device, 0);
-          if (e != cudaSuccess) cudaGetLastError();  // already enabled: fine; otherwise the copy is staged by the driver
-        }
-        std::vector<Piece> pieces;
-        plan_pieces((size_t)cam->height, (size_t)cam->width * 3, q.shard_index, q.shard_count, q.shard_rows, (size_t)1 << 40, pieces);
-        for (const Piece& pc : pieces) {
-          if (pc.height == 1) CU(cudaMemcpyAsync(root->out_rgb8.p + pc.off, c->out_rgb8.p + pc.off, pc.width, cudaMemcpyDefault, c->own_stream));
-          else CU(cudaMemcpy2DAsync(root->out_rgb8.p + pc.off, pc.pitch, c->out_rgb8.p + pc.off, pc.pitch, pc.width, pc.height, cudaMemcpyDefault, c->own_stream));
-        }
-      }
-      return rtclj_ctx_stats(c, c->own_stream, &st[(size_t)d]);  // synchronises: render and copies are done
-    });
+    rtclj_ctx* root = nullptr;
+    rtclj_stats total;
+    rc = render_to_root(scene, cam, prm, devices, n_devices, locks, &root, &total);
     if (rc) return rc;
-    rtclj_stats total = sum_stats(st);
     // the write-color! loop on the assembled image, then the text alone goes to the host
-    CU(cudaSetDevice(root->device));
+    CU(root->p3_text.reserve(worst));
     size_t need = 0;
     rc = rtclj_ctx_encode_ppm_p3(root, root->out_rgb8.p, cam->width, cam->height, reinterpret_cast<char*>(root->p3_text.p), worst, &need, root->own_stream);
     if (rc) return rc;
     *len = need;
     if (need > capacity) return fail(RTCLJ_E_BUFFER, "P3 text needs %zu bytes, capacity is %zu", need, capacity);
     CU(cudaMemcpyAsync(out, root->p3_text.p, need, cudaMemcpyDeviceToHost, root->own_stream));
+    CU(cudaStreamSynchronize(root->own_stream));
+    total.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = total;
+    return RTCLJ_OK;
+  });
+}
+
+// The same render with the compressed PNG writer in place of the P3 writer: only the PNG crosses PCIe.
+int rtclj_render_multi_png(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm,
+                           const int32_t* devices, int32_t n_devices, uint8_t* out, size_t capacity, size_t* len,
+                           rtclj_stats* stats) {
+  return guarded([&]() -> int {
+    const auto t0 = std::chrono::steady_clock::now();
+    if (!scene || !len) return fail(RTCLJ_E_INVALID, "null scene or len");
+    int rc = validate(cam, prm);
+    if (rc) return rc;
+    size_t nf = 0, bound = 0;
+    rc = png_sizes(cam->width, cam->height, &nf, &bound);
+    if (rc) return rc;
+    if (!out) { *len = bound; return RTCLJ_OK; }  // sizing call: the stored bound, nothing is rendered
+    std::vector<std::unique_lock<std::mutex>> locks;
+    rtclj_ctx* root = nullptr;
+    rtclj_stats total;
+    rc = render_to_root(scene, cam, prm, devices, n_devices, locks, &root, &total);
+    if (rc) return rc;
+    CU(root->png_out.reserve(bound));
+    size_t need = 0;
+    rc = rtclj_ctx_encode_png(root, root->out_rgb8.p, cam->width, cam->height, root->png_out.p, bound, &need, root->own_stream);
+    if (rc) return rc;
+    *len = need;
+    if (need > capacity) return fail(RTCLJ_E_BUFFER, "PNG needs %zu bytes, capacity is %zu", need, capacity);
+    CU(cudaMemcpyAsync(out, root->png_out.p, need, cudaMemcpyDeviceToHost, root->own_stream));
     CU(cudaStreamSynchronize(root->own_stream));
     total.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (stats) *stats = total;
@@ -1549,6 +1624,82 @@ int rtclj_encode_ppm_p3_gpu(int32_t device, const uint8_t* rgb8, int32_t width, 
   CU(cudaMemcpyAsync(out, c->p3_text.p, need, cudaMemcpyDeviceToHost, c->own_stream));
   CU(cudaStreamSynchronize(c->own_stream));
   return RTCLJ_OK;
+}
+
+// ---- the compressed PNG writer on the device (DESIGN.md section 4.11; the format: include/rtclj_b200.h)
+int rtclj_ctx_encode_png(rtclj_ctx* c, const uint8_t* d_rgb8, int32_t width, int32_t height, uint8_t* d_out,
+                         size_t capacity, size_t* len, void* stream_) {
+  return guarded([&]() -> int {
+    if (!c || !len) return fail(RTCLJ_E_INVALID, "null ctx or len");
+    size_t N = 0, bound = 0;
+    int rc = png_sizes(width, height, &N, &bound);
+    if (rc) return rc;
+    if (!d_out) { *len = bound; return RTCLJ_OK; }
+    if (!d_rgb8) return fail(RTCLJ_E_INVALID, "null image");
+    cudaStream_t stream = (cudaStream_t)stream_;
+    CU(cudaSetDevice(c->device));
+    if (!c->png_attr) {
+      CU(cudaFuncSetAttribute(png_deflate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PngDeflateSmem)));
+      CU(cudaFuncSetAttribute(png_place_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PngPlaceSmem)));
+      c->png_attr = true;
+    }
+    static const PngCrcShifts shifts = png_crc_shifts();
+    const size_t nseg = (N + kPngSeg - 1) / kPngSeg;
+    CU(c->png_f.reserve(nseg * kPngSeg));
+    CU(c->png_stage.reserve(nseg * kPngSlot));
+    CU(c->png_rec.reserve(nseg));
+    CU(c->png_state.reserve(1));
+    png_filter_kernel<<<(unsigned)height, kPngFilterThreads, 0, stream>>>(d_rgb8, (size_t)width * 3, c->png_f.p);
+    CU(cudaGetLastError());
+    png_deflate_kernel<<<(unsigned)nseg, kPngThreads, sizeof(PngDeflateSmem), stream>>>(c->png_f.p, N, c->png_stage.p, c->png_rec.p);
+    CU(cudaGetLastError());
+    unsigned long long total = 0;
+    if (capacity < bound) {  // the exact length first: the buffer may be too small for it
+      png_place_kernel<<<(unsigned)nseg + 1, kPngThreads, sizeof(PngPlaceSmem), stream>>>(
+          c->png_f.p, N, c->png_stage.p, c->png_rec.p, (unsigned)nseg, (unsigned)width, (unsigned)height, nullptr, c->png_state.p, 1, shifts);
+      CU(cudaGetLastError());
+      CU(cudaMemcpyAsync(&total, c->png_state.p, sizeof total, cudaMemcpyDeviceToHost, stream));
+      CU(cudaStreamSynchronize(stream));
+      *len = (size_t)total;
+      if ((size_t)total > capacity) return fail(RTCLJ_E_BUFFER, "PNG needs %llu bytes, capacity is %zu", total, capacity);
+    }
+    png_place_kernel<<<(unsigned)nseg + 1, kPngThreads, sizeof(PngPlaceSmem), stream>>>(
+        c->png_f.p, N, c->png_stage.p, c->png_rec.p, (unsigned)nseg, (unsigned)width, (unsigned)height, d_out, c->png_state.p, 0, shifts);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(&total, c->png_state.p, sizeof total, cudaMemcpyDeviceToHost, stream));
+    CU(cudaStreamSynchronize(stream));
+    *len = (size_t)total;
+    return RTCLJ_OK;
+  });
+}
+
+int rtclj_encode_png_gpu(int32_t device, const uint8_t* rgb8, int32_t width, int32_t height, uint8_t* out,
+                         size_t capacity, size_t* len) {
+  return guarded([&]() -> int {
+    if (!len) return fail(RTCLJ_E_INVALID, "null len");
+    size_t N = 0, bound = 0;
+    int rc = png_sizes(width, height, &N, &bound);
+    if (rc) return rc;
+    if (!out) { *len = bound; return RTCLJ_OK; }
+    if (!rgb8) return fail(RTCLJ_E_INVALID, "null image");
+    std::unique_lock<std::mutex> lock;
+    rtclj_ctx* c = nullptr;
+    rc = cached_ctx(device, lock, &c);
+    if (rc) return rc;
+    CU(cudaSetDevice(c->device));
+    const size_t bytes = (size_t)width * (size_t)height * 3;
+    CU(c->png_in.reserve(bytes));
+    CU(c->png_out.reserve(bound));
+    CU(cudaMemcpyAsync(c->png_in.p, rgb8, bytes, cudaMemcpyHostToDevice, c->own_stream));
+    size_t need = 0;
+    rc = rtclj_ctx_encode_png(c, c->png_in.p, width, height, c->png_out.p, bound, &need, c->own_stream);
+    if (rc) return rc;
+    *len = need;
+    if (need > capacity) return fail(RTCLJ_E_BUFFER, "PNG needs %zu bytes, capacity is %zu", need, capacity);
+    CU(cudaMemcpyAsync(out, c->png_out.p, need, cudaMemcpyDeviceToHost, c->own_stream));
+    CU(cudaStreamSynchronize(c->own_stream));
+    return RTCLJ_OK;
+  });
 }
 
 int rtclj_calibrate_peaks(int32_t device, double* ffma, double* ffma2, double* dfma, int32_t* sm_count) {

@@ -7,6 +7,7 @@
     python -m raytracing_clj_b200.main main [spp] [depth] --every N --tolerance ABS,REL
                                                               -> the same with adaptive sampling, and
                                                                  scene-samples.png (samples per pixel)
+    python -m raytracing_clj_b200.main main ... --gpu-png     -> the same files, the PNGs compressed on the GPU
     python -m raytracing_clj_b200.main realm                  -> scene-realm.ppm
     python -m raytracing_clj_b200.main i                      -> scene-i.ppm
 
@@ -20,7 +21,11 @@ last files are byte for byte those of a run without --every.
 With --tolerance ABS,REL the passes trace only the pixels whose noise estimate is still above
 ABS + REL * |pixel mean| (adaptive sampling, DESIGN.md section 4.10; every pixel gets at least two pass
 units), and the run ends once no pixel is left.  scene-samples.png shows the samples each pixel received
-(white: spp)."""
+(white: spp).
+
+With --gpu-png scene.png (and scene-samples.png) are written by the device PNG writer from the render's 8-bit
+image (DESIGN.md section 4.11): the same pixels, compressed, and only the compressed bytes leave the GPU.  Without
+it every file is the one the host writer produces."""
 from __future__ import annotations
 
 import os
@@ -47,9 +52,10 @@ def samples_image(samples: np.ndarray, spp: int) -> np.ndarray:
 
 
 def main_variant(spp: int = 100, depth: int = 50, out: str = "scene.ppm", seed: int = 1, every: int = 0,
-                 tolerance=None):
+                 tolerance=None, gpu_png: bool = False):
     print("config:", {"samples-per-px": spp, "max-depth": depth})
     t0 = time.perf_counter()
+    png_device = 0 if gpu_png else None  # the render's device (devices default to [0])
     if tolerance is not None and every <= 0:
         every = max(1, spp // 10)
     if every > 0:
@@ -68,12 +74,12 @@ def main_variant(spp: int = 100, depth: int = 50, out: str = "scene.ppm", seed: 
                     samples, _, active = p.noise()
                 if p.samples_done < spp and active > 0:  # the last image goes out below, as without --every
                     _replace(out, render.encode_ppm(rgb8))
-                    _replace(png, render.encode_png(rgb8))
+                    _replace(png, render.encode_png(rgb8, png_device))
                 left = f", {active} pixels active" if p.adaptive else ""
                 print(f"{p.samples_done}/{spp} samples per pixel{left}: {out} ({1e3 * (time.perf_counter() - t0):.0f} ms)")
             if p.adaptive:
                 grey = out[:-4] + "-samples.png" if out.endswith(".ppm") else out + "-samples.png"
-                render.write_png(grey, samples_image(samples, spp))
+                render.write_png(grey, samples_image(samples, spp), png_device)
                 full = spp * cam.width * cam.height
                 print(f"samples traced: {traced} of {full} ({100.0 * traced / full:.1f} %); sample counts in {grey}")
         st["segments"] = segments
@@ -81,7 +87,11 @@ def main_variant(spp: int = 100, depth: int = 50, out: str = "scene.ppm", seed: 
         _, rgb8, st = render.render(scenes.main_hittables(), camera.main_camera(), spp, depth, seed=seed,
                                     flags=_abi.FLAGS_MAIN, want_linear=False)
     render.write_ppm(out, rgb8)
-    render.ppm_to_png(out, out[:-4] + ".png" if out.endswith(".ppm") else out + ".png")  # (ppm->png "scene.ppm" "scene.png"), raytracing.clj:176
+    png = out[:-4] + ".png" if out.endswith(".ppm") else out + ".png"
+    if gpu_png:
+        render.write_png(png, rgb8, png_device)
+    else:
+        render.ppm_to_png(out, png)  # (ppm->png "scene.ppm" "scene.png"), raytracing.clj:176
     print(f'"Elapsed time: {1e3 * (time.perf_counter() - t0):.3f} msecs"  ({st["segments"]} ray segments)')
     return st
 
@@ -106,6 +116,8 @@ def _cli(argv):
     which = argv[0] if argv else "main"
     if which == "main":
         every, tolerance = 0, None
+        gpu_png = "--gpu-png" in argv
+        argv = [a for a in argv if a != "--gpu-png"]
         if "--tolerance" in argv:
             i = argv.index("--tolerance")
             try:
@@ -122,7 +134,7 @@ def _cli(argv):
             every = int(argv[i + 1])
             argv = argv[:i] + argv[i + 2:]
         main_variant(int(argv[1]) if len(argv) > 1 else 100, int(argv[2]) if len(argv) > 2 else 50, every=every,
-                     tolerance=tolerance)
+                     tolerance=tolerance, gpu_png=gpu_png)
     elif which == "realm":
         realm_variant()
     elif which == "i":

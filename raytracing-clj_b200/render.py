@@ -119,6 +119,28 @@ def render_ppm(world, cam: Camera, samples_per_px: int = 100, max_depth: int = 5
     return bytes(memoryview(store)[: n.value]), st.as_dict()
 
 
+def render_png(world, cam: Camera, samples_per_px: int = 100, max_depth: int = 50, *, seed: int = 1,
+               flags: int = _abi.FLAGS_MAIN, samples_per_unit: int = 0, devices: Optional[Sequence[int]] = None):
+    """The render loop and ppm->png in one call: returns (bytes of a compressed PNG, stats).  The image never visits
+    the host: the shards are assembled on devices[0] and the device PNG writer runs there (rtclj_render_multi_png);
+    the bytes are those of encode_png(rgb8, device=k) on the rendered image."""
+    lib = _abi.lib()
+    soa = _as_soa(world)
+    sc, cm = _scene_struct(soa), _camera_struct(cam)
+    prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit), 0, 0, 0, 0, 0)
+    devs = list(devices) if devices else [0]
+    arr = (C.c_int32 * len(devs))(*devs)
+    n = C.c_size_t()
+    _abi.check(lib.rtclj_render_multi_png(C.byref(sc), C.byref(cm), C.byref(prm), arr, len(devs), None, 0, C.byref(n), None))
+    store = bytearray(n.value)
+    buf = (C.c_char * n.value).from_buffer(store)
+    st = _abi.Stats()
+    _abi.check(lib.rtclj_render_multi_png(C.byref(sc), C.byref(cm), C.byref(prm), arr, len(devs), buf, n.value,
+                                          C.byref(n), C.byref(st)))
+    del buf
+    return bytes(memoryview(store)[: n.value]), st.as_dict()
+
+
 def pass_unit(width: int, height: int, samples_per_px: int, max_depth: int, flags: int = _abi.FLAGS_MAIN,
               samples_per_unit: int = 0) -> int:
     """The pass unit an accumulation of these params reports (rtclj_ctx_accum_begin): 1 in strict order, else the
@@ -222,6 +244,17 @@ class Context:
         _abi.check(_abi.lib().rtclj_ctx_encode_ppm_p3(self._h, C.c_void_p(d_rgb8), int(width), int(height),
                                                       C.c_void_p(d_out or None), int(capacity), C.byref(n),
                                                       C.c_void_p(stream or None)))
+        return n.value
+
+    def encode_png(self, d_rgb8: int, width: int, height: int, d_out: int = 0, capacity: int = 0,
+                   stream: int = 0) -> int:
+        """The compressed PNG writer (rtclj_ctx_encode_png) on device pointers: d_rgb8 -> PNG at d_out.  d_out = 0
+        is the sizing call (a sufficient capacity, no GPU work).  Returns the PNG length in bytes; synchronises
+        `stream`."""
+        n = C.c_size_t()
+        _abi.check(_abi.lib().rtclj_ctx_encode_png(self._h, C.c_void_p(d_rgb8), int(width), int(height),
+                                                   C.c_void_p(d_out or None), int(capacity), C.byref(n),
+                                                   C.c_void_p(stream or None)))
         return n.value
 
     def encode_ms(self) -> tuple:
@@ -356,10 +389,14 @@ def encode_ppm(rgb8: np.ndarray, device: int | None = None) -> bytes:
     return _two_call(lib.rtclj_encode_ppm_p3_gpu, img, int(device))
 
 
-def encode_png(rgb8: np.ndarray) -> bytes:
-    """The PNG `ppm->png` writes next to the PPM (raytracing.clj:176)."""
+def encode_png(rgb8: np.ndarray, device: int | None = None) -> bytes:
+    """The PNG `ppm->png` writes next to the PPM (raytracing.clj:176).
+    device = None: the host writer (stored deflate blocks); device = k: the compressed PNG writer on GPU k
+    (rtclj_encode_png_gpu: filtered rows, run-length deflate, DESIGN.md section 4.11)."""
     img = np.ascontiguousarray(rgb8, dtype=np.uint8)
-    return _two_call(_abi.lib().rtclj_encode_png, img)
+    if device is None:
+        return _two_call(_abi.lib().rtclj_encode_png, img)
+    return _two_call(_abi.lib().rtclj_encode_png_gpu, img, int(device))
 
 
 def decode_ppm(text: bytes) -> np.ndarray:
@@ -380,9 +417,9 @@ def ppm_to_png(source: str, dest: str) -> None:
     print(f"Processed {source} into {dest}")
 
 
-def write_png(path: str, rgb8: np.ndarray) -> None:
+def write_png(path: str, rgb8: np.ndarray, device: int | None = None) -> None:
     with open(path, "wb") as f:
-        f.write(encode_png(rgb8))
+        f.write(encode_png(rgb8, device))
 
 
 def write_ppm(path: str, rgb8: np.ndarray, device: int | None = None) -> None:
