@@ -16,6 +16,8 @@
  *                           several GPUs in, the text of scene.ppm out
  *   rtclj_ctx_*             the same loop with device-resident buffers (scene upload
  *                           once, many renders; what bench.py times as `value`)
+ *   rtclj_ctx_render_frames, rtclj_render_frames
+ *                           the same loop for a sequence of cameras (one scene), every frame in shared launches
  *   rtclj_ctx_accum_*, rtclj_progressive_*
  *                           the same loop run in passes of samples (progressive rendering),
  *                           bit-identical to a one-shot render after every pass
@@ -238,8 +240,35 @@ int rtclj_ctx_set_scene(rtclj_ctx *ctx, const rtclj_scene *scene);
  * carries its cull table with it (kernel parameters), the library holds no per-device state. */
 int rtclj_ctx_render(rtclj_ctx *ctx, const rtclj_camera *camera, const rtclj_params *params,
                      void *d_out_linear, void *d_out_rgb8, void *stream);
-/* Synchronises `stream` and reads the counters of the last rtclj_ctx_render (or accumulation pass). */
+/* Synchronises `stream` and reads the counters of the last rtclj_ctx_render (or accumulation pass, or sequence). */
 int rtclj_ctx_stats(rtclj_ctx *ctx, void *stream, rtclj_stats *stats);
+
+/* ---- Camera sequences: n_frames frames of one scene (a turntable, a fly-through, a focus pull) in shared launches --
+ * one ticket queue and one kernel tail per launch instead of one per frame (DESIGN.md section 4.12).
+ *   - A sequence is one scene, one rtclj_params and n_frames >= 1 cameras of equal width x height; defocus angles may
+ *     differ between frames, with and without the disk in one sequence.
+ *   - Frame f's images (linear and 8-bit) are bit-identical to rtclj_ctx_render with cameras[f] and the same params,
+ *     for every kernel choice, device list, shard_* setting and frame count.  The seed is shared by all frames (per-frame
+ *     seeds: one call per frame).
+ *   - The output buffers hold n_frames consecutive full-size images, frame stride W*H*3 values; a sharded call writes
+ *     only its own rows of each frame.  Either buffer may be NULL.
+ *   - Every camera passes the checks of rtclj_ctx_render before anything runs; otherwise RTCLJ_E_INVALID with a message
+ *     naming the frame, and nothing is written.  RTCLJ_E_INVALID as well: n_frames <= 0, a null camera array, sizes that
+ *     differ between frames, RTCLJ_F_WAVE_KERNEL or RTCLJ_F_SPLIT_KERNEL.  max_depth <= 0 renders black frames.
+ *   - Stats (rtclj_ctx_stats after rtclj_ctx_render_frames, or the stats of rtclj_render_frames) cover the whole call:
+ *     counters summed over the frames; samples_per_unit is the one every frame used.
+ *   - A launch takes at most 128 frames (their cameras travel as kernel parameters), at most 2 GiB of scratch (unit
+ *     sums, or per-sample colours in strict order) and fewer than 2^32 work units; longer sequences take several
+ *     launches, and a frame that alone needs more scratch renders exactly as rtclj_ctx_render renders it. */
+/* Device-resident, like rtclj_ctx_render: enqueues on `stream` without synchronising, honours shard_*; one context
+ * serves one stream at a time.  d_out_linear / d_out_rgb8 are DEVICE pointers to n_frames full-size images. */
+int rtclj_ctx_render_frames(rtclj_ctx *ctx, const rtclj_camera *cameras, int32_t n_frames,
+                            const rtclj_params *params, void *d_out_linear, void *d_out_rgb8, void *stream);
+/* Host buffers, like rtclj_render_multi: rows interleaved over `n_devices` GPUs (tiles of params->shard_rows rows,
+ * <= 0: 1), one worker per device renders its rows of every frame; out_linear / out_rgb8 hold n_frames images. */
+int rtclj_render_frames(const rtclj_scene *scene, const rtclj_camera *cameras, int32_t n_frames,
+                        const rtclj_params *params, const int32_t *devices, int32_t n_devices,
+                        double *out_linear, uint8_t *out_rgb8, rtclj_stats *stats);
 
 /* ---- Progressive rendering: the compute-pixel loop (src/raytracing.clj:141-171) run in passes, so that
  * an image can be shown while it refines, stopped early or extended without tracing its samples again.

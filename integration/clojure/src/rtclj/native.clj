@@ -47,6 +47,13 @@
   (downcall "rtclj_render_multi"
             (fd-int ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS
                     ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS)))
+;; int rtclj_render_frames(const rtclj_scene*, const rtclj_camera* cameras, int32_t n_frames,
+;;                         const rtclj_params*, const int32_t* devices, int32_t n_devices,
+;;                         double* out_linear, uint8_t* out_rgb8, rtclj_stats*)
+(def ^:private rtclj-render-frames
+  (downcall "rtclj_render_frames"
+            (fd-int ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/ADDRESS
+                    ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS)))
 ;; int rtclj_render_multi_ppm(const rtclj_scene*, const rtclj_camera*, const rtclj_params*,
 ;;                            const int32_t* devices, int32_t n_devices,
 ;;                            char* out, size_t capacity, size_t* len, rtclj_stats*)
@@ -94,6 +101,20 @@
         ^MemorySegment p (.reinterpret (.get slot ValueLayout/ADDRESS 0) (* 8 n-doubles))]
     [p #(.invokeWithArguments rtclj-host-free [p])]))
 
+(defn- fill-camera!
+  "Writes the camera map `cam` (see `render`) into the rtclj_camera at `camera`."
+  [^MemorySegment camera cam]
+  (let [put3 (fn [field ^doubles v]
+               (dotimes [k 3]
+                 (.set camera ValueLayout/JAVA_DOUBLE (+ (off :rtclj_camera field) (* 8 k)) (aget v k))))]
+    (put3 :pixel00 (:pixel-00-loc cam)) (put3 :pixel_du (:pixel-du cam))
+    (put3 :pixel_dv (:pixel-dv cam)) (put3 :center (:camera-center cam))
+    (put3 :defocus_u (:defocus-disk-u cam)) (put3 :defocus_v (:defocus-disk-v cam))
+    (.set camera ValueLayout/JAVA_DOUBLE (off :rtclj_camera :defocus_angle) (double (:defocus-angle cam)))
+    (.set camera ValueLayout/JAVA_INT (off :rtclj_camera :width) (int (:image-width cam)))
+    (.set camera ValueLayout/JAVA_INT (off :rtclj_camera :height) (int (:image-height cam)))
+    camera))
+
 (defn- marshal
   "Fills rtclj_scene / rtclj_camera / rtclj_params in arena `a`; returns [scene camera params]."
   [^Arena a bodies cam samples-per-px max-depth {:keys [seed flags device samples-per-unit]
@@ -107,16 +128,7 @@
                  (.set ValueLayout/ADDRESS (off :rtclj_scene :albedo_rgb) (doubles-seg a (mapcat :rtclj/albedo bodies)))
                  (.set ValueLayout/ADDRESS (off :rtclj_scene :fuzz) (doubles-seg a (map :rtclj/fuzz bodies)))
                  (.set ValueLayout/ADDRESS (off :rtclj_scene :ior) (doubles-seg a (map :rtclj/ior bodies))))
-        camera (.allocate a (size :rtclj_camera) 8)
-        put3   (fn [field ^doubles v]
-                 (dotimes [k 3]
-                   (.set camera ValueLayout/JAVA_DOUBLE (+ (off :rtclj_camera field) (* 8 k)) (aget v k))))
-        _      (do (put3 :pixel00 (:pixel-00-loc cam)) (put3 :pixel_du (:pixel-du cam))
-                   (put3 :pixel_dv (:pixel-dv cam)) (put3 :center (:camera-center cam))
-                   (put3 :defocus_u (:defocus-disk-u cam)) (put3 :defocus_v (:defocus-disk-v cam))
-                   (.set camera ValueLayout/JAVA_DOUBLE (off :rtclj_camera :defocus_angle) (double (:defocus-angle cam)))
-                   (.set camera ValueLayout/JAVA_INT (off :rtclj_camera :width) (int (:image-width cam)))
-                   (.set camera ValueLayout/JAVA_INT (off :rtclj_camera :height) (int (:image-height cam))))
+        camera (fill-camera! (.allocate a (size :rtclj_camera) 8) cam)
         params (doto (.allocate a (size :rtclj_params) 8)
                  (.set ValueLayout/JAVA_INT (off :rtclj_params :spp) (int samples-per-px))
                  (.set ValueLayout/JAVA_INT (off :rtclj_params :max_depth) (int max-depth))
@@ -161,6 +173,38 @@
                                (.getAtIndex out ValueLayout/JAVA_DOUBLE (+ 1 (* 3 p)))
                                (.getAtIndex out ValueLayout/JAVA_DOUBLE (+ 2 (* 3 p)))]))
               (range (* w h)))
+        (finally (free!))))))
+
+(defn render-frames
+  "A camera sequence of one scene (rtclj_render_frames): `cams` is a seq of camera maps (see `render`) of one image
+   size -- a turntable, a fly-through, a focus pull.  All frames share the GPU launches (one kernel tail per launch
+   instead of one per frame); frame f is bit-identical to (render bodies (nth cams f) ...) with the same options,
+   which `render` takes as well (:devices, :seed, :flags, :samples-per-unit).  One seed for every frame.  Returns a
+   vector with one frame per camera, each frame what `render` returns."
+  [bodies cams samples-per-px max-depth & {:keys [devices] :or {devices [0]} :as opts}]
+  (with-open [a (Arena/ofConfined)]
+    (let [cam0    (first cams)
+          w       (long (:image-width cam0))
+          h       (long (:image-height cam0))
+          k       (count cams)
+          [scene _ params] (marshal a bodies cam0 samples-per-px max-depth opts)
+          cameras (.allocate a (* k (size :rtclj_camera)) 8)
+          _       (doseq [[i cam] (map-indexed vector cams)]
+                    (fill-camera! (.asSlice cameras (* i (size :rtclj_camera)) (size :rtclj_camera)) cam))
+          [^MemorySegment out free!] (pinned-doubles a (* 3 w h k))]
+      (try
+        (check! (.invokeWithArguments rtclj-render-frames
+                                      [scene cameras (int k) params
+                                       (.allocateFrom a ValueLayout/JAVA_INT (int-array devices)) (int (count devices))
+                                       out MemorySegment/NULL MemorySegment/NULL]))
+        (mapv (fn [^long f]
+                (mapv (fn [^long p]
+                        (let [q (* 3 (+ p (* f w h)))]
+                          (double-array [(.getAtIndex out ValueLayout/JAVA_DOUBLE q)
+                                         (.getAtIndex out ValueLayout/JAVA_DOUBLE (+ 1 q))
+                                         (.getAtIndex out ValueLayout/JAVA_DOUBLE (+ 2 q))])))
+                      (range (* w h))))
+              (range k))
         (finally (free!))))))
 
 (defn render-ppm!

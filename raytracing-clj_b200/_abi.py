@@ -72,6 +72,10 @@ SYMBOLS = {
     "rtclj_ctx_render": (C.c_int, [C.c_void_p, C.POINTER(Camera), C.POINTER(Params), C.c_void_p,
                                    C.c_void_p, C.c_void_p]),
     "rtclj_ctx_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
+    "rtclj_ctx_render_frames": (C.c_int, [C.c_void_p, C.POINTER(Camera), C.c_int32, C.POINTER(Params), C.c_void_p,
+                                          C.c_void_p, C.c_void_p]),
+    "rtclj_render_frames": (C.c_int, [C.POINTER(Scene), C.POINTER(Camera), C.c_int32, C.POINTER(Params),
+                                      C.POINTER(C.c_int32), C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(Stats)]),
     "rtclj_ctx_accum_begin": (C.c_int, [C.c_void_p, C.POINTER(Camera), C.POINTER(Params), C.POINTER(C.c_int32),
                                         C.c_void_p]),
     "rtclj_ctx_accum_step": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32),

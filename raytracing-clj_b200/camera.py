@@ -134,6 +134,23 @@ def main_camera(
     )
 
 
+def turntable_look_from(k: int, n: int, look_from: Sequence[float] = (-2.0, 2.0, 1.0),
+                        look_at: Sequence[float] = (0.0, 0.0, -1.0)) -> tuple:
+    """look_from rotated by k * 360/n degrees about the vertical axis through look_at (frame k of an n-frame
+    turntable); k = 0 is look_from itself."""
+    look_from, look_at = tuple(map(float, look_from)), tuple(map(float, look_at))
+    if k % n == 0:
+        return look_from
+    a = 2.0 * math.pi * k / n
+    dx, dz = look_from[0] - look_at[0], look_from[2] - look_at[2]
+    return (look_at[0] + dx * math.cos(a) + dz * math.sin(a), look_from[1], look_at[2] - dx * math.sin(a) + dz * math.cos(a))
+
+
+def turntable_cameras(n: int, width: int = 400, height: int | None = None) -> list:
+    """The reference's main camera on an n-frame turntable around its look_at: frame 0 is main_camera()."""
+    return [main_camera(width, height, look_from=turntable_look_from(k, n)) for k in range(n)]
+
+
 def realm_camera(
     width: int = 400,
     height: int | None = None,

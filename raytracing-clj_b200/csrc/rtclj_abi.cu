@@ -82,6 +82,7 @@ struct rtclj_ctx {
   DevBuf<double> sample_buf;            // strict order on long paths: one colour per sample (kept between renders)
   std::vector<float> ctab_host;         // the cull table of a small scene: launched as a kernel parameter
   KParams kparams;                      // launch parameters of the last render (8.4 KB with the table)
+  FrameKParams fparams;                 // launch parameters of the last camera-sequence launch (28 KB)
   DevBuf<double> out_linear;            // used by the host-buffer entry points
   DevBuf<unsigned char> out_rgb8;
   DevBuf<unsigned long long> p3_state;  // P3 writer: ticket, total, text bytes per CTA run
@@ -214,13 +215,27 @@ const KernelFn kPrimaryFns[2][2][2] = {
     {{render_primary_listed_kernel<false>, render_primary_listed_kernel<true>},
      {render_primary_seeded_listed_kernel<false>, render_primary_seeded_listed_kernel<true>}}};
 
+// The frame twins of a camera sequence (FrameKParams), one per instantiation the library can choose for it:
+// render_frames_kernel [const_tab][sample_buf][packed] as kRenderFns[0], render_lane2_frames_kernel [sample_buf],
+// render_primary_frames_kernel [some frame has the defocus disk].  (The wave and split kernels render no sequences.)
+using FramesFn = void (*)(FrameKParams);
+const FramesFn kRenderFramesFns[2][2][2] = {
+    {{render_frames_kernel<false, false, false>, nullptr}, {render_frames_kernel<false, true, false>, nullptr}},
+    {{render_frames_kernel<true, false, false>, render_frames_kernel<true, false, true>},
+     {render_frames_kernel<true, true, false>, render_frames_kernel<true, true, true>}}};
+const FramesFn kLane2FramesFns[2] = {render_lane2_frames_kernel<false>, render_lane2_frames_kernel<true>};
+const FramesFn kPrimaryFramesFns[2] = {render_primary_frames_kernel<false>, render_primary_frames_kernel<true>};
+
 // the tables of kernels with dynamic shared memory, and the most a launch asks for (0: the device's opt-in limit)
-struct SmemLimit { const KernelFn* fns; size_t count; size_t bytes; };
-const SmemLimit kSmemLimits[] = {
+template <class Fn> struct SmemLimit { const Fn* fns; size_t count; size_t bytes; };
+const SmemLimit<KernelFn> kSmemLimits[] = {
     {&kRenderFns[0][0][0][0], sizeof kRenderFns / sizeof(KernelFn), 0},
     {&kLane2Fns[0][0], sizeof kLane2Fns / sizeof(KernelFn), Lane2Smem::total},
     {kSplitFns, sizeof kSplitFns / sizeof(KernelFn), SplitSmem::total},
     {kWaveFns, sizeof kWaveFns / sizeof(KernelFn), WaveSmem::total}};
+const SmemLimit<FramesFn> kFramesSmemLimits[] = {
+    {&kRenderFramesFns[0][0][0], sizeof kRenderFramesFns / sizeof(FramesFn), 0},
+    {kLane2FramesFns, sizeof kLane2FramesFns / sizeof(FramesFn), Lane2Smem::total}};
 
 }  // namespace
 
@@ -306,7 +321,11 @@ int rtclj_ctx_create(int32_t device, rtclj_ctx** out) {
   CU(cudaEventCreateWithFlags(&c->pin_ev[1], cudaEventDisableTiming));
   CU(cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking));
   CU(c->counters.reserve(8));
-  for (const SmemLimit& t : kSmemLimits)
+  for (const SmemLimit<KernelFn>& t : kSmemLimits)
+    for (size_t i = 0; i < t.count; ++i)
+      if (t.fns[i])
+        CU(cudaFuncSetAttribute(t.fns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(t.bytes ? t.bytes : c->smem_optin)));
+  for (const SmemLimit<FramesFn>& t : kFramesSmemLimits)
     for (size_t i = 0; i < t.count; ++i)
       if (t.fns[i])
         CU(cudaFuncSetAttribute(t.fns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(t.bytes ? t.bytes : c->smem_optin)));
@@ -526,6 +545,10 @@ struct Pass {
   bool decide = true;            // listed: the last launch of the pass applies the stopping rule and relists
   double* out_linear = nullptr;
   unsigned char* out_rgb8 = nullptr;
+  // a camera sequence: the launch traces the units of frames[0 .. n_frames) (frame twins, FrameKParams), and the
+  // images above hold n_frames full-size frames.  n_frames = 0: the single camera of launch_pass.
+  const rtclj_camera* frames = nullptr;
+  int n_frames = 0;
 };
 
 // the fold and stopping rule of an adaptive accumulation's pass, shard `sh` (finalize_adaptive_kernel)
@@ -551,7 +574,8 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
                 const Pass& ps, cudaStream_t stream) {
   const int grid = c->sm_count;
   const int nchunks = (ps.samples + ps.spu - 1) / ps.spu;
-  const unsigned long long total_units = sh.local_pixels * (unsigned long long)nchunks;
+  const int nframes = ps.n_frames > 0 ? ps.n_frames : 1;
+  const unsigned long long total_units = sh.local_pixels * (unsigned long long)nchunks * (unsigned long long)nframes;
   if (total_units > 0xffffffffull) {
     return fail(RTCLJ_E_INVALID, "%llu work units: raise samples_per_unit", total_units);
   }
@@ -585,13 +609,16 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
     P.nchunks = nchunks; P.spu = ps.spu; P.sample_base = ps.sample_base; P.total_units = total_units;
     P.geom32 = c->geom32.p; P.geomA = c->geomA.p; P.geom64 = c->geom64.p; P.mat = c->mat.p;
     P.partial = c->partial.p; P.acc = ps.acc; P.queue = c->counters.p; P.stats = c->counters.p + 1;
-    P.sample_buf = ps.sample_buf; P.sample_stride = sh.local_pixels;
+    P.sample_buf = ps.sample_buf; P.sample_stride = sh.local_pixels * (unsigned long long)nframes;
     P.list = ps.listed ? c->list.p : nullptr; P.list_count = ps.listed ? c->list_aux.p : nullptr;
     P.acc2 = ps.listed ? c->acc2.p : nullptr;
     const bool const_tab = ch.kernel != Kernel::render_smem, sample_buf = ps.sample_buf != nullptr;
     if (const_tab && !c->ctab_host.empty())
       std::memcpy(P.ctab, c->ctab_host.data(), std::min(sizeof P.ctab, c->ctab_host.size() * sizeof(float)));
     KernelFn fn = nullptr;
+    FramesFn frames_fn = nullptr;
+    bool any_defocus = false;  // a sequence: some frame has the defocus disk
+    for (int f = 0; f < ps.n_frames; ++f) any_defocus = any_defocus || !(ps.frames[f].defocus_angle <= 0.0);
     unsigned blocks = (unsigned)grid, paths = 0;  // paths in flight per CTA: the rows of the attenuation stack
     int threads = 0;
     size_t sm = 0;
@@ -602,6 +629,7 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
         const unsigned long long want = (total_units + kPrimaryThreads - 1) / kPrimaryThreads;
         blocks = (unsigned)std::min<unsigned long long>(want, (unsigned long long)grid * (unsigned long long)(2048 / kPrimaryThreads));
         fn = kPrimaryFns[ps.listed][ps.seeded][P.use_defocus]; threads = kPrimaryThreads; stack = false;
+        frames_fn = kPrimaryFramesFns[any_defocus];
         break;
       }
       case Kernel::wave:
@@ -618,10 +646,12 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
         break;
       case Kernel::lane2:
         fn = kLane2Fns[ps.listed][sample_buf]; threads = kT2; sm = Lane2Smem::total; paths = 2u * kT2;
+        frames_fn = kLane2FramesFns[sample_buf];
         break;
       default:  // render_kernel
         fn = kRenderFns[ps.listed][const_tab][sample_buf][ch.packed]; threads = threads_of(const_tab, ch.packed);
         sm = smem_needed(c->nhalf, const_tab, c->smem_optin, ch.packed); paths = (unsigned)threads;
+        frames_fn = kRenderFramesFns[const_tab][sample_buf][ch.packed];
         stack = prm->flags & RTCLJ_F_REVERSE_PRODUCT;
     }
     P.stack_stride = (unsigned)grid * paths;
@@ -637,7 +667,26 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
       P.arrive = c->arrive.p;
     }
 #endif
-    fn<<<blocks, threads, sm, stream>>>(P);
+    if (ps.n_frames > 0) {
+      if (!frames_fn) return fail(RTCLJ_E_INVALID, "this kernel renders no camera sequences");
+      FrameKParams& F = c->fparams;
+      F.P = P;
+      F.frame_pixels = (unsigned)sh.local_pixels;
+      F.frame_units = (unsigned)(sh.local_pixels * (unsigned long long)nchunks);
+      for (int f = 0; f < ps.n_frames; ++f) {  // the fields launch_pass sets from a camera, in the same way
+        const rtclj_camera& fc = ps.frames[f];
+        FrameCam& fr = F.cam[f];
+        for (int a = 0; a < 3; ++a) {
+          fr.p00[a] = fc.pixel00[a]; fr.du[a] = fc.pixel_du[a]; fr.dv[a] = fc.pixel_dv[a];
+          fr.center[a] = fc.center[a]; fr.ddu[a] = fc.defocus_u[a]; fr.ddv[a] = fc.defocus_v[a];
+        }
+        fr.use_defocus = !(fc.defocus_angle <= 0.0);
+        fr.pad = 0;
+      }
+      frames_fn<<<blocks, threads, sm, stream>>>(F);
+    } else {
+      fn<<<blocks, threads, sm, stream>>>(P);
+    }
 #ifdef RTCLJ_TAIL_PROBE
     if (const char* path = std::getenv("RTCLJ_TAIL_PROBE_FILE"); path && ch.kernel == Kernel::lane2) {
       std::vector<unsigned> host(probe_words);
@@ -661,19 +710,72 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
       if (rc) return rc;
     }
   } else if (ps.finalize) {
-    FParams F;
-    F.sample_buf = ps.sample_buf; F.sample_stride = sh.local_pixels;
-    F.partial = c->partial.p; F.out_linear = ps.out_linear; F.out_rgb8 = ps.out_rgb8;
-    F.W = cam->width; F.spp = ps.samples; F.nchunks = nchunks;
-    F.shard_index = sh.index; F.shard_count = sh.count; F.shard_rows = sh.rows;
-    F.flags = prm->flags; F.local_pixels = sh.local_pixels;
-    F.acc = ps.acc; F.seeded = ps.seeded; F.mean_n = ps.mean_n;
-    const unsigned blocks = (unsigned)((sh.local_pixels + 255) / 256);
-    finalize_kernel<<<blocks, 256, 0, stream>>>(F);
-    CU(cudaGetLastError());
+    // one finalize_kernel per frame, on that frame's unit sums / sample colours and full-size images
+    const size_t frame_values = (size_t)cam->width * (size_t)cam->height * 3u;
+    for (int f = 0; f < nframes; ++f) {
+      FParams F;
+      F.sample_buf = ps.sample_buf ? ps.sample_buf + (size_t)f * sh.local_pixels * 4u : nullptr;
+      F.sample_stride = sh.local_pixels * (unsigned long long)nframes;
+      F.partial = c->partial.p + (size_t)f * sh.local_pixels * (size_t)nchunks * 3u;
+      F.out_linear = ps.out_linear ? ps.out_linear + (size_t)f * frame_values : nullptr;
+      F.out_rgb8 = ps.out_rgb8 ? ps.out_rgb8 + (size_t)f * frame_values : nullptr;
+      F.W = cam->width; F.spp = ps.samples; F.nchunks = nchunks;
+      F.shard_index = sh.index; F.shard_count = sh.count; F.shard_rows = sh.rows;
+      F.flags = prm->flags; F.local_pixels = sh.local_pixels;
+      F.acc = ps.acc; F.seeded = ps.seeded; F.mean_n = ps.mean_n;
+      const unsigned blocks = (unsigned)((sh.local_pixels + 255) / 256);
+      finalize_kernel<<<blocks, 256, 0, stream>>>(F);
+      CU(cudaGetLastError());
+    }
   }
   CU(cudaEventRecord(c->ev2, stream));
   c->render_pending = true;
+  return RTCLJ_OK;
+}
+
+// The strict order of the general kernels goes through sample_buf (32 B per pixel and sample); an
+// accumulation's pass that needs more is cut into sub-passes of at most this many bytes, each followed by its
+// fold, and a camera sequence groups no more frames into one launch than this buffer -- or their unit sums -- holds.
+// A one-shot strict render of 1920x1080 x 500 spp holds 33 GB; a strict accumulation or sequence never more than this.
+constexpr size_t kAccumSampleBufBytes = (size_t)2 << 30;
+
+// The strict order on long paths: one 500-sample unit lasts as long as its pixel's paths, the last ones run alone
+// (measured: 622 vs 543 ms on one GPU, 162 vs 72 ms per GPU on eight).  Instead the samples are traced in small units
+// and each sample's colour is STORED (32 B); finalize_kernel then adds them in sample order -- the same additions in
+// the same order.  33 GB at 1920x1080 x 500 spp; HBM has 180 GB.  Returns the buffer of `need` doubles for a render
+// that wants it (nullptr if it does not fit: one unit per pixel then); a render that does not gives a large one back.
+double* strict_sample_buf(rtclj_ctx* c, bool wanted, size_t need) {
+  if (wanted) {
+    size_t free_b = 0, total_b = 0;
+    // kept in the context between renders (allocating 33 GB per frame costs more than the frame)
+    if (need <= c->sample_buf.cap ||
+        (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need * 8 < (free_b + c->sample_buf.cap * 8) / 2 &&
+         c->sample_buf.reserve(need) == cudaSuccess))
+      return c->sample_buf.p;
+    cudaGetLastError();  // too large: fall back to one unit per pixel
+  } else if (c->sample_buf.cap * 8 > ((size_t)1 << 30)) {
+    c->sample_buf.release();  // (synchronises the device; only on a strict -> chunked change of mode)
+  }
+  return nullptr;
+}
+
+// The checks of a camera sequence, before any device is touched: frame f fails validate() under its own number
+int check_frames(const rtclj_camera* cams, int32_t n_frames, const rtclj_params* prm) {
+  if (n_frames <= 0) return fail(RTCLJ_E_INVALID, "n_frames must be positive, got %d", n_frames);
+  if (!cams) return fail(RTCLJ_E_INVALID, "null camera array");
+  if (!prm) return fail(RTCLJ_E_INVALID, "null params");
+  if (prm->flags & (RTCLJ_F_WAVE_KERNEL | RTCLJ_F_SPLIT_KERNEL))
+    return fail(RTCLJ_E_INVALID, "the wavefront and split kernels do not render camera sequences");
+  for (int f = 0; f < n_frames; ++f) {
+    if (validate(&cams[f], prm)) {
+      char why[256];
+      std::snprintf(why, sizeof why, "%s", rtclj_error_get());
+      return fail(RTCLJ_E_INVALID, "frame %d: %s", f, why);
+    }
+    if (cams[f].width != cams[0].width || cams[f].height != cams[0].height)
+      return fail(RTCLJ_E_INVALID, "frame %d is %dx%d, frame 0 %dx%d: a sequence has one image size", f, cams[f].width,
+                  cams[f].height, cams[0].width, cams[0].height);
+  }
   return RTCLJ_OK;
 }
 
@@ -702,32 +804,66 @@ int rtclj_ctx_render(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* 
                                       : (ch.primary_only ? prm->spp : auto_samples_per_unit(W, H, prm->spp));
   if (spu > prm->spp) spu = prm->spp;
   c->last_spu = spu;
-  // The strict order on long paths: one 500-sample unit lasts as long as its pixel's paths, the last ones
-  // run alone (measured: 622 vs 543 ms on one GPU, 162 vs 72 ms per GPU on eight).  Instead the samples are
-  // traced in small units and each sample's colour is STORED (32 B); finalize_kernel then adds them in
-  // sample order -- the same additions in the same order.  33 GB at 1920x1080 x 500 spp; HBM has 180 GB.
-  double* sample_buf = nullptr;
-  if (spu == prm->spp && !ch.primary_only && prm->spp >= 64 && ch.sample_buf_ok && want_out && sh.local_pixels > 0) {
-    const size_t need = (size_t)sh.local_pixels * (size_t)prm->spp * 4u;  // doubles
-    size_t free_b = 0, total_b = 0;
-    // kept in the context between renders (allocating 33 GB per frame costs more than the frame); a render
-    // that does not need it gives a large one back (below)
-    if (need <= c->sample_buf.cap ||
-        (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && need * 8 < (free_b + c->sample_buf.cap * 8) / 2 &&
-         c->sample_buf.reserve(need) == cudaSuccess)) {
-      sample_buf = c->sample_buf.p;
-      spu = auto_samples_per_unit(W, H, prm->spp);  // scheduling units; the arithmetic stays strict
-    } else {
-      cudaGetLastError();  // too large: fall back to one unit per pixel
-    }
-  } else if (c->sample_buf.cap * 8 > ((size_t)1 << 30)) {
-    c->sample_buf.release();  // (synchronises the device; only on a strict -> chunked change of mode)
-  }
+  const bool strict_long = spu == prm->spp && !ch.primary_only && prm->spp >= 64 && ch.sample_buf_ok && want_out &&
+                           sh.local_pixels > 0;
+  double* sample_buf = strict_sample_buf(c, strict_long, (size_t)sh.local_pixels * (size_t)prm->spp * 4u);
+  if (sample_buf) spu = auto_samples_per_unit(W, H, prm->spp);  // scheduling units; the arithmetic stays strict
   Pass ps;
   ps.samples = prm->spp; ps.spu = spu; ps.sample_buf = sample_buf; ps.mean_n = prm->spp;
   ps.finalize = !ch.finishes && want_out;
   ps.out_linear = (double*)d_out_linear; ps.out_rgb8 = (unsigned char*)d_out_rgb8;
   return launch_pass(c, cam, prm, ch, sh, ps, stream);
+}
+
+// A camera sequence (DESIGN.md section 4.12): the frames share launches -- one ticket queue, one tail -- in groups
+// whose scratch (unit sums, or sample colours in strict order) stays within kAccumSampleBufBytes, whose units stay
+// below 2^32 and whose cameras fit the kernel parameters (kMaxFrames).  The summation unit and the strict-order
+// decision are the single frame's, so frame f is bit-identical to rtclj_ctx_render with cameras[f]; a frame that
+// alone needs more scratch runs as a group of one under rtclj_ctx_render's rules.
+int rtclj_ctx_render_frames(rtclj_ctx* c, const rtclj_camera* cams, int32_t n_frames, const rtclj_params* prm,
+                            void* d_out_linear, void* d_out_rgb8, void* stream_) {
+  if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
+  if (!c->have_scene) return fail(RTCLJ_E_INVALID, "rtclj_ctx_set_scene has not been called");
+  int rc = check_frames(cams, n_frames, prm);
+  if (rc) return rc;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  CU(cudaSetDevice(c->device));
+
+  const int W = cams[0].width, H = cams[0].height;
+  const Shard sh = shard_of(&cams[0], prm);
+  const bool want_out = d_out_linear || d_out_rgb8;
+  // every kernel gives the same bits: the choice may see the whole batch
+  const KernelChoice ch = choose_kernel(c, prm, (double)n_frames * (double)sh.local_pixels * (double)prm->spp);
+  // the summation unit of ONE frame, as rtclj_ctx_render computes it
+  int spu = prm->samples_per_unit > 0 ? prm->samples_per_unit
+                                      : (ch.primary_only ? prm->spp : auto_samples_per_unit(W, H, prm->spp));
+  if (spu > prm->spp) spu = prm->spp;
+  c->last_spu = spu;
+  const bool strict_long = spu == prm->spp && !ch.primary_only && prm->spp >= 64 && ch.sample_buf_ok && want_out &&
+                           sh.local_pixels > 0;
+  const int sched_spu = strict_long ? auto_samples_per_unit(W, H, prm->spp) : spu;
+  const unsigned long long frame_units =
+      sh.local_pixels * (unsigned long long)((prm->spp + sched_spu - 1) / sched_spu);
+  const unsigned long long frame_bytes = strict_long ? sh.local_pixels * (unsigned long long)prm->spp * 32ull
+                                                     : frame_units * 24ull;
+  unsigned long long group = std::min<unsigned long long>((unsigned long long)n_frames, kMaxFrames);
+  if (frame_bytes > 0) group = std::min(group, std::max(1ull, kAccumSampleBufBytes / frame_bytes));
+  if (frame_units > 0) group = std::min(group, std::max(1ull, 0xffffffffull / frame_units));
+  const size_t frame_values = (size_t)W * (size_t)H * 3u;
+  for (int f0 = 0; f0 < n_frames; f0 += (int)group) {
+    const int g = std::min((int)group, n_frames - f0);
+    double* sample_buf = strict_sample_buf(c, strict_long, (size_t)g * (size_t)sh.local_pixels * (size_t)prm->spp * 4u);
+    Pass ps;
+    ps.samples = prm->spp; ps.spu = sample_buf ? sched_spu : spu; ps.sample_buf = sample_buf; ps.mean_n = prm->spp;
+    ps.first = f0 == 0;
+    ps.finalize = !ch.finishes && want_out;
+    ps.out_linear = d_out_linear ? (double*)d_out_linear + (size_t)f0 * frame_values : nullptr;
+    ps.out_rgb8 = d_out_rgb8 ? (unsigned char*)d_out_rgb8 + (size_t)f0 * frame_values : nullptr;
+    ps.frames = cams + f0; ps.n_frames = g;
+    rc = launch_pass(c, &cams[f0], prm, ch, sh, ps, stream);
+    if (rc) return rc;
+  }
+  return RTCLJ_OK;
 }
 
 int rtclj_ctx_stats(rtclj_ctx* c, void* stream_, rtclj_stats* st) {
@@ -827,19 +963,21 @@ int download_image(rtclj_ctx* c, const std::vector<Piece>& pieces, char* host, c
   return RTCLJ_OK;
 }
 
+// frame f of a camera sequence: the f-th full-size image of the device buffers and of the caller's
 int download_rows(rtclj_ctx* c, const rtclj_camera* cam, int shard_index, int shard_count, int shard_rows,
-                  double* out_linear, uint8_t* out_rgb8, cudaStream_t stream) {
+                  double* out_linear, uint8_t* out_rgb8, cudaStream_t stream, int frame = 0) {
   const size_t W = (size_t)cam->width, H = (size_t)cam->height;
+  const size_t frame_values = W * H * 3 * (size_t)frame;
   std::vector<Piece> pieces;
   if (out_linear) {
     plan_pieces(H, W * 3 * sizeof(double), shard_index, shard_count, shard_rows, kStageBytes, pieces);
-    int rc = download_image(c, pieces, (char*)out_linear, (const char*)c->out_linear.p, stream);
+    int rc = download_image(c, pieces, (char*)(out_linear + frame_values), (const char*)(c->out_linear.p + frame_values), stream);
     if (rc) return rc;
   }
   if (out_rgb8) {
     pieces.clear();
     plan_pieces(H, W * 3, shard_index, shard_count, shard_rows, kStageBytes, pieces);
-    int rc = download_image(c, pieces, (char*)out_rgb8, (const char*)c->out_rgb8.p, stream);
+    int rc = download_image(c, pieces, (char*)(out_rgb8 + frame_values), (const char*)(c->out_rgb8.p + frame_values), stream);
     if (rc) return rc;
   }
   return RTCLJ_OK;
@@ -872,9 +1010,10 @@ int cached_ctx(int device, std::unique_lock<std::mutex>& lock, rtclj_ctx** ctx) 
   return RTCLJ_OK;
 }
 
-// scene upload + render of one shard + download into the caller's images, on one device
+// scene upload + render of one shard + download into the caller's images, on one device.  n_frames > 0: the camera
+// sequence cam[0 .. n_frames) (rtclj_ctx_render_frames), the images hold n_frames frames
 int render_shard_hostbuf(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm, double* out_linear,
-                         uint8_t* out_rgb8, rtclj_stats* stats) {
+                         uint8_t* out_rgb8, rtclj_stats* stats, int n_frames = 0) {
   const auto t0 = std::chrono::steady_clock::now();
   std::unique_lock<std::mutex> lock;
   rtclj_ctx* c = nullptr;
@@ -882,13 +1021,18 @@ int render_shard_hostbuf(const rtclj_scene* scene, const rtclj_camera* cam, cons
   if (rc) return rc;
   rc = rtclj_ctx_set_scene(c, scene);
   if (rc) return rc;
-  const size_t npix = (size_t)cam->width * (size_t)cam->height;
-  if (out_linear) CU(c->out_linear.reserve(npix * 3));
-  if (out_rgb8) CU(c->out_rgb8.reserve(npix * 3));
-  rc = rtclj_ctx_render(c, cam, prm, out_linear ? c->out_linear.p : nullptr, out_rgb8 ? c->out_rgb8.p : nullptr, c->own_stream);
+  const size_t nimg = (size_t)cam->width * (size_t)cam->height * 3 * (size_t)std::max(n_frames, 1);
+  if (out_linear) CU(c->out_linear.reserve(nimg));
+  if (out_rgb8) CU(c->out_rgb8.reserve(nimg));
+  double* d_lin = out_linear ? c->out_linear.p : nullptr;
+  unsigned char* d_rgb = out_rgb8 ? c->out_rgb8.p : nullptr;
+  rc = n_frames > 0 ? rtclj_ctx_render_frames(c, cam, n_frames, prm, d_lin, d_rgb, c->own_stream)
+                    : rtclj_ctx_render(c, cam, prm, d_lin, d_rgb, c->own_stream);
   if (rc) return rc;
-  rc = download_rows(c, cam, prm->shard_index, prm->shard_count, prm->shard_rows, out_linear, out_rgb8, c->own_stream);
-  if (rc) return rc;
+  for (int f = 0; f < std::max(n_frames, 1); ++f) {
+    rc = download_rows(c, cam, prm->shard_index, prm->shard_count, prm->shard_rows, out_linear, out_rgb8, c->own_stream, f);
+    if (rc) return rc;
+  }
   rtclj_stats s;
   rc = rtclj_ctx_stats(c, c->own_stream, &s);  // synchronises the stream: the direct copies have landed
   if (rc) return rc;
@@ -1010,6 +1154,31 @@ int rtclj_render_multi(const rtclj_scene* scene, const rtclj_camera* cam, const 
   });
 }
 
+// A camera sequence on host buffers: rtclj_render_multi's rows and workers, each device renders its rows of every
+// frame with rtclj_ctx_render_frames and downloads them frame by frame.
+int rtclj_render_frames(const rtclj_scene* scene, const rtclj_camera* cams, int32_t n_frames, const rtclj_params* prm,
+                        const int32_t* devices, int32_t n_devices, double* out_linear, uint8_t* out_rgb8,
+                        rtclj_stats* stats) {
+  return guarded([&]() -> int {
+    const auto t0 = std::chrono::steady_clock::now();
+    if (!scene) return fail(RTCLJ_E_INVALID, "null scene");
+    int rc = check_frames(cams, n_frames, prm);
+    if (rc) return rc;
+    rc = check_devices(devices, n_devices);
+    if (rc) return rc;
+    std::vector<rtclj_stats> st((size_t)n_devices);
+    rc = run_on_devices(n_devices, [&](int d) {
+      const rtclj_params q = shard_params(prm, devices, d, n_devices);
+      return render_shard_hostbuf(scene, cams, &q, out_linear, out_rgb8, &st[(size_t)d], n_frames);
+    });
+    if (rc) return rc;
+    rtclj_stats total = sum_stats(st);
+    total.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = total;
+    return RTCLJ_OK;
+  });
+}
+
 int rtclj_render(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm, double* out_linear,
                  uint8_t* out_rgb8, rtclj_stats* stats) {
   return guarded([&]() -> int {
@@ -1025,11 +1194,6 @@ int rtclj_render(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_
 // ---------------------------------------------------------------- accumulation over passes
 // The compute-pixel loop (src/raytracing.clj:141-171) run in passes: a pass adds samples [d, d + n) of every
 // pixel to the pixel's running sum, in the order a one-shot render adds them (DESIGN.md section 4.9).
-
-// The strict order of the general kernels goes through sample_buf (32 B per pixel and sample); an
-// accumulation's pass that needs more is cut into sub-passes of at most this many bytes, each followed by its
-// fold.  A one-shot strict render of 1920x1080 x 500 spp holds 33 GB; a strict accumulation never more than this.
-constexpr size_t kAccumSampleBufBytes = (size_t)2 << 30;
 
 }  // extern "C"
 

@@ -33,9 +33,10 @@ struct Lane2Smem {
 };
 
 // kSampleBuf: strict order through the per-sample buffer, its own instantiation (rtclj_kernels.cuh); kListed: the
-// pixels of KParams::list only (render_lane2_listed_kernel)
-template <bool kSampleBuf, bool kListed>
-__device__ __forceinline__ void render_lane2_body(const KParams& P) {
+// pixels of KParams::list only (render_lane2_listed_kernel); kFrames: a camera sequence, P = FP->P
+// (render_lane2_frames_kernel)
+template <bool kSampleBuf, bool kListed, bool kFrames = false>
+__device__ __forceinline__ void render_lane2_body(const KParams& P, const FrameKParams* FP = nullptr) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int tid = threadIdx.x, lane = tid & 31;
   const unsigned gtid = blockIdx.x * kT2 + tid;
@@ -122,9 +123,9 @@ __device__ __forceinline__ void render_lane2_body(const KParams& P) {
 #pragma unroll 1
     for (int path = 0; path < 2; ++path) {
       const unsigned mask_shift = path ? 16u : 0u;
-      path_step<kSampleBuf, kT2, kListed>(P, pr, pc, path ? bany1 : bany0,
-                                          [&](int j) { return ~(my_mask[j * kT2] >> mask_shift) & 0xffffu; },
-                                          my_sums + path * 3 * kT2, (size_t)gtid * 2u + (size_t)path, lane, total_units);
+      path_step<kSampleBuf, kT2, kListed, kFrames>(P, pr, pc, path ? bany1 : bany0,
+                                                   [&](int j) { return ~(my_mask[j * kT2] >> mask_shift) & 0xffffu; },
+                                                   my_sums + path * 3 * kT2, (size_t)gtid * 2u + (size_t)path, lane, total_units, FP);
 
       // ---- swap: this path waits in shared memory while the other one is processed / both are culled
       {
@@ -169,6 +170,11 @@ __global__ void __launch_bounds__(kT2, 1) render_lane2_kernel(const __grid_const
 template <bool kSampleBuf>
 __global__ void __launch_bounds__(kT2, 1) render_lane2_listed_kernel(const __grid_constant__ KParams P) {
   render_lane2_body<kSampleBuf, true>(P);
+}
+
+template <bool kSampleBuf>
+__global__ void __launch_bounds__(kT2, 1) render_lane2_frames_kernel(const __grid_constant__ FrameKParams FP) {
+  render_lane2_body<kSampleBuf, false, true>(FP.P, &FP);
 }
 
 // (The same loop with ONE path per lane built on path_step() was measured against render_kernel<true>: equal on

@@ -44,10 +44,11 @@ struct PathCounters { unsigned samples, seg, exact, pref; };
 // survivors_of_block(j): the 16 survivor bits of block j (sphere s of the block -> bit 15 - s);
 // sums: the path's three unit sums, kSumStride doubles apart; stack_col: its column of the attenuation stack.
 // kListed: tickets go to the pixels of KParams::list, `total_units` of them (total_units_of, read once per kernel).
-template <bool kSampleBuf, int kSumStride, bool kListed = false, class SurvivorsOfBlock>
+// kFrames: the units of a camera sequence, P = FP->P (unit_of_frame_ticket, frame_camera_ray).
+template <bool kSampleBuf, int kSumStride, bool kListed = false, bool kFrames = false, class SurvivorsOfBlock>
 __device__ __forceinline__ void path_step(const KParams& P, PathRegs& pr, PathCounters& pc, unsigned bany,
                                           SurvivorsOfBlock survivors_of_block, double* sums, size_t stack_col, int lane,
-                                          unsigned long long total_units = 0) {
+                                          unsigned long long total_units = 0, const FrameKParams* FP = nullptr) {
   d3& O = pr.O; d3& D = pr.D;
   unsigned& pixel = pr.pixel; unsigned& unit = pr.unit;
   int& k = pr.k; int& k_end = pr.k_end; int& depth_left = pr.depth_left; int& nstack = pr.nstack; int& status = pr.status;
@@ -286,9 +287,11 @@ __device__ __forceinline__ void path_step(const KParams& P, PathRegs& pr, PathCo
         if (ticket >= (kListed ? total_units : P.total_units)) {
           status = PS_DEAD;
         } else {
-          const unsigned p_local = kListed ? unit_of_listed_ticket(P, (unsigned)ticket, unit)
-                                           : unit_of_ticket(P, (unsigned)ticket, unit);
-          const int chunk = (int)(unit - p_local * (unsigned)P.nchunks);
+          int chunk = 0;
+          const unsigned p_local = kFrames ? unit_of_frame_ticket(*FP, (unsigned)ticket, unit, chunk)
+                                   : kListed ? unit_of_listed_ticket(P, (unsigned)ticket, unit)
+                                             : unit_of_ticket(P, (unsigned)ticket, unit);
+          if (!kFrames) chunk = (int)(unit - p_local * (unsigned)P.nchunks);
           const int lr = (int)(p_local / (unsigned)P.W);
           const int pi = (int)(p_local - (unsigned)lr * (unsigned)P.W);
           const int tile = lr / P.shard_rows;
@@ -309,22 +312,26 @@ __device__ __forceinline__ void path_step(const KParams& P, PathRegs& pr, PathCo
     uint4 w = wq;  // usually drawn by the merged call above; a new unit / an absorbed path draws here
     if (!have_wq) w = philox_ni(pixel, (unsigned)k, 0u, 0u, P.k0, P.k1);
     const unsigned pj = pixel / (unsigned)P.W, pi = pixel - pj * (unsigned)P.W;
-    const double sx = (double)pi + (u24(w.x) - 0.5);
-    const double sy = (double)pj + (u24(w.y) - 0.5);
-    const d3 ps = add(add(ld3(P.p00), muls(ld3(P.du), sx)), muls(ld3(P.dv), sy));
-    O = ld3(P.center);
-    if (P.use_defocus) {  // vec3a/random-in-unit-disk, vec3a.clj:81-86
-      double px = sym24(w.z), py = sym24(w.w);
-      unsigned block = 0;
-      int half = 1;
-      while (!(px * px + py * py < 1.0) && block < 0xffffffu) {
-        if (half == 1) { w = philox_ni(pixel, (unsigned)k, 0u, ++block, P.k0, P.k1); half = 0; } else half = 1;
-        px = sym24(half ? w.z : w.x);
-        py = sym24(half ? w.w : w.y);
+    if (kFrames) {
+      frame_camera_ray<true>(P, FP->cam[unit / FP->frame_units], pixel, (int)pi, (int)pj, k, w, O, D);
+    } else {
+      const double sx = (double)pi + (u24(w.x) - 0.5);
+      const double sy = (double)pj + (u24(w.y) - 0.5);
+      const d3 ps = add(add(ld3(P.p00), muls(ld3(P.du), sx)), muls(ld3(P.dv), sy));
+      O = ld3(P.center);
+      if (P.use_defocus) {  // vec3a/random-in-unit-disk, vec3a.clj:81-86
+        double px = sym24(w.z), py = sym24(w.w);
+        unsigned block = 0;
+        int half = 1;
+        while (!(px * px + py * py < 1.0) && block < 0xffffffu) {
+          if (half == 1) { w = philox_ni(pixel, (unsigned)k, 0u, ++block, P.k0, P.k1); half = 0; } else half = 1;
+          px = sym24(half ? w.z : w.x);
+          py = sym24(half ? w.w : w.y);
+        }
+        O = add(add(O, muls(ld3(P.ddu), px)), muls(ld3(P.ddv), py));  // raytracing.clj:89-93
       }
-      O = add(add(O, muls(ld3(P.ddu), px)), muls(ld3(P.ddv), py));  // raytracing.clj:89-93
+      D = sub(ps, O);
     }
-    D = sub(ps, O);
     depth_left = P.max_depth;
     nstack = 0;
     n_samples++;

@@ -35,8 +35,10 @@ constexpr int kPrimaryThreads = RTCLJ_PRIM_THREADS;
 // kListed: the pixels of KParams::list only (an adaptive accumulation's pass, DESIGN.md section 4.10).  Seeded and
 // listed, the kernel also continues the pixel's sums of squared sample colours (KParams::acc2) in three more
 // registers, in sample order, and stores them back in place: the fold's S2 in strict order without a sample buffer.
-template <bool kDefocus, bool kSeeded, bool kListed = false>
-__device__ __forceinline__ void render_primary_body(const KParams& P) {
+// kFrames: the units of a camera sequence, P = FP->P (render_primary_frames_kernel).  Unit u belongs to frame
+// u / frame_units, tickets in unit order as here; kDefocus: some frame of the launch has the defocus disk.
+template <bool kDefocus, bool kSeeded, bool kListed = false, bool kFrames = false>
+__device__ __forceinline__ void render_primary_body(const KParams& P, const FrameKParams* FP = nullptr) {
   constexpr unsigned FULL = 0xffffffffu;
   constexpr bool kMoments = kSeeded && kListed;
   const int lane = threadIdx.x & 31;
@@ -58,8 +60,10 @@ __device__ __forceinline__ void render_primary_body(const KParams& P) {
     if (ticket >= total_units) continue;  // (tail of the last ticket: the lane waits at the next shuffle, which ends the loop)
 
     unsigned unit = (unsigned)ticket;
-    const unsigned p_local = kListed ? unit_of_listed_ticket(P, (unsigned)ticket, unit) : unit / (unsigned)P.nchunks;
-    const int chunk = (int)(unit - p_local * (unsigned)P.nchunks);
+    const unsigned frame = kFrames ? unit / FP->frame_units : 0u;
+    const unsigned frame_unit = kFrames ? unit - frame * FP->frame_units : unit;  // the unit within its frame
+    const unsigned p_local = kListed ? unit_of_listed_ticket(P, (unsigned)ticket, unit) : frame_unit / (unsigned)P.nchunks;
+    const int chunk = (int)((kListed ? unit : frame_unit) - p_local * (unsigned)P.nchunks);
     const int lr = (int)(p_local / (unsigned)P.W);
     const int pi = (int)(p_local - (unsigned)lr * (unsigned)P.W);
     const int tile = lr / P.shard_rows;
@@ -76,22 +80,27 @@ __device__ __forceinline__ void render_primary_body(const KParams& P) {
     for (int k = k_begin; k < k_end; ++k) {
       // ---- camera ray: raytracing.clj:144-151, realm/raytracing.clj:332-339, raytracing_i.clj:150-158
       uint4 w = RTCLJ_PHILOX(P, pixel, (unsigned)k, 0u, 0u);
-      const double sx = (double)pi + (u24(w.x) - 0.5);
-      const double sy = (double)pj + (u24(w.y) - 0.5);
-      const d3 ps = add(add(ld3(P.p00), muls(ld3(P.du), sx)), muls(ld3(P.dv), sy));
-      d3 O = ld3(P.center);
-      if (kDefocus) {  // vec3a/random-in-unit-disk, vec3a.clj:81-86
-        double px = sym24(w.z), py = sym24(w.w);
-        unsigned block = 0;
-        int half = 1;
-        while (!(px * px + py * py < 1.0) && block < 0xffffffu) {
-          if (half == 1) { w = philox_ni(pixel, (unsigned)k, 0u, ++block, P.k0, P.k1); half = 0; } else half = 1;
-          px = sym24(half ? w.z : w.x);
-          py = sym24(half ? w.w : w.y);
+      d3 O, D;
+      if (kFrames) {
+        frame_camera_ray<kDefocus>(P, FP->cam[frame], pixel, pi, pj, k, w, O, D);
+      } else {
+        const double sx = (double)pi + (u24(w.x) - 0.5);
+        const double sy = (double)pj + (u24(w.y) - 0.5);
+        const d3 ps = add(add(ld3(P.p00), muls(ld3(P.du), sx)), muls(ld3(P.dv), sy));
+        O = ld3(P.center);
+        if (kDefocus) {  // vec3a/random-in-unit-disk, vec3a.clj:81-86
+          double px = sym24(w.z), py = sym24(w.w);
+          unsigned block = 0;
+          int half = 1;
+          while (!(px * px + py * py < 1.0) && block < 0xffffffu) {
+            if (half == 1) { w = philox_ni(pixel, (unsigned)k, 0u, ++block, P.k0, P.k1); half = 0; } else half = 1;
+            px = sym24(half ? w.z : w.x);
+            py = sym24(half ? w.w : w.y);
+          }
+          O = add(add(O, muls(ld3(P.ddu), px)), muls(ld3(P.ddv), py));  // raytracing.clj:89-93
         }
-        O = add(add(O, muls(ld3(P.ddu), px)), muls(ld3(P.ddv), py));  // raytracing.clj:89-93
+        D = sub(ps, O);
       }
-      const d3 D = sub(ps, O);
 
       // ---- closest hit over every sphere in list order (hit-anything, raytracing.clj:33-43;
       // raytracing_i.clj:48-57): the operations of exact_test_lex, geometry from the parameters, with the
@@ -182,6 +191,11 @@ __global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_prima
 template <bool kDefocus>
 __global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_primary_seeded_listed_kernel(const __grid_constant__ KParams P) {
   render_primary_body<kDefocus, true, true>(P);
+}
+
+template <bool kDefocus>
+__global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_primary_frames_kernel(const __grid_constant__ FrameKParams FP) {
+  render_primary_body<kDefocus, false, false, true>(FP.P, &FP);
 }
 
 }  // namespace rtclj

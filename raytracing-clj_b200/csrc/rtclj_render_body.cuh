@@ -1,5 +1,6 @@
-// rtclj_render_body.cuh -- the body of render_kernel and render_listed_kernel (rtclj_kernels.cuh), included
-// inside each __global__ function, which defines kConstTab, kSampleBuf, kPacked and kListed and its parameter P.
+// rtclj_render_body.cuh -- the body of render_kernel, render_listed_kernel and render_frames_kernel (rtclj_kernels.cuh),
+// included inside each __global__ function, which defines kConstTab, kSampleBuf, kPacked and kListed and its parameter P
+// (render_frames_kernel: FP, whose P it is, and RTCLJ_FRAMES_BODY, so the other kernels compile from unchanged text).
 // Textual rather than a shared __forceinline__ device function: inlined, the body compiled to different code for
 // the 512-thread instantiation (the launch bounds no longer bound threadIdx.x where it is read, and loops were
 // rotated differently), whereas render_kernel must stay the kernel that was measured (DESIGN.md section 4.10).
@@ -440,9 +441,14 @@
           if (ticket >= (kListed ? (unsigned long long)listed_units : P.total_units)) {
             active = false;
           } else {
+#if RTCLJ_FRAMES_BODY
+            int chunk;
+            const unsigned p_local = unit_of_frame_ticket(FP, (unsigned)ticket, unit, chunk);
+#else
             const unsigned p_local = kListed ? unit_of_listed_ticket(P, (unsigned)ticket, unit)
                                              : unit_of_ticket(P, (unsigned)ticket, unit);
             const int chunk = (int)(unit - p_local * (unsigned)P.nchunks);
+#endif
             const int lr = (int)(p_local / (unsigned)P.W);
             pi = (int)(p_local - (unsigned)lr * (unsigned)P.W);
             const int tile = lr / P.shard_rows;
@@ -465,6 +471,9 @@
       has_ray = true;
       uint4 w = wq;  // usually drawn by the merged call above; a new unit / an absorbed path draws here
       if (!have_wq) w = philox_ni(pixel, (unsigned)k, 0u, 0u, P.k0, P.k1);
+#if RTCLJ_FRAMES_BODY
+      frame_camera_ray<true>(P, FP.cam[unit / FP.frame_units], pixel, pi, pj, k, w, O, D);
+#else
       const double sx = (double)pi + (u24(w.x) - 0.5);
       const double sy = (double)pj + (u24(w.y) - 0.5);
       d3 ps = add(add(ld3(P.p00), muls(ld3(P.du), sx)), muls(ld3(P.dv), sy));
@@ -481,6 +490,7 @@
         O = add(add(O, muls(ld3(P.ddu), px)), muls(ld3(P.ddv), py));  // raytracing.clj:89-93
       }
       D = sub(ps, O);
+#endif
       depth_left = P.max_depth;
       stage = 0;
       nstack = 0;

@@ -8,6 +8,8 @@
                                                               -> the same with adaptive sampling, and
                                                                  scene-samples.png (samples per pixel)
     python -m raytracing_clj_b200.main main ... --gpu-png     -> the same files, the PNGs compressed on the GPU
+    python -m raytracing_clj_b200.main main [spp] [depth] --frames N [--gpu-png]
+                                                              -> scene-0000.png ... scene-{N-1}.png, a turntable
     python -m raytracing_clj_b200.main realm                  -> scene-realm.ppm
     python -m raytracing_clj_b200.main i                      -> scene-i.ppm
 
@@ -25,7 +27,12 @@ units), and the run ends once no pixel is left.  scene-samples.png shows the sam
 
 With --gpu-png scene.png (and scene-samples.png) are written by the device PNG writer from the render's 8-bit
 image (DESIGN.md section 4.11): the same pixels, compressed, and only the compressed bytes leave the GPU.  Without
-it every file is the one the host writer produces."""
+it every file is the one the host writer produces.
+
+With --frames N the camera circles the scene: look_from turns about the vertical axis through look_at in N steps of
+360/N degrees, frame 0 being the reference's camera, and all N frames are rendered as one camera sequence
+(rtclj_render_frames, DESIGN.md section 4.12).  Each frame is written as a PNG only; frame 0 has the pixels of
+scene.png from a run without --frames."""
 from __future__ import annotations
 
 import os
@@ -96,6 +103,20 @@ def main_variant(spp: int = 100, depth: int = 50, out: str = "scene.ppm", seed: 
     return st
 
 
+def frames_variant(spp: int = 100, depth: int = 50, n_frames: int = 60, out: str = "scene", seed: int = 1,
+                   gpu_png: bool = False):
+    print("config:", {"samples-per-px": spp, "max-depth": depth, "frames": n_frames})
+    t0 = time.perf_counter()
+    _, rgb8, st = render.render_frames(scenes.main_hittables(), camera.turntable_cameras(n_frames), spp, depth,
+                                       seed=seed, flags=_abi.FLAGS_MAIN, want_linear=False)
+    t1 = time.perf_counter()
+    for k in range(n_frames):
+        render.write_png(f"{out}-{k:04d}.png", rgb8[k], 0 if gpu_png else None)
+    print(f'"Elapsed time: {1e3 * (time.perf_counter() - t0):.3f} msecs"  (render {1e3 * (t1 - t0):.3f} ms, '
+          f'{st["segments"]} ray segments, {out}-0000.png .. {out}-{n_frames - 1:04d}.png)')
+    return st
+
+
 def realm_variant(out: str = "scene-realm.ppm", seed: int = 1):
     t0 = time.perf_counter()
     _, rgb8, st = render.render(scenes.realm_hittables(), camera.realm_camera(), 100, 50, seed=seed,
@@ -118,6 +139,15 @@ def _cli(argv):
         every, tolerance = 0, None
         gpu_png = "--gpu-png" in argv
         argv = [a for a in argv if a != "--gpu-png"]
+        if "--frames" in argv:
+            i = argv.index("--frames")
+            if i + 1 >= len(argv) or not argv[i + 1].isdigit() or int(argv[i + 1]) <= 0:
+                raise SystemExit("--frames needs a positive number of frames")
+            n_frames = int(argv[i + 1])
+            argv = argv[:i] + argv[i + 2:]
+            frames_variant(int(argv[1]) if len(argv) > 1 else 100, int(argv[2]) if len(argv) > 2 else 50, n_frames,
+                           gpu_png=gpu_png)
+            return
         if "--tolerance" in argv:
             i = argv.index("--tolerance")
             try:

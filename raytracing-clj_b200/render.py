@@ -97,6 +97,36 @@ def render(world, cam: Camera, samples_per_px: int = 100, max_depth: int = 50, *
     return out_linear, out_rgb8, st.as_dict()
 
 
+def _camera_array(cameras):
+    cams = [_camera_struct(c) for c in cameras]
+    arr = (_abi.Camera * max(1, len(cams)))(*cams)
+    return arr, len(cams)
+
+
+def render_frames(world, cameras: Sequence, samples_per_px: int = 100, max_depth: int = 50, *, seed: int = 1,
+                  flags: int = _abi.FLAGS_MAIN, samples_per_unit: int = 0, devices: Optional[Sequence[int]] = None,
+                  want_linear: bool = True, want_rgb8: bool = True):
+    """A camera sequence of one scene (rtclj_render_frames): every frame in shared launches, rows interleaved over
+    `devices` (default [0]).  Returns (linear float64 [K,H,W,3] | None, rgb8 uint8 [K,H,W,3] | None, stats dict);
+    frame f is bit-identical to `render(world, cameras[f], ...)` with the same arguments, and the stats cover the
+    whole sequence."""
+    lib = _abi.lib()
+    soa = _as_soa(world)
+    sc = _scene_struct(soa)
+    arr, n = _camera_array(cameras)
+    H, W = (arr[0].height, arr[0].width) if n else (0, 0)
+    out_linear = np.zeros((n, H, W, 3), dtype=np.float64) if want_linear else None
+    out_rgb8 = np.zeros((n, H, W, 3), dtype=np.uint8) if want_rgb8 else None
+    prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit), 0, 0, 0, 0, 0)
+    devs = list(devices) if devices else [0]
+    darr = (C.c_int32 * len(devs))(*devs)
+    st = _abi.Stats()
+    _abi.check(lib.rtclj_render_frames(C.byref(sc), arr, n, C.byref(prm), darr, len(devs),
+                                       out_linear.ctypes.data if out_linear is not None else None,
+                                       out_rgb8.ctypes.data if out_rgb8 is not None else None, C.byref(st)))
+    return out_linear, out_rgb8, st.as_dict()
+
+
 def render_ppm(world, cam: Camera, samples_per_px: int = 100, max_depth: int = 50, *, seed: int = 1,
                flags: int = _abi.FLAGS_MAIN, samples_per_unit: int = 0, devices: Optional[Sequence[int]] = None):
     """The render loop and the write-color! loop in one call (raytracing.clj:141-175): returns
@@ -189,6 +219,20 @@ class Context:
         _abi.check(_abi.lib().rtclj_ctx_render(self._h, C.byref(cm), C.byref(prm),
                                                C.c_void_p(d_out_linear or None), C.c_void_p(d_out_rgb8 or None),
                                                C.c_void_p(stream or None)))
+
+    def render_frames(self, cameras: Sequence, samples_per_px: int, max_depth: int, *, seed: int = 1,
+                      flags: int = _abi.FLAGS_MAIN, samples_per_unit: int = 0, shard: Optional[tuple] = None,
+                      d_out_linear: int = 0, d_out_rgb8: int = 0, stream: int = 0) -> None:
+        """Enqueues a camera sequence (rtclj_ctx_render_frames): the device images hold len(cameras) full-size
+        frames, frame f bit-identical to render(cameras[f], ...)."""
+        arr, n = _camera_array(cameras)
+        prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit),
+                          0, 0, 0, int(self.device), 0)
+        if shard is not None:
+            prm.shard_index, prm.shard_count, prm.shard_rows = (int(x) for x in shard)
+        _abi.check(_abi.lib().rtclj_ctx_render_frames(self._h, arr, n, C.byref(prm),
+                                                      C.c_void_p(d_out_linear or None), C.c_void_p(d_out_rgb8 or None),
+                                                      C.c_void_p(stream or None)))
 
     def stats(self, stream: int = 0) -> dict:
         st = _abi.Stats()
