@@ -8,6 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 import math
+import operator
 from typing import Iterable, List, Optional, Sequence
 
 import numpy as np
@@ -58,6 +59,18 @@ def _camera_struct(cam) -> _abi.Camera:
     return c
 
 
+def _params(samples_per_px, max_depth, seed, flags, samples_per_unit, device=0) -> _abi.Params:
+    """The rtclj_params of a call.  The seed is the 64-bit Philox key (low word k0, high word k1): a seed outside
+    [0, 2^64) is refused rather than wrapped, since ctypes would silently keep its low 64 bits only."""
+    try:
+        s = operator.index(seed)
+    except TypeError:
+        raise ValueError(f"seed must be an integer in [0, 2^64), got {seed!r}") from None
+    if not 0 <= s < 1 << 64:
+        raise ValueError(f"seed must be an integer in [0, 2^64), got {s}")
+    return _abi.Params(int(samples_per_px), int(max_depth), s, int(flags), int(samples_per_unit), 0, 0, 0, int(device), 0)
+
+
 def _as_soa(world):
     if isinstance(world, tuple) and len(world) == 6 and isinstance(world[0], np.ndarray):
         return world
@@ -80,8 +93,7 @@ def render(world, cam: Camera, samples_per_px: int = 100, max_depth: int = 50, *
         out_linear = np.zeros((H, W, 3), dtype=np.float64)
     if want_rgb8 and out_rgb8 is None:
         out_rgb8 = np.zeros((H, W, 3), dtype=np.uint8)
-    prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit),
-                      0, 0, 0, 0, 0)
+    prm = _params(samples_per_px, max_depth, seed, flags, samples_per_unit)
     st = _abi.Stats()
     lin_p = out_linear.ctypes.data if out_linear is not None else None
     rgb_p = out_rgb8.ctypes.data if out_rgb8 is not None else None
@@ -117,7 +129,7 @@ def render_frames(world, cameras: Sequence, samples_per_px: int = 100, max_depth
     H, W = (arr[0].height, arr[0].width) if n else (0, 0)
     out_linear = np.zeros((n, H, W, 3), dtype=np.float64) if want_linear else None
     out_rgb8 = np.zeros((n, H, W, 3), dtype=np.uint8) if want_rgb8 else None
-    prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit), 0, 0, 0, 0, 0)
+    prm = _params(samples_per_px, max_depth, seed, flags, samples_per_unit)
     devs = list(devices) if devices else [0]
     darr = (C.c_int32 * len(devs))(*devs)
     st = _abi.Stats()
@@ -135,7 +147,7 @@ def render_ppm(world, cam: Camera, samples_per_px: int = 100, max_depth: int = 5
     lib = _abi.lib()
     soa = _as_soa(world)
     sc, cm = _scene_struct(soa), _camera_struct(cam)
-    prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit), 0, 0, 0, 0, 0)
+    prm = _params(samples_per_px, max_depth, seed, flags, samples_per_unit)
     devs = list(devices) if devices else [0]
     arr = (C.c_int32 * len(devs))(*devs)
     n = C.c_size_t()
@@ -157,7 +169,7 @@ def render_png(world, cam: Camera, samples_per_px: int = 100, max_depth: int = 5
     lib = _abi.lib()
     soa = _as_soa(world)
     sc, cm = _scene_struct(soa), _camera_struct(cam)
-    prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit), 0, 0, 0, 0, 0)
+    prm = _params(samples_per_px, max_depth, seed, flags, samples_per_unit)
     devs = list(devices) if devices else [0]
     arr = (C.c_int32 * len(devs))(*devs)
     n = C.c_size_t()
@@ -212,8 +224,7 @@ class Context:
                samples_per_unit: int = 0, shard: Optional[tuple] = None, d_out_linear: int = 0,
                d_out_rgb8: int = 0, stream: int = 0) -> None:
         cm = _camera_struct(cam)
-        prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit),
-                          0, 0, 0, int(self.device), 0)
+        prm = _params(samples_per_px, max_depth, seed, flags, samples_per_unit, self.device)
         if shard is not None:
             prm.shard_index, prm.shard_count, prm.shard_rows = (int(x) for x in shard)
         _abi.check(_abi.lib().rtclj_ctx_render(self._h, C.byref(cm), C.byref(prm),
@@ -226,8 +237,7 @@ class Context:
         """Enqueues a camera sequence (rtclj_ctx_render_frames): the device images hold len(cameras) full-size
         frames, frame f bit-identical to render(cameras[f], ...)."""
         arr, n = _camera_array(cameras)
-        prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit),
-                          0, 0, 0, int(self.device), 0)
+        prm = _params(samples_per_px, max_depth, seed, flags, samples_per_unit, self.device)
         if shard is not None:
             prm.shard_index, prm.shard_count, prm.shard_rows = (int(x) for x in shard)
         _abi.check(_abi.lib().rtclj_ctx_render_frames(self._h, arr, n, C.byref(prm),
@@ -247,8 +257,7 @@ class Context:
         adaptive accumulation (rtclj_ctx_accum_begin_adaptive) whose passes trace only the pixels whose noise
         estimate is still above abs + rel * |mean|, after at least min_samples samples (<= 0: two pass units)."""
         cm = _camera_struct(cam)
-        prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit),
-                          0, 0, 0, int(self.device), 0)
+        prm = _params(samples_per_px, max_depth, seed, flags, samples_per_unit, self.device)
         if shard is not None:
             prm.shard_index, prm.shard_count, prm.shard_rows = (int(x) for x in shard)
         unit = C.c_int32()
@@ -340,8 +349,7 @@ class Progressive:
         self.height, self.width = cm.height, cm.width
         self.samples_per_px = int(samples_per_px)
         self.adaptive = tolerance is not None
-        prm = _abi.Params(int(samples_per_px), int(max_depth), int(seed), int(flags), int(samples_per_unit),
-                          0, 0, 0, 0, 0)
+        prm = _params(samples_per_px, max_depth, seed, flags, samples_per_unit)
         devs = list(devices) if devices else [0]
         arr = (C.c_int32 * len(devs))(*devs)
         unit = C.c_int32()

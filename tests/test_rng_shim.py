@@ -20,6 +20,24 @@ def test_philox_model_equals_oracle_philox():
         assert list(M.philox4x32_10(*c, *k)) == [int(x) for x in O.philox(c, k)]
 
 
+# Random123's published known-answer vectors for philox4x32-10 (kat_vectors): counter, key -> output
+PHILOX_KAT = [
+    ((0x00000000, 0x00000000, 0x00000000, 0x00000000), (0x00000000, 0x00000000),
+     (0x6627e8d5, 0xe169c58d, 0xbc57ac4c, 0x9b00dbd8)),
+    ((0xffffffff, 0xffffffff, 0xffffffff, 0xffffffff), (0xffffffff, 0xffffffff),
+     (0x408f276d, 0x41c83b0e, 0xa20bc7c6, 0x6d5451fd)),
+    ((0x243f6a88, 0x85a308d3, 0x13198a2e, 0x03707344), (0xa4093822, 0x299f31d0),
+     (0xd16cfe09, 0x94fdcceb, 0x5001e420, 0x24126ea1)),
+]
+
+
+def test_philox_known_answers():
+    """Both implementations against the published vectors, not only against each other."""
+    for ctr, key, out in PHILOX_KAT:
+        assert O.philox(ctr, key) == out
+        assert tuple(M.philox4x32_10(*ctr, *key)) == out
+
+
 def test_camera_stage_is_sequential_words():
     st = M.ShimStream(seed=0x1234567890ABCDEF)
     st.begin_sample(77, 5)
@@ -58,6 +76,9 @@ def test_sequential_reference_loop_reproduces_the_oracle_render():
     _compare(S.cover_hittables(7)[:40], CAM.main_camera(12, 7, **S.COVER_CAMERA), 2, 50, seed=5)
     # depth cap reached inside glass
     _compare(S.main_hittables(), CAM.main_camera(10), 2, 3, seed=2)
+    # seeds with the high word of the key set: both words of the key reach every draw
+    _compare(S.main_hittables(), CAM.main_camera(10), 2, 50, seed=(1 << 64) - 1)
+    _compare(S.main_hittables(), CAM.main_camera(10), 2, 50, seed=0xFFFFFFFF00000000)
 
 
 def test_sequential_realm_loop_reproduces_the_oracle_render():
