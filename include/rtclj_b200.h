@@ -32,6 +32,9 @@
  *   rtclj_ctx_encode_png, rtclj_encode_png_gpu
  *                           a compressed PNG of the same image, written by device kernels (device / host buffers)
  *   rtclj_render_multi_png  the render loop and ppm->png as one call: several GPUs in, a compressed PNG out
+ *   rtclj_ctx_denoise, rtclj_denoise_gpu, rtclj_render_denoised
+ *                           not in the reference: an edge-avoiding filter of the rendered image, guided by
+ *                           the normal-shaded primary render (device / host buffers / render + guide + filter)
  *   rtclj_camera_main/_realm/_i
  *                           the camera let-blocks, src/raytracing.clj:105-139 ;
  *                           realm/raytracing.clj:264-280,306-322 ;
@@ -435,6 +438,51 @@ int rtclj_encode_png_gpu(int32_t device, const uint8_t *rgb8, int32_t width, int
 int rtclj_render_multi_png(const rtclj_scene *scene, const rtclj_camera *camera, const rtclj_params *params,
                            const int32_t *devices, int32_t n_devices, uint8_t *out, size_t capacity, size_t *len,
                            rtclj_stats *stats);
+
+/* ---- Denoising: an edge-avoiding a-trous filter of a linear image, guided by a second image -- the normal-shaded
+ * primary render (RTCLJ_F_NORMAL_SHADING, max_depth 1) of the same camera and seed, whose first samples are the colour
+ * render's camera rays bit for bit, so its silhouettes line up with the colour's jitter and defocus (DESIGN.md section
+ * 4.13).  A new output next to the reference's image; no render changes.  The output is exactly this definition
+ * (tests/denoise_model.py reproduces it bit for bit); every operation is an IEEE float32 operation in the order given:
+ *   1. c_0 = float32(C), g = float32(G), rounded to nearest (C: colour, G: guide, both W*H*3 linear doubles).  A
+ *      pixel whose c_0 or g has a non-finite component (NaN, +-inf, or a double beyond the float32 range) is never
+ *      filtered and never used as a tap.
+ *   2. For level i = 0 .. L-1: step s = 2^i, sc2 = (float32(sigma_c) * 2^-i)^2, sg2 = float32(sigma_g)^2.  For each
+ *      pixel p whose c_i and g are finite: acc_r = acc_g = acc_b = W = 0; for dy = -2..2, then dx = -2..2 (row-major),
+ *      the tap q = p + s (dx, dy) is skipped if it lies outside the image or its c_i or g is not finite; otherwise
+ *        dc = ((dr*dr + dg*dg) + db*db) of c_i(q) - c_i(p), dgd the same of g(q) - g(p),
+ *        w  = ((h[dx] * h[dy]) * k(dc / sc2)) * k(dgd / sg2),  h = {1/16, 1/4, 3/8, 1/4, 1/16} for -2..2,
+ *        k(x) = t * t with t = fmax(1 - x, 0),
+ *        acc_ch = acc_ch + w * c_i(q)_ch per channel, W = W + w;
+ *      c_(i+1)(p) = acc_ch / W per channel (the centre tap has weight 9/64 > 0).  Any other pixel keeps c_i.
+ *   3. Linear output: (double)c_L, except a pixel not filtered at level 0, which keeps its input double.  (A pixel
+ *      whose float32 sums overflow becomes non-finite and is then kept as that float.)  8-bit output: write-color! of
+ *      the linear output (flags & RTCLJ_F_QUANT_LINEAR: int(255.999 c); else gamma 2; the only flag read).
+ * RTCLJ_E_INVALID, with a message, before any device work: levels outside 1..8; sigma values that are not finite and
+ * positive, or for which sc2 at level 0 is not finite, sc2 at level L-1 is not a normal float32, or sg2 is not a finite
+ * normal float32 (a subnormal or zero sc2 would turn the centre tap's 0/0 into a NaN); non-positive sizes; null
+ * pointers.  sigma[2] = {sigma_color, sigma_guide} (an array, as the adaptive tolerance).  Pixel indices are 64-bit.
+ * Scratch: 48 bytes per pixel (two float32 colour buffers and the float32 guide) kept in the context.
+ *
+ * Device-resident, enqueued on `stream` without synchronising: d_linear, d_guide, d_out_linear (W*H*3 doubles) and
+ * d_out_rgb8 (W*H*3 bytes) are DEVICE pointers; either output may be NULL; d_out_linear == d_linear (in place) is
+ * allowed.  One context serves one stream at a time. */
+int rtclj_ctx_denoise(rtclj_ctx *ctx, const double *d_linear, const double *d_guide, int32_t width, int32_t height,
+                      int32_t levels, const double sigma[2], uint32_t flags, double *d_out_linear, uint8_t *d_out_rgb8,
+                      void *stream);
+/* Host buffers in and out, the filter on `device` (copies inside the call). */
+int rtclj_denoise_gpu(int32_t device, const double *linear, const double *guide, int32_t width, int32_t height,
+                      int32_t levels, const double sigma[2], uint32_t flags, double *out_linear, uint8_t *out_rgb8);
+/* Render, guide and filter in one call: renders the colour image as rtclj_render_multi does (rows interleaved over
+ * `n_devices` GPUs in tiles of params->shard_rows rows), then the guide -- the same camera, seed and shard_rows,
+ * spp = guide_samples, max_depth = 1, flags RTCLJ_F_NORMAL_SHADING plus the caller's kernel-selection flags (bits 16
+ * and up), samples_per_unit 0 (the strict order) -- assembles both linear images on devices[0] by device-to-device
+ * copies and runs rtclj_ctx_denoise there with params->flags.  out_linear / out_rgb8 (either may be NULL) receive the
+ * denoised image, identical for every device list and shard_rows.  stats (may be NULL) covers the colour render;
+ * its total_ms covers the whole call. */
+int rtclj_render_denoised(const rtclj_scene *scene, const rtclj_camera *camera, const rtclj_params *params,
+                          int32_t guide_samples, int32_t levels, const double sigma[2], const int32_t *devices,
+                          int32_t n_devices, double *out_linear, uint8_t *out_rgb8, rtclj_stats *stats);
 
 /* The reader half of ppm->png (src/ppm2png.clj:35-87 reads "P3", "W H", a maximum <= 255 and one
  * "r g b" line per pixel; this parser accepts any whitespace between the tokens).  Call with

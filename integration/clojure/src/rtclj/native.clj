@@ -437,3 +437,69 @@
           out (.allocate a cap 16)]
       (check! (.invokeWithArguments rtclj-encode-png-gpu [(int device) src w h out cap len]))
       (.toArray (.asSlice out 0 (.get len ValueLayout/JAVA_LONG 0)) ValueLayout/JAVA_BYTE))))
+
+;; ---- denoising (DESIGN.md section 4.13): an edge-avoiding filter guided by the normal-shaded primary render
+;; int rtclj_denoise_gpu(int32_t device, const double* linear, const double* guide, int32_t width, int32_t height,
+;;                       int32_t levels, const double sigma[2], uint32_t flags, double* out_linear, uint8_t* out_rgb8)
+(def ^:private rtclj-denoise-gpu
+  (downcall "rtclj_denoise_gpu"
+            (fd-int ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/JAVA_INT ValueLayout/JAVA_INT
+                    ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/ADDRESS)))
+;; int rtclj_render_denoised(const rtclj_scene*, const rtclj_camera*, const rtclj_params*, int32_t guide_samples,
+;;                           int32_t levels, const double sigma[2], const int32_t* devices, int32_t n_devices,
+;;                           double* out_linear, uint8_t* out_rgb8, rtclj_stats*)
+(def ^:private rtclj-render-denoised
+  (downcall "rtclj_render_denoised"
+            (fd-int ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/JAVA_INT ValueLayout/JAVA_INT
+                    ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/ADDRESS
+                    ValueLayout/ADDRESS)))
+
+(def denoise-defaults
+  "levels, sigma-color, sigma-guide and guide samples chosen by the sweep of DESIGN.md section 4.13 (the Python
+   defaults, render.DENOISE_*)."
+  {:levels 3 :sigma-color 0.5 :sigma-guide 0.4 :guide-samples 4})
+
+(defn- colors-of
+  "W*H double[3] pixels of a W*H*3 double segment, as `render` returns them."
+  [^MemorySegment out ^long n]
+  (mapv (fn [^long p]
+          (double-array [(.getAtIndex out ValueLayout/JAVA_DOUBLE (* 3 p))
+                         (.getAtIndex out ValueLayout/JAVA_DOUBLE (+ 1 (* 3 p)))
+                         (.getAtIndex out ValueLayout/JAVA_DOUBLE (+ 2 (* 3 p)))]))
+        (range n)))
+
+(defn denoise
+  "The filter alone on GPU :device (default 0): `colors` and `guide` are what `render` returns (W*H double[3], the
+   guide rendered with :flags flags-i, max-depth 1 and the same seed).  Returns the denoised pixels in the same form."
+  [colors guide width height & {:keys [device levels sigma-color sigma-guide flags]
+                                :or {device 0 flags 0} :as opts}]
+  (let [{:keys [levels sigma-color sigma-guide]} (merge denoise-defaults (select-keys opts [:levels :sigma-color :sigma-guide]))]
+    (with-open [a (Arena/ofConfined)]
+      (let [n   (* (long width) (long height))
+            lin (doubles-seg a (mapcat seq colors))
+            gd  (doubles-seg a (mapcat seq guide))
+            out (.allocate a (* 24 n) 8)]
+        (check! (.invokeWithArguments rtclj-denoise-gpu
+                                      [(int device) lin gd (int width) (int height) (int levels)
+                                       (doubles-seg a [sigma-color sigma-guide]) (int flags) out MemorySegment/NULL]))
+        (colors-of out n)))))
+
+(defn render-denoised
+  "`render` followed by the denoiser, in one native call (rtclj_render_denoised): the colour render on :devices
+   (default [0]), the guide (the same camera and seed, :guide-samples samples, max-depth 1, normal shading), both
+   assembled on the first device and filtered there.  Options as `render`, plus :guide-samples :levels :sigma-color
+   :sigma-guide (defaults: denoise-defaults).  Returns the denoised pixels as `render` returns its image."
+  [bodies cam samples-per-px max-depth & {:keys [devices] :or {devices [0]} :as opts}]
+  (let [{:keys [guide-samples levels sigma-color sigma-guide]} (merge denoise-defaults opts)]
+    (with-open [a (Arena/ofConfined)]
+      (let [n (* (long (:image-width cam)) (long (:image-height cam)))
+            [scene camera params] (marshal a bodies cam samples-per-px max-depth opts)
+            [^MemorySegment out free!] (pinned-doubles a (* 3 n))]
+        (try
+          (check! (.invokeWithArguments rtclj-render-denoised
+                                        [scene camera params (int guide-samples) (int levels)
+                                         (doubles-seg a [sigma-color sigma-guide])
+                                         (.allocateFrom a ValueLayout/JAVA_INT (int-array devices)) (int (count devices))
+                                         out MemorySegment/NULL MemorySegment/NULL]))
+          (colors-of out n)
+          (finally (free!)))))))

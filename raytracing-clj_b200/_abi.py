@@ -114,6 +114,13 @@ SYMBOLS = {
     "rtclj_render_multi_png": (C.c_int, [C.POINTER(Scene), C.POINTER(Camera), C.POINTER(Params),
                                          C.POINTER(C.c_int32), C.c_int32, C.c_void_p, C.c_size_t,
                                          C.POINTER(C.c_size_t), C.POINTER(Stats)]),
+    "rtclj_ctx_denoise": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
+                                    C.POINTER(C.c_double), C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rtclj_denoise_gpu": (C.c_int, [C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
+                                    C.POINTER(C.c_double), C.c_uint32, C.c_void_p, C.c_void_p]),
+    "rtclj_render_denoised": (C.c_int, [C.POINTER(Scene), C.POINTER(Camera), C.POINTER(Params), C.c_int32, C.c_int32,
+                                        C.POINTER(C.c_double), C.POINTER(C.c_int32), C.c_int32, C.c_void_p, C.c_void_p,
+                                        C.POINTER(Stats)]),
     "rtclj_ratio_to_double": (C.c_double, [C.c_int64, C.c_int64]),
     "rtclj_camera_main": (C.c_int, [C.c_int32, C.c_int32, C.c_double, C.POINTER(C.c_double),
                                     C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_double,

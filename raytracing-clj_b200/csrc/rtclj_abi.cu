@@ -9,11 +9,13 @@
 #include "rtclj_split_kernel.cuh"
 #include "rtclj_p3_kernels.cuh"
 #include "rtclj_png_kernels.cuh"
+#include "rtclj_denoise_kernels.cuh"
 #include "rtclj_adaptive.cuh"
 #include "rtclj_error.h"
 
 #include <algorithm>
 #include <chrono>
+#include <cfloat>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -24,6 +26,7 @@
 #include <new>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 using namespace rtclj;
@@ -95,6 +98,10 @@ struct rtclj_ctx {
   DevBuf<unsigned long long> png_state;
   DevBuf<unsigned char> png_in, png_out;  // staging for the host-buffer entry points
   bool png_attr = false;                   // the PNG kernels' shared-memory limit is raised
+  // denoiser (rtclj_ctx_denoise): the ping-pong float32 colour images and the float32 guide; the f64 guide of the
+  // host-buffer entry points (rtclj_denoise_gpu stages the colour in out_linear)
+  DevBuf<float4> dn_c0, dn_c1, dn_g;
+  DevBuf<double> dn_guide64;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev2 = nullptr;  // render: start, kernel end, finalize end
   cudaEvent_t p3_ev0 = nullptr, p3_ev1 = nullptr;           // the P3 writer's own timing events
   cudaStream_t own_stream = nullptr;
@@ -343,6 +350,7 @@ void rtclj_ctx_destroy(rtclj_ctx* c) {
   c->noise_samples.release(); c->noise_stderr.release();
   c->p3_state.release(); c->p3_in.release(); c->p3_text.release();
   c->png_f.release(); c->png_stage.release(); c->png_rec.release(); c->png_state.release(); c->png_in.release(); c->png_out.release();
+  c->dn_c0.release(); c->dn_c1.release(); c->dn_g.release(); c->dn_guide64.release();
   for (cudaEvent_t e : {c->ev0, c->ev1, c->ev2, c->p3_ev0, c->p3_ev1, c->pin_ev[0], c->pin_ev[1]})
     if (e) cudaEventDestroy(e);
   for (void* h : c->pin) if (h) cudaFreeHost(h);
@@ -1522,19 +1530,16 @@ int rtclj_progressive_destroy(rtclj_progressive* p) {
 
 namespace {
 
-// The render loop on several GPUs with the 8-bit image assembled on devices[0]: each device renders its shard and
-// copies its rows into the root's out_rgb8 over NVLink.  Every device of the call is locked in `locks` until the
-// caller lets go of them (the root's image is written by its peers); locks are taken in ordinal order, so two such
-// calls cannot deadlock.  *root receives devices[0]'s context, *total the summed counters.
-int render_to_root(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm, const int32_t* devices,
-                   int32_t n_devices, std::vector<std::unique_lock<std::mutex>>& locks, rtclj_ctx** root_out,
-                   rtclj_stats* total) {
+// The cached contexts of a multi-GPU call's devices, ctxs[d] being devices[d]'s.  Every device is locked in `locks`
+// until the caller lets go of them (the root's images are written by its peers); locks are taken in ordinal order, so
+// two such calls cannot deadlock.
+int lock_devices(const int32_t* devices, int32_t n_devices, std::vector<std::unique_lock<std::mutex>>& locks,
+                 std::vector<rtclj_ctx*>& ctxs) {
   int rc = check_devices(devices, n_devices);
   if (rc) return rc;
-  const size_t npix = (size_t)cam->width * (size_t)cam->height;
   std::vector<int> order(devices, devices + n_devices);
   std::sort(order.begin(), order.end());
-  std::vector<rtclj_ctx*> ctxs((size_t)n_devices, nullptr);
+  ctxs.assign((size_t)n_devices, nullptr);
   for (int dev : order) {
     rtclj_ctx* c = nullptr;
     locks.emplace_back();
@@ -1542,17 +1547,29 @@ int render_to_root(const rtclj_scene* scene, const rtclj_camera* cam, const rtcl
     if (rc) return rc;
     for (int d = 0; d < n_devices; ++d) if (devices[d] == dev) ctxs[(size_t)d] = c;
   }
+  return RTCLJ_OK;
+}
+
+// The render loop on the locked devices ctxs (lock_devices) with one image assembled on devices[0]: each device renders
+// its shard into its own buffer `img` (out_rgb8: the 8-bit image; a DevBuf<double>: the linear one) and copies its rows
+// into the root's over NVLink.  *total receives the summed counters.
+template <class T>
+int render_to_root(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm, const int32_t* devices,
+                   int32_t n_devices, const std::vector<rtclj_ctx*>& ctxs, DevBuf<T> rtclj_ctx::*img, rtclj_stats* total) {
+  constexpr bool kLinear = std::is_same<T, double>::value;
+  const size_t npix = (size_t)cam->width * (size_t)cam->height;
   rtclj_ctx* root = ctxs[0];
   CU(cudaSetDevice(root->device));
-  CU(root->out_rgb8.reserve(npix * 3));
+  CU((root->*img).reserve(npix * 3));
   std::vector<rtclj_stats> st((size_t)n_devices);
-  rc = run_on_devices(n_devices, [&](int d) -> int {
+  int rc = run_on_devices(n_devices, [&](int d) -> int {
     rtclj_ctx* c = ctxs[(size_t)d];
     const rtclj_params q = shard_params(prm, devices, d, n_devices);
     int r = rtclj_ctx_set_scene(c, scene);
     if (r) return r;
-    if (c != root) CU(c->out_rgb8.reserve(npix * 3));
-    r = rtclj_ctx_render(c, cam, &q, nullptr, c->out_rgb8.p, c->own_stream);
+    if (c != root) CU((c->*img).reserve(npix * 3));
+    T* mine = (c->*img).p;
+    r = rtclj_ctx_render(c, cam, &q, kLinear ? (void*)mine : nullptr, kLinear ? nullptr : (void*)mine, c->own_stream);
     if (r) return r;
     if (c != root) {  // this shard's rows -> the root's image, device to device
       int can = 0;
@@ -1560,20 +1577,45 @@ int render_to_root(const rtclj_scene* scene, const rtclj_camera* cam, const rtcl
         const cudaError_t e = cudaDeviceEnablePeerAccess(root->device, 0);
         if (e != cudaSuccess) cudaGetLastError();  // already enabled: fine; otherwise the copy is staged by the driver
       }
+      char* dst = (char*)(root->*img).p;
+      const char* src = (const char*)mine;
       std::vector<Piece> pieces;
-      plan_pieces((size_t)cam->height, (size_t)cam->width * 3, q.shard_index, q.shard_count, q.shard_rows, (size_t)1 << 40, pieces);
+      plan_pieces((size_t)cam->height, (size_t)cam->width * 3 * sizeof(T), q.shard_index, q.shard_count, q.shard_rows, (size_t)1 << 40, pieces);
       for (const Piece& pc : pieces) {
-        if (pc.height == 1) CU(cudaMemcpyAsync(root->out_rgb8.p + pc.off, c->out_rgb8.p + pc.off, pc.width, cudaMemcpyDefault, c->own_stream));
-        else CU(cudaMemcpy2DAsync(root->out_rgb8.p + pc.off, pc.pitch, c->out_rgb8.p + pc.off, pc.pitch, pc.width, pc.height, cudaMemcpyDefault, c->own_stream));
+        if (pc.height == 1) CU(cudaMemcpyAsync(dst + pc.off, src + pc.off, pc.width, cudaMemcpyDefault, c->own_stream));
+        else CU(cudaMemcpy2DAsync(dst + pc.off, pc.pitch, src + pc.off, pc.pitch, pc.width, pc.height, cudaMemcpyDefault, c->own_stream));
       }
     }
     return rtclj_ctx_stats(c, c->own_stream, &st[(size_t)d]);  // synchronises: render and copies are done
   });
   if (rc) return rc;
   *total = sum_stats(st);
-  *root_out = root;
   CU(cudaSetDevice(root->device));
   return RTCLJ_OK;
+}
+
+// The host-side checks of a denoise call (include/rtclj_b200.h): nothing runs on a device before they pass.
+int check_denoise(int32_t width, int32_t height, int32_t levels, const double* sigma) {
+  if (width <= 0 || height <= 0) return fail(RTCLJ_E_INVALID, "image size must be positive (%d x %d)", width, height);
+  if (levels < 1 || levels > 8) return fail(RTCLJ_E_INVALID, "levels must be in 1..8, got %d", levels);
+  if (!sigma) return fail(RTCLJ_E_INVALID, "null sigma");
+  const char* names[2] = {"sigma_color", "sigma_guide"};
+  for (int k = 0; k < 2; ++k)
+    if (!std::isfinite(sigma[k]) || !(sigma[k] > 0.0))
+      return fail(RTCLJ_E_INVALID, "%s must be finite and positive, got %g", names[k], sigma[k]);
+  const float c = (float)sigma[0], g = (float)sigma[1];
+  const float c_last = std::ldexp(c, -(levels - 1));
+  if (!std::isfinite(c * c) || !(c_last * c_last >= FLT_MIN))
+    return fail(RTCLJ_E_INVALID, "sigma_color = %g: (sigma_color 2^-i)^2 must be a normal float32 at levels 0..%d",
+                sigma[0], levels - 1);
+  if (!std::isfinite(g * g) || !(g * g >= FLT_MIN))
+    return fail(RTCLJ_E_INVALID, "sigma_guide = %g: sigma_guide^2 must be a normal float32", sigma[1]);
+  return RTCLJ_OK;
+}
+
+bool overlaps(const void* a, const void* b, size_t bytes) {
+  const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
+  return x < y + bytes && y < x + bytes;
 }
 
 // The filtered stream's length and the sizing call's answer (every segment stored) of a W x H PNG;
@@ -1609,10 +1651,13 @@ int rtclj_render_multi_ppm(const rtclj_scene* scene, const rtclj_camera* cam, co
     const size_t worst = 64 + npix * 12;  // "255 255 255\n" per pixel + header
     if (!out) { *len = worst; return RTCLJ_OK; }  // sizing call: an upper bound, nothing is rendered
     std::vector<std::unique_lock<std::mutex>> locks;
-    rtclj_ctx* root = nullptr;
+    std::vector<rtclj_ctx*> ctxs;
     rtclj_stats total;
-    rc = render_to_root(scene, cam, prm, devices, n_devices, locks, &root, &total);
+    rc = lock_devices(devices, n_devices, locks, ctxs);
     if (rc) return rc;
+    rc = render_to_root(scene, cam, prm, devices, n_devices, ctxs, &rtclj_ctx::out_rgb8, &total);
+    if (rc) return rc;
+    rtclj_ctx* const root = ctxs[0];
     // the write-color! loop on the assembled image, then the text alone goes to the host
     CU(root->p3_text.reserve(worst));
     size_t need = 0;
@@ -1642,10 +1687,13 @@ int rtclj_render_multi_png(const rtclj_scene* scene, const rtclj_camera* cam, co
     if (rc) return rc;
     if (!out) { *len = bound; return RTCLJ_OK; }  // sizing call: the stored bound, nothing is rendered
     std::vector<std::unique_lock<std::mutex>> locks;
-    rtclj_ctx* root = nullptr;
+    std::vector<rtclj_ctx*> ctxs;
     rtclj_stats total;
-    rc = render_to_root(scene, cam, prm, devices, n_devices, locks, &root, &total);
+    rc = lock_devices(devices, n_devices, locks, ctxs);
     if (rc) return rc;
+    rc = render_to_root(scene, cam, prm, devices, n_devices, ctxs, &rtclj_ctx::out_rgb8, &total);
+    if (rc) return rc;
+    rtclj_ctx* const root = ctxs[0];
     CU(root->png_out.reserve(bound));
     size_t need = 0;
     rc = rtclj_ctx_encode_png(root, root->out_rgb8.p, cam->width, cam->height, root->png_out.p, bound, &need, root->own_stream);
@@ -1862,6 +1910,127 @@ int rtclj_encode_png_gpu(int32_t device, const uint8_t* rgb8, int32_t width, int
     if (need > capacity) return fail(RTCLJ_E_BUFFER, "PNG needs %zu bytes, capacity is %zu", need, capacity);
     CU(cudaMemcpyAsync(out, c->png_out.p, need, cudaMemcpyDeviceToHost, c->own_stream));
     CU(cudaStreamSynchronize(c->own_stream));
+    return RTCLJ_OK;
+  });
+}
+
+// ---- the denoiser (DESIGN.md section 4.13; the definition: include/rtclj_b200.h)
+int rtclj_ctx_denoise(rtclj_ctx* c, const double* d_linear, const double* d_guide, int32_t width, int32_t height,
+                      int32_t levels, const double* sigma, uint32_t flags, double* d_out_linear, uint8_t* d_out_rgb8,
+                      void* stream_) {
+  return guarded([&]() -> int {
+    if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
+    int rc = check_denoise(width, height, levels, sigma);
+    if (rc) return rc;
+    if (!d_linear || !d_guide) return fail(RTCLJ_E_INVALID, "null image or guide");
+    cudaStream_t stream = (cudaStream_t)stream_;
+    CU(cudaSetDevice(c->device));
+    const long long npix = (long long)width * (long long)height;
+    const size_t bytes = (size_t)npix * 3 * sizeof(double);
+    // one level in place: the folded conversion would read C's neighbours after other threads overwrote them
+    const bool convert = levels == 1 && d_out_linear &&
+                         (overlaps(d_out_linear, d_linear, bytes) || overlaps(d_out_linear, d_guide, bytes));
+    if (levels > 1 || convert) { CU(c->dn_c0.reserve((size_t)npix)); CU(c->dn_g.reserve((size_t)npix)); }
+    if (levels > 2) CU(c->dn_c1.reserve((size_t)npix));
+    if (convert) {
+      const long long blocks = std::min<long long>((npix + 255) / 256, kDenoiseMaxBlocks);
+      denoise_convert_kernel<<<(unsigned)blocks, 256, 0, stream>>>(d_linear, d_guide, c->dn_c0.p, c->dn_g.p, npix);
+      CU(cudaGetLastError());
+    }
+    DenoiseParams P;
+    std::memset(&P, 0, sizeof P);
+    P.lin64 = d_linear; P.guide64 = d_guide; P.guide = c->dn_g.p;
+    P.out_linear = d_out_linear; P.out_rgb8 = d_out_rgb8;
+    P.W = width; P.H = height;
+    const float sc = (float)sigma[0], sg = (float)sigma[1];
+    P.sigma2_g = sg * sg;
+    P.quant_linear = (flags & RTCLJ_F_QUANT_LINEAR) != 0;
+    const long long tiles = ((width + kDenoiseTileW - 1) / kDenoiseTileW) * (long long)((height + kDenoiseTileH - 1) / kDenoiseTileH);
+    const unsigned blocks = (unsigned)std::min<long long>(tiles, kDenoiseMaxBlocks);
+    const dim3 block(kDenoiseTileW, kDenoiseTileH);
+    float4* const bufs[2] = {c->dn_c0.p, c->dn_c1.p};
+    const float4* src = convert ? c->dn_c0.p : nullptr;
+    for (int i = 0; i < levels; ++i) {
+      const bool first = i == 0 && !convert, last = i + 1 == levels;
+      const float s = std::ldexp(sc, -i);
+      P.step = 1 << i;
+      P.sigma2_c = s * s;
+      P.src = src;
+      P.dst = last ? nullptr : bufs[i & 1];
+      if (first && last) denoise_level_kernel<true, true><<<blocks, block, 0, stream>>>(P);
+      else if (first) denoise_level_kernel<true, false><<<blocks, block, 0, stream>>>(P);
+      else if (last) denoise_level_kernel<false, true><<<blocks, block, 0, stream>>>(P);
+      else denoise_level_kernel<false, false><<<blocks, block, 0, stream>>>(P);
+      CU(cudaGetLastError());
+      src = P.dst;
+    }
+    return RTCLJ_OK;
+  });
+}
+
+int rtclj_denoise_gpu(int32_t device, const double* linear, const double* guide, int32_t width, int32_t height,
+                      int32_t levels, const double* sigma, uint32_t flags, double* out_linear, uint8_t* out_rgb8) {
+  return guarded([&]() -> int {
+    int rc = check_denoise(width, height, levels, sigma);
+    if (rc) return rc;
+    if (!linear || !guide) return fail(RTCLJ_E_INVALID, "null image or guide");
+    std::unique_lock<std::mutex> lock;
+    rtclj_ctx* c = nullptr;
+    rc = cached_ctx(device, lock, &c);
+    if (rc) return rc;
+    CU(cudaSetDevice(c->device));
+    const size_t n = (size_t)width * (size_t)height * 3;
+    CU(c->out_linear.reserve(n));
+    CU(c->dn_guide64.reserve(n));
+    if (out_rgb8) CU(c->out_rgb8.reserve(n));
+    CU(cudaMemcpyAsync(c->out_linear.p, linear, n * sizeof(double), cudaMemcpyHostToDevice, c->own_stream));
+    CU(cudaMemcpyAsync(c->dn_guide64.p, guide, n * sizeof(double), cudaMemcpyHostToDevice, c->own_stream));
+    rc = rtclj_ctx_denoise(c, c->out_linear.p, c->dn_guide64.p, width, height, levels, sigma, flags, c->out_linear.p,
+                           out_rgb8 ? c->out_rgb8.p : nullptr, c->own_stream);
+    if (rc) return rc;
+    if (out_linear) CU(cudaMemcpyAsync(out_linear, c->out_linear.p, n * sizeof(double), cudaMemcpyDeviceToHost, c->own_stream));
+    if (out_rgb8) CU(cudaMemcpyAsync(out_rgb8, c->out_rgb8.p, n, cudaMemcpyDeviceToHost, c->own_stream));
+    CU(cudaStreamSynchronize(c->own_stream));
+    return RTCLJ_OK;
+  });
+}
+
+int rtclj_render_denoised(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm,
+                          int32_t guide_samples, int32_t levels, const double* sigma, const int32_t* devices,
+                          int32_t n_devices, double* out_linear, uint8_t* out_rgb8, rtclj_stats* stats) {
+  return guarded([&]() -> int {
+    const auto t0 = std::chrono::steady_clock::now();
+    if (!scene) return fail(RTCLJ_E_INVALID, "null scene");
+    int rc = validate(cam, prm);
+    if (rc) return rc;
+    if (guide_samples <= 0) return fail(RTCLJ_E_INVALID, "guide_samples must be positive, got %d", guide_samples);
+    rc = check_denoise(cam->width, cam->height, levels, sigma);
+    if (rc) return rc;
+    // the guide: the colour render's camera rays (Philox stage 0 is keyed by pixel, sample and seed), shaded by normal
+    rtclj_params gp = *prm;
+    gp.spp = guide_samples;
+    gp.max_depth = 1;
+    gp.flags = RTCLJ_F_NORMAL_SHADING | (prm->flags & ~0xffffu);  // + the caller's kernel selection
+    gp.samples_per_unit = 0;
+    std::vector<std::unique_lock<std::mutex>> locks;
+    std::vector<rtclj_ctx*> ctxs;
+    rtclj_stats total, guide_total;
+    rc = lock_devices(devices, n_devices, locks, ctxs);
+    if (rc) return rc;
+    rc = render_to_root(scene, cam, prm, devices, n_devices, ctxs, &rtclj_ctx::out_linear, &total);
+    if (rc) return rc;
+    rc = render_to_root(scene, cam, &gp, devices, n_devices, ctxs, &rtclj_ctx::dn_guide64, &guide_total);
+    if (rc) return rc;
+    rtclj_ctx* const root = ctxs[0];
+    if (out_rgb8) CU(root->out_rgb8.reserve((size_t)cam->width * (size_t)cam->height * 3));
+    rc = rtclj_ctx_denoise(root, root->out_linear.p, root->dn_guide64.p, cam->width, cam->height, levels, sigma,
+                           prm->flags, root->out_linear.p, out_rgb8 ? root->out_rgb8.p : nullptr, root->own_stream);
+    if (rc) return rc;
+    rc = download_rows(root, cam, 0, 1, 0, out_linear, out_rgb8, root->own_stream);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(root->own_stream));
+    total.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = total;
     return RTCLJ_OK;
   });
 }

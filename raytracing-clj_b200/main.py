@@ -8,6 +8,7 @@
                                                               -> the same with adaptive sampling, and
                                                                  scene-samples.png (samples per pixel)
     python -m raytracing_clj_b200.main main ... --gpu-png     -> the same files, the PNGs compressed on the GPU
+    python -m raytracing_clj_b200.main main ... --denoise     -> the same files, and scene-denoised.ppm / .png
     python -m raytracing_clj_b200.main main [spp] [depth] --frames N [--gpu-png]
                                                               -> scene-0000.png ... scene-{N-1}.png, a turntable
     python -m raytracing_clj_b200.main realm                  -> scene-realm.ppm
@@ -28,6 +29,10 @@ units), and the run ends once no pixel is left.  scene-samples.png shows the sam
 With --gpu-png scene.png (and scene-samples.png) are written by the device PNG writer from the render's 8-bit
 image (DESIGN.md section 4.11): the same pixels, compressed, and only the compressed bytes leave the GPU.  Without
 it every file is the one the host writer produces.
+
+With --denoise the image is also denoised (an edge-avoiding filter guided by the normal-shaded primary render of the
+same camera and seed, DESIGN.md section 4.13) and written as scene-denoised.ppm and scene-denoised.png; with --every N
+every pass's image is denoised and written too (the guide is rendered once).  The other files do not change.
 
 With --frames N the camera circles the scene: look_from turns about the vertical axis through look_at in N steps of
 360/N degrees, frame 0 being the reference's camera, and all N frames are rendered as one camera sequence
@@ -58,11 +63,29 @@ def samples_image(samples: np.ndarray, spp: int) -> np.ndarray:
     return np.repeat(v[:, :, None], 3, axis=2)
 
 
+def _write(path: str, data: bytes) -> None:
+    with open(path, "wb") as f:
+        f.write(data)
+
+
+def _stem(out: str) -> str:
+    return out[:-4] if out.endswith(".ppm") else out
+
+
 def main_variant(spp: int = 100, depth: int = 50, out: str = "scene.ppm", seed: int = 1, every: int = 0,
-                 tolerance=None, gpu_png: bool = False):
+                 tolerance=None, gpu_png: bool = False, denoise: bool = False):
     print("config:", {"samples-per-px": spp, "max-depth": depth})
     t0 = time.perf_counter()
     png_device = 0 if gpu_png else None  # the render's device (devices default to [0])
+    guide = None
+    if denoise:  # the colour render's camera rays, shaded by normal: rendered once, for every pass
+        guide, _, _ = render.render(scenes.main_hittables(), camera.main_camera(), render.DENOISE_GUIDE_SAMPLES, 1,
+                                    seed=seed, flags=_abi.FLAGS_I, want_rgb8=False)
+
+    def write_denoised(lin, write=_write):
+        _, drgb8 = render.denoise(lin, guide, flags=_abi.FLAGS_MAIN)
+        write(_stem(out) + "-denoised.ppm", render.encode_ppm(drgb8))
+        write(_stem(out) + "-denoised.png", render.encode_png(drgb8, png_device))
     if tolerance is not None and every <= 0:
         every = max(1, spp // 10)
     if every > 0:
@@ -74,7 +97,7 @@ def main_variant(spp: int = 100, depth: int = 50, out: str = "scene.ppm", seed: 
             segments = traced = 0
             active = cam.width * cam.height
             while p.samples_done < spp and active > 0:
-                _, rgb8, st = p.step(min(n, spp - p.samples_done), want_linear=False)
+                lin, rgb8, st = p.step(min(n, spp - p.samples_done), want_linear=denoise)
                 segments += st["segments"]
                 traced += st["samples"]
                 if p.adaptive:
@@ -82,6 +105,8 @@ def main_variant(spp: int = 100, depth: int = 50, out: str = "scene.ppm", seed: 
                 if p.samples_done < spp and active > 0:  # the last image goes out below, as without --every
                     _replace(out, render.encode_ppm(rgb8))
                     _replace(png, render.encode_png(rgb8, png_device))
+                    if denoise:
+                        write_denoised(lin, _replace)
                 left = f", {active} pixels active" if p.adaptive else ""
                 print(f"{p.samples_done}/{spp} samples per pixel{left}: {out} ({1e3 * (time.perf_counter() - t0):.0f} ms)")
             if p.adaptive:
@@ -91,9 +116,11 @@ def main_variant(spp: int = 100, depth: int = 50, out: str = "scene.ppm", seed: 
                 print(f"samples traced: {traced} of {full} ({100.0 * traced / full:.1f} %); sample counts in {grey}")
         st["segments"] = segments
     else:
-        _, rgb8, st = render.render(scenes.main_hittables(), camera.main_camera(), spp, depth, seed=seed,
-                                    flags=_abi.FLAGS_MAIN, want_linear=False)
+        lin, rgb8, st = render.render(scenes.main_hittables(), camera.main_camera(), spp, depth, seed=seed,
+                                      flags=_abi.FLAGS_MAIN, want_linear=denoise)
     render.write_ppm(out, rgb8)
+    if denoise:
+        write_denoised(lin)
     png = out[:-4] + ".png" if out.endswith(".ppm") else out + ".png"
     if gpu_png:
         render.write_png(png, rgb8, png_device)
@@ -137,8 +164,8 @@ def _cli(argv):
     which = argv[0] if argv else "main"
     if which == "main":
         every, tolerance = 0, None
-        gpu_png = "--gpu-png" in argv
-        argv = [a for a in argv if a != "--gpu-png"]
+        gpu_png, denoise = "--gpu-png" in argv, "--denoise" in argv
+        argv = [a for a in argv if a not in ("--gpu-png", "--denoise")]
         if "--frames" in argv:
             i = argv.index("--frames")
             if i + 1 >= len(argv) or not argv[i + 1].isdigit() or int(argv[i + 1]) <= 0:
@@ -164,7 +191,7 @@ def _cli(argv):
             every = int(argv[i + 1])
             argv = argv[:i] + argv[i + 2:]
         main_variant(int(argv[1]) if len(argv) > 1 else 100, int(argv[2]) if len(argv) > 2 else 50, every=every,
-                     tolerance=tolerance, gpu_png=gpu_png)
+                     tolerance=tolerance, gpu_png=gpu_png, denoise=denoise)
     elif which == "realm":
         realm_variant()
     elif which == "i":

@@ -183,6 +183,61 @@ def render_png(world, cam: Camera, samples_per_px: int = 100, max_depth: int = 5
     return bytes(memoryview(store)[: n.value]), st.as_dict()
 
 
+#: the denoiser's defaults (DESIGN.md section 4.13: the sweep that chose them)
+DENOISE_LEVELS, DENOISE_SIGMA_COLOR, DENOISE_SIGMA_GUIDE, DENOISE_GUIDE_SAMPLES = 3, 0.5, 0.4, 4
+
+
+def _sigma(sigma_color, sigma_guide):
+    return (C.c_double * 2)(float(sigma_color), float(sigma_guide))
+
+
+def denoise(linear: np.ndarray, guide: np.ndarray, *, device: int = 0, levels: int = DENOISE_LEVELS,
+            sigma_color: float = DENOISE_SIGMA_COLOR, sigma_guide: float = DENOISE_SIGMA_GUIDE, flags: int = 0):
+    """The edge-avoiding a-trous filter of include/rtclj_b200.h on GPU `device` (rtclj_denoise_gpu): `linear` (the
+    colour, float64 [H,W,3]) filtered under the edges of `guide` (float64 [H,W,3], the normal-shaded primary render of
+    the same camera and seed: render(..., flags=FLAGS_I, max_depth=1)).  flags: only F_QUANT_LINEAR is read, for the
+    8-bit image.  Returns (linear float64 [H,W,3], rgb8 uint8 [H,W,3])."""
+    lin = np.ascontiguousarray(linear, dtype=np.float64)
+    gd = np.ascontiguousarray(guide, dtype=np.float64)
+    if lin.ndim != 3 or lin.shape[2] != 3 or gd.shape != lin.shape:
+        raise ValueError(f"linear and guide must be [H,W,3] images of one size, got {lin.shape} and {gd.shape}")
+    H, W, _ = lin.shape
+    out_linear = np.empty_like(lin)
+    out_rgb8 = np.empty(lin.shape, dtype=np.uint8)
+    _abi.check(_abi.lib().rtclj_denoise_gpu(int(device), lin.ctypes.data, gd.ctypes.data, W, H, int(levels),
+                                            _sigma(sigma_color, sigma_guide), int(flags), out_linear.ctypes.data,
+                                            out_rgb8.ctypes.data))
+    return out_linear, out_rgb8
+
+
+def render_denoised(world, cam: Camera, samples_per_px: int = 100, max_depth: int = 50, *, seed: int = 1,
+                    flags: int = _abi.FLAGS_MAIN, samples_per_unit: int = 0, devices: Optional[Sequence[int]] = None,
+                    shard_rows: int = 0, guide_samples: int = DENOISE_GUIDE_SAMPLES, levels: int = DENOISE_LEVELS,
+                    sigma_color: float = DENOISE_SIGMA_COLOR, sigma_guide: float = DENOISE_SIGMA_GUIDE,
+                    want_linear: bool = True, want_rgb8: bool = True):
+    """Render, guide and filter in one call (rtclj_render_denoised): the colour render as `render`, rows interleaved
+    over `devices` (default [0]) in tiles of `shard_rows` rows; the guide rendered with the same camera and seed,
+    guide_samples samples, max_depth 1 and normal shading; both assembled on devices[0] and denoised there.  Returns
+    (linear float64 [H,W,3] | None, rgb8 uint8 [H,W,3] | None, stats dict): the stats are the colour render's, except
+    total_ms, which covers the whole call."""
+    lib = _abi.lib()
+    soa = _as_soa(world)
+    sc, cm = _scene_struct(soa), _camera_struct(cam)
+    H, W = cm.height, cm.width
+    out_linear = np.zeros((H, W, 3), dtype=np.float64) if want_linear else None
+    out_rgb8 = np.zeros((H, W, 3), dtype=np.uint8) if want_rgb8 else None
+    prm = _params(samples_per_px, max_depth, seed, flags, samples_per_unit)
+    prm.shard_rows = int(shard_rows)
+    devs = list(devices) if devices else [0]
+    arr = (C.c_int32 * len(devs))(*devs)
+    st = _abi.Stats()
+    _abi.check(lib.rtclj_render_denoised(C.byref(sc), C.byref(cm), C.byref(prm), int(guide_samples), int(levels),
+                                         _sigma(sigma_color, sigma_guide), arr, len(devs),
+                                         out_linear.ctypes.data if out_linear is not None else None,
+                                         out_rgb8.ctypes.data if out_rgb8 is not None else None, C.byref(st)))
+    return out_linear, out_rgb8, st.as_dict()
+
+
 def pass_unit(width: int, height: int, samples_per_px: int, max_depth: int, flags: int = _abi.FLAGS_MAIN,
               samples_per_unit: int = 0) -> int:
     """The pass unit an accumulation of these params reports (rtclj_ctx_accum_begin): 1 in strict order, else the
@@ -309,6 +364,16 @@ class Context:
                                                    C.c_void_p(d_out or None), int(capacity), C.byref(n),
                                                    C.c_void_p(stream or None)))
         return n.value
+
+    def denoise(self, d_linear: int, d_guide: int, width: int, height: int, *, levels: int = DENOISE_LEVELS,
+                sigma_color: float = DENOISE_SIGMA_COLOR, sigma_guide: float = DENOISE_SIGMA_GUIDE, flags: int = 0,
+                d_out_linear: int = 0, d_out_rgb8: int = 0, stream: int = 0) -> None:
+        """Enqueues the denoiser (rtclj_ctx_denoise) on device pointers: d_linear / d_guide (float64 [H,W,3]) ->
+        d_out_linear (float64, may equal d_linear) and d_out_rgb8 (uint8); either output may be 0."""
+        _abi.check(_abi.lib().rtclj_ctx_denoise(self._h, C.c_void_p(d_linear or None), C.c_void_p(d_guide or None),
+                                                int(width), int(height), int(levels), _sigma(sigma_color, sigma_guide),
+                                                int(flags), C.c_void_p(d_out_linear or None),
+                                                C.c_void_p(d_out_rgb8 or None), C.c_void_p(stream or None)))
 
     def encode_ms(self) -> tuple:
         """(line lengths + scan, text write) device milliseconds of the last encode_ppm call."""
