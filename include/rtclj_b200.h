@@ -32,6 +32,9 @@
  *   rtclj_ctx_encode_png, rtclj_encode_png_gpu
  *                           a compressed PNG of the same image, written by device kernels (device / host buffers)
  *   rtclj_render_multi_png  the render loop and ppm->png as one call: several GPUs in, a compressed PNG out
+ *   rtclj_ctx_encode_apng, rtclj_encode_apng_gpu, rtclj_render_frames_apng
+ *                           not in the reference: a camera sequence as one animated PNG, encoded on the device
+ *                           (device / host buffers / render + encode)
  *   rtclj_ctx_denoise, rtclj_denoise_gpu, rtclj_render_denoised
  *                           not in the reference: an edge-avoiding filter of the rendered image, guided by
  *                           the normal-shaded primary render (device / host buffers / render + guide + filter)
@@ -438,6 +441,50 @@ int rtclj_encode_png_gpu(int32_t device, const uint8_t *rgb8, int32_t width, int
 int rtclj_render_multi_png(const rtclj_scene *scene, const rtclj_camera *camera, const rtclj_params *params,
                            const int32_t *devices, int32_t n_devices, uint8_t *out, size_t capacity, size_t *len,
                            rtclj_stats *stats);
+
+/* An animated PNG (APNG) of K >= 1 frames of one size W x H, encoded on the device (DESIGN.md section 4.14):
+ * every frame's data chunks are those of rtclj_ctx_encode_png above, so the per-frame filter, token, Huffman and
+ * stored-fallback rules are exactly that definition's.  The frames are 8-bit RGB, stored consecutively (frame stride
+ * W*H*3 bytes).  delay_num / delay_den (each 0..65535; a delay_den of 0 means 1/100 s) is every frame's duration,
+ * plays the number of loops (0: forever).  The file is, in this order:
+ *   1. the signature and IHDR exactly as rtclj_encode_png writes them;
+ *   2. acTL {num_frames K, num_plays plays};
+ *   3. frame 0: fcTL {sequence number 0, width W, height H, x 0, y 0, the delay, dispose_op 0 (NONE), blend_op 0
+ *      (SOURCE)}, then the IDAT chunks of rtclj_ctx_encode_png on frame 0, unchanged (the zlib header 78 01, one per
+ *      segment, the Adler-32);
+ *   4. each frame f >= 1: an fcTL with frame 0's fields but its own sequence number, then one fdAT per IDAT that frame f
+ *      would have in its own PNG (zlib header, each segment, Adler-32), each fdAT a 4-byte sequence number followed by
+ *      that IDAT's data;
+ *   5. IEND.
+ * fcTL and fdAT chunks share one sequence counter, from 0 in file order: with nseg = ceil(H (1 + 3W) / 65536) segments
+ * per frame, frame f >= 1 has its fcTL at 1 + (f - 1)(nseg + 3) and its fdATs follow.  Every CRC covers the chunk type
+ * and data, sequence number included.  So: without its acTL, fcTL and fdAT chunks the file is byte for byte
+ * rtclj_encode_png_gpu's PNG of frame 0, and frame f's fdAT payloads after their sequence numbers are the IDAT data of
+ * frame f's own PNG.
+ * out == NULL (d_out == NULL) is the sizing call, with no GPU work: *len receives the size with every segment stored,
+ * B + 58 + (K - 1)(B + 4 nseg + 1), B being rtclj_encode_png_gpu's sizing answer for one W x H frame.  A capacity below
+ * the exact length returns RTCLJ_E_BUFFER with *len set to the exact length.  RTCLJ_E_INVALID before any device work:
+ * K <= 0, null pointers, a delay or plays out of range, a last sequence number (K - 1)(nseg + 3) above 2^31 - 1, and
+ * whatever rtclj_ctx_encode_png refuses.  Scratch (filtered streams, staging slots) lives in the context; the frames are
+ * encoded in groups of at most 2 GiB of it (a frame that alone needs more is a group of its own), and the bytes do not
+ * depend on the grouping.  rtclj_ctx_encode_apng reads the DEVICE frames d_frames, writes DEVICE memory d_out and
+ * synchronises `stream` (the length comes back from the device). */
+int rtclj_ctx_encode_apng(rtclj_ctx *ctx, const uint8_t *d_frames, int32_t width, int32_t height, int32_t n_frames,
+                          int32_t delay_num, int32_t delay_den, int32_t plays, uint8_t *d_out, size_t capacity,
+                          size_t *len, void *stream);
+/* Host buffers in and out, the encoding on `device` (copies inside the call). */
+int rtclj_encode_apng_gpu(int32_t device, const uint8_t *frames, int32_t width, int32_t height, int32_t n_frames,
+                          int32_t delay_num, int32_t delay_den, int32_t plays, uint8_t *out, size_t capacity,
+                          size_t *len);
+/* A camera sequence as one animation: renders it as rtclj_render_frames does (rows interleaved over `n_devices` GPUs in
+ * tiles of params->shard_rows rows), assembles every frame's 8-bit rows on devices[0] by device-to-device copies and
+ * encodes them there; only the APNG crosses PCIe.  The bytes are those of rtclj_encode_apng_gpu on rtclj_render_frames'
+ * rgb8 frames, for every device list and shard_rows.  Refuses what rtclj_render_frames refuses (naming the failing
+ * frame) and what rtclj_encode_apng_gpu refuses; out == NULL is the sizing call (nothing is rendered). */
+int rtclj_render_frames_apng(const rtclj_scene *scene, const rtclj_camera *cameras, int32_t n_frames,
+                             const rtclj_params *params, int32_t delay_num, int32_t delay_den, int32_t plays,
+                             const int32_t *devices, int32_t n_devices, uint8_t *out, size_t capacity, size_t *len,
+                             rtclj_stats *stats);
 
 /* ---- Denoising: an edge-avoiding a-trous filter of a linear image, guided by a second image -- the normal-shaded
  * primary render (RTCLJ_F_NORMAL_SHADING, max_depth 1) of the same camera and seed, whose first samples are the colour

@@ -438,6 +438,65 @@
       (check! (.invokeWithArguments rtclj-encode-png-gpu [(int device) src w h out cap len]))
       (.toArray (.asSlice out 0 (.get len ValueLayout/JAVA_LONG 0)) ValueLayout/JAVA_BYTE))))
 
+;; ---- animated PNG of a camera sequence (DESIGN.md section 4.14)
+;; int rtclj_encode_apng_gpu(int32_t device, const uint8_t* frames, int32_t width, int32_t height, int32_t n_frames,
+;;                           int32_t delay_num, int32_t delay_den, int32_t plays, uint8_t* out, size_t capacity,
+;;                           size_t* len)
+(def ^:private rtclj-encode-apng-gpu
+  (downcall "rtclj_encode_apng_gpu"
+            (fd-int ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/JAVA_INT ValueLayout/JAVA_INT ValueLayout/JAVA_INT
+                    ValueLayout/JAVA_INT ValueLayout/JAVA_INT ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/JAVA_LONG
+                    ValueLayout/ADDRESS)))
+;; int rtclj_render_frames_apng(const rtclj_scene*, const rtclj_camera* cameras, int32_t n_frames, const rtclj_params*,
+;;                              int32_t delay_num, int32_t delay_den, int32_t plays, const int32_t* devices,
+;;                              int32_t n_devices, uint8_t* out, size_t capacity, size_t* len, rtclj_stats*)
+(def ^:private rtclj-render-frames-apng
+  (downcall "rtclj_render_frames_apng"
+            (fd-int ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/JAVA_INT
+                    ValueLayout/JAVA_INT ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/JAVA_INT ValueLayout/ADDRESS
+                    ValueLayout/JAVA_LONG ValueLayout/ADDRESS ValueLayout/ADDRESS)))
+
+(defn encode-apng-gpu
+  "An animated PNG of n-frames frames on the GPU: rgb8 is a byte[] of n-frames consecutive W*H*3 images (row-major
+   from the top-left pixel), the result a byte[] whose every frame carries the compressed PNG data encode-png-gpu
+   writes for it.  :delay [num den] seconds per frame (default [1 30]), :plays loops (default 0: forever)."
+  ^bytes [^bytes rgb8 width height n-frames & {:keys [device delay plays] :or {device 0 delay [1 30] plays 0}}]
+  (with-open [a (Arena/ofConfined)]
+    (let [[num den] delay
+          args (fn [out cap len] [(int device) (.allocateFrom a ValueLayout/JAVA_BYTE rgb8) (int width) (int height)
+                                  (int n-frames) (int num) (int den) (int plays) out (long cap) len])
+          len  (.allocate a 8 8)
+          _    (check! (.invokeWithArguments rtclj-encode-apng-gpu (args MemorySegment/NULL 0 len)))
+          cap  (.get len ValueLayout/JAVA_LONG 0)
+          out  (.allocate a cap 16)]
+      (check! (.invokeWithArguments rtclj-encode-apng-gpu (args out cap len)))
+      (.toArray (.asSlice out 0 (.get len ValueLayout/JAVA_LONG 0)) ValueLayout/JAVA_BYTE))))
+
+(defn render-frames-apng!
+  "render-frames and encode-apng-gpu as ONE native call (rtclj_render_frames_apng): the camera sequence `cams` rendered
+   on :devices (default [0]), every frame assembled on the first of them and encoded there as one animated PNG, which
+   comes back and is handed to a single .write.  Options as render-frames, plus :delay [num den] (default [1 30]) and
+   :plays (default 0: loop forever)."
+  [^String path bodies cams samples-per-px max-depth
+   & {:keys [devices delay plays] :or {devices [0] delay [1 30] plays 0} :as opts}]
+  (with-open [a (Arena/ofConfined)]
+    (let [k       (count cams)
+          [scene _ params] (marshal a bodies (first cams) samples-per-px max-depth opts)
+          cameras (.allocate a (* k (size :rtclj_camera)) 8)
+          _       (doseq [[i cam] (map-indexed vector cams)]
+                    (fill-camera! (.asSlice cameras (* i (size :rtclj_camera)) (size :rtclj_camera)) cam))
+          devs    (.allocateFrom a ValueLayout/JAVA_INT (int-array devices))
+          [num den] delay
+          args    (fn [out cap len] [scene cameras (int k) params (int num) (int den) (int plays) devs
+                                     (int (count devices)) out (long cap) len MemorySegment/NULL])
+          len     (.allocate a 8 8)
+          _       (check! (.invokeWithArguments rtclj-render-frames-apng (args MemorySegment/NULL 0 len)))  ; sizing
+          cap     (.get len ValueLayout/JAVA_LONG 0)
+          out     (.allocate a cap 16)]
+      (check! (.invokeWithArguments rtclj-render-frames-apng (args out cap len)))
+      (with-open [o (java.io.FileOutputStream. path)]
+        (.write (.getChannel o) (.asByteBuffer (.asSlice out 0 (.get len ValueLayout/JAVA_LONG 0))))))))
+
 ;; ---- denoising (DESIGN.md section 4.13): an edge-avoiding filter guided by the normal-shaded primary render
 ;; int rtclj_denoise_gpu(int32_t device, const double* linear, const double* guide, int32_t width, int32_t height,
 ;;                       int32_t levels, const double sigma[2], uint32_t flags, double* out_linear, uint8_t* out_rgb8)

@@ -114,6 +114,13 @@ SYMBOLS = {
     "rtclj_render_multi_png": (C.c_int, [C.POINTER(Scene), C.POINTER(Camera), C.POINTER(Params),
                                          C.POINTER(C.c_int32), C.c_int32, C.c_void_p, C.c_size_t,
                                          C.POINTER(C.c_size_t), C.POINTER(Stats)]),
+    "rtclj_ctx_encode_apng": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                        C.c_int32, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t), C.c_void_p]),
+    "rtclj_encode_apng_gpu": (C.c_int, [C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                        C.c_int32, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]),
+    "rtclj_render_frames_apng": (C.c_int, [C.POINTER(Scene), C.POINTER(Camera), C.c_int32, C.POINTER(Params), C.c_int32,
+                                           C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.c_void_p, C.c_size_t,
+                                           C.POINTER(C.c_size_t), C.POINTER(Stats)]),
     "rtclj_ctx_denoise": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                     C.POINTER(C.c_double), C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rtclj_denoise_gpu": (C.c_int, [C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,

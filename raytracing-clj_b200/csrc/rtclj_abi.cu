@@ -98,6 +98,7 @@ struct rtclj_ctx {
   DevBuf<unsigned long long> png_state;
   DevBuf<unsigned char> png_in, png_out;  // staging for the host-buffer entry points
   bool png_attr = false;                   // the PNG kernels' shared-memory limit is raised
+  bool apng_attr = false;                  // ... and the APNG kernels'
   // denoiser (rtclj_ctx_denoise): the ping-pong float32 colour images and the float32 guide; the f64 guide of the
   // host-buffer entry points (rtclj_denoise_gpu stages the colour in out_linear)
   DevBuf<float4> dn_c0, dn_c1, dn_g;
@@ -1552,24 +1553,30 @@ int lock_devices(const int32_t* devices, int32_t n_devices, std::vector<std::uni
 
 // The render loop on the locked devices ctxs (lock_devices) with one image assembled on devices[0]: each device renders
 // its shard into its own buffer `img` (out_rgb8: the 8-bit image; a DevBuf<double>: the linear one) and copies its rows
-// into the root's over NVLink.  *total receives the summed counters.
+// into the root's over NVLink.  *total receives the summed counters.  n_frames > 0: the camera sequence
+// cam[0 .. n_frames) (rtclj_ctx_render_frames), `img` holds n_frames consecutive images.
 template <class T>
 int render_to_root(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm, const int32_t* devices,
-                   int32_t n_devices, const std::vector<rtclj_ctx*>& ctxs, DevBuf<T> rtclj_ctx::*img, rtclj_stats* total) {
+                   int32_t n_devices, const std::vector<rtclj_ctx*>& ctxs, DevBuf<T> rtclj_ctx::*img, rtclj_stats* total,
+                   int n_frames = 0) {
   constexpr bool kLinear = std::is_same<T, double>::value;
   const size_t npix = (size_t)cam->width * (size_t)cam->height;
+  const int nimg = std::max(n_frames, 1);
   rtclj_ctx* root = ctxs[0];
   CU(cudaSetDevice(root->device));
-  CU((root->*img).reserve(npix * 3));
+  CU((root->*img).reserve(npix * 3 * (size_t)nimg));
   std::vector<rtclj_stats> st((size_t)n_devices);
   int rc = run_on_devices(n_devices, [&](int d) -> int {
     rtclj_ctx* c = ctxs[(size_t)d];
     const rtclj_params q = shard_params(prm, devices, d, n_devices);
     int r = rtclj_ctx_set_scene(c, scene);
     if (r) return r;
-    if (c != root) CU((c->*img).reserve(npix * 3));
+    if (c != root) CU((c->*img).reserve(npix * 3 * (size_t)nimg));
     T* mine = (c->*img).p;
-    r = rtclj_ctx_render(c, cam, &q, kLinear ? (void*)mine : nullptr, kLinear ? nullptr : (void*)mine, c->own_stream);
+    void* lin = kLinear ? (void*)mine : nullptr;
+    void* rgb = kLinear ? nullptr : (void*)mine;
+    r = n_frames > 0 ? rtclj_ctx_render_frames(c, cam, n_frames, &q, lin, rgb, c->own_stream)
+                     : rtclj_ctx_render(c, cam, &q, lin, rgb, c->own_stream);
     if (r) return r;
     if (c != root) {  // this shard's rows -> the root's image, device to device
       int can = 0;
@@ -1577,13 +1584,15 @@ int render_to_root(const rtclj_scene* scene, const rtclj_camera* cam, const rtcl
         const cudaError_t e = cudaDeviceEnablePeerAccess(root->device, 0);
         if (e != cudaSuccess) cudaGetLastError();  // already enabled: fine; otherwise the copy is staged by the driver
       }
-      char* dst = (char*)(root->*img).p;
-      const char* src = (const char*)mine;
       std::vector<Piece> pieces;
       plan_pieces((size_t)cam->height, (size_t)cam->width * 3 * sizeof(T), q.shard_index, q.shard_count, q.shard_rows, (size_t)1 << 40, pieces);
-      for (const Piece& pc : pieces) {
-        if (pc.height == 1) CU(cudaMemcpyAsync(dst + pc.off, src + pc.off, pc.width, cudaMemcpyDefault, c->own_stream));
-        else CU(cudaMemcpy2DAsync(dst + pc.off, pc.pitch, src + pc.off, pc.pitch, pc.width, pc.height, cudaMemcpyDefault, c->own_stream));
+      for (int f = 0; f < nimg; ++f) {
+        char* dst = (char*)((root->*img).p + npix * 3 * (size_t)f);
+        const char* src = (const char*)(mine + npix * 3 * (size_t)f);
+        for (const Piece& pc : pieces) {
+          if (pc.height == 1) CU(cudaMemcpyAsync(dst + pc.off, src + pc.off, pc.width, cudaMemcpyDefault, c->own_stream));
+          else CU(cudaMemcpy2DAsync(dst + pc.off, pc.pitch, src + pc.off, pc.pitch, pc.width, pc.height, cudaMemcpyDefault, c->own_stream));
+        }
       }
     }
     return rtclj_ctx_stats(c, c->own_stream, &st[(size_t)d]);  // synchronises: render and copies are done
@@ -1628,6 +1637,25 @@ int png_sizes(int32_t width, int32_t height, size_t* nf, size_t* bound) {
   const size_t full = N / kPngSeg, rest = N - full * kPngSeg;
   *nf = N;
   *bound = kPngHead + kPngTail + full * (12 + kPngSeg + 10) + (rest ? 12 + rest + 5 * ((rest + 65534) / 65535) : 0);
+  return RTCLJ_OK;
+}
+
+// The checks of an APNG (include/rtclj_b200.h) and the sizing call's answer: the filtered bytes *nf and segments *nseg
+// of one frame, and *bound, the file with every segment stored: B + 58 + (K - 1)(B + 4 nseg + 1), B being png_sizes'
+// bound of one frame.
+int apng_sizes(int32_t width, int32_t height, int32_t n_frames, int32_t delay_num, int32_t delay_den, int32_t plays,
+               size_t* nf, size_t* nseg, size_t* bound) {
+  if (n_frames <= 0) return fail(RTCLJ_E_INVALID, "n_frames must be positive, got %d", n_frames);
+  if (delay_num < 0 || delay_num > 65535 || delay_den < 0 || delay_den > 65535)
+    return fail(RTCLJ_E_INVALID, "delay %d/%d: numerator and denominator must be in 0..65535", delay_num, delay_den);
+  if (plays < 0) return fail(RTCLJ_E_INVALID, "plays must be >= 0 (0: loop forever), got %d", plays);
+  size_t B = 0;
+  int rc = png_sizes(width, height, nf, &B);
+  if (rc) return rc;
+  *nseg = (*nf + kPngSeg - 1) / kPngSeg;
+  if ((unsigned long long)(n_frames - 1) * (*nseg + 3) > 0x7fffffffull)
+    return fail(RTCLJ_E_INVALID, "%d frames of %zu segments: the last sequence number would exceed 2^31 - 1", n_frames, *nseg);
+  *bound = B + 58 + (size_t)(n_frames - 1) * (B + 4 * *nseg + 1);
   return RTCLJ_OK;
 }
 
@@ -1910,6 +1938,143 @@ int rtclj_encode_png_gpu(int32_t device, const uint8_t* rgb8, int32_t width, int
     if (need > capacity) return fail(RTCLJ_E_BUFFER, "PNG needs %zu bytes, capacity is %zu", need, capacity);
     CU(cudaMemcpyAsync(out, c->png_out.p, need, cudaMemcpyDeviceToHost, c->own_stream));
     CU(cudaStreamSynchronize(c->own_stream));
+    return RTCLJ_OK;
+  });
+}
+
+// ---- animated PNG of a sequence of frames (DESIGN.md section 4.14; the format: include/rtclj_b200.h).  The frames
+// are encoded in groups whose scratch -- filtered streams, staging slots, records -- stays within
+// kAccumSampleBufBytes; three launches per group, and each group's place kernel finds where it starts in the device
+// state its predecessor left, so nothing waits for the host between groups.
+int rtclj_ctx_encode_apng(rtclj_ctx* c, const uint8_t* d_frames, int32_t width, int32_t height, int32_t n_frames,
+                          int32_t delay_num, int32_t delay_den, int32_t plays, uint8_t* d_out, size_t capacity,
+                          size_t* len, void* stream_) {
+  return guarded([&]() -> int {
+    if (!c || !len) return fail(RTCLJ_E_INVALID, "null ctx or len");
+    size_t N = 0, nseg = 0, bound = 0;
+    int rc = apng_sizes(width, height, n_frames, delay_num, delay_den, plays, &N, &nseg, &bound);
+    if (rc) return rc;
+    if (!d_out) { *len = bound; return RTCLJ_OK; }
+    if (!d_frames) return fail(RTCLJ_E_INVALID, "null frames");
+    cudaStream_t stream = (cudaStream_t)stream_;
+    CU(cudaSetDevice(c->device));
+    if (!c->apng_attr) {
+      CU(cudaFuncSetAttribute(png_deflate_frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PngDeflateSmem)));
+      CU(cudaFuncSetAttribute(png_place_frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PngPlaceSmem)));
+      c->apng_attr = true;
+    }
+    static const PngCrcShifts shifts = png_crc_shifts();
+    const size_t frame_scratch = nseg * ((size_t)kPngSeg + kPngSlot + sizeof(PngSegRec));
+    const size_t group = std::max<size_t>(1, std::min<size_t>((size_t)n_frames, kAccumSampleBufBytes / frame_scratch));
+    CU(c->png_f.reserve(group * nseg * kPngSeg));
+    CU(c->png_stage.reserve(group * nseg * kPngSlot));
+    CU(c->png_rec.reserve(group * nseg));
+    CU(c->png_state.reserve(3));
+    const size_t row_bytes = (size_t)width * 3, frame_bytes = row_bytes * (size_t)height;
+    auto pass = [&](uint8_t* out) -> int {  // out == nullptr: the length only
+      for (size_t f0 = 0, i = 0; f0 < (size_t)n_frames; f0 += group, ++i) {
+        const size_t g = std::min(group, (size_t)n_frames - f0);
+        png_filter_frames_kernel<<<(unsigned)(g * (size_t)height), kPngFilterThreads, 0, stream>>>(
+            d_frames + f0 * frame_bytes, row_bytes, (unsigned)height, nseg * kPngSeg, c->png_f.p);
+        CU(cudaGetLastError());
+        png_deflate_frames_kernel<<<(unsigned)(g * nseg), kPngThreads, sizeof(PngDeflateSmem), stream>>>(
+            c->png_f.p, N, nseg, c->png_stage.p, c->png_rec.p);
+        CU(cudaGetLastError());
+        ApngGroup a;
+        a.F = c->png_f.p; a.staging = c->png_stage.p; a.rec = c->png_rec.p; a.out = out; a.state = c->png_state.p;
+        a.N = N; a.nseg = (unsigned)nseg;
+        a.frames = (unsigned)g; a.first = (unsigned)f0; a.total = (unsigned)n_frames;
+        a.width = (unsigned)width; a.height = (unsigned)height;
+        a.delay_num = (unsigned)delay_num; a.delay_den = (unsigned)delay_den; a.plays = (unsigned)plays;
+        a.parity = (int)(i & 1); a.count_only = out == nullptr;
+        png_place_frames_kernel<<<(unsigned)(g * nseg + g + 1), kPngThreads, sizeof(PngPlaceSmem), stream>>>(a, shifts);
+        CU(cudaGetLastError());
+      }
+      return RTCLJ_OK;
+    };
+    unsigned long long total = 0;
+    if (capacity < bound) {  // the exact length first: the buffer may be too small for it
+      rc = pass(nullptr);
+      if (rc) return rc;
+      CU(cudaMemcpyAsync(&total, c->png_state.p + 2, sizeof total, cudaMemcpyDeviceToHost, stream));
+      CU(cudaStreamSynchronize(stream));
+      *len = (size_t)total;
+      if ((size_t)total > capacity) return fail(RTCLJ_E_BUFFER, "APNG needs %llu bytes, capacity is %zu", total, capacity);
+    }
+    rc = pass(d_out);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(&total, c->png_state.p + 2, sizeof total, cudaMemcpyDeviceToHost, stream));
+    CU(cudaStreamSynchronize(stream));
+    *len = (size_t)total;
+    return RTCLJ_OK;
+  });
+}
+
+int rtclj_encode_apng_gpu(int32_t device, const uint8_t* frames, int32_t width, int32_t height, int32_t n_frames,
+                          int32_t delay_num, int32_t delay_den, int32_t plays, uint8_t* out, size_t capacity,
+                          size_t* len) {
+  return guarded([&]() -> int {
+    if (!len) return fail(RTCLJ_E_INVALID, "null len");
+    size_t N = 0, nseg = 0, bound = 0;
+    int rc = apng_sizes(width, height, n_frames, delay_num, delay_den, plays, &N, &nseg, &bound);
+    if (rc) return rc;
+    if (!out) { *len = bound; return RTCLJ_OK; }
+    if (!frames) return fail(RTCLJ_E_INVALID, "null frames");
+    std::unique_lock<std::mutex> lock;
+    rtclj_ctx* c = nullptr;
+    rc = cached_ctx(device, lock, &c);
+    if (rc) return rc;
+    CU(cudaSetDevice(c->device));
+    const size_t bytes = (size_t)width * (size_t)height * 3 * (size_t)n_frames;
+    CU(c->png_in.reserve(bytes));
+    CU(c->png_out.reserve(bound));
+    CU(cudaMemcpyAsync(c->png_in.p, frames, bytes, cudaMemcpyHostToDevice, c->own_stream));
+    size_t need = 0;
+    rc = rtclj_ctx_encode_apng(c, c->png_in.p, width, height, n_frames, delay_num, delay_den, plays, c->png_out.p,
+                               bound, &need, c->own_stream);
+    if (rc) return rc;
+    *len = need;
+    if (need > capacity) return fail(RTCLJ_E_BUFFER, "APNG needs %zu bytes, capacity is %zu", need, capacity);
+    CU(cudaMemcpyAsync(out, c->png_out.p, need, cudaMemcpyDeviceToHost, c->own_stream));
+    CU(cudaStreamSynchronize(c->own_stream));
+    return RTCLJ_OK;
+  });
+}
+
+// A camera sequence rendered as rtclj_render_frames renders it, every frame's 8-bit rows assembled on devices[0] by
+// device-to-device copies and encoded there: only the APNG crosses PCIe.
+int rtclj_render_frames_apng(const rtclj_scene* scene, const rtclj_camera* cams, int32_t n_frames,
+                             const rtclj_params* prm, int32_t delay_num, int32_t delay_den, int32_t plays,
+                             const int32_t* devices, int32_t n_devices, uint8_t* out, size_t capacity, size_t* len,
+                             rtclj_stats* stats) {
+  return guarded([&]() -> int {
+    const auto t0 = std::chrono::steady_clock::now();
+    if (!scene || !len) return fail(RTCLJ_E_INVALID, "null scene or len");
+    int rc = check_frames(cams, n_frames, prm);
+    if (rc) return rc;
+    size_t N = 0, nseg = 0, bound = 0;
+    rc = apng_sizes(cams[0].width, cams[0].height, n_frames, delay_num, delay_den, plays, &N, &nseg, &bound);
+    if (rc) return rc;
+    if (!out) { *len = bound; return RTCLJ_OK; }  // sizing call: the stored bound, nothing is rendered
+    std::vector<std::unique_lock<std::mutex>> locks;
+    std::vector<rtclj_ctx*> ctxs;
+    rtclj_stats total;
+    rc = lock_devices(devices, n_devices, locks, ctxs);
+    if (rc) return rc;
+    rc = render_to_root(scene, cams, prm, devices, n_devices, ctxs, &rtclj_ctx::out_rgb8, &total, n_frames);
+    if (rc) return rc;
+    rtclj_ctx* const root = ctxs[0];
+    CU(root->png_out.reserve(bound));
+    size_t need = 0;
+    rc = rtclj_ctx_encode_apng(root, root->out_rgb8.p, cams[0].width, cams[0].height, n_frames, delay_num, delay_den,
+                               plays, root->png_out.p, bound, &need, root->own_stream);
+    if (rc) return rc;
+    *len = need;
+    if (need > capacity) return fail(RTCLJ_E_BUFFER, "APNG needs %zu bytes, capacity is %zu", need, capacity);
+    CU(cudaMemcpyAsync(out, root->png_out.p, need, cudaMemcpyDeviceToHost, root->own_stream));
+    CU(cudaStreamSynchronize(root->own_stream));
+    total.total_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = total;
     return RTCLJ_OK;
   });
 }

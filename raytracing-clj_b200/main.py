@@ -11,6 +11,8 @@
     python -m raytracing_clj_b200.main main ... --denoise     -> the same files, and scene-denoised.ppm / .png
     python -m raytracing_clj_b200.main main [spp] [depth] --frames N [--gpu-png]
                                                               -> scene-0000.png ... scene-{N-1}.png, a turntable
+    python -m raytracing_clj_b200.main main [spp] [depth] --frames N --apng
+                                                              -> scene.apng, the turntable as one animation
     python -m raytracing_clj_b200.main realm                  -> scene-realm.ppm
     python -m raytracing_clj_b200.main i                      -> scene-i.ppm
 
@@ -37,7 +39,11 @@ every pass's image is denoised and written too (the guide is rendered once).  Th
 With --frames N the camera circles the scene: look_from turns about the vertical axis through look_at in N steps of
 360/N degrees, frame 0 being the reference's camera, and all N frames are rendered as one camera sequence
 (rtclj_render_frames, DESIGN.md section 4.12).  Each frame is written as a PNG only; frame 0 has the pixels of
-scene.png from a run without --frames."""
+scene.png from a run without --frames.
+
+With --frames N --apng the turntable is written as one animated PNG instead, scene.apng: 1/30 s per frame, looping
+forever, rendered and encoded on the GPU in one call (rtclj_render_frames_apng, DESIGN.md section 4.14); its frames
+have the pixels of the scene-NNNN.png files.  --apng needs --frames."""
 from __future__ import annotations
 
 import os
@@ -131,9 +137,16 @@ def main_variant(spp: int = 100, depth: int = 50, out: str = "scene.ppm", seed: 
 
 
 def frames_variant(spp: int = 100, depth: int = 50, n_frames: int = 60, out: str = "scene", seed: int = 1,
-                   gpu_png: bool = False):
+                   gpu_png: bool = False, apng: bool = False):
     print("config:", {"samples-per-px": spp, "max-depth": depth, "frames": n_frames})
     t0 = time.perf_counter()
+    if apng:
+        data = render.render_frames_apng(scenes.main_hittables(), camera.turntable_cameras(n_frames), spp, depth,
+                                         seed=seed, flags=_abi.FLAGS_MAIN, delay=(1, 30), plays=0)
+        _write(f"{out}.apng", data)
+        print(f'"Elapsed time: {1e3 * (time.perf_counter() - t0):.3f} msecs"  ({out}.apng, {n_frames} frames, '
+              f'{len(data)} bytes)')
+        return
     _, rgb8, st = render.render_frames(scenes.main_hittables(), camera.turntable_cameras(n_frames), spp, depth,
                                        seed=seed, flags=_abi.FLAGS_MAIN, want_linear=False)
     t1 = time.perf_counter()
@@ -164,8 +177,10 @@ def _cli(argv):
     which = argv[0] if argv else "main"
     if which == "main":
         every, tolerance = 0, None
-        gpu_png, denoise = "--gpu-png" in argv, "--denoise" in argv
-        argv = [a for a in argv if a not in ("--gpu-png", "--denoise")]
+        gpu_png, denoise, apng = "--gpu-png" in argv, "--denoise" in argv, "--apng" in argv
+        argv = [a for a in argv if a not in ("--gpu-png", "--denoise", "--apng")]
+        if apng and "--frames" not in argv:
+            raise SystemExit("--apng writes a camera sequence: it needs --frames N")
         if "--frames" in argv:
             i = argv.index("--frames")
             if i + 1 >= len(argv) or not argv[i + 1].isdigit() or int(argv[i + 1]) <= 0:
@@ -173,7 +188,7 @@ def _cli(argv):
             n_frames = int(argv[i + 1])
             argv = argv[:i] + argv[i + 2:]
             frames_variant(int(argv[1]) if len(argv) > 1 else 100, int(argv[2]) if len(argv) > 2 else 50, n_frames,
-                           gpu_png=gpu_png)
+                           gpu_png=gpu_png, apng=apng)
             return
         if "--tolerance" in argv:
             i = argv.index("--tolerance")

@@ -183,6 +183,33 @@ def render_png(world, cam: Camera, samples_per_px: int = 100, max_depth: int = 5
     return bytes(memoryview(store)[: n.value]), st.as_dict()
 
 
+def render_frames_apng(world, cameras: Sequence, samples_per_px: int = 100, max_depth: int = 50, *, seed: int = 1,
+                       flags: int = _abi.FLAGS_MAIN, samples_per_unit: int = 0, devices: Optional[Sequence[int]] = None,
+                       shard_rows: int = 0, delay=(1, 30), plays: int = 0) -> bytes:
+    """A camera sequence as one animated PNG (rtclj_render_frames_apng): the frames rendered as `render_frames` renders
+    them, rows interleaved over `devices` (default [0]) in tiles of `shard_rows` rows, assembled on devices[0] and
+    encoded there; only the file leaves the GPU.  delay = (numerator, denominator) seconds per frame, plays = loops
+    (0: forever).  The bytes are those of encode_apng(rgb8 of render_frames(...), delay=delay, plays=plays)."""
+    lib = _abi.lib()
+    soa = _as_soa(world)
+    sc = _scene_struct(soa)
+    arr, n = _camera_array(cameras)
+    prm = _params(samples_per_px, max_depth, seed, flags, samples_per_unit)
+    prm.shard_rows = int(shard_rows)
+    devs = list(devices) if devices else [0]
+    darr = (C.c_int32 * len(devs))(*devs)
+    num, den = (int(x) for x in delay)
+    size = C.c_size_t()
+    _abi.check(lib.rtclj_render_frames_apng(C.byref(sc), arr, n, C.byref(prm), num, den, int(plays), darr, len(devs),
+                                            None, 0, C.byref(size), None))
+    store = bytearray(size.value)
+    buf = (C.c_char * size.value).from_buffer(store)
+    _abi.check(lib.rtclj_render_frames_apng(C.byref(sc), arr, n, C.byref(prm), num, den, int(plays), darr, len(devs),
+                                            buf, size.value, C.byref(size), None))
+    del buf
+    return bytes(memoryview(store)[: size.value])
+
+
 #: the denoiser's defaults (DESIGN.md section 4.13: the sweep that chose them)
 DENOISE_LEVELS, DENOISE_SIGMA_COLOR, DENOISE_SIGMA_GUIDE, DENOISE_GUIDE_SAMPLES = 3, 0.5, 0.4, 4
 
@@ -365,6 +392,18 @@ class Context:
                                                    C.c_void_p(stream or None)))
         return n.value
 
+    def encode_apng(self, d_frames: int, width: int, height: int, n_frames: int, d_out: int = 0, capacity: int = 0, *,
+                    delay=(1, 30), plays: int = 0, stream: int = 0) -> int:
+        """The animated PNG writer (rtclj_ctx_encode_apng) on device pointers: n_frames consecutive uint8 [H,W,3]
+        frames at d_frames -> APNG at d_out.  d_out = 0 is the sizing call (a sufficient capacity, no GPU work).
+        Returns the file's length in bytes; synchronises `stream`."""
+        n = C.c_size_t()
+        num, den = (int(x) for x in delay)
+        _abi.check(_abi.lib().rtclj_ctx_encode_apng(self._h, C.c_void_p(d_frames or None), int(width), int(height),
+                                                    int(n_frames), num, den, int(plays), C.c_void_p(d_out or None),
+                                                    int(capacity), C.byref(n), C.c_void_p(stream or None)))
+        return n.value
+
     def denoise(self, d_linear: int, d_guide: int, width: int, height: int, *, levels: int = DENOISE_LEVELS,
                 sigma_color: float = DENOISE_SIGMA_COLOR, sigma_guide: float = DENOISE_SIGMA_GUIDE, flags: int = 0,
                 d_out_linear: int = 0, d_out_rgb8: int = 0, stream: int = 0) -> None:
@@ -514,6 +553,26 @@ def encode_png(rgb8: np.ndarray, device: int | None = None) -> bytes:
     if device is None:
         return _two_call(_abi.lib().rtclj_encode_png, img)
     return _two_call(_abi.lib().rtclj_encode_png_gpu, img, int(device))
+
+
+def encode_apng(frames: np.ndarray, device: int = 0, delay=(1, 30), plays: int = 0) -> bytes:
+    """An animated PNG of `frames` (uint8 [K,H,W,3]) written by the device PNG writer on GPU `device`
+    (rtclj_encode_apng_gpu, DESIGN.md section 4.14): each frame's data are those of encode_png(frame, device).
+    delay = (numerator, denominator) seconds per frame, plays = loops (0: forever)."""
+    img = np.ascontiguousarray(frames, dtype=np.uint8)
+    if img.ndim != 4 or img.shape[3] != 3:
+        raise ValueError(f"frames must be a [K,H,W,3] array, got shape {img.shape}")
+    K, H, W, _ = img.shape
+    num, den = (int(x) for x in delay)
+    lib = _abi.lib()
+    n = C.c_size_t()
+    _abi.check(lib.rtclj_encode_apng_gpu(int(device), img.ctypes.data, W, H, K, num, den, int(plays), None, 0, C.byref(n)))
+    store = bytearray(n.value)
+    buf = (C.c_char * n.value).from_buffer(store)
+    _abi.check(lib.rtclj_encode_apng_gpu(int(device), img.ctypes.data, W, H, K, num, den, int(plays), buf, n.value,
+                                         C.byref(n)))
+    del buf
+    return bytes(memoryview(store)[: n.value])
 
 
 def decode_ppm(text: bytes) -> np.ndarray:
