@@ -21,6 +21,8 @@
  *   rtclj_ctx_accum_*, rtclj_progressive_*
  *                           the same loop run in passes of samples (progressive rendering),
  *                           bit-identical to a one-shot render after every pass
+ *   rtclj_ctx_accum_begin_frames, rtclj_progressive_create_frames
+ *                           the same passes over a camera sequence, every frame's live pixels in shared launches
  *   rtclj_quantise_rgb8     write-color! / linear->gamma / clamp,
  *                           src/raytracing.clj:19-26 ; realm/raytracing.clj:246-249,356-357
  *   rtclj_encode_ppm_p3     the P3 writer, src/raytracing.clj:172-175 ;
@@ -355,6 +357,35 @@ int rtclj_progressive_create_adaptive(const rtclj_scene *scene, const rtclj_came
                                       const int32_t *devices, int32_t n_devices, int32_t *pass_unit,
                                       rtclj_progressive **out);
 int rtclj_progressive_noise(rtclj_progressive *p, int32_t *samples, double *noise, uint64_t *active_pixels);
+
+/* ---- Accumulations over frames: a plain or adaptive accumulation of a camera sequence (n_frames >= 1 cameras of one
+ * scene and one size, as rtclj_ctx_render_frames takes them), every frame's live pixels in shared launches
+ * (DESIGN.md section 4.15).  A turntable rendered to a noise target: each pixel of each frame stops once it is clean.
+ *   - tolerance == NULL: a plain accumulation (rtclj_ctx_accum_begin's rules); else an adaptive one with this tolerance
+ *     and min_samples (rtclj_ctx_accum_begin_adaptive's rules).  The pass unit is the single frame's.
+ *   - Stepping, noise and teardown are the calls above, unchanged: rtclj_ctx_accum_step / rtclj_ctx_accum_noise /
+ *     rtclj_ctx_stats and rtclj_progressive_step / rtclj_progressive_noise / rtclj_progressive_destroy.  Their buffers
+ *     hold the n_frames frames one after the other: images W*H*3 values per frame, the sample-count map W*H int32 per
+ *     frame, the noise estimate W*H*3 doubles per frame; active_pixels is the sum over the frames.
+ *   - After every step frame f -- linear image, 8-bit image, sample-count map and noise estimate -- is bit-identical to
+ *     a single-camera accumulation of cameras[f] with the same params, tolerance and min_samples stepped with the same
+ *     pass sizes, for every kernel choice, device list, shard_rows and n_frames.
+ *   - RTCLJ_E_INVALID before any device work, nothing begun: whatever rtclj_ctx_render_frames refuses (the message names
+ *     the frame), whatever an accumulation refuses (RTCLJ_F_WAVE_KERNEL, RTCLJ_F_SPLIT_KERNEL, spp > 2^30) and whatever
+ *     an adaptive accumulation refuses (tolerance, min_samples).
+ *   - Lifetime as above: rtclj_ctx_set_scene ends the accumulation, a failed pass ends it, a new begin replaces it.
+ *   - Memory: the state of every frame stays resident, 24 B per pixel of the shard per frame (+ 33 B adaptive); a failed
+ *     allocation returns RTCLJ_E_CUDA and leaves no accumulation active.  A pass runs in launches of at most 128 frames
+ *     and fewer than 2^32 work units (strict order: sub-passes within the 2 GiB of per-sample colours); no output bit
+ *     depends on this grouping. */
+int rtclj_ctx_accum_begin_frames(rtclj_ctx *ctx, const rtclj_camera *cameras, int32_t n_frames,
+                                 const rtclj_params *params, const double *tolerance /* NULL: plain; else abs, rel */,
+                                 int32_t min_samples, int32_t *pass_unit, void *stream);
+/* host buffers, rows interleaved over `n_devices` GPUs as rtclj_progressive_create does */
+int rtclj_progressive_create_frames(const rtclj_scene *scene, const rtclj_camera *cameras, int32_t n_frames,
+                                    const rtclj_params *params, const double *tolerance, int32_t min_samples,
+                                    const int32_t *devices, int32_t n_devices, int32_t *pass_unit,
+                                    rtclj_progressive **out);
 
 /* Measures this GPU's arithmetic peaks with pure-FMA kernels (no memory traffic): scalar
  * FFMA, packed FFMA2 and fp64 DFMA, in TFLOP/s (2 flops per FMA), plus the SM count.

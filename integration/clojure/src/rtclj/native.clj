@@ -362,12 +362,73 @@
             (.invokeWithArguments rtclj-progressive-destroy [handle])
             (throw t)))))))
 
+;; ---- accumulations over frames: a camera sequence accumulated in shared launches (DESIGN.md 4.15)
+;; int rtclj_progressive_create_frames(const rtclj_scene*, const rtclj_camera* cameras, int32_t n_frames,
+;;                                     const rtclj_params*, const double* tolerance, int32_t min_samples,
+;;                                     const int32_t* devices, int32_t n_devices, int32_t* pass_unit,
+;;                                     rtclj_progressive** out)
+(def ^:private rtclj-progressive-create-frames
+  (downcall "rtclj_progressive_create_frames"
+            (fd-int ValueLayout/ADDRESS ValueLayout/ADDRESS ValueLayout/JAVA_INT ValueLayout/ADDRESS
+                    ValueLayout/ADDRESS ValueLayout/JAVA_INT ValueLayout/ADDRESS ValueLayout/JAVA_INT
+                    ValueLayout/ADDRESS ValueLayout/ADDRESS)))
+
+(defn- progressive-frames*
+  "rtclj_progressive_create_frames with tolerance `tol` ([abs rel], or nil: plain) and min-samples `least`."
+  [bodies cams samples-per-px max-depth tol least {:keys [devices] :or {devices [0]} :as opts}]
+  (with-open [a (Arena/ofConfined)]
+    (let [cam0    (first cams)
+          w       (long (:image-width cam0))
+          h       (long (:image-height cam0))
+          k       (count cams)
+          [scene _ params] (marshal a bodies cam0 samples-per-px max-depth opts)
+          cameras (.allocate a (* (max k 1) (size :rtclj_camera)) 8)
+          _       (doseq [[i cam] (map-indexed vector cams)]
+                    (fill-camera! (.asSlice cameras (* i (size :rtclj_camera)) (size :rtclj_camera)) cam))
+          unit    (.allocate a 4 4)
+          slot    (.allocate a 8 8)]
+      (check! (.invokeWithArguments rtclj-progressive-create-frames
+                                    [scene cameras (int k) params
+                                     (if tol (.allocateFrom a ValueLayout/JAVA_DOUBLE (double-array tol)) MemorySegment/NULL)
+                                     (int least)
+                                     (.allocateFrom a ValueLayout/JAVA_INT (int-array devices)) (int (count devices))
+                                     unit slot]))
+      (let [handle (.get slot ValueLayout/ADDRESS 0)]
+        (try
+          (let [[linear free-linear!] (pinned-doubles a (* 3 w h k))
+                [rgb8 free-rgb8!]     (pinned-bytes a (* 3 w h k))]
+            {:handle handle :pass-unit (.get unit ValueLayout/JAVA_INT 0) :samples-per-px samples-per-px
+             :width w :height h :frames k :linear linear :rgb8 rgb8 :free! (fn [] (free-linear!) (free-rgb8!))})
+          (catch Throwable t
+            (.invokeWithArguments rtclj-progressive-destroy [handle])
+            (throw t)))))))
+
+(defn progressive-frames
+  "Begins a progressive render of a camera sequence (`cams`, camera maps of one image size, as render-frames takes
+   them): all frames accumulate in shared launches, and after every step frame f is bit-identical to (progressive
+   bodies (nth cams f) ...) stepped alike.  Use progressive-step! (its images hold the frames one after the other,
+   W*H*3 values each) and progressive-close! on the handle."
+  [bodies cams samples-per-px max-depth & {:as opts}]
+  (progressive-frames* bodies cams samples-per-px max-depth nil 0 opts))
+
+(defn progressive-frames-adaptive
+  "progressive-frames with adaptive sampling: every pass traces only the pixels of every frame whose noise estimate
+   is still above abs-tol + rel-tol * |mean| (see progressive-adaptive, whose :min-samples default it shares); frame f
+   is bit-identical to (progressive-adaptive bodies (nth cams f) ...) stepped alike.  progressive-noise returns the
+   frames' sample counts and noise one after the other and the active pixels of all frames."
+  [bodies cams samples-per-px max-depth abs-tol rel-tol & {:keys [min-samples] :as opts}]
+  (let [least (or min-samples
+                  (let [probe (progressive-frames bodies (take 1 cams) samples-per-px max-depth opts)]
+                    (try (* 2 (:pass-unit probe)) (finally (progressive-close! probe)))))]
+    (progressive-frames* bodies cams samples-per-px max-depth [abs-tol rel-tol] least opts)))
+
 (defn progressive-noise
   "After a step of a progressive-adaptive render: {:samples int[W*H], the samples each pixel has, :stderr
-   double[W*H*3], its noise estimate, :active, the pixels the next pass traces (0: the render is done)}."
+   double[W*H*3], its noise estimate, :active, the pixels the next pass traces (0: the render is done)}.  A render of
+   frames returns every frame's, one after the other."
   [p]
   (with-open [a (Arena/ofConfined)]
-    (let [n       (* (long (:width p)) (long (:height p)))
+    (let [n       (* (long (:width p)) (long (:height p)) (long (:frames p 1)))
           samples (.allocate a (* 4 n) 8)
           stderr  (.allocate a (* 24 n) 8)
           active  (.allocate a 8 8)]

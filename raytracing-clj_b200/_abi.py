@@ -93,6 +93,11 @@ SYMBOLS = {
                                                     C.POINTER(C.c_double), C.c_int32, C.POINTER(C.c_int32), C.c_int32,
                                                     C.POINTER(C.c_int32), C.POINTER(C.c_void_p)]),
     "rtclj_progressive_noise": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)]),
+    "rtclj_ctx_accum_begin_frames": (C.c_int, [C.c_void_p, C.POINTER(Camera), C.c_int32, C.POINTER(Params),
+                                               C.POINTER(C.c_double), C.c_int32, C.POINTER(C.c_int32), C.c_void_p]),
+    "rtclj_progressive_create_frames": (C.c_int, [C.POINTER(Scene), C.POINTER(Camera), C.c_int32, C.POINTER(Params),
+                                                  C.POINTER(C.c_double), C.c_int32, C.POINTER(C.c_int32), C.c_int32,
+                                                  C.POINTER(C.c_int32), C.POINTER(C.c_void_p)]),
     "rtclj_calibrate_peaks": (C.c_int, [C.c_int32, C.POINTER(C.c_double), C.POINTER(C.c_double),
                                         C.POINTER(C.c_double), C.POINTER(C.c_int32)]),
     "rtclj_quantise_rgb8": (C.c_int, [C.c_void_p, C.c_size_t, C.c_uint32, C.c_void_p]),

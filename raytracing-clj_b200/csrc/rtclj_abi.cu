@@ -119,10 +119,18 @@ struct rtclj_ctx {
     bool adaptive = false;
     double abs_tol = 0.0, rel_tol = 0.0;
     int min_samples = 0;
+    // an accumulation over frames (rtclj_ctx_accum_begin_frames; DESIGN.md section 4.15): cam is cams[0].  Its state
+    // holds the frames one after the other; a pass runs in launch groups of frames [f0, f0 + n), whose state starts at
+    // local pixel f0 * (pixels of a frame) and whose list count is list_aux[aux].  One group {0, 1, 0}: one camera.
+    bool frames = false;
+    std::vector<rtclj_camera> cams;
+    struct Group { int f0, n; size_t aux; };
+    std::vector<Group> groups;
   } accum;
   DevBuf<double> acc;                   // the accumulation's running sums: 3 per local pixel
   // adaptive accumulation, per local pixel: sums of squared unit sums (3 doubles), sample count, live flag, and
   // the list of the live pixels (descending) that the listed kernels trace; list_aux = [count, tile counts...]
+  // (over frames: per launch group, the group's list at its first pixel, its count and tile counts at Group::aux)
   DevBuf<double> acc2;
   DevBuf<int> nsamp;
   DevBuf<unsigned char> live;
@@ -223,16 +231,26 @@ const KernelFn kPrimaryFns[2][2][2] = {
     {{render_primary_listed_kernel<false>, render_primary_listed_kernel<true>},
      {render_primary_seeded_listed_kernel<false>, render_primary_seeded_listed_kernel<true>}}};
 
-// The frame twins of a camera sequence (FrameKParams), one per instantiation the library can choose for it:
-// render_frames_kernel [const_tab][sample_buf][packed] as kRenderFns[0], render_lane2_frames_kernel [sample_buf],
-// render_primary_frames_kernel [some frame has the defocus disk].  (The wave and split kernels render no sequences.)
+// The frame twins of a camera sequence (FrameKParams), one per instantiation the library can choose for it, indexed
+// as the tables above: render_frames_kernel / render_listed_frames_kernel [listed][const_tab][sample_buf][packed],
+// render_lane2_frames_kernel / render_lane2_listed_frames_kernel [listed][sample_buf], the primary-ray twins
+// [listed][seeded][some frame has the defocus disk].  The listed and seeded twins run the passes of an accumulation over
+// frames (DESIGN.md section 4.15).  (The wave and split kernels render no sequences.)
 using FramesFn = void (*)(FrameKParams);
-const FramesFn kRenderFramesFns[2][2][2] = {
-    {{render_frames_kernel<false, false, false>, nullptr}, {render_frames_kernel<false, true, false>, nullptr}},
-    {{render_frames_kernel<true, false, false>, render_frames_kernel<true, false, true>},
-     {render_frames_kernel<true, true, false>, render_frames_kernel<true, true, true>}}};
-const FramesFn kLane2FramesFns[2] = {render_lane2_frames_kernel<false>, render_lane2_frames_kernel<true>};
-const FramesFn kPrimaryFramesFns[2] = {render_primary_frames_kernel<false>, render_primary_frames_kernel<true>};
+const FramesFn kRenderFramesFns[2][2][2][2] = {
+    {{{render_frames_kernel<false, false, false>, nullptr}, {render_frames_kernel<false, true, false>, nullptr}},
+     {{render_frames_kernel<true, false, false>, render_frames_kernel<true, false, true>},
+      {render_frames_kernel<true, true, false>, render_frames_kernel<true, true, true>}}},
+    {{{render_listed_frames_kernel<false, false, false>, nullptr}, {render_listed_frames_kernel<false, true, false>, nullptr}},
+     {{render_listed_frames_kernel<true, false, false>, render_listed_frames_kernel<true, false, true>},
+      {render_listed_frames_kernel<true, true, false>, render_listed_frames_kernel<true, true, true>}}}};
+const FramesFn kLane2FramesFns[2][2] = {{render_lane2_frames_kernel<false>, render_lane2_frames_kernel<true>},
+                                        {render_lane2_listed_frames_kernel<false>, render_lane2_listed_frames_kernel<true>}};
+const FramesFn kPrimaryFramesFns[2][2][2] = {
+    {{render_primary_frames_kernel<false>, render_primary_frames_kernel<true>},
+     {render_primary_seeded_frames_kernel<false>, render_primary_seeded_frames_kernel<true>}},
+    {{render_primary_listed_frames_kernel<false>, render_primary_listed_frames_kernel<true>},
+     {render_primary_seeded_listed_frames_kernel<false>, render_primary_seeded_listed_frames_kernel<true>}}};
 
 // the tables of kernels with dynamic shared memory, and the most a launch asks for (0: the device's opt-in limit)
 template <class Fn> struct SmemLimit { const Fn* fns; size_t count; size_t bytes; };
@@ -242,8 +260,8 @@ const SmemLimit<KernelFn> kSmemLimits[] = {
     {kSplitFns, sizeof kSplitFns / sizeof(KernelFn), SplitSmem::total},
     {kWaveFns, sizeof kWaveFns / sizeof(KernelFn), WaveSmem::total}};
 const SmemLimit<FramesFn> kFramesSmemLimits[] = {
-    {&kRenderFramesFns[0][0][0], sizeof kRenderFramesFns / sizeof(FramesFn), 0},
-    {kLane2FramesFns, sizeof kLane2FramesFns / sizeof(FramesFn), Lane2Smem::total}};
+    {&kRenderFramesFns[0][0][0][0], sizeof kRenderFramesFns / sizeof(FramesFn), 0},
+    {&kLane2FramesFns[0][0], sizeof kLane2FramesFns / sizeof(FramesFn), Lane2Smem::total}};
 
 }  // namespace
 
@@ -558,6 +576,9 @@ struct Pass {
   // images above hold n_frames full-size frames.  n_frames = 0: the single camera of launch_pass.
   const rtclj_camera* frames = nullptr;
   int n_frames = 0;
+  // an accumulation over frames: the local pixel of the running state (acc, acc2, sample counts, live flags, list) where
+  // the launch's first frame starts, and the launch group's list count at list_aux[aux0]
+  size_t state0 = 0, aux0 = 0;
 };
 
 // the fold and stopping rule of an adaptive accumulation's pass, shard `sh` (finalize_adaptive_kernel)
@@ -573,9 +594,10 @@ AParams adaptive_params(const rtclj_ctx* c, const Shard& sh) {
   return A;
 }
 
-// rebuilds the list of live pixels and its count on the device (rtclj_adaptive.cuh)
-int relist(rtclj_ctx* c, unsigned long long local_pixels, cudaStream_t stream) {
-  CU(launch_relist(c->live.p, local_pixels, c->list_aux.p, c->list.p, stream));
+// rebuilds the list of live pixels and its count on the device (rtclj_adaptive.cuh): the `pixels` local pixels of the
+// running state from `state0` (a launch group of an accumulation over frames, whose count is list_aux[aux0])
+int relist(rtclj_ctx* c, size_t state0, unsigned long long pixels, size_t aux0, cudaStream_t stream) {
+  CU(launch_relist(c->live.p + state0, pixels, c->list_aux.p + aux0, c->list.p + state0, stream));
   return RTCLJ_OK;
 }
 
@@ -619,8 +641,8 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
     P.geom32 = c->geom32.p; P.geomA = c->geomA.p; P.geom64 = c->geom64.p; P.mat = c->mat.p;
     P.partial = c->partial.p; P.acc = ps.acc; P.queue = c->counters.p; P.stats = c->counters.p + 1;
     P.sample_buf = ps.sample_buf; P.sample_stride = sh.local_pixels * (unsigned long long)nframes;
-    P.list = ps.listed ? c->list.p : nullptr; P.list_count = ps.listed ? c->list_aux.p : nullptr;
-    P.acc2 = ps.listed ? c->acc2.p : nullptr;
+    P.list = ps.listed ? c->list.p + ps.state0 : nullptr; P.list_count = ps.listed ? c->list_aux.p + ps.aux0 : nullptr;
+    P.acc2 = ps.listed ? c->acc2.p + 3u * ps.state0 : nullptr;
     const bool const_tab = ch.kernel != Kernel::render_smem, sample_buf = ps.sample_buf != nullptr;
     if (const_tab && !c->ctab_host.empty())
       std::memcpy(P.ctab, c->ctab_host.data(), std::min(sizeof P.ctab, c->ctab_host.size() * sizeof(float)));
@@ -638,7 +660,7 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
         const unsigned long long want = (total_units + kPrimaryThreads - 1) / kPrimaryThreads;
         blocks = (unsigned)std::min<unsigned long long>(want, (unsigned long long)grid * (unsigned long long)(2048 / kPrimaryThreads));
         fn = kPrimaryFns[ps.listed][ps.seeded][P.use_defocus]; threads = kPrimaryThreads; stack = false;
-        frames_fn = kPrimaryFramesFns[any_defocus];
+        frames_fn = kPrimaryFramesFns[ps.listed][ps.seeded][any_defocus];
         break;
       }
       case Kernel::wave:
@@ -655,12 +677,12 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
         break;
       case Kernel::lane2:
         fn = kLane2Fns[ps.listed][sample_buf]; threads = kT2; sm = Lane2Smem::total; paths = 2u * kT2;
-        frames_fn = kLane2FramesFns[sample_buf];
+        frames_fn = kLane2FramesFns[ps.listed][sample_buf];
         break;
       default:  // render_kernel
         fn = kRenderFns[ps.listed][const_tab][sample_buf][ch.packed]; threads = threads_of(const_tab, ch.packed);
         sm = smem_needed(c->nhalf, const_tab, c->smem_optin, ch.packed); paths = (unsigned)threads;
-        frames_fn = kRenderFramesFns[const_tab][sample_buf][ch.packed];
+        frames_fn = kRenderFramesFns[ps.listed][const_tab][sample_buf][ch.packed];
         stack = prm->flags & RTCLJ_F_REVERSE_PRODUCT;
     }
     P.stack_stride = (unsigned)grid * paths;
@@ -708,14 +730,25 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
   }
   CU(cudaEventRecord(c->ev1, stream));
   if (ps.finalize && ps.listed) {
-    AParams A = adaptive_params(c, sh);
-    A.sample_buf = ps.sample_buf; A.partial = c->partial.p; A.out_linear = ps.out_linear; A.out_rgb8 = ps.out_rgb8;
-    A.spp = ps.samples; A.nchunks = nchunks; A.seeded = ps.seeded; A.mean_n = ps.mean_n; A.decide = ps.decide;
-    const unsigned blocks = (unsigned)((sh.local_pixels + 255) / 256);
-    finalize_adaptive_kernel<<<blocks, 256, 0, stream>>>(A);
-    CU(cudaGetLastError());
+    // one finalize_adaptive_kernel per frame, on that frame's unit sums / sample colours, state and full-size images,
+    // then one compaction of the launch's frames
+    const size_t frame_values = (size_t)cam->width * (size_t)cam->height * 3u;
+    for (int f = 0; f < nframes; ++f) {
+      const size_t at = ps.state0 + (size_t)f * sh.local_pixels;
+      AParams A = adaptive_params(c, sh);
+      A.acc += 3u * at; A.acc2 += 3u * at; A.samples += at; A.live += at;
+      A.sample_buf = ps.sample_buf ? ps.sample_buf + (size_t)f * sh.local_pixels * 4u : nullptr;
+      A.sample_stride = sh.local_pixels * (unsigned long long)nframes;
+      A.partial = c->partial.p + (size_t)f * sh.local_pixels * (size_t)nchunks * 3u;
+      A.out_linear = ps.out_linear ? ps.out_linear + (size_t)f * frame_values : nullptr;
+      A.out_rgb8 = ps.out_rgb8 ? ps.out_rgb8 + (size_t)f * frame_values : nullptr;
+      A.spp = ps.samples; A.nchunks = nchunks; A.seeded = ps.seeded; A.mean_n = ps.mean_n; A.decide = ps.decide;
+      const unsigned blocks = (unsigned)((sh.local_pixels + 255) / 256);
+      finalize_adaptive_kernel<<<blocks, 256, 0, stream>>>(A);
+      CU(cudaGetLastError());
+    }
     if (ps.decide) {
-      int rc = relist(c, sh.local_pixels, stream);
+      int rc = relist(c, ps.state0, sh.local_pixels * (unsigned long long)nframes, ps.aux0, stream);
       if (rc) return rc;
     }
   } else if (ps.finalize) {
@@ -731,7 +764,7 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
       F.W = cam->width; F.spp = ps.samples; F.nchunks = nchunks;
       F.shard_index = sh.index; F.shard_count = sh.count; F.shard_rows = sh.rows;
       F.flags = prm->flags; F.local_pixels = sh.local_pixels;
-      F.acc = ps.acc; F.seeded = ps.seeded; F.mean_n = ps.mean_n;
+      F.acc = ps.acc ? ps.acc + (size_t)f * sh.local_pixels * 3u : nullptr; F.seeded = ps.seeded; F.mean_n = ps.mean_n;
       const unsigned blocks = (unsigned)((sh.local_pixels + 255) / 256);
       finalize_kernel<<<blocks, 256, 0, stream>>>(F);
       CU(cudaGetLastError());
@@ -1231,52 +1264,147 @@ int check_adaptive(const rtclj_camera* cam, const rtclj_params* prm, const doubl
   return RTCLJ_OK;
 }
 
-// tol == nullptr: a plain accumulation
-int accum_begin(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, const double* tol, int32_t min_samples,
-                int32_t* pass_unit, cudaStream_t stream) {
-  if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
-  if (!c->have_scene) return fail(RTCLJ_E_INVALID, "rtclj_ctx_set_scene has not been called");
-  int rc = tol ? check_adaptive(cam, prm, tol, min_samples) : validate(cam, prm);
-  if (rc) return rc;
+// what every accumulation refuses besides validate(), checked before any device is touched
+int check_accum(const rtclj_params* prm) {
   if (prm->flags & (RTCLJ_F_WAVE_KERNEL | RTCLJ_F_SPLIT_KERNEL))
     return fail(RTCLJ_E_INVALID, "the wavefront and split kernels do not accumulate over passes");
   // the kernels hold sample indices in 32-bit ints (render_lane2_kernel keeps k and k_end in shared memory
   // as 32-bit words) and compute k + samples_per_unit: keep that sum below 2^31
   if (prm->spp > (1 << 30)) return fail(RTCLJ_E_INVALID, "target of %d samples per pixel: at most 2^30", prm->spp);
+  return RTCLJ_OK;
+}
+
+// every check of an accumulation's begin, before any device is touched.  n_frames == 0: the single camera cams[0]
+// (rtclj_ctx_accum_begin[_adaptive]); else a sequence (rtclj_ctx_accum_begin_frames), whose frames are checked as
+// rtclj_ctx_render_frames checks them.  tol == nullptr: a plain accumulation
+int check_accum_begin(const rtclj_camera* cams, int32_t n_frames, const rtclj_params* prm, const double* tol,
+                      int32_t min_samples) {
+  int rc = n_frames > 0 ? check_frames(cams, n_frames, prm) : RTCLJ_OK;
+  if (rc) return rc;
+  rc = tol ? check_adaptive(cams, prm, tol, min_samples) : validate(cams, prm);
+  if (rc) return rc;
+  return check_accum(prm);
+}
+
+// An allocation of an accumulation's state: a failure leaves no error behind for the next CUDA call to report.
+template <class T>
+int reserve_state(DevBuf<T>& buf, size_t n, const char* what) {
+  const cudaError_t e = buf.reserve(n);
+  if (e == cudaSuccess) return RTCLJ_OK;
+  cudaGetLastError();
+  return fail(RTCLJ_E_CUDA, "%s of the accumulation (%zu bytes): %s", what, n * sizeof(T), cudaGetErrorString(e));
+}
+
+int accum_begin(rtclj_ctx* c, const rtclj_camera* cams, int32_t n_frames, const rtclj_params* prm, const double* tol,
+                int32_t min_samples, int32_t* pass_unit, cudaStream_t stream) {
+  if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
+  if (!c->have_scene) return fail(RTCLJ_E_INVALID, "rtclj_ctx_set_scene has not been called");
+  int rc = check_accum_begin(cams, n_frames, prm, tol, min_samples);
+  if (rc) return rc;
   c->accum.active = false;
   CU(cudaSetDevice(c->device));
+  const rtclj_camera* cam = cams;
   bool strict = false;
   const int unit = accum_pass_unit(cam, prm, &strict);
   const Shard sh = shard_of(cam, prm);
-  const size_t npix = (size_t)sh.local_pixels;
-  CU(c->acc.reserve(std::max<size_t>(npix * 3, 1)));
+  const int K = std::max(n_frames, 1);
+  const size_t fp = (size_t)sh.local_pixels, npix = fp * (size_t)K;
+  // The launch groups of a pass: at most kMaxFrames frames (their cameras are kernel parameters) and fewer than 2^32
+  // work units at the most chunks a pass can give a pixel -- chunked, ceil(spp / pass_unit); strict, the scheduling
+  // units of a sub-pass (auto_samples_per_unit), at most spp / 8 -- and in strict order one sample of every pixel within
+  // the kAccumSampleBufBytes of a sub-pass.  Fixed here: each group keeps its own list between passes.
+  std::vector<rtclj_ctx::Accum::Group> groups;
+  size_t aux = 0;
+  {
+    unsigned long long group = std::min<unsigned long long>((unsigned long long)K, kMaxFrames);
+    const unsigned long long chunks =
+        strict ? (unsigned long long)std::max(1, prm->spp / 8) : (unsigned long long)((prm->spp + unit - 1) / unit);
+    if (fp > 0) {
+      group = std::min(group, std::max(1ull, 0xffffffffull / (fp * chunks)));
+      if (strict) group = std::min(group, std::max(1ull, (unsigned long long)(kAccumSampleBufBytes / (fp * 32u))));
+    }
+    for (int f0 = 0; f0 < K; f0 += (int)group) {
+      const int g = std::min((int)group, K - f0);
+      groups.push_back({f0, g, aux});
+      aux += 1 + (fp * (size_t)g + kListTile - 1) / kListTile;  // count, then the compaction's tile counts
+    }
+  }
+  rc = reserve_state(c->acc, std::max<size_t>(npix * 3, 1), "running sums");
+  if (rc) return rc;
   CU(cudaMemsetAsync(c->acc.p, 0, npix * 3 * sizeof(double), stream));
   if (tol) {
     // every pixel starts live, with no samples and S2 = 0; the list of all pixels is built by the compaction
-    const size_t tiles = (npix + kListTile - 1) / kListTile;
-    CU(c->acc2.reserve(std::max<size_t>(npix * 3, 1)));
-    CU(c->nsamp.reserve(std::max<size_t>(npix, 1)));
-    CU(c->live.reserve(std::max<size_t>(npix, 1)));
-    CU(c->list.reserve(std::max<size_t>(npix, 1)));
-    CU(c->list_aux.reserve(1 + tiles));
+    if ((rc = reserve_state(c->acc2, std::max<size_t>(npix * 3, 1), "sums of squares")) ||
+        (rc = reserve_state(c->nsamp, std::max<size_t>(npix, 1), "sample counts")) ||
+        (rc = reserve_state(c->live, std::max<size_t>(npix, 1), "live flags")) ||
+        (rc = reserve_state(c->list, std::max<size_t>(npix, 1), "pixel list")) ||
+        (rc = reserve_state(c->list_aux, aux, "pixel list counts")))
+      return rc;
     CU(cudaMemsetAsync(c->acc2.p, 0, npix * 3 * sizeof(double), stream));
     CU(cudaMemsetAsync(c->nsamp.p, 0, npix * sizeof(int), stream));
     CU(cudaMemsetAsync(c->live.p, 1, npix, stream));
-    CU(cudaMemsetAsync(c->list_aux.p, 0, sizeof(unsigned), stream));
-    rc = relist(c, sh.local_pixels, stream);
+    CU(cudaMemsetAsync(c->list_aux.p, 0, aux * sizeof(unsigned), stream));
+    for (const auto& g : groups) {
+      rc = relist(c, (size_t)g.f0 * fp, (unsigned long long)fp * (unsigned long long)g.n, g.aux, stream);
+      if (rc) return rc;
+    }
+  }
+  auto& A = c->accum;
+  A.strict = strict;
+  A.cam = *cam;
+  A.prm = *prm;
+  A.done = 0;
+  A.pass_unit = unit;
+  A.adaptive = tol != nullptr;
+  A.abs_tol = tol ? tol[0] : 0.0;
+  A.rel_tol = tol ? tol[1] : 0.0;
+  A.min_samples = tol ? min_samples : 0;
+  A.frames = n_frames > 0;
+  A.cams.assign(cams, cams + K);
+  A.groups = std::move(groups);
+  A.active = true;
+  if (pass_unit) *pass_unit = unit;
+  return RTCLJ_OK;
+}
+
+// One pass of the accumulation on launch group `ps` (rtclj_ctx_accum_step); ps.frames / ps.n_frames: its cameras
+int accum_pass(rtclj_ctx* c, const rtclj_camera* cam, const KernelChoice& ch, const Shard& sh, const Pass& ps,
+               cudaStream_t stream) {
+  const auto& A = c->accum;
+  const rtclj_params* prm = &A.prm;
+  const int samples = ps.samples;
+  if (!A.strict || ch.kernel == Kernel::none) {
+    // chunks of pass_unit samples, folded onto the running sums in chunk order (depth <= 0: one unit of black)
+    Pass p = ps;
+    p.spu = ch.kernel != Kernel::none ? std::min(A.pass_unit, samples) : samples;
+    return launch_pass(c, cam, prm, ch, sh, p, stream);
+  }
+  if (ch.kernel == Kernel::primary) {
+    // one unit per pixel whose sums continue from the running sums: the reference's sequential sum in registers
+    Pass p = ps;
+    p.spu = samples; p.seeded = true;
+    return launch_pass(c, cam, prm, ch, sh, p, stream);
+  }
+  // every sample's colour through sample_buf, added in sample order by the fold: sub-passes of at most
+  // kAccumSampleBufBytes, the fold is sequential per sample, so the cut changes no bit
+  const size_t per_sample = (size_t)sh.local_pixels * 32u * (size_t)std::max(ps.n_frames, 1);
+  const int per = per_sample ? (int)std::min<size_t>(kAccumSampleBufBytes / per_sample, (size_t)samples) : samples;
+  if (per <= 0)
+    return fail(RTCLJ_E_TOO_LARGE, "%llu pixels: one sample of each exceeds the %zu-byte strict buffer; use chunks "
+                "(samples_per_unit < spp)", sh.local_pixels, kAccumSampleBufBytes);
+  CU(c->sample_buf.reserve(std::max<size_t>((size_t)per * per_sample / 8u, 1)));
+  for (int b = 0; b < samples; b += per) {
+    Pass sub = ps;
+    sub.sample_base = ps.sample_base + b;
+    sub.samples = std::min(per, samples - b);
+    sub.spu = auto_samples_per_unit(cam->width, cam->height, sub.samples);  // scheduling units only
+    sub.sample_buf = c->sample_buf.p;
+    sub.first = ps.first && b == 0;
+    sub.decide = b + per >= samples;
+    if (b + per < samples) { sub.out_linear = nullptr; sub.out_rgb8 = nullptr; }  // fold only
+    const int rc = launch_pass(c, cam, prm, ch, sh, sub, stream);
     if (rc) return rc;
   }
-  c->accum.strict = strict;
-  c->accum.cam = *cam;
-  c->accum.prm = *prm;
-  c->accum.done = 0;
-  c->accum.pass_unit = unit;
-  c->accum.adaptive = tol != nullptr;
-  c->accum.abs_tol = tol ? tol[0] : 0.0;
-  c->accum.rel_tol = tol ? tol[1] : 0.0;
-  c->accum.min_samples = tol ? min_samples : 0;
-  c->accum.active = true;
-  if (pass_unit) *pass_unit = unit;
   return RTCLJ_OK;
 }
 
@@ -1286,7 +1414,7 @@ extern "C" {
 
 int rtclj_ctx_accum_begin(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, int32_t* pass_unit,
                           void* stream_) {
-  return guarded([&]() -> int { return accum_begin(c, cam, prm, nullptr, 0, pass_unit, (cudaStream_t)stream_); });
+  return guarded([&]() -> int { return accum_begin(c, cam, 0, prm, nullptr, 0, pass_unit, (cudaStream_t)stream_); });
 }
 
 int rtclj_ctx_accum_begin_adaptive(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm,
@@ -1294,7 +1422,16 @@ int rtclj_ctx_accum_begin_adaptive(rtclj_ctx* c, const rtclj_camera* cam, const 
   return guarded([&]() -> int {
     if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
     if (!tolerance) return fail(RTCLJ_E_INVALID, "null tolerance");
-    return accum_begin(c, cam, prm, tolerance, min_samples, pass_unit, (cudaStream_t)stream_);
+    return accum_begin(c, cam, 0, prm, tolerance, min_samples, pass_unit, (cudaStream_t)stream_);
+  });
+}
+
+int rtclj_ctx_accum_begin_frames(rtclj_ctx* c, const rtclj_camera* cameras, int32_t n_frames, const rtclj_params* prm,
+                                 const double* tolerance, int32_t min_samples, int32_t* pass_unit, void* stream_) {
+  return guarded([&]() -> int {
+    if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
+    if (n_frames <= 0) return fail(RTCLJ_E_INVALID, "n_frames must be positive, got %d", n_frames);
+    return accum_begin(c, cameras, n_frames, prm, tolerance, min_samples, pass_unit, (cudaStream_t)stream_);
   });
 }
 
@@ -1305,46 +1442,27 @@ int rtclj_ctx_accum_step(rtclj_ctx* c, int32_t samples, void* d_out_linear, void
     auto& A = c->accum;
     if (!A.active) return fail(RTCLJ_E_INVALID, "no accumulation: call rtclj_ctx_accum_begin (rtclj_ctx_set_scene ends one)");
     const rtclj_params* prm = &A.prm;
-    const rtclj_camera* cam = &A.cam;
     int rc = check_pass(A.done, samples, prm->spp, A.pass_unit);
     if (rc) return rc;
     cudaStream_t stream = (cudaStream_t)stream_;
     CU(cudaSetDevice(c->device));
-    const Shard sh = shard_of(cam, prm);
-    const KernelChoice ch = choose_kernel(c, prm, (double)sh.local_pixels * (double)samples);
+    const Shard sh = shard_of(&A.cam, prm);
+    // every kernel gives the same bits: over frames the choice may see the whole sequence
+    const KernelChoice ch = choose_kernel(c, prm, (double)A.cams.size() * (double)sh.local_pixels * (double)samples);
     const int d = A.done + samples;  // samples per pixel after this pass: the mean's divisor
-    Pass ps;
-    ps.sample_base = A.done; ps.samples = samples; ps.acc = c->acc.p; ps.mean_n = d; ps.finalize = true;
-    ps.listed = A.adaptive;  // only the live pixels, each folded and tested (finalize_adaptive_kernel)
-    ps.out_linear = (double*)d_out_linear; ps.out_rgb8 = (unsigned char*)d_out_rgb8;
-    if (!A.strict || ch.kernel == Kernel::none) {
-      // chunks of pass_unit samples, folded onto the running sums in chunk order (depth <= 0: one unit of black)
-      ps.spu = ch.kernel != Kernel::none ? std::min(A.pass_unit, samples) : samples;
-      rc = launch_pass(c, cam, prm, ch, sh, ps, stream);
-    } else if (ch.kernel == Kernel::primary) {
-      // one unit per pixel whose sums continue from the running sums: the reference's sequential sum in registers
-      ps.spu = samples; ps.seeded = true;
-      rc = launch_pass(c, cam, prm, ch, sh, ps, stream);
-    } else {
-      // every sample's colour through sample_buf, added in sample order by the fold: sub-passes of at most
-      // kAccumSampleBufBytes, the fold is sequential per sample, so the cut changes no bit
-      const size_t per_sample = (size_t)sh.local_pixels * 32u;
-      const int per = per_sample ? (int)std::min<size_t>(kAccumSampleBufBytes / per_sample, (size_t)samples) : samples;
-      if (per <= 0)
-        return fail(RTCLJ_E_TOO_LARGE, "%llu pixels: one sample of each exceeds the %zu-byte strict buffer; use chunks "
-                    "(samples_per_unit < spp)", sh.local_pixels, kAccumSampleBufBytes);
-      CU(c->sample_buf.reserve(std::max<size_t>((size_t)per * per_sample / 8u, 1)));
-      for (int b = 0; b < samples && rc == RTCLJ_OK; b += per) {
-        Pass sub = ps;
-        sub.sample_base = A.done + b;
-        sub.samples = std::min(per, samples - b);
-        sub.spu = auto_samples_per_unit(cam->width, cam->height, sub.samples);  // scheduling units only
-        sub.sample_buf = c->sample_buf.p;
-        sub.first = b == 0;
-        sub.decide = b + per >= samples;
-        if (b + per < samples) { sub.out_linear = nullptr; sub.out_rgb8 = nullptr; }  // fold only
-        rc = launch_pass(c, cam, prm, ch, sh, sub, stream);
-      }
+    const size_t frame_values = (size_t)A.cam.width * (size_t)A.cam.height * 3u;
+    for (size_t gi = 0; gi < A.groups.size() && rc == RTCLJ_OK; ++gi) {
+      const auto& g = A.groups[gi];
+      Pass ps;
+      ps.sample_base = A.done; ps.samples = samples; ps.mean_n = d; ps.finalize = true;
+      ps.first = gi == 0;
+      ps.state0 = (size_t)g.f0 * (size_t)sh.local_pixels; ps.aux0 = g.aux;
+      ps.acc = c->acc.p + 3u * ps.state0;
+      ps.listed = A.adaptive;  // only the live pixels, each folded and tested (finalize_adaptive_kernel)
+      ps.out_linear = d_out_linear ? (double*)d_out_linear + (size_t)g.f0 * frame_values : nullptr;
+      ps.out_rgb8 = d_out_rgb8 ? (unsigned char*)d_out_rgb8 + (size_t)g.f0 * frame_values : nullptr;
+      if (A.frames) { ps.frames = &A.cams[(size_t)g.f0]; ps.n_frames = g.n; }
+      rc = accum_pass(c, &A.cams[(size_t)g.f0], ch, sh, ps, stream);
     }
     if (rc) { A.active = false; return rc; }  // the running sums may hold part of the pass
     c->last_spu = A.strict ? d : A.pass_unit;
@@ -1357,21 +1475,32 @@ int rtclj_ctx_accum_step(rtclj_ctx* c, int32_t samples, void* d_out_linear, void
 int rtclj_ctx_accum_noise(rtclj_ctx* c, int32_t* d_samples, double* d_stderr, uint64_t* active_pixels, void* stream_) {
   return guarded([&]() -> int {
     if (!c) return fail(RTCLJ_E_INVALID, "null ctx");
-    if (!c->accum.active || !c->accum.adaptive)
+    const auto& Acc = c->accum;
+    if (!Acc.active || !Acc.adaptive)
       return fail(RTCLJ_E_INVALID, "no adaptive accumulation: call rtclj_ctx_accum_begin_adaptive");
     cudaStream_t stream = (cudaStream_t)stream_;
     CU(cudaSetDevice(c->device));
-    const Shard sh = shard_of(&c->accum.cam, &c->accum.prm);
+    const Shard sh = shard_of(&Acc.cam, &Acc.prm);
     if ((d_samples || d_stderr) && sh.local_pixels > 0) {
-      const unsigned blocks = (unsigned)((sh.local_pixels + 255) / 256);
-      noise_export_kernel<<<blocks, 256, 0, stream>>>(adaptive_params(c, sh), d_samples, d_stderr);
-      CU(cudaGetLastError());
+      const size_t frame_pixels = (size_t)Acc.cam.width * (size_t)Acc.cam.height;
+      for (size_t f = 0; f < Acc.cams.size(); ++f) {  // frame f's state -> its full-size maps
+        const size_t at = f * (size_t)sh.local_pixels;
+        AParams A = adaptive_params(c, sh);
+        A.acc += 3u * at; A.acc2 += 3u * at; A.samples += at; A.live += at;
+        const unsigned blocks = (unsigned)((sh.local_pixels + 255) / 256);
+        noise_export_kernel<<<blocks, 256, 0, stream>>>(A, d_samples ? d_samples + f * frame_pixels : nullptr,
+                                                        d_stderr ? d_stderr + f * frame_pixels * 3u : nullptr);
+        CU(cudaGetLastError());
+      }
     }
-    if (active_pixels) {
-      unsigned n = 0;
-      CU(cudaMemcpyAsync(&n, c->list_aux.p, sizeof n, cudaMemcpyDeviceToHost, stream));
+    if (active_pixels) {  // the launch groups' counts
+      std::vector<unsigned> n(Acc.groups.size(), 0u);
+      for (size_t g = 0; g < n.size(); ++g)
+        CU(cudaMemcpyAsync(&n[g], c->list_aux.p + Acc.groups[g].aux, sizeof(unsigned), cudaMemcpyDeviceToHost, stream));
       CU(cudaStreamSynchronize(stream));
-      *active_pixels = n;
+      uint64_t total = 0;
+      for (unsigned v : n) total += v;
+      *active_pixels = total;
     }
     return RTCLJ_OK;
   });
@@ -1383,7 +1512,8 @@ int rtclj_ctx_accum_noise(rtclj_ctx* c, int32_t* d_samples, double* d_stderr, ui
 struct rtclj_progressive {
   std::vector<rtclj_ctx*> ctxs;
   std::vector<rtclj_params> prm;  // per device: its shard
-  rtclj_camera cam;
+  rtclj_camera cam;               // (a sequence: the first camera; every frame has its size)
+  int n_frames = 1;               // the images of a step: frames of W*H pixels one after the other
   int spp = 0, pass_unit = 1, done = 0;
   bool adaptive = false;
   bool failed = false;  // a step failed on some device: the devices' running sums no longer agree
@@ -1394,24 +1524,21 @@ struct rtclj_progressive {
 
 namespace {
 
-// tol == nullptr: a plain accumulation
-int progressive_create(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm, const double* tol,
-                       int32_t min_samples, const int32_t* devices, int32_t n_devices, int32_t* pass_unit,
-                       rtclj_progressive** out) {
+// tol == nullptr: a plain accumulation; n_frames == 0: the single camera cams[0], else a sequence
+int progressive_create(const rtclj_scene* scene, const rtclj_camera* cams, int32_t n_frames, const rtclj_params* prm,
+                       const double* tol, int32_t min_samples, const int32_t* devices, int32_t n_devices,
+                       int32_t* pass_unit, rtclj_progressive** out) {
   return guarded([&]() -> int {
     if (!out) return fail(RTCLJ_E_INVALID, "null out");
     *out = nullptr;
     if (!scene) return fail(RTCLJ_E_INVALID, "null scene");
-    int rc = validate(cam, prm);
+    int rc = check_accum_begin(cams, n_frames, prm, tol, min_samples);
     if (rc) return rc;
-    if (tol) {
-      rc = check_adaptive(cam, prm, tol, min_samples);
-      if (rc) return rc;
-    }
     rc = check_devices(devices, n_devices);
     if (rc) return rc;
     std::unique_ptr<rtclj_progressive> p(new rtclj_progressive());
-    p->cam = *cam;
+    p->cam = *cams;
+    p->n_frames = std::max(n_frames, 1);
     p->spp = prm->spp;
     p->adaptive = tol != nullptr;
     for (int d = 0; d < n_devices; ++d) {
@@ -1423,7 +1550,7 @@ int progressive_create(const rtclj_scene* scene, const rtclj_camera* cam, const 
       p->prm.push_back(q);
       rc = rtclj_ctx_set_scene(c, scene);
       if (rc) return rc;
-      rc = accum_begin(c, cam, &q, tol, min_samples, &p->pass_unit, c->own_stream);
+      rc = accum_begin(c, cams, n_frames, &q, tol, min_samples, &p->pass_unit, c->own_stream);
       if (rc) return rc;
     }
     if (pass_unit) *pass_unit = p->pass_unit;
@@ -1438,7 +1565,7 @@ extern "C" {
 
 int rtclj_progressive_create(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm,
                              const int32_t* devices, int32_t n_devices, int32_t* pass_unit, rtclj_progressive** out) {
-  return progressive_create(scene, cam, prm, nullptr, 0, devices, n_devices, pass_unit, out);
+  return progressive_create(scene, cam, 0, prm, nullptr, 0, devices, n_devices, pass_unit, out);
 }
 
 int rtclj_progressive_create_adaptive(const rtclj_scene* scene, const rtclj_camera* cam, const rtclj_params* prm,
@@ -1446,7 +1573,16 @@ int rtclj_progressive_create_adaptive(const rtclj_scene* scene, const rtclj_came
                                       int32_t n_devices, int32_t* pass_unit, rtclj_progressive** out) {
   if (out) *out = nullptr;
   if (!tolerance) return fail(RTCLJ_E_INVALID, "null tolerance");
-  return progressive_create(scene, cam, prm, tolerance, min_samples, devices, n_devices, pass_unit, out);
+  return progressive_create(scene, cam, 0, prm, tolerance, min_samples, devices, n_devices, pass_unit, out);
+}
+
+int rtclj_progressive_create_frames(const rtclj_scene* scene, const rtclj_camera* cameras, int32_t n_frames,
+                                    const rtclj_params* prm, const double* tolerance, int32_t min_samples,
+                                    const int32_t* devices, int32_t n_devices, int32_t* pass_unit,
+                                    rtclj_progressive** out) {
+  if (out) *out = nullptr;
+  if (n_frames <= 0) return fail(RTCLJ_E_INVALID, "n_frames must be positive, got %d", n_frames);
+  return progressive_create(scene, cameras, n_frames, prm, tolerance, min_samples, devices, n_devices, pass_unit, out);
 }
 
 int rtclj_progressive_step(rtclj_progressive* p, int32_t samples, double* out_linear, uint8_t* out_rgb8,
@@ -1458,19 +1594,21 @@ int rtclj_progressive_step(rtclj_progressive* p, int32_t samples, double* out_li
     // rtclj_ctx_accum_step's checks, made before any device starts, so that the devices stay in step
     int rc = check_pass(p->done, samples, p->spp, p->pass_unit);
     if (rc) return rc;
-    const size_t npix = (size_t)p->cam.width * (size_t)p->cam.height;
+    const size_t nval = (size_t)p->cam.width * (size_t)p->cam.height * 3u * (size_t)p->n_frames;
     std::vector<rtclj_stats> st(p->ctxs.size());
     rc = run_on_devices((int)p->ctxs.size(), [&](int d) -> int {  // pass -> this device's rows of the caller's images
       rtclj_ctx* c = p->ctxs[d];
       const rtclj_params& q = p->prm[d];
       CU(cudaSetDevice(c->device));
-      if (out_linear) CU(c->out_linear.reserve(npix * 3));
-      if (out_rgb8) CU(c->out_rgb8.reserve(npix * 3));
+      if (out_linear) CU(c->out_linear.reserve(nval));
+      if (out_rgb8) CU(c->out_rgb8.reserve(nval));
       int r = rtclj_ctx_accum_step(c, samples, out_linear ? c->out_linear.p : nullptr, out_rgb8 ? c->out_rgb8.p : nullptr,
                                    nullptr, c->own_stream);
       if (r) return r;
-      r = download_rows(c, &p->cam, q.shard_index, q.shard_count, q.shard_rows, out_linear, out_rgb8, c->own_stream);
-      if (r) return r;
+      for (int f = 0; f < p->n_frames; ++f) {
+        r = download_rows(c, &p->cam, q.shard_index, q.shard_count, q.shard_rows, out_linear, out_rgb8, c->own_stream, f);
+        if (r) return r;
+      }
       return rtclj_ctx_stats(c, c->own_stream, &st[(size_t)d]);  // synchronises the stream: the direct copies have landed
     });
     if (rc) { p->failed = true; return rc; }
@@ -1488,14 +1626,14 @@ int rtclj_progressive_noise(rtclj_progressive* p, int32_t* samples, double* stde
     if (!p) return fail(RTCLJ_E_INVALID, "null progressive handle");
     if (!p->adaptive) return fail(RTCLJ_E_INVALID, "not an adaptive progressive render");
     if (p->failed) return fail(RTCLJ_E_INVALID, "an earlier step failed: destroy this handle and create a new one");
-    const size_t W = (size_t)p->cam.width, H = (size_t)p->cam.height;
+    const size_t W = (size_t)p->cam.width, H = (size_t)p->cam.height, K = (size_t)p->n_frames;
     uint64_t total = 0;
     for (size_t d = 0; d < p->ctxs.size(); ++d) {  // (small images: one device after the other)
       rtclj_ctx* c = p->ctxs[d];
       const rtclj_params& q = p->prm[d];
       CU(cudaSetDevice(c->device));
-      if (samples) CU(c->noise_samples.reserve(W * H));
-      if (stderr_) CU(c->noise_stderr.reserve(W * H * 3));
+      if (samples) CU(c->noise_samples.reserve(W * H * K));
+      if (stderr_) CU(c->noise_stderr.reserve(W * H * 3 * K));
       uint64_t n = 0;
       int rc = rtclj_ctx_accum_noise(c, samples ? c->noise_samples.p : nullptr, stderr_ ? c->noise_stderr.p : nullptr, &n,
                                      c->own_stream);
@@ -1504,14 +1642,20 @@ int rtclj_progressive_noise(rtclj_progressive* p, int32_t* samples, double* stde
       std::vector<Piece> pieces;
       if (samples) {
         plan_pieces(H, W * sizeof(int32_t), q.shard_index, q.shard_count, q.shard_rows, kStageBytes, pieces);
-        rc = download_image(c, pieces, (char*)samples, (const char*)c->noise_samples.p, c->own_stream);
-        if (rc) return rc;
+        for (size_t f = 0; f < K; ++f) {
+          rc = download_image(c, pieces, (char*)(samples + f * W * H), (const char*)(c->noise_samples.p + f * W * H),
+                              c->own_stream);
+          if (rc) return rc;
+        }
       }
       if (stderr_) {
         pieces.clear();
         plan_pieces(H, W * 3 * sizeof(double), q.shard_index, q.shard_count, q.shard_rows, kStageBytes, pieces);
-        rc = download_image(c, pieces, (char*)stderr_, (const char*)c->noise_stderr.p, c->own_stream);
-        if (rc) return rc;
+        for (size_t f = 0; f < K; ++f) {
+          rc = download_image(c, pieces, (char*)(stderr_ + f * W * H * 3), (const char*)(c->noise_stderr.p + f * W * H * 3),
+                              c->own_stream);
+          if (rc) return rc;
+        }
       }
       CU(cudaStreamSynchronize(c->own_stream));  // the direct copies into pinned memory have landed
     }

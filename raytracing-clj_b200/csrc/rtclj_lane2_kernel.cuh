@@ -177,6 +177,11 @@ __global__ void __launch_bounds__(kT2, 1) render_lane2_frames_kernel(const __gri
   render_lane2_body<kSampleBuf, false, true>(FP.P, &FP);
 }
 
+template <bool kSampleBuf>
+__global__ void __launch_bounds__(kT2, 1) render_lane2_listed_frames_kernel(const __grid_constant__ FrameKParams FP) {
+  render_lane2_body<kSampleBuf, true, true>(FP.P, &FP);
+}
+
 // (The same loop with ONE path per lane built on path_step() was measured against render_kernel<true>: equal on
 // the cover scene, 6 % slower on realm's forward product -- formed from the stack instead of a running product
 // in registers -- and on primary-ray renders, which pay path_step's pixel / W division per sample.  So short

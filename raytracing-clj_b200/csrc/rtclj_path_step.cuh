@@ -44,7 +44,8 @@ struct PathCounters { unsigned samples, seg, exact, pref; };
 // survivors_of_block(j): the 16 survivor bits of block j (sphere s of the block -> bit 15 - s);
 // sums: the path's three unit sums, kSumStride doubles apart; stack_col: its column of the attenuation stack.
 // kListed: tickets go to the pixels of KParams::list, `total_units` of them (total_units_of, read once per kernel).
-// kFrames: the units of a camera sequence, P = FP->P (unit_of_frame_ticket, frame_camera_ray).
+// kFrames: the units of a camera sequence, P = FP->P (unit_of_frame_ticket, frame_camera_ray); with kListed, the listed
+// pixels of an adaptive accumulation over frames (unit_of_listed_frame_ticket).
 template <bool kSampleBuf, int kSumStride, bool kListed = false, bool kFrames = false, class SurvivorsOfBlock>
 __device__ __forceinline__ void path_step(const KParams& P, PathRegs& pr, PathCounters& pc, unsigned bany,
                                           SurvivorsOfBlock survivors_of_block, double* sums, size_t stack_col, int lane,
@@ -288,7 +289,8 @@ __device__ __forceinline__ void path_step(const KParams& P, PathRegs& pr, PathCo
           status = PS_DEAD;
         } else {
           int chunk = 0;
-          const unsigned p_local = kFrames ? unit_of_frame_ticket(*FP, (unsigned)ticket, unit, chunk)
+          const unsigned p_local = kFrames && kListed ? unit_of_listed_frame_ticket(*FP, (unsigned)ticket, unit, chunk)
+                                   : kFrames ? unit_of_frame_ticket(*FP, (unsigned)ticket, unit, chunk)
                                    : kListed ? unit_of_listed_ticket(P, (unsigned)ticket, unit)
                                              : unit_of_ticket(P, (unsigned)ticket, unit);
           if (!kFrames) chunk = (int)(unit - p_local * (unsigned)P.nchunks);

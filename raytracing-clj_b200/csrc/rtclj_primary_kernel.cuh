@@ -60,10 +60,16 @@ __device__ __forceinline__ void render_primary_body(const KParams& P, const Fram
     if (ticket >= total_units) continue;  // (tail of the last ticket: the lane waits at the next shuffle, which ends the loop)
 
     unsigned unit = (unsigned)ticket;
-    const unsigned frame = kFrames ? unit / FP->frame_units : 0u;
-    const unsigned frame_unit = kFrames ? unit - frame * FP->frame_units : unit;  // the unit within its frame
-    const unsigned p_local = kListed ? unit_of_listed_ticket(P, (unsigned)ticket, unit) : frame_unit / (unsigned)P.nchunks;
+    unsigned frame = kFrames && !kListed ? unit / FP->frame_units : 0u;
+    const unsigned frame_unit = kFrames && !kListed ? unit - frame * FP->frame_units : unit;  // the unit within its frame
+    unsigned p_local = kListed ? unit_of_listed_ticket(P, (unsigned)ticket, unit) : frame_unit / (unsigned)P.nchunks;
     const int chunk = (int)((kListed ? unit : frame_unit) - p_local * (unsigned)P.nchunks);
+    if (kFrames && kListed) {  // the list entry is frame * frame_pixels + local pixel
+      frame = p_local / FP->frame_pixels;
+      p_local -= frame * FP->frame_pixels;
+    }
+    // frames: the running sums are indexed by unit / nchunks = frame * frame_pixels + local pixel
+    const unsigned sum_at = kFrames ? unit / (unsigned)P.nchunks : p_local;
     const int lr = (int)(p_local / (unsigned)P.W);
     const int pi = (int)(p_local - (unsigned)lr * (unsigned)P.W);
     const int tile = lr / P.shard_rows;
@@ -72,9 +78,9 @@ __device__ __forceinline__ void render_primary_body(const KParams& P, const Fram
     const int k_begin = P.sample_base + chunk * P.spu;
     const int k_end = min(k_begin + P.spu, P.spp);
     double sum_r = 0.0, sum_g = 0.0, sum_b = 0.0;
-    if (kSeeded) { const double* a = P.acc + (size_t)p_local * 3u; sum_r = a[0]; sum_g = a[1]; sum_b = a[2]; }
+    if (kSeeded) { const double* a = P.acc + (size_t)sum_at * 3u; sum_r = a[0]; sum_g = a[1]; sum_b = a[2]; }
     double sq_r = 0.0, sq_g = 0.0, sq_b = 0.0;
-    if (kMoments) { const double* a = P.acc2 + (size_t)p_local * 3u; sq_r = a[0]; sq_g = a[1]; sq_b = a[2]; }
+    if (kMoments) { const double* a = P.acc2 + (size_t)sum_at * 3u; sq_r = a[0]; sq_g = a[1]; sq_b = a[2]; }
 
 #pragma unroll 1
     for (int k = k_begin; k < k_end; ++k) {
@@ -158,7 +164,10 @@ __device__ __forceinline__ void render_primary_body(const KParams& P, const Fram
     }
     double* out = P.partial + (size_t)unit * 3u;
     out[0] = sum_r; out[1] = sum_g; out[2] = sum_b;
-    if (kMoments) { double* a = P.acc2 + (size_t)p_local * 3u; a[0] = sq_r; a[1] = sq_g; a[2] = sq_b; }
+    if (kMoments) {
+      double* a = P.acc2 + (size_t)(kFrames ? unit / (unsigned)P.nchunks : p_local) * 3u;  // (frames: from the unit just re-read)
+      a[0] = sq_r; a[1] = sq_g; a[2] = sq_b;
+    }
   }
 
   // ---- counters: samples = segments; every sphere is tested for every segment
@@ -196,6 +205,23 @@ __global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_prima
 template <bool kDefocus>
 __global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_primary_frames_kernel(const __grid_constant__ FrameKParams FP) {
   render_primary_body<kDefocus, false, false, true>(FP.P, &FP);
+}
+
+// the twins of an accumulation over frames (DESIGN.md section 4.15): a strict pass (seeded), an adaptive pass (listed,
+// list entries frame * frame_pixels + local pixel) and an adaptive strict pass (both)
+template <bool kDefocus>
+__global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_primary_seeded_frames_kernel(const __grid_constant__ FrameKParams FP) {
+  render_primary_body<kDefocus, true, false, true>(FP.P, &FP);
+}
+
+template <bool kDefocus>
+__global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_primary_listed_frames_kernel(const __grid_constant__ FrameKParams FP) {
+  render_primary_body<kDefocus, false, true, true>(FP.P, &FP);
+}
+
+template <bool kDefocus>
+__global__ void __launch_bounds__(kPrimaryThreads, RTCLJ_PRIM_MINB) render_primary_seeded_listed_frames_kernel(const __grid_constant__ FrameKParams FP) {
+  render_primary_body<kDefocus, true, true, true>(FP.P, &FP);
 }
 
 }  // namespace rtclj

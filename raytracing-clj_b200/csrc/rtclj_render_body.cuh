@@ -1,6 +1,8 @@
-// rtclj_render_body.cuh -- the body of render_kernel, render_listed_kernel and render_frames_kernel (rtclj_kernels.cuh),
+// rtclj_render_body.cuh -- the body of render_kernel, render_listed_kernel, render_frames_kernel and
+// render_listed_frames_kernel (rtclj_kernels.cuh),
 // included inside each __global__ function, which defines kConstTab, kSampleBuf, kPacked and kListed and its parameter P
-// (render_frames_kernel: FP, whose P it is, and RTCLJ_FRAMES_BODY, so the other kernels compile from unchanged text).
+// (render_frames_kernel: FP, whose P it is, and RTCLJ_FRAMES_BODY, so the other kernels compile from unchanged text;
+// render_listed_frames_kernel: RTCLJ_LISTED_FRAMES_BODY as well).
 // Textual rather than a shared __forceinline__ device function: inlined, the body compiled to different code for
 // the 512-thread instantiation (the launch bounds no longer bound threadIdx.x where it is read, and loops were
 // rotated differently), whereas render_kernel must stay the kernel that was measured (DESIGN.md section 4.10).
@@ -441,7 +443,10 @@
           if (ticket >= (kListed ? (unsigned long long)listed_units : P.total_units)) {
             active = false;
           } else {
-#if RTCLJ_FRAMES_BODY
+#if RTCLJ_LISTED_FRAMES_BODY
+            int chunk;
+            const unsigned p_local = unit_of_listed_frame_ticket(FP, (unsigned)ticket, unit, chunk);
+#elif RTCLJ_FRAMES_BODY
             int chunk;
             const unsigned p_local = unit_of_frame_ticket(FP, (unsigned)ticket, unit, chunk);
 #else

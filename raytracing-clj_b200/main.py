@@ -13,6 +13,8 @@
                                                               -> scene-0000.png ... scene-{N-1}.png, a turntable
     python -m raytracing_clj_b200.main main [spp] [depth] --frames N --apng
                                                               -> scene.apng, the turntable as one animation
+    python -m raytracing_clj_b200.main main [spp] [depth] --frames N --tolerance ABS,REL [--every M] [--apng]
+                                                              -> the same files, every frame adaptively sampled
     python -m raytracing_clj_b200.main realm                  -> scene-realm.ppm
     python -m raytracing_clj_b200.main i                      -> scene-i.ppm
 
@@ -43,7 +45,13 @@ scene.png from a run without --frames.
 
 With --frames N --apng the turntable is written as one animated PNG instead, scene.apng: 1/30 s per frame, looping
 forever, rendered and encoded on the GPU in one call (rtclj_render_frames_apng, DESIGN.md section 4.14); its frames
-have the pixels of the scene-NNNN.png files.  --apng needs --frames."""
+have the pixels of the scene-NNNN.png files.  --apng needs --frames.
+
+With --frames N --tolerance ABS,REL the turntable is rendered as one adaptive accumulation over its frames
+(rtclj_progressive_create_frames, DESIGN.md section 4.15): every pass traces the pixels of every frame that are still
+noisy, in passes of --every M samples (default spp/10, rounded up to the pass unit), until no pixel is left.  The same
+files are written at the end, and the share of the samples traced is printed.  Each frame has the pixels of the
+single-image run with --tolerance and the same --every at that frame's camera."""
 from __future__ import annotations
 
 import os
@@ -137,9 +145,11 @@ def main_variant(spp: int = 100, depth: int = 50, out: str = "scene.ppm", seed: 
 
 
 def frames_variant(spp: int = 100, depth: int = 50, n_frames: int = 60, out: str = "scene", seed: int = 1,
-                   gpu_png: bool = False, apng: bool = False):
+                   gpu_png: bool = False, apng: bool = False, tolerance=None, every: int = 0):
     print("config:", {"samples-per-px": spp, "max-depth": depth, "frames": n_frames})
     t0 = time.perf_counter()
+    if tolerance is not None:
+        return _adaptive_frames(spp, depth, n_frames, out, seed, gpu_png, apng, tolerance, every, t0)
     if apng:
         data = render.render_frames_apng(scenes.main_hittables(), camera.turntable_cameras(n_frames), spp, depth,
                                          seed=seed, flags=_abi.FLAGS_MAIN, delay=(1, 30), plays=0)
@@ -155,6 +165,39 @@ def frames_variant(spp: int = 100, depth: int = 50, n_frames: int = 60, out: str
     print(f'"Elapsed time: {1e3 * (time.perf_counter() - t0):.3f} msecs"  (render {1e3 * (t1 - t0):.3f} ms, '
           f'{st["segments"]} ray segments, {out}-0000.png .. {out}-{n_frames - 1:04d}.png)')
     return st
+
+
+def _adaptive_frames(spp, depth, n_frames, out, seed, gpu_png, apng, tolerance, every, t0):
+    """--frames N --tolerance ABS,REL: the turntable as one adaptive accumulation, run until no pixel is active."""
+    if every <= 0:
+        every = max(1, spp // 10)
+    cams = camera.turntable_cameras(n_frames)
+    with render.ProgressiveFrames(scenes.main_hittables(), cams, spp, depth, seed=seed, flags=_abi.FLAGS_MAIN,
+                                  tolerance=tolerance) as p:
+        n = -(-every // p.pass_unit) * p.pass_unit
+        segments = traced = 0
+        active = n_frames * p.width * p.height
+        while p.samples_done < spp and active > 0:
+            _, rgb8, st = p.step(min(n, spp - p.samples_done), want_linear=False)
+            segments += st["segments"]
+            traced += st["samples"]
+            _, _, active = p.noise()
+            print(f"{p.samples_done}/{spp} samples per pixel, {active} pixels active "
+                  f"({1e3 * (time.perf_counter() - t0):.0f} ms)")
+        full = spp * n_frames * p.width * p.height
+    t1 = time.perf_counter()
+    if apng:
+        data = render.encode_apng(rgb8, device=0, delay=(1, 30), plays=0)
+        _write(f"{out}.apng", data)
+        files = f"{out}.apng, {len(data)} bytes"
+    else:
+        for k in range(n_frames):
+            render.write_png(f"{out}-{k:04d}.png", rgb8[k], 0 if gpu_png else None)
+        files = f"{out}-0000.png .. {out}-{n_frames - 1:04d}.png"
+    print(f"samples traced: {traced} of {full} ({100.0 * traced / full:.1f} %)")
+    print(f'"Elapsed time: {1e3 * (time.perf_counter() - t0):.3f} msecs"  (render {1e3 * (t1 - t0):.3f} ms, '
+          f'{segments} ray segments, {files})')
+    return {"samples": traced, "segments": segments}
 
 
 def realm_variant(out: str = "scene-realm.ppm", seed: int = 1):
@@ -181,15 +224,17 @@ def _cli(argv):
         argv = [a for a in argv if a not in ("--gpu-png", "--denoise", "--apng")]
         if apng and "--frames" not in argv:
             raise SystemExit("--apng writes a camera sequence: it needs --frames N")
+        n_frames = 0
         if "--frames" in argv:
             i = argv.index("--frames")
             if i + 1 >= len(argv) or not argv[i + 1].isdigit() or int(argv[i + 1]) <= 0:
                 raise SystemExit("--frames needs a positive number of frames")
             n_frames = int(argv[i + 1])
             argv = argv[:i] + argv[i + 2:]
-            frames_variant(int(argv[1]) if len(argv) > 1 else 100, int(argv[2]) if len(argv) > 2 else 50, n_frames,
-                           gpu_png=gpu_png, apng=apng)
-            return
+            if "--tolerance" not in argv:
+                frames_variant(int(argv[1]) if len(argv) > 1 else 100, int(argv[2]) if len(argv) > 2 else 50, n_frames,
+                               gpu_png=gpu_png, apng=apng)
+                return
         if "--tolerance" in argv:
             i = argv.index("--tolerance")
             try:
@@ -205,8 +250,11 @@ def _cli(argv):
                 raise SystemExit("--every needs a positive number of samples")
             every = int(argv[i + 1])
             argv = argv[:i] + argv[i + 2:]
-        main_variant(int(argv[1]) if len(argv) > 1 else 100, int(argv[2]) if len(argv) > 2 else 50, every=every,
-                     tolerance=tolerance, gpu_png=gpu_png, denoise=denoise)
+        spp, depth = int(argv[1]) if len(argv) > 1 else 100, int(argv[2]) if len(argv) > 2 else 50
+        if n_frames:
+            frames_variant(spp, depth, n_frames, gpu_png=gpu_png, apng=apng, tolerance=tolerance, every=every)
+            return
+        main_variant(spp, depth, every=every, tolerance=tolerance, gpu_png=gpu_png, denoise=denoise)
     elif which == "realm":
         realm_variant()
     elif which == "i":

@@ -287,6 +287,15 @@ def _adaptive_args(cam, samples_per_px, max_depth, flags, samples_per_unit, tole
     return (C.c_double * 2)(abs_tol, rel_tol), int(min_samples)
 
 
+def _frames_adaptive_args(arr, n, samples_per_px, max_depth, flags, samples_per_unit, tolerance, min_samples):
+    """(double[2] tolerance or None, min_samples) of an accumulation over frames: tolerance None is a plain one."""
+    if tolerance is None:
+        return None, 0
+    cam = arr[0] if n else _abi.Camera()
+    return _adaptive_args(cam, int(samples_per_px), int(max_depth), int(flags), int(samples_per_unit), tolerance,
+                          int(min_samples))
+
+
 class Context:
     """Device-resident rendering: scene uploaded once, output left in device memory
     (pointers come from the caller, e.g. torch tensors), launches enqueued on the caller's
@@ -351,6 +360,24 @@ class Context:
                                         tolerance, int(min_samples))
             _abi.check(_abi.lib().rtclj_ctx_accum_begin_adaptive(self._h, C.byref(cm), C.byref(prm), tol, least,
                                                                  C.byref(unit), C.c_void_p(stream or None)))
+        return unit.value
+
+    def accum_begin_frames(self, cameras: Sequence, samples_per_px: int, max_depth: int, *, seed: int = 1,
+                           flags: int = _abi.FLAGS_MAIN, samples_per_unit: int = 0, shard: Optional[tuple] = None,
+                           stream: int = 0, tolerance: Optional[Sequence[float]] = None, min_samples: int = 0) -> int:
+        """Begins an accumulation over the frames of a camera sequence (rtclj_ctx_accum_begin_frames; plain, or
+        adaptive with `tolerance` as in accum_begin) and returns the pass unit, the single frame's.  accum_step,
+        accum_noise and stats then serve all frames: the device buffers hold len(cameras) full-size frames one after
+        the other, frame f bit-identical to an accumulation of cameras[f] alone stepped alike."""
+        arr, n = _camera_array(cameras)
+        prm = _params(samples_per_px, max_depth, seed, flags, samples_per_unit, self.device)
+        if shard is not None:
+            prm.shard_index, prm.shard_count, prm.shard_rows = (int(x) for x in shard)
+        tol, least = _frames_adaptive_args(arr, n, samples_per_px, max_depth, flags, samples_per_unit, tolerance,
+                                           min_samples)
+        unit = C.c_int32()
+        _abi.check(_abi.lib().rtclj_ctx_accum_begin_frames(self._h, arr, n, C.byref(prm), tol, least, C.byref(unit),
+                                                           C.c_void_p(stream or None)))
         return unit.value
 
     def accum_noise(self, d_samples: int = 0, d_stderr: int = 0, stream: int = 0) -> int:
@@ -513,6 +540,63 @@ class Progressive:
             self.close()
         except Exception:
             pass
+
+
+class ProgressiveFrames(Progressive):
+    """A camera sequence of one scene that refines pass by pass (rtclj_progressive_create_frames): every frame's pixels
+    (adaptive: its live pixels) in shared launches, rows interleaved over `devices` (default [0]).  `Progressive`'s
+    interface with arrays of K = len(cameras) frames: step returns linear float64 [K,H,W,3] and rgb8 uint8 [K,H,W,3],
+    noise returns samples int32 [K,H,W], stderr float64 [K,H,W,3] and the active pixels of all frames.  After every
+    step frame f is bit-identical to a `Progressive` of cameras[f] with the same arguments stepped alike.
+
+        with ProgressiveFrames(world, turntable_cameras(60), 500, 50, tolerance=(0.004, 0.04)) as p:
+            while p.samples_done < p.samples_per_px:
+                lin, rgb8, st = p.step(min(50, p.samples_per_px - p.samples_done))
+                if p.adaptive and p.noise()[2] == 0:
+                    break   # every pixel of every frame has stopped
+    """
+
+    def __init__(self, world, cameras: Sequence, samples_per_px: int = 100, max_depth: int = 50, *, seed: int = 1,
+                 flags: int = _abi.FLAGS_MAIN, samples_per_unit: int = 0, devices: Optional[Sequence[int]] = None,
+                 tolerance: Optional[Sequence[float]] = None, min_samples: int = 0):
+        self._h = C.c_void_p()
+        soa = _as_soa(world)
+        sc = _scene_struct(soa)
+        arr, n = _camera_array(cameras)
+        self.frames = n
+        self.height, self.width = (arr[0].height, arr[0].width) if n else (0, 0)
+        self.samples_per_px = int(samples_per_px)
+        self.adaptive = tolerance is not None
+        prm = _params(samples_per_px, max_depth, seed, flags, samples_per_unit)
+        tol, least = _frames_adaptive_args(arr, n, samples_per_px, max_depth, flags, samples_per_unit, tolerance,
+                                           min_samples)
+        devs = list(devices) if devices else [0]
+        darr = (C.c_int32 * len(devs))(*devs)
+        unit = C.c_int32()
+        _abi.check(_abi.lib().rtclj_progressive_create_frames(C.byref(sc), arr, n, C.byref(prm), tol, least, darr,
+                                                              len(devs), C.byref(unit), C.byref(self._h)))
+        self.pass_unit = unit.value
+        self.samples_done = 0
+
+    def step(self, samples: int, *, want_linear: bool = True, want_rgb8: bool = True,
+             out_linear: Optional[np.ndarray] = None, out_rgb8: Optional[np.ndarray] = None):
+        K, H, W = self.frames, self.height, self.width
+        if want_linear and out_linear is None:
+            out_linear = np.zeros((K, H, W, 3), dtype=np.float64)
+        if want_rgb8 and out_rgb8 is None:
+            out_rgb8 = np.zeros((K, H, W, 3), dtype=np.uint8)
+        return super().step(samples, want_linear=want_linear, want_rgb8=want_rgb8, out_linear=out_linear,
+                            out_rgb8=out_rgb8)
+
+    def noise(self):
+        if not self._h:
+            raise _abi.RtcljError(_abi.E_INVALID, "progressive render is closed")
+        K, H, W = self.frames, self.height, self.width
+        samples = np.zeros((K, H, W), dtype=np.int32)
+        stderr = np.zeros((K, H, W, 3), dtype=np.float64)
+        active = C.c_uint64()
+        _abi.check(_abi.lib().rtclj_progressive_noise(self._h, samples.ctypes.data, stderr.ctypes.data, C.byref(active)))
+        return samples, stderr, active.value
 
 
 def quantise_rgb8(linear: np.ndarray, flags: int = 0) -> np.ndarray:
