@@ -21,6 +21,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <memory>
 #include <mutex>
 #include <new>
@@ -66,6 +67,95 @@ float round_up_to_float(double v) {
   return f;
 }
 
+// The slot order, table and group records of render_lane2_kernel's two-level cull (KParams::ltab / gtab,
+// DESIGN.md section 4.2, "group bound").  Group 0 holds the n - 16 (ng - 1) spheres of largest radius (the ground of
+// a scene) and the padding; every other group 16 spheres of a recursive median split of the centres.  Members keep
+// list order within their group.  gA: the spheres' cull records {c, Ws}; r: their radii.
+struct CullGroups { std::vector<float> ltab; std::vector<unsigned short> lslot; float gtab[kGroups * 4]; };  // ltab: kLtabUint4 * 4
+CullGroups cull_groups(int n, const std::vector<float4>& gA, const double* r) {
+  const int ng = (n + kGroupSpheres - 1) / kGroupSpheres;
+  CullGroups G;
+  std::vector<int> order((size_t)n);
+  for (int i = 0; i < n; ++i) order[(size_t)i] = i;
+  const int n0 = n - kGroupSpheres * std::max(ng - 1, 0);
+  std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return std::fabs(r[a]) > std::fabs(r[b]); });
+  std::function<void(int, int)> split = [&](int lo, int hi) {  // [lo, hi) holds a multiple of 16 spheres
+    const int m = (hi - lo) / kGroupSpheres;
+    if (m <= 1) return;
+    float ext[3];
+    for (int a = 0; a < 3; ++a) {
+      float mn = INFINITY, mx = -INFINITY;
+      for (int q = lo; q < hi; ++q) { const float4 g = gA[(size_t)order[(size_t)q]]; const float v = a == 0 ? g.x : a == 1 ? g.y : g.z; mn = std::min(mn, v); mx = std::max(mx, v); }
+      ext[a] = mx - mn;
+    }
+    const int a = ext[0] >= ext[1] && ext[0] >= ext[2] ? 0 : ext[1] >= ext[2] ? 1 : 2;
+    const int mid = lo + m / 2 * kGroupSpheres;
+    auto key = [&](int i) { const float4 g = gA[(size_t)i]; return std::make_pair(a == 0 ? g.x : a == 1 ? g.y : g.z, i); };
+    std::nth_element(order.begin() + lo, order.begin() + mid, order.begin() + hi, [&](int x, int y) { return key(x) < key(y); });
+    split(lo, mid);
+    split(mid, hi);
+  };
+  split(n0, n);
+  std::sort(order.begin(), order.begin() + n0);
+  for (int g = 1; g < ng; ++g) std::sort(order.begin() + n0 + (g - 1) * kGroupSpheres, order.begin() + n0 + g * kGroupSpheres);
+  // slots: group 0's members, its padding, then the other groups
+  G.lslot.assign((size_t)ng * kGroupSpheres, (unsigned short)0xffff);
+  for (int q = 0; q < n; ++q) G.lslot[(size_t)(q < n0 ? q : q + kGroupSpheres - n0)] = (unsigned short)order[(size_t)q];
+  // table in the layout of geom32 / ctab, kGroupStride uint4s per group: pair p = s/2, half h = s&1 -> {cx[h], cy[2+h]},
+  // {cz[h], Ws[2+h]}
+  auto put = [](float* tab, int s, float cx, float cy, float cz, float ws) {
+    float* v = tab + (size_t)(s / kGroupSpheres) * kGroupStride * 4 + (size_t)((s % kGroupSpheres) >> 1) * 8;
+    const int h = s & 1;
+    v[0 + h] = cx; v[2 + h] = cy; v[4 + h] = cz; v[6 + h] = ws;
+  };
+  G.ltab.assign((size_t)kLtabUint4 * 4, 0.f);
+  for (int s = 0; s < ng * kGroupSpheres; ++s) {
+    const int i = G.lslot[(size_t)s];
+    if (i == 0xffff) put(G.ltab.data(), s, 0.f, 0.f, 0.f, -1e30f);
+    else put(G.ltab.data(), s, gA[(size_t)i].x, gA[(size_t)i].y, gA[(size_t)i].z, gA[(size_t)i].w);
+  }
+  std::memcpy(G.ltab.data() + (size_t)kLtabSlots * 4, G.lslot.data(), G.lslot.size() * sizeof(unsigned short));
+  // Group records (the proof: DESIGN.md 4.2).  A member's fp32 cull value is >= 0 only where its line passes within
+  // sqrt(r^2 + lambda (r^2 + |c|^2 + |o|^2)) of c, lambda = 2^-15; so the line passes within Q + sqrt(lambda) |o| of
+  // the record's centre C, Q = max (sqrt(r^2 (1 + lambda) + lambda |c|^2) + |c - C|), and its square is below
+  // (1 + t) Q^2 + (1 + 1/t) lambda |o|^2, t = 2^-5.  The record is the sphere of squared radius
+  // A = (1 + t) Q^2 (1 + 2^-14) + 2^-14 |C|^2 (its own rounding), the per-ray term kGroupKq leaves 2^-9 |o|^2 for the rest.
+  const double lambda = std::ldexp(1.0, -15), t = std::ldexp(1.0, -5), slack = std::ldexp(1.0, -14);
+  for (int g = 0; g < kGroups; ++g) {
+    float cx = 0.f, cy = 0.f, cz = 0.f, ws = -3e38f;  // no group: never reached
+    if (g < ng) {
+      double mn[3] = {INFINITY, INFINITY, INFINITY}, mx[3] = {-INFINITY, -INFINITY, -INFINITY};
+      bool never = false;  // a member the cull never rejects (Ws = 3e38): so is the group
+      for (int s = g * kGroupSpheres; s < (g + 1) * kGroupSpheres; ++s) {
+        const int i = G.lslot[(size_t)s];
+        if (i == 0xffff) continue;
+        const float4 c = gA[(size_t)i];
+        never = never || c.w >= 3.0e38f;
+        const double v[3] = {c.x, c.y, c.z};
+        for (int a = 0; a < 3; ++a) { mn[a] = std::min(mn[a], v[a]); mx[a] = std::max(mx[a], v[a]); }
+      }
+      cx = (float)(0.5 * (mn[0] + mx[0])); cy = (float)(0.5 * (mn[1] + mx[1])); cz = (float)(0.5 * (mn[2] + mx[2]));
+      double Q = 0.0;
+      for (int s = g * kGroupSpheres; s < (g + 1) * kGroupSpheres; ++s) {
+        const int i = G.lslot[(size_t)s];
+        if (i == 0xffff) continue;
+        const float4 c = gA[(size_t)i];
+        const double c2 = (double)c.x * c.x + (double)c.y * c.y + (double)c.z * c.z;
+        const double dx = (double)c.x - cx, dy = (double)c.y - cy, dz = (double)c.z - cz;
+        Q = std::max(Q, std::sqrt(r[i] * r[i] * (1.0 + lambda) + lambda * c2) + std::sqrt(dx * dx + dy * dy + dz * dz));
+      }
+      const double C2 = (double)cx * cx + (double)cy * cy + (double)cz * cz;
+      const double A = (1.0 + t) * Q * Q * (1.0 + slack) + slack * C2;
+      if (never || !(A < 1e36 && C2 < 1e36)) { cx = cy = cz = 0.f; ws = 3.0e38f; }
+      else ws = round_up_to_float(A - C2);
+    }
+    float* v = G.gtab + (size_t)(g >> 1) * 8;
+    const int h = g & 1;
+    v[0 + h] = cx; v[2 + h] = cy; v[4 + h] = cz; v[6 + h] = ws;
+  }
+  return G;
+}
+
 }  // namespace
 
 struct rtclj_ctx {
@@ -84,6 +174,8 @@ struct rtclj_ctx {
   DevBuf<unsigned> arrive;              // wavefront kernel: chunk arrival counters per pixel
   DevBuf<double> sample_buf;            // strict order on long paths: one colour per sample (kept between renders)
   std::vector<float> ctab_host;         // the cull table of a small scene: launched as a kernel parameter
+  DevBuf<float4> ltab;                  // render_lane2_kernel's cull table in group order and its slot -> index map
+  float gtab_host[kGroups * 4] = {};    // ... and its group records (kernel parameter)
   KParams kparams;                      // launch parameters of the last render (8.4 KB with the table)
   FrameKParams fparams;                 // launch parameters of the last camera-sequence launch (28 KB)
   DevBuf<double> out_linear;            // used by the host-buffer entry points
@@ -364,6 +456,7 @@ void rtclj_ctx_destroy(rtclj_ctx* c) {
   cudaSetDevice(c->device);
   if (c->own_stream) cudaStreamSynchronize(c->own_stream);
   c->geom32.release(); c->geomA.release(); c->geom64.release(); c->mat.release(); c->partial.release();
+  c->ltab.release();
   c->counters.release(); c->stack.release(); c->arrive.release(); c->sample_buf.release(); c->out_linear.release(); c->out_rgb8.release();
   c->acc.release(); c->acc2.release(); c->nsamp.release(); c->live.release(); c->list.release(); c->list_aux.release();
   c->noise_samples.release(); c->noise_stderr.release();
@@ -477,7 +570,13 @@ int rtclj_ctx_set_scene(rtclj_ctx* c, const rtclj_scene* s) {
     c->prim_geom[4 * i + 2] = g64[(size_t)i].cz; c->prim_geom[4 * i + 3] = g64[(size_t)i].r;
   }
   c->ctab_host.clear();
-  if (use_const_table(nhalf)) c->ctab_host.assign(g32.begin(), g32.begin() + (size_t)npad * 4);
+  if (use_const_table(nhalf)) {
+    c->ctab_host.assign(g32.begin(), g32.begin() + (size_t)npad * 4);
+    const CullGroups G = cull_groups(n, gA, s->radius);
+    CU(c->ltab.reserve((size_t)kLtabUint4));
+    CU(cudaMemcpy(c->ltab.p, G.ltab.data(), sizeof(float) * G.ltab.size(), cudaMemcpyHostToDevice));
+    std::memcpy(c->gtab_host, G.gtab, sizeof G.gtab);
+  }
   std::memcpy(c->shift, shift, sizeof shift);
   c->have_scene = true;
   return RTCLJ_OK;
@@ -514,7 +613,9 @@ KernelChoice choose_kernel(const rtclj_ctx* c, const rtclj_params* prm, double t
   // 71.40 ms, 16 spp (3.3e7 samples) 19.6 vs 18.6 ms; 5 spheres: 11.7 vs 11.0 ms.  Break-even near 9e7 samples.
   // (final build of round 2, 16 / 24 / 32 / 48 spp at 1920x1080: 18.48 / 26.71 / 34.86 / 51.25 against 18.50 / 27.23 /
   // 35.77 / 53.28 ms -- the break-even moved down to 3.3e7 samples; at 2e6 samples the single-path kernel is 30 % faster)
-  int small = (c->n >= 64 && total_samples >= 4.0e7) ? SMALL_LANE2 : SMALL_LANE1;
+  // (two-level cull, round 3, one B200 at 1000 W: the cover scene at 16 / 24 / 32 spp, 3.3e7 samples and up, 16.1 / 23.2 /
+  // 30.2 ms against 18.4 / 27.1 / 35.6 ms with one path per lane -- the break-even moved below 3.3e7 samples)
+  int small = (c->n >= 64 && total_samples >= 3.0e7) ? SMALL_LANE2 : SMALL_LANE1;
 #ifdef RTCLJ_DEFAULT_SMALL_KERNEL
   small = RTCLJ_DEFAULT_SMALL_KERNEL;
 #endif
@@ -677,6 +778,8 @@ int launch_pass(rtclj_ctx* c, const rtclj_camera* cam, const rtclj_params* prm, 
         break;
       case Kernel::lane2:
         fn = kLane2Fns[ps.listed][sample_buf]; threads = kT2; sm = Lane2Smem::total; paths = 2u * kT2;
+        P.ltab = c->ltab.p;
+        std::memcpy(P.gtab, c->gtab_host, sizeof P.gtab);
         frames_fn = kLane2FramesFns[ps.listed][sample_buf];
         break;
       default:  // render_kernel

@@ -8,6 +8,9 @@
 // pipe busy (one warp culling alone reaches only half the FFMA2 rate).  Resolve / shade / sampling stay
 // exactly the code of render_kernel<true>, run for path 0 and then for path 1: the path that is not being
 // processed waits in shared memory (76 bytes), the two are swapped between the passes.
+// The cull has two levels (DESIGN.md 4.2): both lines against one bounding record per group of 16 spheres (uniform
+// operands), then each lane against the members of the groups its lines reach -- the flat cull's survivors.  The
+// camera-sequence twins keep the flat cull.
 //
 // Reference: src/raytracing.clj:141-171, src/realm/raytracing.clj:325-346 and the functions they call
 // (cited at each step below).  Arithmetic, draw order and results are those of render_kernel<true>.
@@ -21,6 +24,7 @@ namespace rtclj {
 #endif
 constexpr int kT2 = RTCLJ_LANE2_THREADS;
 
+
 // dynamic shared memory layout (bytes)
 // (unit sums accumulating in global memory instead -- 30 KB less shared memory, 96 instead of 64 KB of L1 --
 // were measured: 552.5 against 543.7 ms per bench frame)
@@ -29,7 +33,8 @@ struct Lane2Smem {
   static constexpr size_t sums = masks + (size_t)32 * kT2 * 4;         // 2 paths x 3 x kT2 doubles: unit sums
   static constexpr size_t f64 = sums + (size_t)2 * 3 * kT2 * 8;        // 6 x kT2 doubles: O, D of the waiting path
   static constexpr size_t u32 = f64 + (size_t)6 * kT2 * 8;             // 7 x kT2 words: its bookkeeping
-  static constexpr size_t total = u32 + (size_t)7 * kT2 * 4;
+  static constexpr size_t table = u32 + (size_t)7 * kT2 * 4;           // KParams::ltab: the groups, then the slot -> index map
+  static constexpr size_t total = table + (size_t)kLtabUint4 * 16;
 };
 
 // kSampleBuf: strict order through the per-sample buffer, its own instantiation (rtclj_kernels.cuh); kListed: the
@@ -44,6 +49,7 @@ __device__ __forceinline__ void render_lane2_body(const KParams& P, const FrameK
   double* const my_sums = reinterpret_cast<double*>(smem_raw + Lane2Smem::sums) + tid;            // [(path * 3 + c) * kT2]
   double* const wO = reinterpret_cast<double*>(smem_raw + Lane2Smem::f64) + tid;                  // [c * kT2]: Ox Oy Oz Dx Dy Dz
   unsigned* const wU = reinterpret_cast<unsigned*>(smem_raw + Lane2Smem::u32) + tid;              // [c * kT2]
+  const unsigned short* const slot_index = reinterpret_cast<const unsigned short*>(smem_raw + Lane2Smem::table) + kLtabSlots * 8;
   const unsigned flags = P.flags;
   const unsigned FULL = 0xffffffffu;
   const unsigned long long total_units = kListed ? total_units_of<true>(P) : 0ull;
@@ -58,6 +64,12 @@ __device__ __forceinline__ void render_lane2_body(const KParams& P, const FrameK
   int& k = pr.k; int& k_end = pr.k_end; int& depth_left = pr.depth_left; int& nstack = pr.nstack; int& status = pr.status;
   // the waiting path starts FRESH as well
   wU[6 * kT2] = (unsigned)PS_FRESH;
+  if (!kFrames) {  // the spatially ordered cull table, for level 2 of the cull
+    uint4* const tab = reinterpret_cast<uint4*>(smem_raw + Lane2Smem::table);
+    static_assert(kLtabUint4 <= kT2, "one uint4 of the table per thread");
+    if (tid < kLtabUint4) tab[tid] = __ldg(reinterpret_cast<const uint4*>(P.ltab) + tid);
+    __syncthreads();
+  }
 
 #ifdef RTCLJ_TAIL_PROBE  // tuning builds only (tools/tail_probe.py): when does each warp start, first run dry, end?
   unsigned long long t_start, t_dry = 0, t_end;
@@ -85,36 +97,81 @@ __device__ __forceinline__ void render_lane2_body(const KParams& P, const FrameK
         const f32x2 b_ox = splat2(2.0f * b.ofx), b_oy = splat2(2.0f * b.ofy), b_oz = splat2(2.0f * b.ofz);
         const f32x2 a_dx = splat2(a.dhx), a_dy = splat2(a.dhy), a_dz = splat2(a.dhz);
         const f32x2 b_dx = splat2(b.dhx), b_dy = splat2(b.dhy), b_dz = splat2(b.dhz);
-        const int nhb = P.nconst;
-        // every block's sign bits are stored unconditionally (warp-uniform index): that keeps the table
-        // loads uniform (LDCU -> UR operands) and the loop free of branches
+        // one pair of cull records against both lines: record s of a block -> sign bit 2 kCBP - 1 - s of acc0 / acc1
+        auto pair = [&](const f32x2 cx, const f32x2 cy, const f32x2 cz, const f32x2 rs, f32x2 akq, f32x2 bkq, unsigned& acc0,
+                        unsigned& acc1) {
+          {
+            const f32x2 bb = fma2(cz, a_dz, fma2(cy, a_dy, fma2(cx, a_dx, a_nb)));
+            const f32x2 ss = fma2(cz, a_oz, fma2(cy, a_oy, fma2(cx, a_ox, add2(rs, akq))));
+            const f32x2 dd = fma2(bb, bb, ss);
+            acc0 = __funnelshift_l((unsigned)dd, acc0, 1);
+            acc0 = __funnelshift_l((unsigned)(dd >> 32), acc0, 1);
+          }
+          {
+            const f32x2 bb = fma2(cz, b_dz, fma2(cy, b_dy, fma2(cx, b_dx, b_nb)));
+            const f32x2 ss = fma2(cz, b_oz, fma2(cy, b_oy, fma2(cx, b_ox, add2(rs, bkq))));
+            const f32x2 dd = fma2(bb, bb, ss);
+            acc1 = __funnelshift_l((unsigned)dd, acc1, 1);
+            acc1 = __funnelshift_l((unsigned)(dd >> 32), acc1, 1);
+          }
+        };
+        const int ng = P.nconst;
+        if constexpr (kFrames) {
+          // the camera-sequence twins keep the flat cull: every block of the list-order table, stored unconditionally
+          // (their chunked instantiation has no room for the second level in the 34 KB instruction-cache budget)
 #pragma unroll 1
-        for (int ub = 0; ub < nhb; ++ub) {
-          unsigned acc0 = 0xffffffffu, acc1 = 0xffffffffu;
+          for (int ub = 0; ub < ng; ++ub) {
+            unsigned acc0 = 0xffffffffu, acc1 = 0xffffffffu;
 #pragma unroll
-          for (int p = 0; p < kCBP; ++p) {
-            const uint4 u = P.ctab[2 * (ub * kCBP + p)], v = P.ctab[2 * (ub * kCBP + p) + 1];
-            const f32x2 cx = ((f32x2)u.y << 32) | u.x, cy = ((f32x2)u.w << 32) | u.z;
-            const f32x2 cz = ((f32x2)v.y << 32) | v.x, rs = ((f32x2)v.w << 32) | v.z;
-            {
-              const f32x2 bb = fma2(cz, a_dz, fma2(cy, a_dy, fma2(cx, a_dx, a_nb)));
-              const f32x2 ss = fma2(cz, a_oz, fma2(cy, a_oy, fma2(cx, a_ox, add2(rs, a_kq))));
-              const f32x2 dd = fma2(bb, bb, ss);
-              acc0 = __funnelshift_l((unsigned)dd, acc0, 1);
-              acc0 = __funnelshift_l((unsigned)(dd >> 32), acc0, 1);
+            for (int p = 0; p < kCBP; ++p) {
+              const uint4 u = P.ctab[2 * (ub * kCBP + p)], v = P.ctab[2 * (ub * kCBP + p) + 1];
+              pair(((f32x2)u.y << 32) | u.x, ((f32x2)u.w << 32) | u.z, ((f32x2)v.y << 32) | v.x, ((f32x2)v.w << 32) | v.z,
+                   a_kq, b_kq, acc0, acc1);
             }
-            {
-              const f32x2 bb = fma2(cz, b_dz, fma2(cy, b_dy, fma2(cx, b_dx, b_nb)));
-              const f32x2 ss = fma2(cz, b_oz, fma2(cy, b_oy, fma2(cx, b_ox, add2(rs, b_kq))));
-              const f32x2 dd = fma2(bb, bb, ss);
-              acc1 = __funnelshift_l((unsigned)dd, acc1, 1);
-              acc1 = __funnelshift_l((unsigned)(dd >> 32), acc1, 1);
+            my_mask[ub * kT2] = __byte_perm(acc0, acc1, 0x5410);
+            bany0 = (bany0 >> 1) | (acc0 != 0xffffffffu ? 0x80000000u : 0u);
+            bany1 = (bany1 >> 1) | (acc1 != 0xffffffffu ? 0x80000000u : 0u);
+          }
+        } else {
+          // level 1: the sign bits of the group records for each line, from uniform operands; one running word per line
+          // (group g at bit 16 nb - 1 - g after nb blocks, set = the record rejects the line, ones above)
+          unsigned rej0 = 0xffffffffu, rej1 = 0xffffffffu;
+          {
+            const f32x2 a_kg = splat2(a.kqf * kGroupKq), b_kg = splat2(b.kqf * kGroupKq);
+#pragma unroll 1
+            for (int ub = 0; ub * kGroupSpheres < ng; ++ub) {
+#pragma unroll
+              for (int p = 0; p < kCBP; ++p) {
+                const uint4 u = P.gtab[2 * (ub * kCBP + p)], v = P.gtab[2 * (ub * kCBP + p) + 1];
+                pair(((f32x2)u.y << 32) | u.x, ((f32x2)u.w << 32) | u.z, ((f32x2)v.y << 32) | v.x, ((f32x2)v.w << 32) | v.z,
+                     a_kg, b_kg, rej0, rej1);
+              }
             }
           }
-          // sphere s of the block -> bit 15 - s (path 0) / 31 - s (path 1); clear = survivor
-          my_mask[ub * kT2] = __byte_perm(acc0, acc1, 0x5410);
-          bany0 = (bany0 >> 1) | (acc0 != 0xffffffffu ? 0x80000000u : 0u);
-          bany1 = (bany1 >> 1) | (acc1 != 0xffffffffu ? 0x80000000u : 0u);
+          // level 2: each lane culls the groups either of its lines reaches, both lines at once, from the shared-memory
+          // table.  A group one line does not reach yields no survivor for it: the same masks as culling every group.
+          const ulonglong2* const tab = reinterpret_cast<const ulonglong2*>(smem_raw + Lane2Smem::table);
+          // (the groups either line reaches, group g at bit 32 - ng + g as in bany; padding groups shift out)
+          const int nb = (ng + kGroupSpheres - 1) / kGroupSpheres;
+          unsigned todo = __brev(~(rej0 & rej1)) << (kGroupSpheres * nb - ng);
+#pragma unroll 1
+          while (todo) {
+            const unsigned bit = todo & (0u - todo);
+            todo ^= bit;
+            const int g = ng - 1 - __clz(bit);
+            const ulonglong2* const t = tab + g * kGroupStride;
+            unsigned acc0 = 0xffffffffu, acc1 = 0xffffffffu;
+#pragma unroll 1
+            for (const ulonglong2* q = t; q != t + 2 * kCBP; q += 2) {
+              const ulonglong2 u = q[0], v = q[1];
+              pair(u.x, u.y, v.x, v.y, a_kq, b_kq, acc0, acc1);
+            }
+            // slot s of the group -> bit 15 - s (path 0) / 31 - s (path 1); clear = survivor
+            my_mask[g * kT2] = __byte_perm(acc0, acc1, 0x5410);
+            bany0 |= acc0 != 0xffffffffu ? bit : 0u;
+            bany1 |= acc1 != 0xffffffffu ? bit : 0u;
+          }
+          __syncwarp();  // (without it ptxas demotes the next segment's level-1 loads to per-lane LDC)
         }
       }
     }
@@ -125,7 +182,8 @@ __device__ __forceinline__ void render_lane2_body(const KParams& P, const FrameK
       const unsigned mask_shift = path ? 16u : 0u;
       path_step<kSampleBuf, kT2, kListed, kFrames>(P, pr, pc, path ? bany1 : bany0,
                                                    [&](int j) { return ~(my_mask[j * kT2] >> mask_shift) & 0xffffu; },
-                                                   my_sums + path * 3 * kT2, (size_t)gtid * 2u + (size_t)path, lane, total_units, FP);
+                                                   my_sums + path * 3 * kT2, (size_t)gtid * 2u + (size_t)path, lane, total_units, FP,
+                                                   [&](int s) { return kFrames ? s : (int)slot_index[s]; });
 
       // ---- swap: this path waits in shared memory while the other one is processed / both are culled
       {

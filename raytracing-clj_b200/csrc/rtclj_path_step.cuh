@@ -40,16 +40,22 @@ enum { PS_FRESH = 0, PS_RAY = 1, PS_DEAD = 2 };  // a path: needs a work unit / 
 struct PathRegs { d3 O, D; unsigned pixel, unit; int k, k_end, depth_left, nstack, status; };
 struct PathCounters { unsigned samples, seg, exact, pref; };
 
+// the list index of cull-table slot s, for a table in list order
+struct SlotIsIndex { __device__ __forceinline__ int operator()(int s) const { return s; } };
+
 // bany: which cull blocks have a survivor for this path (block j at bit 32 - nconst + j);
-// survivors_of_block(j): the 16 survivor bits of block j (sphere s of the block -> bit 15 - s);
+// survivors_of_block(j): the 16 survivor bits of block j (slot s of the block -> bit 15 - s);
+// index_of_slot(s): the list index of table slot s (>= P.n for padding);
 // sums: the path's three unit sums, kSumStride doubles apart; stack_col: its column of the attenuation stack.
 // kListed: tickets go to the pixels of KParams::list, `total_units` of them (total_units_of, read once per kernel).
 // kFrames: the units of a camera sequence, P = FP->P (unit_of_frame_ticket, frame_camera_ray); with kListed, the listed
 // pixels of an adaptive accumulation over frames (unit_of_listed_frame_ticket).
-template <bool kSampleBuf, int kSumStride, bool kListed = false, bool kFrames = false, class SurvivorsOfBlock>
+template <bool kSampleBuf, int kSumStride, bool kListed = false, bool kFrames = false, class SurvivorsOfBlock,
+          class IndexOfSlot = SlotIsIndex>
 __device__ __forceinline__ void path_step(const KParams& P, PathRegs& pr, PathCounters& pc, unsigned bany,
                                           SurvivorsOfBlock survivors_of_block, double* sums, size_t stack_col, int lane,
-                                          unsigned long long total_units = 0, const FrameKParams* FP = nullptr) {
+                                          unsigned long long total_units = 0, const FrameKParams* FP = nullptr,
+                                          IndexOfSlot index_of_slot = IndexOfSlot()) {
   d3& O = pr.O; d3& D = pr.D;
   unsigned& pixel = pr.pixel; unsigned& unit = pr.unit;
   int& k = pr.k; int& k_end = pr.k_end; int& depth_left = pr.depth_left; int& nstack = pr.nstack; int& status = pr.status;
@@ -94,7 +100,7 @@ __device__ __forceinline__ void path_step(const KParams& P, PathRegs& pr, PathCo
         }
         const int bit = __clz(cur);
         cur &= ~(0x80000000u >> bit);
-        int i = bbase + bit;
+        int i = index_of_slot(bbase + bit);
         if (i >= P.n) continue;
         const float4 g4 = __ldg(P.geomA + i);
         const float cx = g4.x, cy = g4.y, cz = g4.z, ws = g4.w;
